@@ -143,11 +143,9 @@ int ssc_destroy(ssc_handle* h);
 /* "batch_pairs" (pairs per kernel launch), "fp64_search" (0/1: use the FP64 linear-search
  * ground-truth kernel instead of the integer-threshold kernel), "force_generic" (0/1), "gzip" (0/1: the slabs
  * handed to the sink hold concatenated gzip members -- a valid .gz stream of the same FASTQ bytes -- compressed on
- * the GPU; the plain bytes of SeqWriter::write are the default), "carry_pass2" (1: the blobs of batch k are moved into the dense slab by the
- * generation kernel of batch k+1; default 0: by a stand-alone kernel after every batch), "concurrent_move" (n > 0: the blobs of batch k are moved by a
+ * the GPU; the plain bytes of SeqWriter::write are the default), "concurrent_move" (n > 0: the blobs of batch k are moved by a
  * bulk-copy kernel on n SMs, on a second stream, while the generation kernel of batch k+1 runs on the others; default 8 of
- * 148 SMs; 0: a stand-alone kernel after every batch), "prefetch_windows" (default 1: the
- * ticket prologue of the generation kernel pulls the haplotype windows of its pairs into the L2), "max_ctas" (> 0 caps the grid of the generation
+ * 148 SMs, 0 below 64 SMs; 0, or n at least the GPU's SM count: a stand-alone kernel after every batch), "max_ctas" (> 0 caps the grid of the generation
  * kernel; 0 = one CTA per SM), "no_splice" (0/1, tests: reads with indel events take the position-by-position path
  * of the fast kernel instead of the spliced packed read). */
 int ssc_set_option(ssc_handle* h, const char* key, int64_t value);

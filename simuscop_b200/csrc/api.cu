@@ -74,16 +74,13 @@ struct ssc_handle {
 	bool forceGeneric = false;
 	bool noSplice = false;        // tests: see GenParams::noSplice
 	int maxCtas = 0;              // > 0: cap the grid of the generation kernel (tests: many tickets per warp on small inputs)
-	int moverCtas = -1;           // "concurrent_move": pass 2b of batch k runs on that many SMs (bulk-copy mover, second stream) under the
-	                              // generation kernel of batch k+1, which leaves them free.  -1 = default: 8 of 148 SMs (measured
-	                              // optimum on the 3 Gb job: 4.30 -> 3.97 ms per step; 6 SMs cannot keep up, 12 cost the generation more)
+	int moverCtas = 0;            // "concurrent_move": pass 2b of batch k runs on that many SMs (bulk-copy mover, second stream) under the
+	                              // generation kernel of batch k+1, which leaves them free; 0 or [1, smCount), 0 = a stand-alone move
+	                              // after every batch.  Default (init_handle): 8 of 148 SMs, 0 below 64 SMs (measured optimum on the
+	                              // 3 Gb job: 4.30 -> 3.97 ms per step; 6 SMs cannot keep up, 12 cost the generation more)
 	cudaStream_t mover = nullptr;
 	cudaEvent_t evPre = nullptr, evScanned[2] = {nullptr, nullptr}, evMoved[2] = {nullptr, nullptr};
 	bool noQ16 = false;           // "no_q16": keep profiles with 9..40 live quality symbols on the diagonal-rows mode (A/B, tests)
-	bool prefetchWindows = true;  // the ticket prologue of the fast kernel prefetches its pairs' haplotype windows into the L2
-	bool carryPass2 = false;      // on: pass 2b (blob moves) of batch k rides on the generation kernel of batch k+1 instead of a stand-alone
-	                              // kernel per batch.  Measured neutral on the 3 Gb job (DESIGN.md section 4): a warp of the generation kernel
-	                              // moves its 21 KB at the latency-bound rate of one warp, which costs what the stand-alone kernel costs
 	bool gzip = false;            // slabs hold gzip members (one per ticket blob) instead of plain FASTQ
 	bool haveGz = false;          // Huffman / CRC tables of the current plan are on the device
 	ssc::GzTables* d_gzTab = nullptr;
@@ -151,9 +148,8 @@ struct ssc_handle {
 	DevBuf<unsigned long long> d_tileState[2];
 	DevBuf<unsigned int> d_ticket[2];
 	uint8_t* d_slots[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};   // [buffer][file] pass-1 blob scratch of the fast kernel; file 2 lies
-	                                                                     // behind file 1 in the same allocation.  Two buffers: the blobs of batch
-	                                                                     // k are moved to their dense slab by the launch that generates batch k+1
-	DevBuf<unsigned int> d_ticket2;
+	                                                                     // behind file 1 in the same allocation.  Two buffers: the mover moves
+	                                                                     // the blobs of batch k while batch k+1 is generated
 	DevBuf<unsigned long long> d_blobPrefix[2];
 	struct { bool valid = false; ssc::GenParams P; } pending;          // generated + scanned, blobs not yet moved
 	cudaEvent_t evDense[2] = {nullptr, nullptr};
@@ -213,7 +209,6 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 			CK(h->d_blobPrefix[b].alloc((size_t)(pairs / 16) + 2));
 		}
 		for (int f = 0; f < 2; f++) { if (h->d_gzBlobs[f]) cudaFree(h->d_gzBlobs[f]); h->d_gzBlobs[f] = nullptr; }
-		CK(h->d_ticket2.alloc(1));
 		int nTiles = (int)(pairs / 16) + 2;   // enough for every kernel's tile size
 		for (int b = 0; b < 2; b++) {
 			for (int f = 0; f < nFiles; f++) CK(cudaMalloc((void**)&h->d_out[b][f], cap));
@@ -272,8 +267,8 @@ int build_gz_tables(ssc_handle* h, const ssc::GenParams& P, int nTiles) {
 	return SSC_OK;
 }
 
-// Moves the blobs of the last launched batch to its dense slab with the stand-alone kernel (the last batch of a call: no
-// later launch carries its moves).
+// Moves the blobs of the last launched batch to its dense slab with the stand-alone kernel (every batch without the mover;
+// with it, the last batch of a call: no later launch runs the mover for it).
 int flush_pending(ssc_handle* h) {
 	if (!h->pending.valid) return SSC_OK;
 	h->pending.valid = false;
@@ -283,8 +278,8 @@ int flush_pending(ssc_handle* h) {
 }
 
 // Launches batch [emitLo, emitHi) into buffer set `buf`.  Fast kernel, plain output: pass 1 + the scan of the blob lengths;
-// the blobs are moved to the dense slab d_out[buf] by the next launch_batch (fused into its generation kernel) or by
-// flush_pending.  Every other mode leaves the finished slab in d_out[buf] when its kernels have run.
+// the blobs are moved to the dense slab d_out[buf] by the mover under the next launch_batch, or by flush_pending (right
+// after the scan when the mover is off).  Every other mode leaves the finished slab in d_out[buf] when its kernels have run.
 int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 	int qsmem = 0; size_t fastSmem = 0;
 	const bool fast = use_fast(h, &qsmem, &fastSmem);
@@ -293,7 +288,6 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 	cudaStream_t s = h->compute;
 	CK(cudaMemsetAsync(h->d_tileState[buf].p, 0, sizeof(unsigned long long) * nTiles, s));
 	CK(cudaMemsetAsync(h->d_ticket[buf].p, 0, sizeof(unsigned int), s));
-	CK(cudaMemsetAsync(h->d_ticket2.p, 0, sizeof(unsigned int), s));
 	CK(cudaMemsetAsync(h->d_result[buf], 0, sizeof(ssc::BatchResult), s));
 	CK(ssc::launch_locate(h->d_emitBase.p, h->nDevBins, emitLo, tp, nTiles, h->d_tileStart[buf].p, s));
 	h->stats.launches += 1;
@@ -319,9 +313,8 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 		P.rk[2 * r] = (uint32_t)h->seed + (uint32_t)r * 0x9E3779B9u;
 		P.rk[2 * r + 1] = (uint32_t)(h->seed >> 32) + (uint32_t)r * 0xBB67AE85u;
 	}
-	P.tileStartBin = h->d_tileStart[buf].p; P.nTiles = nTiles; P.nLoop = nTiles; P.nTilesPrev = 0;
-	P.prefetchWindows = h->prefetchWindows ? 1 : 0;
-	P.tileState = h->d_tileState[buf].p; P.ticket = h->d_ticket[buf].p; P.ticket2 = h->d_ticket2.p; P.blobPrefix = h->d_blobPrefix[buf].p;
+	P.tileStartBin = h->d_tileStart[buf].p; P.nTiles = nTiles;
+	P.tileState = h->d_tileState[buf].p; P.ticket = h->d_ticket[buf].p; P.blobPrefix = h->d_blobPrefix[buf].p;
 	P.out1 = h->d_out[buf][0]; P.out2 = h->d_out[buf][1];
 	P.cap1 = h->slabCap; P.cap2 = h->slabCap;
 	P.result = h->d_result[buf];
@@ -340,8 +333,9 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 		}
 		if (!h->gzip) {
 			int movedBuf = -1;
-			if (h->pending.valid && h->moverCtas > 0 && h->moverCtas < h->smCount) {
-				// pass 2b of the previous batch on the mover stream, under this batch's generation kernel (which leaves it the SMs)
+			if (h->pending.valid) {
+				// pass 2b of the previous batch on the mover stream, under this batch's generation kernel (which leaves it the SMs);
+				// only the mover leaves a batch pending between launches
 				const ssc::GenParams& Q = h->pending.P;
 				movedBuf = buf ^ 1;
 				CK(cudaEventRecord(h->evPre, s));                          // everything this launch had to wait for (copies, ...)
@@ -352,24 +346,14 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 				h->pending.valid = false;
 				h->stats.launches += 1;
 			}
-			if (h->pending.valid && h->carryPass2) {
-				// this launch carries pass 2b of the previous batch
-				const ssc::GenParams& Q = h->pending.P;
-				P.nTilesPrev = Q.nTiles; P.nLoop = std::max(nTiles, Q.nTiles);
-				P.prevBlobs = Q.out1; P.prevFile2Off = Q.file2Off; P.prevBlobPitch = Q.blobPitch;
-				P.prevTileState = Q.tileState; P.prevPrefix = Q.blobPrefix;
-				P.prevDense1 = Q.dense1; P.prevDense2 = Q.dense2; P.prevCap1 = Q.cap1; P.prevCap2 = Q.cap2;
-				h->pending.valid = false;
-			}
-			if (h->pending.valid) { int rc = flush_pending(h); if (rc) return rc; }     // (neither carried nor moved concurrently)
-			grid = std::min((P.nLoop + FG_GEN - 1) / FG_GEN, h->smCount - (movedBuf >= 0 ? h->moverCtas : 0));
+			grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount - (movedBuf >= 0 ? h->moverCtas : 0));
 			if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
 			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, e0, e1));
 			CK(ssc::launch_scan_blobs(P, s));
 			CK(cudaEventRecord(h->evScanned[buf], s));
 			h->pending.P = P; h->pending.valid = true;
 			h->stats.launches += 2;
-			if (!h->carryPass2 && h->moverCtas <= 0) { int rc = flush_pending(h); if (rc) return rc; }
+			if (h->moverCtas == 0) { int rc = flush_pending(h); if (rc) return rc; }     // stand-alone move right after the scan
 			if (e2) CK(cudaEventRecord(e2, s));
 			// later work on this stream (the next launch reuses the blob scratch, copies read the dense slab) comes after the mover
 			if (movedBuf >= 0) CK(cudaStreamWaitEvent(s, h->evMoved[movedBuf], 0));
@@ -404,11 +388,14 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 	return SSC_OK;
 }
 
-// error exit of a pipelined call: nothing of it may still be running when the caller sees the code
+// error exit of a pipelined call: nothing of it may still be running when the caller sees the code, no batch stays pending
+// for the next call, and the kernel timing of ssc_generate_device ends with the call
 int bail(ssc_handle* h, int rc) {
 	const std::string msg = g_err;
 	cudaDeviceSynchronize();
 	h->pending.valid = false;
+	h->timeKernels = false;
+	h->kevUsed = 0;
 	g_err = msg;
 	return rc;
 }
@@ -440,7 +427,7 @@ static int init_handle(ssc_handle* h, int device) {
 	cudaDeviceProp prop;
 	CK(cudaGetDeviceProperties(&prop, device));
 	h->smCount = prop.multiProcessorCount;
-	if (h->moverCtas < 0) h->moverCtas = h->smCount >= 64 ? (h->smCount * 8 + 74) / 148 : 0;
+	h->moverCtas = h->smCount >= 64 ? (h->smCount * 8 + 74) / 148 : 0;   // < smCount
 	h->smemLimit = (int)prop.sharedMemPerBlockOptin - 1024;
 	CK(cudaStreamCreateWithFlags(&h->compute, cudaStreamNonBlocking));
 	CK(cudaStreamCreateWithFlags(&h->copy, cudaStreamNonBlocking));
@@ -518,7 +505,7 @@ int ssc_destroy(ssc_handle* h) {
 	h->d_ref2.release(); h->d_raw2.release(); h->d_other2.release();
 	if (h->upload) cudaStreamDestroy(h->upload);
 	if (h->evRefFree) cudaEventDestroy(h->evRefFree);
-	h->d_ticket2.release(); h->d_gzLens.release();
+	h->d_gzLens.release();
 	for (int f = 0; f < 2; f++) if (h->d_gzBlobs[f]) cudaFree(h->d_gzBlobs[f]);
 	if (h->d_gzTab) cudaFree(h->d_gzTab);
 	h->d_cenStarts.release(); h->d_cenLens.release(); h->d_cenGc.release(); h->d_cenNn.release();
@@ -543,13 +530,11 @@ int ssc_set_option(ssc_handle* h, const char* key, int64_t value) {
 		return SSC_OK;
 	}
 	if (!strcmp(key, "gzip")) { h->gzip = value != 0; return SSC_OK; }
-	if (!strcmp(key, "carry_pass2")) { h->carryPass2 = value != 0; return SSC_OK; }
 	if (!strcmp(key, "concurrent_move")) {
 		if (value < 0 || value > 64) return fail(SSC_ERR_INVALID, "concurrent_move: 0 (off) .. 64 SMs");
-		h->moverCtas = (int)value;
+		h->moverCtas = value < h->smCount ? (int)value : 0;     // the generation kernel needs SMs beside the mover
 		return SSC_OK;
 	}
-	if (!strcmp(key, "prefetch_windows")) { h->prefetchWindows = value != 0; return SSC_OK; }
 	if (!strcmp(key, "no_q16")) {
 		if (h->haveProfile) return fail(SSC_ERR_STATE, "no_q16 must be set before ssc_set_profile");
 		h->noQ16 = value != 0;
@@ -1088,11 +1073,8 @@ int ssc_set_plan(ssc_handle* h, uint64_t seed, const ssc_bin* bins, int64_t n_bi
 	return SSC_OK;
 }
 
-int ssc_generate(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc_sink_fn sink, void* user) {
-	if (!h || !sink) return fail(SSC_ERR_INVALID, "null argument");
-	if (!h->havePlan) return fail(SSC_ERR_STATE, "ssc_set_plan must precede ssc_generate");
-	if (pair_lo < 0 || pair_hi < pair_lo) return fail(SSC_ERR_INVALID, "bad pair range");
-	CK(cudaSetDevice(h->device));
+// The pipeline of ssc_generate.  Every error return goes through bail() in ssc_generate.
+static int generate_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc_sink_fn sink, void* user) {
 	int rc = ensure_batch_resources(h, true);
 	if (rc) return rc;
 	const int64_t eLo = emit_index_of_plan(h, pair_lo), eHi = emit_index_of_plan(h, pair_hi);
@@ -1102,35 +1084,35 @@ int ssc_generate(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc_sink_fn si
 	std::vector<Batch> batches;
 	for (int64_t e = eLo; e < eHi; e += h->slabPairs) batches.push_back({e, std::min(eHi, e + h->slabPairs)});
 	const int nb = (int)batches.size();
-	// pipeline: the launch of batch k+1 (which also completes the dense slab of batch k) runs under the device->host copies of
-	// batch k-1 (file 1 / file 2 on two streams), which run under the sink of batch k-2.  h_out[k & 1] was consumed by the
-	// sink of batch k-2 an iteration before the copy of batch k is issued.
+	// pipeline: the launch of batch k+1 (under which the mover completes the dense slab of batch k) runs under the device->host
+	// copies of batch k-1 (file 1 / file 2 on two streams), which run under the sink of batch k-2.  h_out[k & 1] was consumed by
+	// the sink of batch k-2 an iteration before the copy of batch k is issued.
 	int qm = 0; size_t sb = 0;
-	const bool carried = use_fast(h, &qm, &sb) && !h->gzip && (h->carryPass2 || h->moverCtas > 0);     // pass 2b of batch k rides on the launch of batch k+1
+	const bool moverCompletes = use_fast(h, &qm, &sb) && !h->gzip && h->moverCtas > 0;   // batch k's dense slab under launch k+1
 	auto launch = [&](int k) -> int {
-		// the dense slab this launch writes: d_out[(k-1) & 1] when it carries the previous batch's moves, else d_out[k & 1];
-		// its last reader is the copy of the batch two before the one that now lands there
-		const int target = carried ? (k + 1) & 1 : k & 1;
+		// the dense slab this launch writes: d_out[(k-1) & 1] when the mover completes the previous batch under it, else
+		// d_out[k & 1]; its last reader is the copy of the batch two before the one that now lands there
+		const int target = moverCompletes ? (k + 1) & 1 : k & 1;
 		CK(cudaStreamWaitEvent(h->compute, h->evCopy[target], 0));
 		CK(cudaStreamWaitEvent(h->compute, h->evCopy2[target], 0));
 		int r = launch_batch(h, k & 1, batches[k].lo, batches[k].hi);
 		if (r) return r;
 		CK(cudaEventRecord(h->evGen[k & 1], h->compute));
-		if (!carried) CK(cudaEventRecord(h->evDense[k & 1], h->compute));     // the dense slab of batch k is complete with its own launch
+		if (!moverCompletes) CK(cudaEventRecord(h->evDense[k & 1], h->compute));     // the dense slab of batch k is complete with its own launch
 		return SSC_OK;
 	};
 	rc = launch(0);
-	if (rc) return bail(h, rc);
+	if (rc) return rc;
 	ssc::BatchResult res[2];
 	for (int k = 0; k < nb; k++) {
 		const int buf = k & 1;
 		rc = k + 1 < nb ? launch(k + 1) : flush_pending(h);         // after this the dense slab of batch k is in the stream
-		if (rc) return bail(h, rc);
-		if (carried) CK(cudaEventRecord(h->evDense[buf], h->compute));    // (its pass 2b came with the launch of batch k+1)
+		if (rc) return rc;
+		if (moverCompletes) CK(cudaEventRecord(h->evDense[buf], h->compute));    // (its pass 2b came with the launch of batch k+1)
 		CK(cudaEventSynchronize(h->evGen[buf]));
 		res[buf] = *h->h_result[buf];
 		rc = check_result(h, res[buf]);
-		if (rc) return bail(h, rc);
+		if (rc) return rc;
 		CK(cudaStreamWaitEvent(h->copy, h->evDense[buf], 0));
 		CK(cudaMemcpyAsync(h->h_out[buf][0], h->d_out[buf][0], res[buf].bytes1, cudaMemcpyDeviceToHost, h->copy));
 		CK(cudaEventRecord(h->evCopy[buf], h->copy));
@@ -1146,7 +1128,7 @@ int ssc_generate(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc_sink_fn si
 			CK(cudaEventSynchronize(h->evCopy2[pb]));
 			int src = sink(user, (const char*)h->h_out[pb][0], res[pb].bytes1, nFiles == 2 ? (const char*)h->h_out[pb][1] : nullptr,
 			               nFiles == 2 ? res[pb].bytes2 : 0, batches[k - 1].lo, batches[k - 1].hi - batches[k - 1].lo);
-			if (src) { fail(SSC_ERR_SINK, "sink returned %d", src); return bail(h, SSC_ERR_SINK); }
+			if (src) return fail(SSC_ERR_SINK, "sink returned %d", src);
 		}
 	}
 	{
@@ -1160,64 +1142,81 @@ int ssc_generate(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc_sink_fn si
 	return SSC_OK;
 }
 
+int ssc_generate(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc_sink_fn sink, void* user) {
+	if (!h || !sink) return fail(SSC_ERR_INVALID, "null argument");
+	if (!h->havePlan) return fail(SSC_ERR_STATE, "ssc_set_plan must precede ssc_generate");
+	if (pair_lo < 0 || pair_hi < pair_lo) return fail(SSC_ERR_INVALID, "bad pair range");
+	CK(cudaSetDevice(h->device));
+	const int rc = generate_batches(h, pair_lo, pair_hi, sink, user);
+	return rc ? bail(h, rc) : SSC_OK;
+}
+
+// The pipeline of ssc_generate_device; the totals are added to *b1, *b2, *nb.  Every error return goes through bail() in
+// ssc_generate_device.
+static int generate_device_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, uint64_t* b1, uint64_t* b2, uint64_t* nb,
+                                   float* ms) {
+	int rc = ensure_batch_resources(h, false);
+	if (rc) return rc;
+	const int64_t eLo = emit_index_of_plan(h, pair_lo), eHi = emit_index_of_plan(h, pair_hi);
+	if (eHi <= eLo) return SSC_OK;
+	h->timeKernels = true; h->kevUsed = 0;
+	CK(cudaEventRecord(h->evStart, h->compute));
+	int k = 0;
+	for (int64_t e = eLo; e < eHi; e += h->slabPairs, k++) {
+		const int buf = k & 1;
+		if (k >= 2) {
+			CK(cudaEventSynchronize(h->evGen[buf]));
+			ssc::BatchResult r = *h->h_result[buf];
+			rc = check_result(h, r);
+			if (rc) return rc;
+			*b1 += r.bytes1; *b2 += r.bytes2; *nb += r.bases;
+		}
+		rc = launch_batch(h, buf, e, std::min(eHi, e + h->slabPairs));
+		if (rc) return rc;
+		CK(cudaEventRecord(h->evGen[buf], h->compute));
+	}
+	// the last batch's blobs: stand-alone move, timed with the scans as "pass 2"
+	while ((int)h->kev.size() < h->kevUsed + 2) { cudaEvent_t e; CK(cudaEventCreate(&e)); h->kev.push_back(e); }
+	const int fl = h->kevUsed;
+	CK(cudaEventRecord(h->kev[fl], h->compute));
+	rc = flush_pending(h);
+	if (rc) return rc;
+	CK(cudaEventRecord(h->kev[fl + 1], h->compute));
+	CK(cudaEventRecord(h->evStop, h->compute));
+	CK(cudaEventSynchronize(h->evStop));
+	for (int j = std::max(0, k - 2); j < k; j++) {
+		ssc::BatchResult r = *h->h_result[j & 1];
+		rc = check_result(h, r);
+		if (rc) return rc;
+		*b1 += r.bytes1; *b2 += r.bytes2; *nb += r.bases;
+	}
+	CK(cudaEventElapsedTime(ms, h->evStart, h->evStop));
+	h->stats.device_ms += *ms;
+	h->timeKernels = false;
+	for (int i = 0; i + 2 < h->kevUsed; i += 3) {
+		float a = 0, b = 0;
+		CK(cudaEventElapsedTime(&a, h->kev[i], h->kev[i + 1]));
+		CK(cudaEventElapsedTime(&b, h->kev[i + 1], h->kev[i + 2]));
+		h->stats.gen_kernel_ms += a; h->stats.compact_kernel_ms += b; h->stats.timed_batches += 1;
+	}
+	{
+		float c = 0;
+		CK(cudaEventElapsedTime(&c, h->kev[fl], h->kev[fl + 1]));
+		h->stats.compact_kernel_ms += c;
+	}
+	return SSC_OK;
+}
+
 int ssc_generate_device(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, uint64_t* bytes1, uint64_t* bytes2,
                         uint64_t* bases, double* device_ms) {
 	if (!h) return fail(SSC_ERR_INVALID, "null handle");
 	if (!h->havePlan) return fail(SSC_ERR_STATE, "ssc_set_plan must precede ssc_generate_device");
 	if (pair_lo < 0 || pair_hi < pair_lo) return fail(SSC_ERR_INVALID, "bad pair range");
 	CK(cudaSetDevice(h->device));
-	int rc = ensure_batch_resources(h, false);
-	if (rc) return rc;
-	const int64_t eLo = emit_index_of_plan(h, pair_lo), eHi = emit_index_of_plan(h, pair_hi);
 	uint64_t b1 = 0, b2 = 0, nb = 0;
 	float ms = 0;
-	if (eHi > eLo) {
-		h->timeKernels = true; h->kevUsed = 0;
-		CK(cudaEventRecord(h->evStart, h->compute));
-		int k = 0;
-		for (int64_t e = eLo; e < eHi; e += h->slabPairs, k++) {
-			const int buf = k & 1;
-			if (k >= 2) {
-				CK(cudaEventSynchronize(h->evGen[buf]));
-				ssc::BatchResult r = *h->h_result[buf];
-				rc = check_result(h, r);
-				if (rc) return bail(h, rc);
-				b1 += r.bytes1; b2 += r.bytes2; nb += r.bases;
-			}
-			rc = launch_batch(h, buf, e, std::min(eHi, e + h->slabPairs));
-			if (rc) return bail(h, rc);
-			CK(cudaEventRecord(h->evGen[buf], h->compute));
-		}
-		// the last batch's blobs: stand-alone move, timed with the scans as "pass 2"
-		while ((int)h->kev.size() < h->kevUsed + 2) { cudaEvent_t e; CK(cudaEventCreate(&e)); h->kev.push_back(e); }
-		const int fl = h->kevUsed;
-		CK(cudaEventRecord(h->kev[fl], h->compute));
-		rc = flush_pending(h);
-		if (rc) return bail(h, rc);
-		CK(cudaEventRecord(h->kev[fl + 1], h->compute));
-		CK(cudaEventRecord(h->evStop, h->compute));
-		CK(cudaEventSynchronize(h->evStop));
-		for (int j = std::max(0, k - 2); j < k; j++) {
-			ssc::BatchResult r = *h->h_result[j & 1];
-			rc = check_result(h, r);
-			if (rc) return rc;
-			b1 += r.bytes1; b2 += r.bytes2; nb += r.bases;
-		}
-		CK(cudaEventElapsedTime(&ms, h->evStart, h->evStop));
-		h->stats.device_ms += ms;
-		h->timeKernels = false;
-		for (int i = 0; i + 2 < h->kevUsed; i += 3) {
-			float a = 0, b = 0;
-			CK(cudaEventElapsedTime(&a, h->kev[i], h->kev[i + 1]));
-			CK(cudaEventElapsedTime(&b, h->kev[i + 1], h->kev[i + 2]));
-			h->stats.gen_kernel_ms += a; h->stats.compact_kernel_ms += b; h->stats.timed_batches += 1;
-		}
-		{
-			float c = 0;
-			CK(cudaEventElapsedTime(&c, h->kev[fl], h->kev[fl + 1]));
-			h->stats.compact_kernel_ms += c;
-		}
-	}
+	const int rc = generate_device_batches(h, pair_lo, pair_hi, &b1, &b2, &nb, &ms);
+	if (rc) return bail(h, rc);
 	if (bytes1) *bytes1 = b1;
 	if (bytes2) *bytes2 = b2;
 	if (bases) *bases = nb;

@@ -79,23 +79,13 @@ struct GenParams {
 	int nTiles;
 	unsigned long long* tileState;
 	unsigned long long* blobPrefix;   // fast kernel: exclusive prefix of the blob lengths (pass 2)
-	unsigned int* ticket;
-	unsigned int* ticket2;      // fast kernel: work counter of pass 1 (tickets of FG_CHUNK pairs)
+	unsigned int* ticket;       // work counter of the generation kernel (tiles / tickets of FG_CHUNK pairs), zeroed per launch
 	uint8_t* out1; uint8_t* out2;       // generic kernel: final slabs; fast kernel: blob scratch (pass 1: out2 == out1 + file2Off)
 	uint32_t blobPitch;                 // fast kernel: bytes from the blob of ticket j to the blob of ticket j + 1 (pass 1 output, pass 2 / deflate input)
 	uint32_t file2Off;                  // fast kernel, pass 1: file 2's blobs start this many bytes behind file 1's (one allocation, 32-bit cursors)
 	uint8_t* dense1; uint8_t* dense2;   // fast kernel: final slabs (pass 2)
 	unsigned long long cap1, cap2;
 	BatchResult* result;
-	// fast kernel, pass 2 folded into the next launch: while a warp generates ticket j of this batch it also moves blob j of
-	// the PREVIOUS batch (lengths and offsets final since that batch's scan) to its place in that batch's dense slab.
-	// nTilesPrev == 0: nothing to move; nLoop = max(nTiles, nTilesPrev) tickets are handed out.
-	int prefetchWindows;                // fast kernel: the ticket prologue pulls the windows of its 32 pairs into the L2
-	int nTilesPrev, nLoop;
-	const uint8_t* prevBlobs; uint32_t prevFile2Off; uint32_t prevBlobPitch;
-	const unsigned long long* prevTileState; const unsigned long long* prevPrefix;
-	uint8_t* prevDense1; uint8_t* prevDense2;
-	unsigned long long prevCap1, prevCap2;
 };
 
 }  // namespace ssc

@@ -558,32 +558,14 @@ __device__ __forceinline__ void emit_mapped(const WarpCtx& w, const IndelPlan& p
 }
 
 // ---------------------------------------------------------------------------------------------
-// blob -> dense slab (the ordered write-out, done by the generating warps with a lag)
+// blob -> dense slab (pass 2)
 // ---------------------------------------------------------------------------------------------
 // copy len bytes from a 16-byte aligned global source to an arbitrarily aligned global destination with 16-byte stores.
-// Vector v of the destination (16-byte aligned) takes source bytes [head + 16 v, head + 16 v + 16): two aligned 16-byte loads
-// (chunks v and v + 1 of the source) and four funnel shifts; the word offset head >> 2 of the window inside the chunk pair is
-// the same for the whole copy, so the loop exists once per offset (Q0).  Streaming accesses (ld.global.cs / st.global.cs): the
-// blob is read once and the slab is not read again on the device, and when the moves ride on a generation kernel they must
-// not push the haplotype windows of that kernel out of the L2.  The source may be read up to 16 bytes past len (blob pitch).
-template <int Q0, int U>
-__device__ __forceinline__ void copy_vectors(const uint4* __restrict__ s16, uint4* __restrict__ dv, int nvec, int r8, int lane) {
-#pragma unroll U
-	for (int v = lane; v < nvec; v += 32) {
-		const uint4 A = __ldcs(s16 + v), B = __ldcs(s16 + v + 1);
-		const uint32_t w[8] = {A.x, A.y, A.z, A.w, B.x, B.y, B.z, B.w};
-		uint4 o;
-		o.x = __funnelshift_r(w[Q0], w[Q0 + 1], r8);
-		o.y = __funnelshift_r(w[Q0 + 1], w[Q0 + 2], r8);
-		o.z = __funnelshift_r(w[Q0 + 2], w[Q0 + 3], r8);
-		o.w = __funnelshift_r(w[Q0 + 3], w[Q0 + 4], r8);
-		__stcs(dv + v, o);
-	}
-}
-
-// The stand-alone move kernel keeps the first form of the copy (five 4-byte loads per vector, 32 registers, 8 CTAs per SM:
-// 5.15 TB/s of DRAM traffic); the two-16-byte-loads form above needs more registers than that kernel has.
-__device__ __forceinline__ void copy_realign_w32(const uint8_t* __restrict__ src, int len, uint8_t* __restrict__ dst, int lane) {
+// Vector v of the destination (16-byte aligned) takes source bytes [head + 16 v, head + 16 v + 16): five 4-byte loads and
+// four funnel shifts (32 registers, 8 CTAs per SM: 5.15 TB/s of DRAM traffic; a form with two 16-byte loads per vector needs
+// more registers than that).  Streaming accesses (ld.global.cs / st.global.cs): the blob is read once and the slab is not
+// read again on the device.  The source may be read up to 4 bytes past len (blob pitch).
+__device__ __forceinline__ void copy_realign(const uint8_t* __restrict__ src, int len, uint8_t* __restrict__ dst, int lane) {
 	int head = (int)((16u - (uint32_t)((uintptr_t)dst & 15u)) & 15u);
 	if (head > len) head = len;
 	if (lane < head) dst[lane] = __ldcs(src + lane);
@@ -602,25 +584,6 @@ __device__ __forceinline__ void copy_realign_w32(const uint8_t* __restrict__ src
 		o.z = __funnelshift_r(w2, w3, r8);
 		o.w = __funnelshift_r(w3, w4, r8);
 		__stcs(dv + v, o);
-	}
-	const int t0 = head + (nvec << 4);
-	if (lane < len - t0) dst[t0 + lane] = __ldcs(src + t0 + lane);
-}
-
-template <int U>
-__device__ __forceinline__ void copy_realign(const uint8_t* __restrict__ src, int len, uint8_t* __restrict__ dst, int lane) {
-	int head = (int)((16u - (uint32_t)((uintptr_t)dst & 15u)) & 15u);
-	if (head > len) head = len;
-	if (lane < head) dst[lane] = __ldcs(src + lane);
-	const int nvec = (len - head) >> 4;
-	const int r8 = (head & 3) * 8;
-	const uint4* s16 = (const uint4*)src;
-	uint4* dv = (uint4*)(dst + head);
-	switch (head >> 2) {
-	case 0: copy_vectors<0, U>(s16, dv, nvec, r8, lane); break;
-	case 1: copy_vectors<1, U>(s16, dv, nvec, r8, lane); break;
-	case 2: copy_vectors<2, U>(s16, dv, nvec, r8, lane); break;
-	default: copy_vectors<3, U>(s16, dv, nvec, r8, lane); break;
 	}
 	const int t0 = head + (nvec << 4);
 	if (lane < len - t0) dst[t0 + lane] = __ldcs(src + t0 + lane);
@@ -678,8 +641,7 @@ __global__ void __launch_bounds__(SC_THREADS) scan_blobs_kernel(const GenParams 
 }
 
 // pass 2b: blob j of a batch -> its place in the dense slabs (one warp)
-template <bool INL>
-__device__ __forceinline__ void move_blob_body(const uint8_t* __restrict__ blobs1, const uint8_t* __restrict__ blobs2, uint32_t blobPitch,
+__device__ __forceinline__ void move_blob(const uint8_t* __restrict__ blobs1, const uint8_t* __restrict__ blobs2, uint32_t blobPitch,
                                           const unsigned long long* __restrict__ tileState, const unsigned long long* __restrict__ prefix,
                                           uint8_t* __restrict__ dense1, uint8_t* __restrict__ dense2, unsigned long long cap1,
                                           unsigned long long cap2, int j, int lane) {
@@ -688,30 +650,11 @@ __device__ __forceinline__ void move_blob_body(const uint8_t* __restrict__ blobs
 	const int l1 = (int)(mine >> 31), l2 = (int)(mine & 0x7fffffffull);
 	if (d1 + (unsigned)l1 > cap1 || d2 + (unsigned)l2 > cap2) return;   // flagged by the scan
 	const size_t blob = (size_t)j * blobPitch;
-	if (INL) {
-		copy_realign_w32(blobs1 + blob, l1, dense1 + d1, lane);
-		if (l2) copy_realign_w32(blobs2 + blob, l2, dense2 + d2, lane);
-	} else {
-		copy_realign<4>(blobs1 + blob, l1, dense1 + d1, lane);
-		if (l2) copy_realign<4>(blobs2 + blob, l2, dense2 + d2, lane);
-	}
-}
-__device__ __forceinline__ void move_blob(const uint8_t* __restrict__ blobs1, const uint8_t* __restrict__ blobs2, uint32_t blobPitch,
-                                          const unsigned long long* __restrict__ tileState, const unsigned long long* __restrict__ prefix,
-                                          uint8_t* __restrict__ dense1, uint8_t* __restrict__ dense2, unsigned long long cap1,
-                                          unsigned long long cap2, int j, int lane) {
-	move_blob_body<true>(blobs1, blobs2, blobPitch, tileState, prefix, dense1, dense2, cap1, cap2, j, lane);
-}
-// Out of line for the generation kernel: once per ticket, and its body must not sit between the hot loops of that kernel
-// (they have to stay in the instruction cache).
-__device__ __noinline__ void move_blob_call(const uint8_t* __restrict__ blobs1, const uint8_t* __restrict__ blobs2, uint32_t blobPitch,
-                                            const unsigned long long* __restrict__ tileState, const unsigned long long* __restrict__ prefix,
-                                            uint8_t* __restrict__ dense1, uint8_t* __restrict__ dense2, unsigned long long cap1,
-                                            unsigned long long cap2, int j, int lane) {
-	move_blob_body<false>(blobs1, blobs2, blobPitch, tileState, prefix, dense1, dense2, cap1, cap2, j, lane);
+	copy_realign(blobs1 + blob, l1, dense1 + d1, lane);
+	if (l2) copy_realign(blobs2 + blob, l2, dense2 + d2, lane);
 }
 
-// stand-alone form: the last batch of a call (nothing follows that could carry its moves) and the gzip members
+// stand-alone form: the last batch of a call, every batch when the concurrent mover is off, and the gzip members
 static constexpr int CP_THREADS = 256;
 __global__ void __launch_bounds__(CP_THREADS, 8) move_blobs_kernel(const GenParams P) {
 	const int lane = threadIdx.x & 31;
@@ -982,11 +925,9 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 	while (true) {
 		// ---- a ticket = FG_CHUNK consecutive pairs
 		int chunk = 0;
-		if (lane == 0) chunk = (int)atomicAdd(P.ticket2, 1u);
+		if (lane == 0) chunk = (int)atomicAdd(P.ticket, 1u);
 		chunk = __shfl_sync(0xffffffffu, chunk, 0);
-		if (chunk >= P.nLoop) break;
-		bool moved = false;
-		if (chunk < P.nTiles) {
+		if (chunk >= P.nTiles) break;
 		// slot = pair index inside the batch (a batch has < 2^31 / FG_SLOT pairs)
 		const uint32_t slot0 = (uint32_t)chunk * FG_CHUNK;
 		const uint32_t nSlots = (uint32_t)(P.emitHi - P.emitLo);
@@ -1044,17 +985,6 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 			const int64_t g0b = fstart + flen - RL;
 			const int64_t g0a = seReverse ? g0b : fstart;
 			k_winA = (uint32_t)((uint64_t)(g0a - 32) >> 4); k_winB = (uint32_t)((uint64_t)(g0b - 32) >> 4);
-			// The windows of the ticket's 32 pairs are scattered over a store of several GB; the pair loop gets to pair p only
-			// p x ~8 us from now.  Pulling the lines into the L2 here turns the HBM latency of every pair's window fetch (which the
-			// ~250 instructions between the cp.async and its wait do not cover) into an L2 hit.
-			if (lane < count && P.prefetchWindows) {
-				const uint32_t* dA = P.hap2 + k_winA; const uint32_t* mA = P.hapN + (k_winA >> 1);
-				const uint32_t* dB = P.hap2 + k_winB; const uint32_t* mB = P.hapN + (k_winB >> 1);
-				asm volatile("prefetch.global.L2 [%0];" ::"l"(dA)); asm volatile("prefetch.global.L2 [%0];" ::"l"(dA + 15));
-				asm volatile("prefetch.global.L2 [%0];" ::"l"(mA)); asm volatile("prefetch.global.L2 [%0];" ::"l"(mA + 8));
-				asm volatile("prefetch.global.L2 [%0];" ::"l"(dB)); asm volatile("prefetch.global.L2 [%0];" ::"l"(dB + 15));
-				asm volatile("prefetch.global.L2 [%0];" ::"l"(mB)); asm volatile("prefetch.global.L2 [%0];" ::"l"(mB + 8));
-			}
 			k_g = ((uint32_t)g0a & 31u) | (((uint32_t)g0b & 31u) << 8) | (seReverse ? 0x80000000u : 0u);
 			k_posmod = posmod; k_frag = fragCount;
 			// name_off (17 bits) | name_len << 17 (7 bits) | digits of posmod << 24 | digits of fragCount << 28
@@ -1063,15 +993,6 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 
 #pragma unroll 1
 		for (int p = 0; p < count; p++) {
-			// ---- pass 2 of the previous batch, carried by this launch: blob `chunk` of that batch to its dense place.  The blob
-			// lies in HBM since the previous launch and its offset is final, so nothing is waited for.  The warps of an SM run
-			// through their tickets almost in lock step; each one does its move in front of a different pair of its ticket
-			// (pair index = warp index), so that at any time only a few of them sit in the copy loop's memory latency.
-			if (p == warp && chunk < P.nTilesPrev) {
-				move_blob_call(P.prevBlobs, P.prevBlobs + P.prevFile2Off, P.prevBlobPitch, P.prevTileState, P.prevPrefix, P.prevDense1, P.prevDense2,
-				               P.prevCap1, P.prevCap2, chunk, lane);
-				moved = true;
-			}
 			w.c0 = __shfl_sync(0xffffffffu, k_pairLo, p); w.c1 = __shfl_sync(0xffffffffu, k_pairHi, p);
 			const uint32_t kg = __shfl_sync(0xffffffffu, k_g, p);
 			const uint32_t posmod = __shfl_sync(0xffffffffu, k_posmod, p), fragCount = __shfl_sync(0xffffffffu, k_frag, p);
@@ -1251,11 +1172,6 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 				atomicAdd(&P.result->rawBytes, (unsigned long long)len1 + len2);
 			}
 		}
-		}
-		// (tickets shorter than the warp's phase, and tickets beyond this batch's own when the previous batch had more)
-		if (!moved && chunk < P.nTilesPrev)
-			move_blob_call(P.prevBlobs, P.prevBlobs + P.prevFile2Off, P.prevBlobPitch, P.prevTileState, P.prevPrefix, P.prevDense1, P.prevDense2,
-			               P.prevCap1, P.prevCap2, chunk, lane);
 	}
 
 }
@@ -1318,8 +1234,8 @@ static cudaError_t launch_fast_variant(const GenParams& P, size_t smemBytes, int
 	return cudaGetLastError();
 }
 
-// P.out1/out2 = blob scratch, P.dense1/dense2 = final slabs, P.nTiles = tickets of FG_CHUNK pairs.  Launches pass 1 (which
-// also carries the moves of the previous batch when P.nTilesPrev > 0); events e0/e1 (optional) bracket the kernel.
+// P.out1/out2 = blob scratch, P.dense1/dense2 = final slabs, P.nTiles = tickets of FG_CHUNK pairs.  Launches pass 1;
+// events e0/e1 (optional) bracket the kernel.
 cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream,
                                  cudaEvent_t e0, cudaEvent_t e1) {
 	const int nch = (P.t.RL + 31) / 32;   // the kernel's chunk count is exact: only the last chunk has idle lanes
@@ -1369,12 +1285,8 @@ cudaError_t launch_move_blobs(const GenParams& P, int smCount, cudaStream_t stre
 // pass 2b on `ctas` SMs (see move_blobs_tma_kernel): meant to run on a second stream under the next batch's generation kernel
 cudaError_t launch_move_blobs_tma(const GenParams& P, int ctas, cudaStream_t stream) {
 	const int smem = MV_WARPS * MV_WARP_BYTES;
-	static bool attr = false;
-	if (!attr) {
-		cudaError_t e = cudaFuncSetAttribute(move_blobs_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-		if (e != cudaSuccess) return e;
-		attr = true;
-	}
+	cudaError_t e = cudaFuncSetAttribute(move_blobs_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+	if (e != cudaSuccess) return e;
 	move_blobs_tma_kernel<<<ctas, MV_THREADS, smem, stream>>>(P);
 	return cudaGetLastError();
 }

@@ -32,13 +32,17 @@ def test_fastq_bit_exact_vs_instrumented_reference(name, gen, workdir):
         assert len(r1) > 0
 
 
-@pytest.mark.parametrize("mode", ["force_generic", "fp64_search", "no_splice", "no_q16", "carry_pass2", "concurrent_move"])
+# pass 2 of the fast kernel: a stand-alone move after every batch (what GPUs with fewer than 64 SMs run), or the bulk-copy mover
+MOVE_MODES = {"standalone_move": ("concurrent_move", 0), "concurrent_move": ("concurrent_move", 8)}
+
+
+@pytest.mark.parametrize("mode", ["force_generic", "fp64_search", "no_splice", "no_q16", "standalone_move", "concurrent_move"])
 @pytest.mark.parametrize("name", ["pe_xten", "pe_tiny", "se_gaiix"])
 def test_fallback_kernels_bit_exact(name, mode, built, workdir):
     """The generic integer kernel, the FP64 linear-search ground-truth kernel, the fast kernel without the spliced indel path,
     without the 16-bit-key shared-memory tables (profiles with 9..40 live quality symbols then keep only the ref == call rows
-    in shared memory), with pass 2 carried by the next batch's generation kernel, and with pass 2 on the bulk-copy mover
-    (8 SMs, second stream, under the next batch's generation) all give the same bytes."""
+    in shared memory), with pass 2 as a stand-alone move after every batch, and with pass 2 on the bulk-copy mover (8 SMs,
+    second stream, under the next batch's generation) all give the same bytes."""
     from simuscop_b200 import cuda_binding
     scn = helpers.build_scenario(name, workdir)
     plans, out = helpers.reference_run(scn, tag=mode)
@@ -47,15 +51,49 @@ def test_fallback_kernels_bit_exact(name, mode, built, workdir):
     r1, r2 = helpers.read_file(r1p), helpers.read_file(r2p)
     g = cuda_binding.Generator(0)
     try:
-        g.set_option(mode, 8 if mode == "concurrent_move" else 1)
-        if mode in ("carry_pass2", "concurrent_move"):
-            g.set_option("batch_pairs", 256)          # many batches: every launch but the first moves its predecessor's blobs
+        key, value = MOVE_MODES.get(mode, (mode, 1))
+        g.set_option(key, value)
+        if mode in MOVE_MODES:
+            g.set_option("batch_pairs", 256)          # many batches: with the mover, every launch but the first moves its predecessor's blobs
         g.load_plan(plan, scn["seed"])
         f1, f2 = g.generate()
     finally:
         g.close()
     assert helpers.first_diff(f1, r1) == -1
     assert helpers.first_diff(f2, r2) == -1
+
+
+def test_error_in_a_pipelined_call_leaves_the_handle_usable(built, workdir):
+    """A sink error in the middle of ssc_generate (later batches generated, scanned or moving on the mover's stream) drains
+    the device and leaves no batch pending: the same handle's next ssc_generate and ssc_generate_device give the reference's
+    bytes and counts."""
+    from simuscop_b200 import cuda_binding
+    scn = helpers.build_scenario("pe_tiny", workdir)
+    plans, out = helpers.reference_run(scn, tag="err")
+    plan = planfile.read_plan(plans[0])
+    r1p, r2p = helpers.sample_files(out, plan, 0, scn)
+    r1, r2 = helpers.read_file(r1p), helpers.read_file(r2p)
+    calls = []
+
+    def failing_sink(user, b1, l1, b2, l2, first, n):
+        calls.append(n)
+        return 1 if len(calls) == 3 else 0
+    g = cuda_binding.Generator(0)
+    try:
+        g.set_option("batch_pairs", 256)
+        g.load_plan(plan, scn["seed"])
+        assert g.emitted > 4 * 256
+        with pytest.raises(cuda_binding.SscError) as e:
+            g.generate(sink=failing_sink)
+        assert "ssc error 5" in str(e.value) and len(calls) == 3
+        f1, f2 = g.generate()
+        assert helpers.first_diff(f1, r1) == -1 and helpers.first_diff(f2, r2) == -1
+        d = g.generate_device()
+        assert (d["bytes1"], d["bytes2"]) == (len(r1), len(r2))
+        f1, f2 = g.generate()
+        assert helpers.first_diff(f1, r1) == -1 and helpers.first_diff(f2, r2) == -1
+    finally:
+        g.close()
 
 
 def test_batching_and_ranges_are_seamless(built, workdir):
@@ -177,11 +215,16 @@ def test_synthetic_profiles_cli_and_abi(name, built, workdir):
 
 def test_reads_beyond_the_scratch_limits_fail_loudly(built, workdir):
     """A profile with 2 % insertion AND deletion rates outgrows the per-read limits (32 events / 128 inserted bases):
-    the library must return SSC_ERR_OVERFLOW, not a silently different FASTQ."""
+    the library must return SSC_ERR_OVERFLOW, not a silently different FASTQ, from both pipelined calls.  The handle stays
+    usable: the next plan loaded on it gives the reference's bytes."""
     from simuscop_b200 import cuda_binding
     scn = helpers.build_stress("overflow", workdir)
     plans, out_ref = helpers.reference_run(scn, tag="ov")
     plan = planfile.read_plan(plans[0])
+    tiny = helpers.build_scenario("pe_tiny", workdir)
+    tiny_plans, tiny_out = helpers.reference_run(tiny, tag="ov")
+    tiny_plan = planfile.read_plan(tiny_plans[0])
+    t1, t2 = (helpers.read_file(p) for p in helpers.sample_files(tiny_out, tiny_plan, 0, tiny))
     for opt in (None, "force_generic", "no_splice"):
         g = cuda_binding.Generator(0)
         try:
@@ -191,6 +234,12 @@ def test_reads_beyond_the_scratch_limits_fail_loudly(built, workdir):
             with pytest.raises(cuda_binding.SscError) as e:
                 g.generate()
             assert "ssc error 6" in str(e.value)
+            with pytest.raises(cuda_binding.SscError) as e:
+                g.generate_device()
+            assert "ssc error 6" in str(e.value)
+            g.load_plan(tiny_plan, tiny["seed"])
+            f1, f2 = g.generate()
+            assert helpers.first_diff(f1, t1) == -1 and helpers.first_diff(f2, t2) == -1
         finally:
             g.close()
 

@@ -21,7 +21,7 @@ g = cuda_binding.Generator(0)
 g.set_option("batch_pairs", int(os.environ.get("QB_BATCH", 1 << 21)))
 if os.environ.get("QB_GZIP"):
     g.set_option("gzip", 1)
-for kv in filter(None, os.environ.get("QB_OPTS", "").split(",")):          # e.g. QB_OPTS=carry_pass2=0
+for kv in filter(None, os.environ.get("QB_OPTS", "").split(",")):          # e.g. QB_OPTS=concurrent_move=0
     g.set_option(kv.split("=")[0], int(kv.split("=")[1]))
 t = time.time()
 g.load_plan(plan, 7)
