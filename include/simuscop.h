@@ -123,6 +123,8 @@ typedef struct ssc_stats {
 	uint64_t timed_batches;    /* launches covered by gen_kernel_ms */
 	uint64_t gz_bytes;         /* gzip mode: compressed bytes written to the slabs (fastq_bytes stays the plain size) */
 	uint64_t bin_bytes;        /* algorithmic bin-record bytes read: 64 bytes per distinct bin of every generated batch */
+	double   mover_kernel_ms;  /* CUDA-event time of the concurrent blob mover (concurrent_move > 0) on its own stream, under the
+	                              generation kernel of the next batch (ssc_generate_device) */
 } ssc_stats;
 
 /*

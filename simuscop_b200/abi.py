@@ -37,7 +37,7 @@ class Stats(C.Structure):
         ("pairs_emitted", C.c_uint64), ("reads_emitted", C.c_uint64), ("bases_emitted", C.c_uint64),
         ("fastq_bytes", C.c_uint64), ("hap_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64), ("h2d_bytes", C.c_uint64),
         ("gen_kernel_ms", C.c_double), ("compact_kernel_ms", C.c_double), ("timed_batches", C.c_uint64),
-        ("gz_bytes", C.c_uint64), ("bin_bytes", C.c_uint64),
+        ("gz_bytes", C.c_uint64), ("bin_bytes", C.c_uint64), ("mover_kernel_ms", C.c_double),
     ]
 
 

@@ -66,7 +66,7 @@ struct ssc_handle {
 	int smCount = 0;
 	int smemLimit = 0;
 	cudaStream_t compute = nullptr, copy = nullptr, copy2 = nullptr;   // copy/copy2: device->host of file 1 / file 2 (two copy engines)
-	cudaEvent_t evStart = nullptr, evStop = nullptr, evGen[2] = {nullptr, nullptr}, evCopy[2] = {nullptr, nullptr}, evCopy2[2] = {nullptr, nullptr};
+	cudaEvent_t evStart = nullptr, evStop = nullptr, evCopy[2] = {nullptr, nullptr}, evCopy2[2] = {nullptr, nullptr};
 
 	// options
 	int64_t batchPairs = 1 << 20;
@@ -76,10 +76,15 @@ struct ssc_handle {
 	int maxCtas = 0;              // > 0: cap the grid of the generation kernel (tests: many tickets per warp on small inputs)
 	int moverCtas = 0;            // "concurrent_move": pass 2b of batch k runs on that many SMs (bulk-copy mover, second stream) under the
 	                              // generation kernel of batch k+1, which leaves them free; 0 or [1, smCount), 0 = a stand-alone move
-	                              // after every batch.  Default (init_handle): 8 of 148 SMs, 0 below 64 SMs (measured optimum on the
-	                              // 3 Gb job: 4.30 -> 3.97 ms per step; 6 SMs cannot keep up, 12 cost the generation more)
-	cudaStream_t mover = nullptr;
-	cudaEvent_t evPre = nullptr, evScanned[2] = {nullptr, nullptr}, evMoved[2] = {nullptr, nullptr};
+	                              // after every batch.  Default: init_handle
+	cudaStream_t mover = nullptr; // pass 2 of the fast kernel's plain output: the scans and the concurrent moves
+	cudaEvent_t evPre = nullptr;  // a point of the compute stream the mover stream waits for (recorded anew for every wait)
+	cudaEvent_t evScanned[2] = {nullptr, nullptr};   // batch of buffer set b: its last kernel (fast kernel, plain output: the scan) done
+	cudaEvent_t evMoved[2] = {nullptr, nullptr};
+	// the device->host copy of a batch's BatchResult: on a stream of its own, because the copy engines may be busy with the
+	// FASTQ slabs of ssc_generate for milliseconds, and no kernel must queue behind it
+	cudaStream_t results = nullptr;
+	cudaEvent_t evResult[2] = {nullptr, nullptr};    // batch of buffer set b: its BatchResult in h_result[b]
 	bool noQ16 = false;           // "no_q16": keep profiles with 9..40 live quality symbols on the diagonal-rows mode (A/B, tests)
 	bool gzip = false;            // slabs hold gzip members (one per ticket blob) instead of plain FASTQ
 	bool haveGz = false;          // Huffman / CRC tables of the current plan are on the device
@@ -151,14 +156,17 @@ struct ssc_handle {
 	                                                                     // behind file 1 in the same allocation.  Two buffers: the mover moves
 	                                                                     // the blobs of batch k while batch k+1 is generated
 	DevBuf<unsigned long long> d_blobPrefix[2];
-	struct { bool valid = false; ssc::GenParams P; } pending;          // generated + scanned, blobs not yet moved
+	struct { bool valid = false; int buf = 0; ssc::GenParams P; } pending;   // generated (scan queued), blobs not yet moved
 	cudaEvent_t evDense[2] = {nullptr, nullptr};
 	DevBuf<int64_t> d_cenStarts;                  // ssc_gc_census scratch (grow-only)
 	DevBuf<int32_t> d_cenLens, d_cenGc, d_cenNn;
 	ssc::BatchResult* d_result[2] = {nullptr, nullptr};
 	ssc::BatchResult* h_result[2] = {nullptr, nullptr};
 
-	std::vector<cudaEvent_t> kev;   // per-batch kernel timing events of ssc_generate_device (3 per batch)
+	// kernel timing of ssc_generate_device: events kev[2 i] and kev[2 i + 1] bracket the i-th timed piece of work of the call,
+	// whose time goes to *kevSum[i] when the call ends (see time_begin)
+	std::vector<cudaEvent_t> kev;
+	std::vector<double*> kevSum;
 	int kevUsed = 0;
 	bool timeKernels = false;
 
@@ -267,30 +275,65 @@ int build_gz_tables(ssc_handle* h, const ssc::GenParams& P, int nTiles) {
 	return SSC_OK;
 }
 
+// Kernel timing of ssc_generate_device: when the call is timed, records the start event of a piece of work on stream s and
+// returns in *end the event the caller records on s after it; the time between the two goes to *sum when the call ends.
+// *end is null when the call is not timed.
+cudaError_t time_begin(ssc_handle* h, cudaStream_t s, double* sum, cudaEvent_t* end) {
+	*end = nullptr;
+	if (!h->timeKernels) return cudaSuccess;
+	while (h->kev.size() < 2 * (size_t)(h->kevUsed + 1)) {
+		cudaEvent_t e;
+		const cudaError_t err = cudaEventCreate(&e);
+		if (err != cudaSuccess) return err;
+		h->kev.push_back(e);
+	}
+	h->kevSum.resize((size_t)h->kevUsed + 1);
+	h->kevSum[h->kevUsed] = sum;
+	*end = h->kev[2 * h->kevUsed + 1];
+	return cudaEventRecord(h->kev[2 * h->kevUsed++], s);
+}
+
 // Moves the blobs of the last launched batch to its dense slab with the stand-alone kernel (every batch without the mover;
-// with it, the last batch of a call: no later launch runs the mover for it).
+// with it, the last batch of a call: no later launch runs the mover for it).  Timed as pass 2.
 int flush_pending(ssc_handle* h) {
 	if (!h->pending.valid) return SSC_OK;
 	h->pending.valid = false;
+	CK(cudaStreamWaitEvent(h->compute, h->evScanned[h->pending.buf], 0));    // the blob offsets, scanned on the mover stream
+	cudaEvent_t te;
+	CK(time_begin(h, h->compute, &h->stats.compact_kernel_ms, &te));
 	CK(ssc::launch_move_blobs(h->pending.P, h->smCount, h->compute));
+	if (te) CK(cudaEventRecord(te, h->compute));
 	h->stats.launches += 1;
 	return SSC_OK;
 }
 
-// Launches batch [emitLo, emitHi) into buffer set `buf`.  Fast kernel, plain output: pass 1 + the scan of the blob lengths;
-// the blobs are moved to the dense slab d_out[buf] by the mover under the next launch_batch, or by flush_pending (right
-// after the scan when the mover is off).  Every other mode leaves the finished slab in d_out[buf] when its kernels have run.
+// Copies the BatchResult of buffer set `buf` to h_result[buf] (evResult[buf]) once the work queued on stream `after`, which
+// writes it last, is done (evScanned[buf]).
+int result_to_host(ssc_handle* h, int buf, cudaStream_t after) {
+	CK(cudaEventRecord(h->evScanned[buf], after));
+	CK(cudaStreamWaitEvent(h->results, h->evScanned[buf], 0));
+	CK(cudaMemcpyAsync(h->h_result[buf], h->d_result[buf], sizeof(ssc::BatchResult), cudaMemcpyDeviceToHost, h->results));
+	CK(cudaEventRecord(h->evResult[buf], h->results));
+	return SSC_OK;
+}
+
+// Launches batch [emitLo, emitHi) into buffer set `buf`; evResult[buf] marks its BatchResult in h_result[buf].  Fast kernel,
+// plain output: pass 1 on the compute stream, then the scan of the blob lengths on the mover stream; the blobs are moved to
+// the dense slab d_out[buf] by the mover under the next launch_batch, or by flush_pending (right after the scan when the
+// mover is off).  Every other mode leaves the finished slab in d_out[buf] when its kernels have run on the compute stream.
 int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 	int qsmem = 0; size_t fastSmem = 0;
 	const bool fast = use_fast(h, &qsmem, &fastSmem);
 	const int tp = fast ? FG_CHUNK : GEN_TILE_PAIRS;
 	int nTiles = (int)((emitHi - emitLo + tp - 1) / tp);
 	cudaStream_t s = h->compute;
+	CK(cudaStreamWaitEvent(s, h->evResult[buf], 0));          // the copy of the BatchResult this buffer set held before
 	CK(cudaMemsetAsync(h->d_tileState[buf].p, 0, sizeof(unsigned long long) * nTiles, s));
 	CK(cudaMemsetAsync(h->d_ticket[buf].p, 0, sizeof(unsigned int), s));
 	CK(cudaMemsetAsync(h->d_result[buf], 0, sizeof(ssc::BatchResult), s));
 	CK(ssc::launch_locate(h->d_emitBase.p, h->nDevBins, emitLo, tp, nTiles, h->d_tileStart[buf].p, s));
 	h->stats.launches += 1;
+	h->stats.gen_launches += 1;
 	{
 		// distinct bins of the batch (statistics: the algorithmic bin-record bytes of the roofline)
 		const std::vector<int64_t>& eb = h->devEmitBase;
@@ -325,45 +368,51 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 		P.out1 = h->d_slots[buf][0]; P.out2 = h->d_slots[buf][1];
 		P.blobPitch = (uint32_t)(FG_CHUNK * FG_SLOT);
 		P.file2Off = (uint32_t)(h->d_slots[buf][1] ? h->d_slots[buf][1] - h->d_slots[buf][0] : 0);
-		cudaEvent_t e0 = nullptr, e1 = nullptr, e2 = nullptr;
-		if (h->timeKernels) {
-			while ((int)h->kev.size() < h->kevUsed + 3) { cudaEvent_t e; CK(cudaEventCreate(&e)); h->kev.push_back(e); }
-			e0 = h->kev[h->kevUsed]; e1 = h->kev[h->kevUsed + 1]; e2 = h->kev[h->kevUsed + 2];
-			h->kevUsed += 3;
-		}
+		cudaEvent_t te;
 		if (!h->gzip) {
 			int movedBuf = -1;
 			if (h->pending.valid) {
 				// pass 2b of the previous batch on the mover stream, under this batch's generation kernel (which leaves it the SMs);
-				// only the mover leaves a batch pending between launches
+				// only the mover leaves a batch pending between launches.  Its scan is ahead of it on that stream.
 				const ssc::GenParams& Q = h->pending.P;
 				movedBuf = buf ^ 1;
 				CK(cudaEventRecord(h->evPre, s));                          // everything this launch had to wait for (copies, ...)
 				CK(cudaStreamWaitEvent(h->mover, h->evPre, 0));
-				CK(cudaStreamWaitEvent(h->mover, h->evScanned[movedBuf], 0));
+				CK(time_begin(h, h->mover, &h->stats.mover_kernel_ms, &te));
 				CK(ssc::launch_move_blobs_tma(Q, h->moverCtas, h->mover));
+				if (te) CK(cudaEventRecord(te, h->mover));
 				CK(cudaEventRecord(h->evMoved[movedBuf], h->mover));
 				h->pending.valid = false;
 				h->stats.launches += 1;
 			}
 			grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount - (movedBuf >= 0 ? h->moverCtas : 0));
 			if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
-			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, e0, e1));
-			CK(ssc::launch_scan_blobs(P, s));
-			CK(cudaEventRecord(h->evScanned[buf], s));
-			h->pending.P = P; h->pending.valid = true;
+			CK(time_begin(h, s, &h->stats.gen_kernel_ms, &te));
+			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, nullptr, te));
+			// pass 2a on the mover stream, behind the previous batch's move: only the moves and the host need its offsets and
+			// totals, so the compute stream goes straight on to the next batch
+			CK(cudaEventRecord(h->evPre, s));
+			CK(cudaStreamWaitEvent(h->mover, h->evPre, 0));
+			CK(time_begin(h, h->mover, &h->stats.compact_kernel_ms, &te));
+			CK(ssc::launch_scan_blobs(P, h->mover));
+			if (te) CK(cudaEventRecord(te, h->mover));
+			const int rc = result_to_host(h, buf, h->mover);
+			if (rc) return rc;
+			h->pending.P = P; h->pending.buf = buf; h->pending.valid = true;
 			h->stats.launches += 2;
-			if (h->moverCtas == 0) { int rc = flush_pending(h); if (rc) return rc; }     // stand-alone move right after the scan
-			if (e2) CK(cudaEventRecord(e2, s));
+			if (h->moverCtas == 0) return flush_pending(h);              // stand-alone move right after the scan
 			// later work on this stream (the next launch reuses the blob scratch, copies read the dense slab) comes after the mover
 			if (movedBuf >= 0) CK(cudaStreamWaitEvent(s, h->evMoved[movedBuf], 0));
+			return SSC_OK;
 		} else {
 			// gzip mode: blobs -> (first batch of a plan: fit the Huffman table to a sample) -> one gzip member per blob -> pass 2 on the members
 			int rc = flush_pending(h);
 			if (rc) return rc;
 			grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount);
 			if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
-			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, e0, e1));
+			CK(time_begin(h, s, &h->stats.gen_kernel_ms, &te));
+			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, nullptr, te));
+			CK(time_begin(h, s, &h->stats.compact_kernel_ms, &te));
 			if (!h->haveGz) { rc = build_gz_tables(h, P, nTiles); if (rc) return rc; }
 			CK(cudaMemsetAsync(h->d_gzLens.p, 0, sizeof(unsigned long long) * nTiles, s));
 			CK(ssc::launch_deflate_blobs(P.out1, P.out2, P.tileState, nTiles, P.blobPitch, h->d_gzBlobs[0], h->d_gzBlobs[1], h->d_gzLens.p,
@@ -371,7 +420,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 			ssc::GenParams P2 = P;
 			P2.out1 = h->d_gzBlobs[0]; P2.out2 = h->d_gzBlobs[1]; P2.tileState = h->d_gzLens.p; P2.blobPitch = FG_CHUNK * FG_SLOT;
 			CK(ssc::launch_pass2(P2, h->smCount, s));
-			if (e2) CK(cudaEventRecord(e2, s));
+			if (te) CK(cudaEventRecord(te, s));
 			h->stats.launches += 4;
 		}
 	} else {
@@ -383,9 +432,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 		CK(ssc::launch_generate(P, v, grid, s));
 		h->stats.launches += 1;
 	}
-	CK(cudaMemcpyAsync(h->h_result[buf], h->d_result[buf], sizeof(ssc::BatchResult), cudaMemcpyDeviceToHost, s));
-	h->stats.gen_launches += 1;
-	return SSC_OK;
+	return result_to_host(h, buf, s);
 }
 
 // error exit of a pipelined call: nothing of it may still be running when the caller sees the code, no batch stays pending
@@ -427,22 +474,28 @@ static int init_handle(ssc_handle* h, int device) {
 	cudaDeviceProp prop;
 	CK(cudaGetDeviceProperties(&prop, device));
 	h->smCount = prop.multiProcessorCount;
-	h->moverCtas = h->smCount >= 64 ? (h->smCount * 8 + 74) / 148 : 0;   // < smCount
+	// 9 of 148 SMs, 0 below 64 SMs.  On the 3 Gb XTen job (B200, tools/pipeline_probe.py) 9 are the fewest under which the scan
+	// and the move of a batch finish before the generation launch on the others does: 8 SMs need 3.88 ms for the move, 9
+	// need 3.46 (+ 0.06 for the scan) under a 3.69 ms launch.  GAIIx and HiSeq2500 move fewer bytes per pair and run 1.4 and
+	// 0.5 % faster on 7 and 8 SMs, but what a profile needs depends on its generation time as much as on its bytes, and one SM
+	// too few costs 4-6 % (the mover sets the step) where one too many costs 0.5-0.7 %: every profile gets the count XTen needs.
+	h->moverCtas = h->smCount >= 64 ? (h->smCount * 9 + 74) / 148 : 0;   // < smCount
 	h->smemLimit = (int)prop.sharedMemPerBlockOptin - 1024;
 	CK(cudaStreamCreateWithFlags(&h->compute, cudaStreamNonBlocking));
 	CK(cudaStreamCreateWithFlags(&h->copy, cudaStreamNonBlocking));
 	CK(cudaStreamCreateWithFlags(&h->copy2, cudaStreamNonBlocking));
 	CK(cudaStreamCreateWithFlags(&h->mover, cudaStreamNonBlocking));
+	CK(cudaStreamCreateWithFlags(&h->results, cudaStreamNonBlocking));
 	CK(cudaEventCreateWithFlags(&h->evPre, cudaEventDisableTiming));
 	CK(cudaEventCreate(&h->evStart));
 	CK(cudaEventCreate(&h->evStop));
 	for (int i = 0; i < 2; i++) {
-		CK(cudaEventCreateWithFlags(&h->evGen[i], cudaEventDisableTiming));
 		CK(cudaEventCreateWithFlags(&h->evCopy[i], cudaEventDisableTiming));
 		CK(cudaEventCreateWithFlags(&h->evCopy2[i], cudaEventDisableTiming));
 		CK(cudaEventCreateWithFlags(&h->evStage[i], cudaEventDisableTiming));
 		CK(cudaEventCreateWithFlags(&h->evDense[i], cudaEventDisableTiming));
 		CK(cudaEventCreateWithFlags(&h->evScanned[i], cudaEventDisableTiming));
+		CK(cudaEventCreateWithFlags(&h->evResult[i], cudaEventDisableTiming));
 		CK(cudaEventCreateWithFlags(&h->evMoved[i], cudaEventDisableTiming));
 		CK(cudaMalloc((void**)&h->d_result[i], sizeof(ssc::BatchResult)));
 		CK(cudaMallocHost((void**)&h->h_result[i], sizeof(ssc::BatchResult)));
@@ -487,11 +540,11 @@ int ssc_destroy(ssc_handle* h) {
 		h->d_blobPrefix[b].release();
 		if (h->evDense[b]) cudaEventDestroy(h->evDense[b]);
 		if (h->evScanned[b]) cudaEventDestroy(h->evScanned[b]);
+		if (h->evResult[b]) cudaEventDestroy(h->evResult[b]);
 		if (h->evMoved[b]) cudaEventDestroy(h->evMoved[b]);
 		if (h->d_result[b]) cudaFree(h->d_result[b]);
 		if (h->h_result[b]) cudaFreeHost(h->h_result[b]);
 		h->d_tileStart[b].release(); h->d_tileState[b].release(); h->d_ticket[b].release();
-		if (h->evGen[b]) cudaEventDestroy(h->evGen[b]);
 		if (h->evCopy[b]) cudaEventDestroy(h->evCopy[b]);
 		if (h->evCopy2[b]) cudaEventDestroy(h->evCopy2[b]);
 		if (h->evStage[b]) cudaEventDestroy(h->evStage[b]);
@@ -517,6 +570,7 @@ int ssc_destroy(ssc_handle* h) {
 	if (h->copy) cudaStreamDestroy(h->copy);
 	if (h->copy2) cudaStreamDestroy(h->copy2);
 	if (h->mover) cudaStreamDestroy(h->mover);
+	if (h->results) cudaStreamDestroy(h->results);
 	if (h->evPre) cudaEventDestroy(h->evPre);
 	delete h;
 	return SSC_OK;
@@ -1097,7 +1151,6 @@ static int generate_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc
 		CK(cudaStreamWaitEvent(h->compute, h->evCopy2[target], 0));
 		int r = launch_batch(h, k & 1, batches[k].lo, batches[k].hi);
 		if (r) return r;
-		CK(cudaEventRecord(h->evGen[k & 1], h->compute));
 		if (!moverCompletes) CK(cudaEventRecord(h->evDense[k & 1], h->compute));     // the dense slab of batch k is complete with its own launch
 		return SSC_OK;
 	};
@@ -1109,7 +1162,7 @@ static int generate_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc
 		rc = k + 1 < nb ? launch(k + 1) : flush_pending(h);         // after this the dense slab of batch k is in the stream
 		if (rc) return rc;
 		if (moverCompletes) CK(cudaEventRecord(h->evDense[buf], h->compute));    // (its pass 2b came with the launch of batch k+1)
-		CK(cudaEventSynchronize(h->evGen[buf]));
+		CK(cudaEventSynchronize(h->evResult[buf]));
 		res[buf] = *h->h_result[buf];
 		rc = check_result(h, res[buf]);
 		if (rc) return rc;
@@ -1165,7 +1218,7 @@ static int generate_device_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_
 	for (int64_t e = eLo; e < eHi; e += h->slabPairs, k++) {
 		const int buf = k & 1;
 		if (k >= 2) {
-			CK(cudaEventSynchronize(h->evGen[buf]));
+			CK(cudaEventSynchronize(h->evResult[buf]));
 			ssc::BatchResult r = *h->h_result[buf];
 			rc = check_result(h, r);
 			if (rc) return rc;
@@ -1173,18 +1226,13 @@ static int generate_device_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_
 		}
 		rc = launch_batch(h, buf, e, std::min(eHi, e + h->slabPairs));
 		if (rc) return rc;
-		CK(cudaEventRecord(h->evGen[buf], h->compute));
 	}
-	// the last batch's blobs: stand-alone move, timed with the scans as "pass 2"
-	while ((int)h->kev.size() < h->kevUsed + 2) { cudaEvent_t e; CK(cudaEventCreate(&e)); h->kev.push_back(e); }
-	const int fl = h->kevUsed;
-	CK(cudaEventRecord(h->kev[fl], h->compute));
-	rc = flush_pending(h);
+	rc = flush_pending(h);                      // the last batch's blobs: stand-alone move, timed with the scans as "pass 2"
 	if (rc) return rc;
-	CK(cudaEventRecord(h->kev[fl + 1], h->compute));
-	CK(cudaEventRecord(h->evStop, h->compute));
+	CK(cudaEventRecord(h->evStop, h->compute));    // the compute stream has waited for the mover stream's last work
 	CK(cudaEventSynchronize(h->evStop));
 	for (int j = std::max(0, k - 2); j < k; j++) {
+		CK(cudaEventSynchronize(h->evResult[j & 1]));
 		ssc::BatchResult r = *h->h_result[j & 1];
 		rc = check_result(h, r);
 		if (rc) return rc;
@@ -1193,16 +1241,11 @@ static int generate_device_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_
 	CK(cudaEventElapsedTime(ms, h->evStart, h->evStop));
 	h->stats.device_ms += *ms;
 	h->timeKernels = false;
-	for (int i = 0; i + 2 < h->kevUsed; i += 3) {
-		float a = 0, b = 0;
-		CK(cudaEventElapsedTime(&a, h->kev[i], h->kev[i + 1]));
-		CK(cudaEventElapsedTime(&b, h->kev[i + 1], h->kev[i + 2]));
-		h->stats.gen_kernel_ms += a; h->stats.compact_kernel_ms += b; h->stats.timed_batches += 1;
-	}
-	{
-		float c = 0;
-		CK(cudaEventElapsedTime(&c, h->kev[fl], h->kev[fl + 1]));
-		h->stats.compact_kernel_ms += c;
+	for (int i = 0; i < h->kevUsed; i++) {
+		float t = 0;
+		CK(cudaEventElapsedTime(&t, h->kev[2 * i], h->kev[2 * i + 1]));
+		*h->kevSum[i] += t;
+		if (h->kevSum[i] == &h->stats.gen_kernel_ms) h->stats.timed_batches += 1;
 	}
 	return SSC_OK;
 }
