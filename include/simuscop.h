@@ -125,6 +125,12 @@ typedef struct ssc_stats {
 	uint64_t bin_bytes;        /* algorithmic bin-record bytes read: 64 bytes per distinct bin of every generated batch */
 	double   mover_kernel_ms;  /* CUDA-event time of the concurrent blob mover (concurrent_move > 0) on its own stream, under the
 	                              generation kernel of the next batch (ssc_generate_device) */
+	/* the generation kernel of the most recent launch (0 before the first): */
+	int32_t  gen_kernel;       /* 1 = fast kernel (K = 3, RL 33..160), 2 = generic kernel with the K = 3 substitution tables in
+	                              shared memory, 3 = generic kernel with the tables in global memory, 4 = FP64 linear search */
+	int32_t  gen_nch;          /* chunks of 32 cycles of the instance: 2..5 for the fast kernel, 10 for the generic kernels */
+	int32_t  gen_qmode;        /* fast kernel: where the quality tables live (8 / 16 / 2 / 0, see "fast_qmode"); -1 otherwise */
+	int32_t  gen_smem_bytes;   /* dynamic shared memory of the launch */
 } ssc_stats;
 
 /*
@@ -149,7 +155,11 @@ int ssc_destroy(ssc_handle* h);
  * bulk-copy kernel on n SMs, on a second stream, while the generation kernel of batch k+1 runs on the others; default 8 of
  * 148 SMs, 0 below 64 SMs; 0, or n at least the GPU's SM count: a stand-alone kernel after every batch), "max_ctas" (> 0 caps the grid of the generation
  * kernel; 0 = one CTA per SM), "no_splice" (0/1, tests: reads with indel events take the position-by-position path
- * of the fast kernel instead of the spliced packed read). */
+ * of the fast kernel instead of the spliced packed read), "fast_qmode" (tests; set before ssc_set_profile: -1 = automatic,
+ * the default; 8 / 16 / 2 / 0 = the fast kernel may only keep its quality tables that way: 8 = every row in shared memory
+ * as 32-bit thresholds (5..8 live symbols per row), 16 = every row as 16-bit keys with an exact repeat on ties (<= 40 live
+ * symbols), 2 = only the ref == call rows in shared memory, 0 = all in global memory.  A mode that does not apply or does
+ * not fit the shared memory leaves the profile to the generic kernel; ssc_stats shows what ran). */
 int ssc_set_option(ssc_handle* h, const char* key, int64_t value);
 
 int ssc_set_profile(ssc_handle* h, const ssc_profile_tables* t);

@@ -38,6 +38,7 @@ class Stats(C.Structure):
         ("fastq_bytes", C.c_uint64), ("hap_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64), ("h2d_bytes", C.c_uint64),
         ("gen_kernel_ms", C.c_double), ("compact_kernel_ms", C.c_double), ("timed_batches", C.c_uint64),
         ("gz_bytes", C.c_uint64), ("bin_bytes", C.c_uint64), ("mover_kernel_ms", C.c_double),
+        ("gen_kernel", C.c_int32), ("gen_nch", C.c_int32), ("gen_qmode", C.c_int32), ("gen_smem_bytes", C.c_int32),
     ]
 
 

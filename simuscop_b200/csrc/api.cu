@@ -85,7 +85,7 @@ struct ssc_handle {
 	// FASTQ slabs of ssc_generate for milliseconds, and no kernel must queue behind it
 	cudaStream_t results = nullptr;
 	cudaEvent_t evResult[2] = {nullptr, nullptr};    // batch of buffer set b: its BatchResult in h_result[b]
-	bool noQ16 = false;           // "no_q16": keep profiles with 9..40 live quality symbols on the diagonal-rows mode (A/B, tests)
+	int fastQmode = -1;           // "fast_qmode": -1 automatic, else the only quality-table mode the fast kernel may use (tests)
 	bool gzip = false;            // slabs hold gzip members (one per ticket blob) instead of plain FASTQ
 	bool haveGz = false;          // Huffman / CRC tables of the current plan are on the device
 	ssc::GzTables* d_gzTab = nullptr;
@@ -363,6 +363,8 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 	P.result = h->d_result[buf];
 	int grid = std::min(nTiles, h->smCount);
 	if (fast) {
+		h->stats.gen_kernel = 1; h->stats.gen_nch = ssc::fast_nch(h->dt.RL); h->stats.gen_qmode = qsmem;
+		h->stats.gen_smem_bytes = (int32_t)fastSmem;
 		// pass 1 writes one blob per ticket and file into the scratch, pass 2 (scan of the blob lengths + one move per blob) the dense slab
 		P.dense1 = P.out1; P.dense2 = P.out2;
 		P.out1 = h->d_slots[buf][0]; P.out2 = h->d_slots[buf][1];
@@ -429,6 +431,8 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 		if (rc) return rc;
 		ssc::GenVariant v = ssc::choose_variant(h->dt, h->fp64, h->smemLimit);
 		if (!v.ok) return fail(SSC_ERR_INVALID, "no kernel variant for read length %d / kmer %d", h->dt.RL, h->dt.K);
+		h->stats.gen_kernel = v.fp64 ? 4 : v.k3 ? 2 : 3; h->stats.gen_nch = v.nch; h->stats.gen_qmode = -1;
+		h->stats.gen_smem_bytes = (int32_t)v.smemBytes;
 		CK(ssc::launch_generate(P, v, grid, s));
 		h->stats.launches += 1;
 	}
@@ -589,9 +593,11 @@ int ssc_set_option(ssc_handle* h, const char* key, int64_t value) {
 		h->moverCtas = value < h->smCount ? (int)value : 0;     // the generation kernel needs SMs beside the mover
 		return SSC_OK;
 	}
-	if (!strcmp(key, "no_q16")) {
-		if (h->haveProfile) return fail(SSC_ERR_STATE, "no_q16 must be set before ssc_set_profile");
-		h->noQ16 = value != 0;
+	if (!strcmp(key, "fast_qmode")) {
+		if (value != -1 && value != 8 && value != 16 && value != 2 && value != 0)
+			return fail(SSC_ERR_INVALID, "fast_qmode must be -1 (automatic), 8, 16, 2 or 0");
+		if (h->haveProfile) return fail(SSC_ERR_STATE, "fast_qmode must be set before ssc_set_profile");
+		h->fastQmode = (int)value;
 		return SSC_OK;
 	}
 	if (!strcmp(key, "max_ctas")) { if (value < 0) return fail(SSC_ERR_INVALID, "max_ctas must be >= 0"); h->maxCtas = (int)value; return SSC_OK; }
@@ -647,7 +653,7 @@ int ssc_set_profile(ssc_handle* h, const ssc_profile_tables* t) {
 	d.delLenT = h->d_delT.p; d.delLenSym = h->d_delSym.p;
 	d.sub = h->d_sub.p; d.nSub = th.nRows * th.B;
 	d.qualT = h->d_qualT.p; d.qualSym = h->d_qualSym.p; d.qualPitch = th.qualPitch; d.nQualRows = 16 * th.B;
-	d.maxQualRow = th.maxQualRow; d.noQ16 = h->noQ16 ? 1 : 0;
+	d.maxQualRow = th.maxQualRow; d.fastQmode = h->fastQmode;
 	d.qualBins = ssc::fast_choose_qbins(th.B, th.RL);
 	d.qualDiagT = h->d_qualDiagT.p; d.qualDiagSym = h->d_qualDiagSym.p; d.qualDiagPitch = th.diagPitch;
 	d.compLut = th.compLut;

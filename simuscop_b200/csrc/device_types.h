@@ -38,7 +38,7 @@ struct DevTables {
 	const uint4* sub; int nSub;              // rows*B per read table; table of read 2 follows when useCdf2
 	const uint32_t* qualT; const uint8_t* qualSym; int qualPitch; int nQualRows;
 	int maxQualRow;                          // live symbols of the longest quality row
-	int noQ16;                               // tests / experiments: do not use the 16-bit-key shared-memory tables
+	int fastQmode;                           // tests: -1 = automatic, else the only quality-table mode fast_supported may choose
 	int qualBins;                            // fast kernel: bins per (ref, call) block of the shared quality image (>= B, see fast_choose_qbins)
 	const uint32_t* qualDiagT; const uint8_t* qualDiagSym; int qualDiagPitch;   // ref == call rows, [N*B][pitch]
 	uint32_t compLut;

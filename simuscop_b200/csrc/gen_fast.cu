@@ -1215,8 +1215,9 @@ bool fast_supported(const DevTables& t, int smemLimit, int* qmode, size_t* smemB
 	// 2: only the ref == call rows; 0: quality table in global memory
 	const int modes[4] = {8, 16, 2, 0};
 	for (int k = 0; k < 4; k++) {
+		if (t.fastQmode >= 0 && modes[k] != t.fastQmode) continue;
 		if (modes[k] == 8 && t.qualPitch != 8) continue;
-		if (modes[k] == 16 && (t.maxQualRow > F_Q16_KEYS || t.noQ16)) continue;
+		if (modes[k] == 16 && t.maxQualRow > F_Q16_KEYS) continue;
 		int qb, qs;
 		fast_qual_bytes(t, modes[k], &qb, &qs);
 		const int total = fast_layout(nSubTotal / t.B * fast_sub_pitch(t.B) * (modes[k] == 16 ? 8 : 16), qb, qs, t.nIsize, t.nInsLen, t.nDelLen).total;
@@ -1234,30 +1235,33 @@ static cudaError_t launch_fast_variant(const GenParams& P, size_t smemBytes, int
 	return cudaGetLastError();
 }
 
+// chunks of 32 cycles of the fast kernel instance for read length RL (33..160): exact, only the last chunk has idle lanes
+int fast_nch(int RL) { return RL <= 64 ? 2 : (RL + 31) / 32; }
+
 // P.out1/out2 = blob scratch, P.dense1/dense2 = final slabs, P.nTiles = tickets of FG_CHUNK pairs.  Launches pass 1;
 // events e0/e1 (optional) bracket the kernel.
 cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream,
                                  cudaEvent_t e0, cudaEvent_t e1) {
-	const int nch = (P.t.RL + 31) / 32;   // the kernel's chunk count is exact: only the last chunk has idle lanes
+	const int nch = fast_nch(P.t.RL);
 	cudaError_t e;
 	if (e0) cudaEventRecord(e0, stream);
 	if (qmode == 8) {
-		if (nch <= 2) e = launch_fast_variant<2, 8>(P, smemBytes, grid, stream);
+		if (nch == 2) e = launch_fast_variant<2, 8>(P, smemBytes, grid, stream);
 		else if (nch == 3) e = launch_fast_variant<3, 8>(P, smemBytes, grid, stream);
 		else if (nch == 4) e = launch_fast_variant<4, 8>(P, smemBytes, grid, stream);
 		else e = launch_fast_variant<5, 8>(P, smemBytes, grid, stream);
 	} else if (qmode == 16) {
-		if (nch <= 2) e = launch_fast_variant<2, 16>(P, smemBytes, grid, stream);
+		if (nch == 2) e = launch_fast_variant<2, 16>(P, smemBytes, grid, stream);
 		else if (nch == 3) e = launch_fast_variant<3, 16>(P, smemBytes, grid, stream);
 		else if (nch == 4) e = launch_fast_variant<4, 16>(P, smemBytes, grid, stream);
 		else e = launch_fast_variant<5, 16>(P, smemBytes, grid, stream);
 	} else if (qmode == 2) {
-		if (nch <= 2) e = launch_fast_variant<2, 2>(P, smemBytes, grid, stream);
+		if (nch == 2) e = launch_fast_variant<2, 2>(P, smemBytes, grid, stream);
 		else if (nch == 3) e = launch_fast_variant<3, 2>(P, smemBytes, grid, stream);
 		else if (nch == 4) e = launch_fast_variant<4, 2>(P, smemBytes, grid, stream);
 		else e = launch_fast_variant<5, 2>(P, smemBytes, grid, stream);
 	} else {
-		if (nch <= 2) e = launch_fast_variant<2, 0>(P, smemBytes, grid, stream);
+		if (nch == 2) e = launch_fast_variant<2, 0>(P, smemBytes, grid, stream);
 		else if (nch == 3) e = launch_fast_variant<3, 0>(P, smemBytes, grid, stream);
 		else if (nch == 4) e = launch_fast_variant<4, 0>(P, smemBytes, grid, stream);
 		else e = launch_fast_variant<5, 0>(P, smemBytes, grid, stream);

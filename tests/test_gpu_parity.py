@@ -32,17 +32,18 @@ def test_fastq_bit_exact_vs_instrumented_reference(name, gen, workdir):
         assert len(r1) > 0
 
 
-# pass 2 of the fast kernel: a stand-alone move after every batch (what GPUs with fewer than 64 SMs run), or the bulk-copy mover
-MOVE_MODES = {"standalone_move": ("concurrent_move", 0), "concurrent_move": ("concurrent_move", 8)}
+# pass 2 of the fast kernel: a stand-alone move after every batch (what GPUs with fewer than 64 SMs run), or the bulk-copy mover;
+# the fast kernel with only the ref == call quality rows in shared memory
+OPTION_MODES = {"standalone_move": ("concurrent_move", 0), "concurrent_move": ("concurrent_move", 8), "fast_qmode2": ("fast_qmode", 2)}
 
 
-@pytest.mark.parametrize("mode", ["force_generic", "fp64_search", "no_splice", "no_q16", "standalone_move", "concurrent_move"])
+@pytest.mark.parametrize("mode", ["force_generic", "fp64_search", "no_splice", "fast_qmode2", "standalone_move", "concurrent_move"])
 @pytest.mark.parametrize("name", ["pe_xten", "pe_tiny", "se_gaiix"])
 def test_fallback_kernels_bit_exact(name, mode, built, workdir):
     """The generic integer kernel, the FP64 linear-search ground-truth kernel, the fast kernel without the spliced indel path,
-    without the 16-bit-key shared-memory tables (profiles with 9..40 live quality symbols then keep only the ref == call rows
-    in shared memory), with pass 2 as a stand-alone move after every batch, and with pass 2 on the bulk-copy mover (8 SMs,
-    second stream, under the next batch's generation) all give the same bytes."""
+    with only the ref == call quality rows in shared memory (the rare substituted bases read the full table in global
+    memory), with pass 2 as a stand-alone move after every batch, and with pass 2 on the bulk-copy mover (8 SMs, second
+    stream, under the next batch's generation) all give the same bytes, and the statistics name the kernel that ran."""
     from simuscop_b200 import cuda_binding
     scn = helpers.build_scenario(name, workdir)
     plans, out = helpers.reference_run(scn, tag=mode)
@@ -51,16 +52,22 @@ def test_fallback_kernels_bit_exact(name, mode, built, workdir):
     r1, r2 = helpers.read_file(r1p), helpers.read_file(r2p)
     g = cuda_binding.Generator(0)
     try:
-        key, value = MOVE_MODES.get(mode, (mode, 1))
+        key, value = OPTION_MODES.get(mode, (mode, 1))
         g.set_option(key, value)
-        if mode in MOVE_MODES:
+        if key == "concurrent_move":
             g.set_option("batch_pairs", 256)          # many batches: with the mover, every launch but the first moves its predecessor's blobs
         g.load_plan(plan, scn["seed"])
         f1, f2 = g.generate()
+        st = g.stats()
     finally:
         g.close()
     assert helpers.first_diff(f1, r1) == -1
     assert helpers.first_diff(f2, r2) == -1
+    kernel = {"force_generic": (2, 3), "fp64_search": (4,)}.get(mode, (1,))
+    assert st["gen_kernel"] in kernel, st
+    if mode == "fast_qmode2":
+        rl = plan.hdr["read_length"]
+        assert (st["gen_nch"], st["gen_qmode"]) == (2 if rl <= 64 else (rl + 31) // 32, 2), st
 
 
 def test_error_in_a_pipelined_call_leaves_the_handle_usable(built, workdir):
