@@ -104,7 +104,7 @@ typedef struct ssc_segment {
 	int64_t first_bin;
 	int64_t n_bins;
 	int32_t name_offset;  /* "@<popu>#<chr>#" inside the name blob (Segment.cpp:780,809,824) */
-	int32_t name_len;
+	int32_t name_len;     /* 1..64 bytes, the first one '@'; the blob is < 2^17 bytes */
 } ssc_segment;
 
 typedef struct ssc_stats {
@@ -167,7 +167,8 @@ int ssc_set_profile(ssc_handle* h, const ssc_profile_tables* t);
 /* Haplotype store: 2-bit codes (in the profile's `bases` order) + 1-bit non-ACGT mask,
  * packed on the device from ASCII (any case; every non-ACGT character behaves as N).
  * Append the haplotype strings contig by contig; *first_base receives the store index of
- * the first appended base. */
+ * the first appended base.  ssc_genome_reserve refuses (SSC_ERR_INVALID, before allocating) a store of more than
+ * 2^36 - 32 bases: the fast kernel addresses a read's window by a 32-bit index of 16-base words. */
 int ssc_genome_reserve(ssc_handle* h, uint64_t total_bases);
 int ssc_genome_append(ssc_handle* h, const char* ascii, uint64_t n, uint64_t* first_base);
 int ssc_genome_size(ssc_handle* h, uint64_t* n_bases);

@@ -679,6 +679,10 @@ int ssc_set_profile(ssc_handle* h, const ssc_profile_tables* t) {
 int ssc_genome_reserve(ssc_handle* h, uint64_t total_bases) {
 	if (!h) return fail(SSC_ERR_INVALID, "null handle");
 	if (!h->haveProfile) return fail(SSC_ERR_STATE, "ssc_set_profile must precede ssc_genome_reserve (codes follow the profile's base order)");
+	// checked before anything is allocated (k_winA / k_winB of gen_fast.cu; the 32-bit index is a deliberate saving)
+	if (total_bases > SSC_MAX_STORE_BASES)
+		return fail(SSC_ERR_INVALID, "haplotype store of %llu bases (limit %llu)", (unsigned long long)total_bases,
+		            (unsigned long long)SSC_MAX_STORE_BASES);
 	CK(cudaSetDevice(h->device));
 	uint64_t groups = (total_bases + SSC_GPAD + 31) / 32 + 2;
 	CK(h->d_hap2.alloc(groups * 2 + 64));
@@ -941,7 +945,7 @@ int ssc_gc_census(ssc_handle* h, const int64_t* starts, const int32_t* lens, int
 
 int ssc_set_plan(ssc_handle* h, uint64_t seed, const ssc_bin* bins, int64_t n_bins, const ssc_segment* segs,
                  int64_t n_segs, const char* names, int64_t names_len, int64_t* planned_pairs, int64_t* emitted_pairs) {
-	if (!h || (!bins && n_bins) || (!segs && n_segs)) return fail(SSC_ERR_INVALID, "null argument");
+	if (!h || (!bins && n_bins) || (!segs && n_segs) || (!names && names_len)) return fail(SSC_ERR_INVALID, "null argument");
 	if (!h->haveProfile) return fail(SSC_ERR_STATE, "ssc_set_profile must precede ssc_set_plan");
 	CK(cudaSetDevice(h->device));
 	const ssc::DevTables& t = h->dt;
@@ -973,8 +977,10 @@ int ssc_set_plan(ssc_handle* h, uint64_t seed, const ssc_bin* bins, int64_t n_bi
 	for (int64_t s = 0; s < n_segs; s++) {
 		if (segs[s].first_bin < 0 || segs[s].n_bins < 0 || segs[s].first_bin + segs[s].n_bins > n_bins)
 			return fail(SSC_ERR_INVALID, "segment %lld: bin range out of bounds", (long long)s);
-		if (segs[s].name_len < 0 || segs[s].name_len > 64 || segs[s].name_offset < 0 || segs[s].name_offset + segs[s].name_len > names_len)
-			return fail(SSC_ERR_INVALID, "segment %lld: bad name (max 64 bytes)", (long long)s);
+		// a name is "@" + popu + "#" + chr + "#" (the '@' is written as part of it, 1..64 bytes)
+		if (segs[s].name_len < 1 || segs[s].name_len > 64 || segs[s].name_offset < 0 || segs[s].name_offset + segs[s].name_len > names_len ||
+		    names[segs[s].name_offset] != '@')
+			return fail(SSC_ERR_INVALID, "segment %lld: bad name (1..64 bytes starting with '@')", (long long)s);
 		maxName = std::max(maxName, (int)segs[s].name_len);
 	}
 	struct BinError { int64_t bin = -1; const char* what = nullptr; };

@@ -20,6 +20,9 @@
 #endif
 #define FG_SLOT 640                               /* bytes of HBM scratch per record (>= 96 + 2*256 + 4) */
 #define SSC_GPAD 64                               /* zero bases in front of the haplotype store */
+/* largest haplotype store: the fast kernel's 32-bit window word index (g - 32) >> 4 of device base g = SSC_GPAD + store
+   index must not wrap for any base, i.e. SSC_GPAD + total_bases - 1 - 32 < 2^36 */
+#define SSC_MAX_STORE_BASES ((1ull << 36) + 32 - SSC_GPAD)
 
 namespace ssc {
 
