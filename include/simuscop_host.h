@@ -35,6 +35,14 @@ const char* ssh_output_dir(ssh_job* job);
 /* dump_path may be NULL; otherwise an SSCPLAN1 file of the sample is written there */
 int ssh_prepare_sample(ssh_job* job, int s, ssc_handle* dev, const char* dump_path,
                        int64_t* planned_pairs, int64_t* emitted_pairs);
+/* The answer key of sample s: a VCFv4.2 file at `path` with every SNV and indel the sample's haplotypes hold, one phased
+ * allele per copy (GT:HCN in the column of every population the sample draws from, '.' in the others; INFO/EAF the expected
+ * allele fraction in this sample) and one <CNV> record per copy-number segment of the variation file (CN:MCN:HCN).  Call it
+ * right after ssh_prepare_sample(job, s, ...) and before the next sample is prepared: it reads the phasing state as it stands
+ * (a segment the reference leaves without a major set is phased again for the next sample).  Draws nothing from the plan RNG,
+ * so the plans of later samples do not change.  The CLI writes it as <output>/<stem>.truth.vcf when SIMUSCOP_TRUTH_VCF=1.
+ * Returns SSC_ERR_STATE unless s is the sample prepared last, SSC_ERR_SINK when the file cannot be written. */
+int ssh_write_truth_vcf(ssh_job* job, int s, const char* path);
 /* Host-only self test (no GPU): the splice lists from which the device assembles haplotypes with insertion / deletion
  * variants, materialised on the host, against the string construction of Segment::generateSegSequences
  * (lib/segment/Segment.cpp:124-460).  Returns the number of differing haplotypes. */

@@ -45,6 +45,7 @@ public:
 	// (lib/mydefine/MyDefine.cpp:279-303) counts only a literal 'N' as unknown, the device mask every non-ACGT character
 	bool other_in(size_t a, size_t b) const;
 	const FastaEntry* entry(const std::string& chr) const;   // .fai geometry of a record, nullptr when unknown
+	std::vector<FastaEntry> records;                         // every .fai record in index order, named by the first word of its header line
 	int fd();                                                // the FASTA file, opened read-only on first use
 	~Fasta();
 private:
@@ -92,6 +93,7 @@ struct ChrLayout {   // where the haplotype strings of one chromosome live in th
 
 struct Segment {
 	int idx; std::string chr; long start, end; int CN, mCN;
+	bool fromCnv = false;                // made from a 'c' record of the variation file (not the ploidy default between them)
 	std::vector<int> seqReps, mIndx, targetIdx;
 	std::vector<Bin> bins; bool weighted = false;
 	std::vector<std::string> hapCache;   // haplotypes kept between the weights pass and materialisation (memory permitting)
@@ -131,6 +133,8 @@ public:
 	void phase_segment(Segment& seg);                        // rand()-driven copy-number phasing (Segment.cpp:140-215)
 	bool segment_is_copy_only(const Segment& seg, const std::string& popu);
 	void segment_copies_and_pokes(Segment& seg, const std::string& popu, std::vector<int>& reps, std::vector<Poke>& pokes);
+	// the same from the phasing state as it stands: draws nothing, for a segment that has been phased
+	void phased_copies_and_pokes(const Segment& seg, const std::string& popu, std::vector<int>& reps, std::vector<Poke>& pokes);
 	// the insert / erase part of Segment::generateSegSequences (Segment.cpp:313-444) on splice lists instead of strings
 	void segment_splices(Segment& seg, const std::string& popu, size_t refLen, const std::vector<int>& reps, std::vector<std::vector<Piece>>& ropes);
 	// bins + weights (Segment::getWeightedLength, Segment.cpp:550-641)
@@ -149,6 +153,12 @@ public:
 	int prepare_sample(int s, ssc_handle* dev, const std::string& dumpPath, int64_t* planned, int64_t* emitted);
 	// same, replicated into several device handles (one per GPU); an empty list = plan-only mode
 	int prepare_sample_multi(int s, const std::vector<ssc_handle*>& devs, const std::string& dumpPath, int64_t* planned, int64_t* emitted);
+	int lastPrepared = -1;                                    // the sample prepared last
+	// truth.cpp: the variants and copy numbers the haplotypes of sample `s` carry, as a phased per-copy VCF (DESIGN.md section 10).
+	// Reads the phasing state as it stands and draws nothing, so it describes sample `s` only while `s` is the sample prepared
+	// last (a segment the reference leaves without a major set is phased again for the next sample).  0, or SSC_ERR_SINK when
+	// `path` cannot be written.
+	int write_truth_vcf(int s, const std::string& path);
 private:
 	void load_variations();
 	void load_snps();
@@ -156,7 +166,7 @@ private:
 	void divide_targets();
 	void load_abundance();
 	void generate_segments();
-	void divide_segment(const std::string& popu, const std::string& chr, long s, long e, int CN, int mCN, int& idx);
+	void divide_segment(const std::string& popu, const std::string& chr, long s, long e, int CN, int mCN, int& idx, bool fromCnv);
 	long rand_int(long a, long b);                            // randomInteger, lib/mydefine/MyDefine.cpp:192-194
 };
 

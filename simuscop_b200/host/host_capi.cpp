@@ -173,6 +173,15 @@ int turn_sink(void* user, const char* b1, size_t l1, const char* b2, size_t l2, 
 	return e ? 1 : 0;
 }
 
+// SIMUSCOP_TRUTH_VCF=1: <output>/<stem>.truth.vcf of sample s, written once the sample is prepared
+int write_truth(sschost::Job& J, int s) {
+	const char* t = getenv("SIMUSCOP_TRUTH_VCF");
+	if (!t || atoi(t) == 0) return 0;
+	const std::string path = J.cfg.str["output"] + "/" + J.samples[s].stem + ".truth.vcf";
+	if (J.write_truth_vcf(s, path)) { std::cerr << "Error: can not write the truth VCF " << path << std::endl; return SSC_ERR_SINK; }
+	return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -196,6 +205,12 @@ const char* ssh_output_dir(ssh_job* job) { return job->job.cfg.str["output"].c_s
 int ssh_prepare_sample(ssh_job* job, int s, ssc_handle* dev, const char* dump_path, int64_t* planned, int64_t* emitted) {
 	if (!job || s < 0 || s >= (int)job->job.samples.size()) return SSC_ERR_INVALID;
 	return job->job.prepare_sample(s, dev, dump_path ? dump_path : "", planned, emitted);
+}
+
+int ssh_write_truth_vcf(ssh_job* job, int s, const char* path) {
+	if (!job || !path || s < 0 || s >= (int)job->job.samples.size()) return SSC_ERR_INVALID;
+	if (s != job->job.lastPrepared) return SSC_ERR_STATE;
+	return job->job.write_truth_vcf(s, path);
 }
 
 int ssh_selftest_splices(ssh_job* job, int64_t* segments_checked, int64_t* with_indels) {
@@ -289,6 +304,8 @@ int ssh_run(ssh_job* job, int device) {
 			int64_t a, b;
 			int r = job->job.prepare_sample(s, nullptr, std::string(prefix) == "none" ? std::string() : std::string(prefix) + "." + std::to_string(s) + ".plan", &a, &b);
 			if (r) return r;
+			r = write_truth(job->job, s);
+			if (r) return r;
 		}
 		return 0;
 	}
@@ -325,6 +342,8 @@ int ssh_run(ssh_job* job, int device) {
 		int64_t planned = 0, emitted = 0;
 		rc = J.prepare_sample_multi(s, devs, dump, &planned, &emitted);
 		if (rc) { std::cerr << "Error: " << ssc_last_error() << std::endl; break; }
+		rc = write_truth(J, s);
+		if (rc) break;
 		// one ordered writer per sample.  One GPU: a single ssc_generate call over the whole job (the library pipelines kernel,
 		// device->host copy and sink).  Several GPUs: the job is cut into batches, batch k goes to GPU k mod G, and every
 		// finished slab waits at the writer's turnstile until all earlier batches are in the file -- one pass of I/O, no part

@@ -170,6 +170,7 @@ void Fasta::open(const std::string& path) {
 			die(1, "Warning: malformed fasta index file " + fai + " does not have enough fields @line " + std::to_string(ln) + "\n" + line);
 		std::string name = abbr_chr(first_token(f5[0]));
 		names.push_back(name);
+		records.push_back(FastaEntry{first_token(f5[0]), atol(f5[1].c_str()), atoll(f5[2].c_str()), atoi(f5[3].c_str()), atoi(f5[4].c_str())});
 		idx_.insert(std::make_pair(name, FastaEntry{f5[0], atol(f5[1].c_str()), atoll(f5[2].c_str()), atoi(f5[3].c_str()), atoi(f5[4].c_str())}));
 	}
 }

@@ -21,12 +21,12 @@ long Job::rand_int(long start, long end) {
 }
 
 // Genome::divideSegment, lib/genome/Genome.cpp:741-763
-void Job::divide_segment(const std::string& popu, const std::string& chr, long s, long e, int CN, int mCN, int& idx) {
+void Job::divide_segment(const std::string& popu, const std::string& chr, long s, long e, int CN, int mCN, int& idx, bool fromCnv) {
 	const unsigned int segMax = 1000000;
 	std::vector<Segment>& v = segs[popu][chr];
 	auto make = [&](long a, long b) {
 		Segment g;
-		g.idx = idx++; g.chr = chr; g.start = a; g.end = b; g.CN = CN; g.mCN = mCN;
+		g.idx = idx++; g.chr = chr; g.start = a; g.end = b; g.CN = CN; g.mCN = mCN; g.fromCnv = fromCnv;
 		auto it = targets.find(chr);                         // Segment::initTargets, Segment.cpp:67-79
 		if (!targets.empty() && it != targets.end())
 			for (size_t i = 0; i < it->second.size(); i++) {
@@ -63,11 +63,11 @@ void Job::generate_segments() {
 			for (auto c : cv) {
 				if (segStart > chrLen) break;
 				c.epos = std::min(c.epos, chrLen);
-				if (segStart < c.spos) divide_segment(popu, chr, segStart, c.spos - 1, ploidy, mCN, idx);
-				divide_segment(popu, chr, c.spos, c.epos, (int)c.cn, (int)c.mcn, idx);
+				if (segStart < c.spos) divide_segment(popu, chr, segStart, c.spos - 1, ploidy, mCN, idx, false);
+				divide_segment(popu, chr, c.spos, c.epos, (int)c.cn, (int)c.mcn, idx, true);
 				segStart = c.epos + 1;
 			}
-			if (segStart <= chrLen) divide_segment(popu, chr, segStart, chrLen, ploidy, mCN, idx);
+			if (segStart <= chrLen) divide_segment(popu, chr, segStart, chrLen, ploidy, mCN, idx, false);
 		}
 	}
 }
@@ -347,9 +347,13 @@ bool Job::segment_is_copy_only(const Segment& seg, const std::string& popu) {
 
 // copies per haplotype index and the substitutions (haplotype, offset in the first copy, allele) in application order
 void Job::segment_copies_and_pokes(Segment& seg, const std::string& popu, std::vector<int>& reps, std::vector<Poke>& pokes) {
-	const int ploidy = cfg.num["ploidy"];
 	if (seg.CN == 0) die(1, "ERROR: copy number 0 segments are not supported (" + popu + " " + seg.chr + ":" + std::to_string(seg.start) + ")");
 	phase_segment(seg);
+	phased_copies_and_pokes(seg, popu, reps, pokes);
+}
+
+void Job::phased_copies_and_pokes(const Segment& seg, const std::string& popu, std::vector<int>& reps, std::vector<Poke>& pokes) {
+	const int ploidy = cfg.num["ploidy"];
 	reps.assign(ploidy, 0);
 	for (int i = 0; i < ploidy; i++)
 		reps[i] = seg.CN < ploidy ? (std::find(seg.seqReps.begin(), seg.seqReps.end(), i) != seg.seqReps.end() ? 1 : 0) : seg.seqReps[i];
@@ -983,13 +987,14 @@ int Job::prepare_sample_multi(int s, const std::vector<ssc_handle*>& devs, const
 		pw.rec(7, names);
 	}
 	if (pw.fp) { pw.rec(9, std::string()); fclose(pw.fp); }
-	if (devs.empty()) { if (planned) *planned = 0; if (emitted) *emitted = 0; return 0; }
+	if (devs.empty()) { if (planned) *planned = 0; if (emitted) *emitted = 0; lastPrepared = s; return 0; }
 	const double ts0 = PhaseTimers::now();
 	for (ssc_handle* dev : devs) {
 		rc = ssc_set_plan(dev, seed, bins.data(), (int64_t)bins.size(), segments.data(), (int64_t)segments.size(),
 		                  names.data(), (int64_t)names.size(), planned, emitted);
 		if (rc) return rc;
 	}
+	lastPrepared = s;
 	g_tm.setPlan += PhaseTimers::now() - ts0;
 	if (getenv("SIMUSCOP_TIMING"))
 		fprintf(stderr, "[simuscop timing] reference upload / haplotype strings %.2f s, append+pack %.2f s, gc census (device, incl. bin enumeration %.2f s) %.2f s, "

@@ -23,6 +23,7 @@ def lib():
         L.ssh_output_dir.argtypes = [C.c_void_p]
         L.ssh_output_dir.restype = C.c_char_p
         L.ssh_prepare_sample.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_char_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+        L.ssh_write_truth_vcf.argtypes = [C.c_void_p, C.c_int, C.c_char_p]
         L.ssh_run.argtypes = [C.c_void_p, C.c_int]
         _lib = L
     return _lib
@@ -62,3 +63,9 @@ class Job:
                 rc, cuda_binding.lib().ssc_last_error().decode(errors="replace")))
         gen.planned, gen.emitted = pp.value, ep.value
         return pp.value, ep.value
+
+    def write_truth_vcf(self, sample, path):
+        """Writes the truth VCF of `sample` (after prepare() of that sample) to `path`."""
+        rc = lib().ssh_write_truth_vcf(self.j, sample, path.encode())
+        if rc:
+            raise RuntimeError("ssh_write_truth_vcf failed (%d)" % rc)
