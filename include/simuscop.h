@@ -151,8 +151,10 @@ int ssc_destroy(ssc_handle* h);
 /* "batch_pairs" (pairs per kernel launch), "fp64_search" (0/1: use the FP64 linear-search
  * ground-truth kernel instead of the integer-threshold kernel), "force_generic" (0/1), "gzip" (0/1: the slabs
  * handed to the sink hold concatenated gzip members -- a valid .gz stream of the same FASTQ bytes -- compressed on
- * the GPU; the plain bytes of SeqWriter::write are the default), "concurrent_move" (n > 0: the blobs of batch k are moved by a
- * bulk-copy kernel on n SMs, on a second stream, while the generation kernel of batch k+1 runs on the others; default 8 of
+ * the GPU, one member per 32 pairs, Huffman-coded with a table fitted to the first batch, or stored where that code would
+ * expand the member past its bytes + 23, so gzip mode fails only where plain output does; the plain bytes of
+ * SeqWriter::write are the default), "concurrent_move" (n > 0: the blobs of batch k are moved by a
+ * bulk-copy kernel on n SMs, on a second stream, while the generation kernel of batch k+1 runs on the others; default 9 of
  * 148 SMs, 0 below 64 SMs; 0, or n at least the GPU's SM count: a stand-alone kernel after every batch), "max_ctas" (> 0 caps the grid of the generation
  * kernel; 0 = one CTA per SM), "no_splice" (0/1, tests: reads with indel events take the position-by-position path
  * of the fast kernel instead of the spliced packed read), "fast_qmode" (tests; set before ssc_set_profile: -1 = automatic,
@@ -236,7 +238,8 @@ int ssc_sub_lookup_host(const double* cdf4, uint32_t u);
 
 /* Host-only diagnostic (no GPU needed): one gzip member of in[0..n) built with the device encoder's own tables
  * (Huffman code fitted to the byte histogram of `sample`, CRC-32 by the kernel's lane-strided algebra) and bit
- * packing.  Returns the member size, or -1.  Tests inflate it with zlib. */
+ * packing, stored instead when coding would make it longer than n + 23 bytes, as on the device.  Returns the member size,
+ * 0 when it does not fit `cap`, or -1.  Tests inflate it with zlib and compare it with the device's members. */
 int64_t ssc_gzip_member_host(const uint8_t* in, uint32_t n, const uint8_t* sample, size_t sample_n, uint8_t* out, size_t cap);
 
 /* Measurement aid (no reference counterpart): the instruction-issue ceiling of the generation kernel on this GPU.

@@ -184,12 +184,15 @@ bool use_fast(const ssc_handle* h, int* qmode, size_t* smemBytes) {
 int ensure_batch_resources(ssc_handle* h, bool needHost) {
 	int64_t pairs = std::min<int64_t>(h->batchPairs, std::max<int64_t>(h->emittedPairs, 1));
 	pairs = ((pairs + GEN_TILE_PAIRS - 1) / GEN_TILE_PAIRS) * GEN_TILE_PAIRS;   // multiple of both tile sizes
-	uint64_t cap = (uint64_t)pairs * (uint64_t)h->maxRecBytes + 4096;
+	// gzip mode: a member is at most its blob plus the bytes of a stored block (gz.cu), and there is one member per ticket
+	const uint64_t perPair = (uint64_t)h->maxRecBytes + (h->gzip ? 1 : 0);
+	auto slab_cap = [&](int64_t n) { return (uint64_t)n * (uint64_t)h->maxRecBytes + 4096 + (h->gzip ? (uint64_t)(n / FG_CHUNK) * ssc::GZ_STORED_EXTRA : 0); };
+	uint64_t cap = slab_cap(pairs);
 	if (cap >= (1ull << 31)) {
-		pairs = (int64_t)(((1ull << 31) - 8192) / (uint64_t)h->maxRecBytes);
+		pairs = (int64_t)(((1ull << 31) - 8192) / perPair);
 		pairs = (pairs / GEN_TILE_PAIRS) * GEN_TILE_PAIRS;
 		if (pairs <= 0) return fail(SSC_ERR_INVALID, "record size too large");
-		cap = (uint64_t)pairs * (uint64_t)h->maxRecBytes + 4096;
+		cap = slab_cap(pairs);
 	}
 	int nFiles = h->dt.paired ? 2 : 1;
 	{
@@ -197,7 +200,7 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 		const int64_t maxFast = (int64_t)(((1ull << 32) - (1ull << 20)) / ((uint64_t)FG_SLOT * (uint64_t)nFiles));
 		if (pairs > maxFast) {
 			pairs = (maxFast / GEN_TILE_PAIRS) * GEN_TILE_PAIRS;
-			cap = (uint64_t)pairs * (uint64_t)h->maxRecBytes + 4096;
+			cap = slab_cap(pairs);
 		}
 	}
 	if (pairs != h->slabPairs || cap != h->slabCap) {
@@ -418,7 +421,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 			if (!h->haveGz) { rc = build_gz_tables(h, P, nTiles); if (rc) return rc; }
 			CK(cudaMemsetAsync(h->d_gzLens.p, 0, sizeof(unsigned long long) * nTiles, s));
 			CK(ssc::launch_deflate_blobs(P.out1, P.out2, P.tileState, nTiles, P.blobPitch, h->d_gzBlobs[0], h->d_gzBlobs[1], h->d_gzLens.p,
-			                             FG_CHUNK * FG_SLOT, h->d_gzTab, &P.result->errorFlags, h->smCount, s));
+			                             FG_CHUNK * FG_SLOT, h->d_gzTab, h->smCount, s));
 			ssc::GenParams P2 = P;
 			P2.out1 = h->d_gzBlobs[0]; P2.out2 = h->d_gzBlobs[1]; P2.tileState = h->d_gzLens.p; P2.blobPitch = FG_CHUNK * FG_SLOT;
 			CK(ssc::launch_pass2(P2, h->smCount, s));
@@ -455,7 +458,6 @@ int check_result(ssc_handle* h, const ssc::BatchResult& r) {
 	if (r.errorFlags & 1u) return fail(SSC_ERR_OVERFLOW, "output slab overflow (internal capacity estimate too small)");
 	if (r.errorFlags & 2u) return fail(SSC_ERR_OVERFLOW, "a read outgrew the per-read scratch (insertions > 96 bases)");
 	if (r.errorFlags & 4u) return fail(SSC_ERR_OVERFLOW, "more than 32 indel events or 128 inserted bases in one read");
-	if (r.errorFlags & 8u) return fail(SSC_ERR_OVERFLOW, "a gzip member outgrew its scratch blob");
 	h->stats.pairs_emitted += r.pairs;
 	h->stats.reads_emitted += r.reads;
 	h->stats.bases_emitted += r.bases;
@@ -1132,7 +1134,7 @@ int ssc_set_plan(ssc_handle* h, uint64_t seed, const ssc_bin* bins, int64_t n_bi
 	CK(cudaStreamSynchronize(s));
 	h->stats.h2d_bytes += nDev * sizeof(ssc::DevBin) + devEmitBase.size() * 8;
 	// worst-case record bytes per pair per file: header + 2*(RL + 96) + 4
-	h->maxRecBytes = maxName + 10 + 1 + 10 + 3 + 2 * (RL + 16) + 4;
+	h->maxRecBytes = maxName + 10 + 1 + 10 + 3 + 2 * (RL + 96) + 4;
 	h->havePlan = true;
 	if (planned_pairs) *planned_pairs = h->plannedPairs;
 	if (emitted_pairs) *emitted_pairs = h->emittedPairs;
@@ -1294,7 +1296,7 @@ int ssc_sub_lookup_host(const double* cdf4, uint32_t u) {
 }
 
 int64_t ssc_gzip_member_host(const uint8_t* in, uint32_t n, const uint8_t* sample, size_t sample_n, uint8_t* out, size_t cap) {
-	if (!in || !out || n < 8) return -1;
+	if (!in || !out || n == 0) return -1;
 	uint64_t hist[256];
 	memset(hist, 0, sizeof(hist));
 	for (size_t i = 0; i < sample_n; i++) hist[sample[i]]++;

@@ -53,7 +53,7 @@ struct DevTables {
 struct BatchResult {
 	unsigned long long bytes1, bytes2;
 	unsigned long long bases, reads, pairs, hapBytes;
-	unsigned int errorFlags;   // bit0: slab overflow, bit1: read outgrew scratch, bit2: too many indel events, bit3: gzip blob overflow
+	unsigned int errorFlags;   // bit0: slab overflow, bit1: read outgrew scratch, bit2: too many indel events
 	unsigned int pad;
 	unsigned long long rawBytes;   // fast kernel: FASTQ bytes generated (bytes1/bytes2 are compressed sizes in gzip mode)
 };

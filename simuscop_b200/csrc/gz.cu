@@ -5,13 +5,18 @@
 // ~2 bits per character.  The table is fitted on the host to a sample of the first batch and shared by all
 // members, so the per-member cost is a ~60-byte block header.  Concatenated members are a valid .gz file
 // (SeqWriter's plain files, lib/seqwriter/SeqWriter.cpp:41-54, remain the default output).
+// Bytes absent from the sample still get codes, of 14-15 bits: a later blob full of them (a 64-byte name that is not in
+// the sample, N-run qualities) can code to nearly twice its size.  So, as zlib does, a member whose coded form would be
+// longer than its raw bytes + 23 is written as one stored block instead (gzip header, 0x01, LEN, NLEN, the raw bytes,
+// CRC-32, ISIZE): no member exceeds its blob + 23 bytes (a blob is at most 32 x 612 = 19 584 bytes, its scratch 20 480).
 //
 // Kernel: one warp per (ticket, file).  A round takes 256 bytes (two 32-bit words per lane): LUT -> up to 2 x 60 bits
 // per lane, warp scan of the bit counts, OR into a shared-memory round buffer (two buffers in turn: the one just
 // written out is zeroed word by word as it is stored), coalesced store of the completed words.  CRC-32 (the gzip
 // trailer) is computed on the fly without a second pass: lane l keeps the pure remainder of its strided word pairs
 // (slice-by-4 tables), advanced by 256 bytes of zeros per round through four 256-entry tables of the linear map
-// x^2048 mod P; the lanes are combined at the end with one GF(2) multiplication each.
+// x^2048 mod P; the lanes are combined at the end with one GF(2) multiplication each.  Coded words past the scratch pitch
+// are counted but not stored: such a member is always rewritten in the stored form.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -208,10 +213,11 @@ const char* gz_build_tables(const uint64_t hist[256], GzTables* t) {
 	return "";
 }
 
-// Host mirror of deflate_blobs_kernel for one blob (same tables, same lane-strided CRC arithmetic, same bit packing):
-// lets the table construction and the CRC algebra be checked against zlib without a GPU.  Returns the member size or 0.
+// Host mirror of deflate_blobs_kernel for one blob (same tables, same lane-strided CRC arithmetic, same bit packing, same
+// choice between the coded and the stored form): lets the table construction and the CRC algebra be checked against zlib
+// without a GPU, and the kernel's members byte for byte.  Returns the member size, or 0 when it does not fit cap.
 size_t gz_member_host(const GzTables* t, const uint8_t* src, uint32_t len, uint8_t* dst, size_t cap) {
-	if (len < 8) return 0;
+	if (len == 0 || len > 0xFFFFu) return 0;
 	std::vector<uint32_t> out(t->prefix, t->prefix + ((t->prefixBits + 31) >> 5));
 	uint64_t bits = t->prefixBits;
 	auto put = [&](uint64_t v, uint32_t n) {
@@ -244,6 +250,15 @@ size_t gz_member_host(const GzTables* t, const uint8_t* src, uint32_t len, uint8
 	while (bits & 7) put(0, 1);
 	put(crc, 32); put(len, 32);
 	const size_t n = (size_t)(bits >> 3);
+	if (n > (size_t)len + GZ_STORED_EXTRA) {              // coding would expand the blob: one stored block
+		if ((size_t)len + GZ_STORED_EXTRA > cap) return 0;
+		memcpy(dst, out.data(), 10);                      // the gzip header of the coded form
+		const uint8_t blk[5] = {0x01, (uint8_t)len, (uint8_t)(len >> 8), (uint8_t)~len, (uint8_t)(~len >> 8)};
+		memcpy(dst + 10, blk, 5);
+		memcpy(dst + 15, src, len);
+		for (int k = 0; k < 4; k++) { dst[15 + len + k] = (uint8_t)(crc >> (8 * k)); dst[19 + len + k] = (uint8_t)(len >> (8 * k)); }
+		return (size_t)len + GZ_STORED_EXTRA;
+	}
 	if (n > cap) return 0;
 	memcpy(dst, out.data(), n);
 	return n;
@@ -279,7 +294,7 @@ __global__ void __launch_bounds__(GZ_WARPS * 32) deflate_blobs_kernel(const uint
                                                                       const unsigned long long* __restrict__ rawLens, int nTiles, uint32_t rawPitch,
                                                                       uint8_t* __restrict__ gz1, uint8_t* __restrict__ gz2,
                                                                       unsigned long long* __restrict__ gzLens, uint32_t gzPitch,
-                                                                      const GzTables* __restrict__ tab, unsigned int* __restrict__ errorFlags) {
+                                                                      const GzTables* __restrict__ tab) {
 	__shared__ uint32_t s_lut[257];
 	__shared__ uint32_t s_T[4][256];
 	__shared__ uint32_t s_S[4][256];
@@ -303,10 +318,11 @@ __global__ void __launch_bounds__(GZ_WARPS * 32) deflate_blobs_kernel(const uint
 		const unsigned long long lens = rawLens[ticket];
 		const uint32_t len = file ? (uint32_t)(lens & 0x7fffffffull) : (uint32_t)(lens >> 31);
 		uint32_t outBytes = 0;
-		if (len >= 8) {
+		if (len > 0) {
 			const uint2* src64 = (const uint2*)((file ? raw2 : raw1) + (size_t)ticket * rawPitch);
 			const uint8_t* src8 = (const uint8_t*)src64;
 			uint32_t* dst32 = (uint32_t*)((file ? gz2 : gz1) + (size_t)ticket * gzPitch);
+			const uint32_t pitchWords = gzPitch >> 2;     // coded words past it are counted, not stored (the member goes stored)
 			// ---- member header + block header
 			uint32_t outWords = prefixBits >> 5, carryBits = prefixBits & 31u;
 			for (uint32_t i = lane; i < outWords; i += 32) dst32[i] = s_prefix[i];
@@ -315,7 +331,6 @@ __global__ void __launch_bounds__(GZ_WARPS * 32) deflate_blobs_kernel(const uint
 			// ---- the word pairs of the blob
 			const uint32_t P2 = len >> 3;
 			uint32_t A = 0, lastIdx = 0xFFFFFFFFu;
-			bool overflow = false;
 			for (uint32_t base = 0; base < P2; base += 32) {
 				const uint32_t idx = base + lane;
 				const bool valid = idx < P2;
@@ -351,52 +366,58 @@ __global__ void __launch_bounds__(GZ_WARPS * 32) deflate_blobs_kernel(const uint
 				put_bits(rbA, off + n0, acc1, n1);
 				__syncwarp();
 				const uint32_t totalBits = carryBits + total, nw = totalBits >> 5;
-				if ((outWords + nw + GZ_RB) * 4u > gzPitch) { overflow = true; break; }
 				// store the completed words, zero them, and move the partial last word to the other (all zero) buffer
 				for (uint32_t i = lane; i <= nw; i += 32) {
 					const uint32_t v = rbA[i];
 					rbA[i] = 0u;
-					if (i < nw) dst32[outWords + i] = v; else rbB[0] = v;
+					if (i < nw) { if (outWords + i < pitchWords) dst32[outWords + i] = v; } else rbB[0] = v;
 				}
 				__syncwarp();
 				{ uint32_t* tswap = rbA; rbA = rbB; rbB = tswap; }
 				carryBits = totalBits & 31u;
 				outWords += nw;
 			}
-			if (overflow) {
-				if (lane == 0) atomicOr(errorFlags, 8u);
-				for (int i = lane; i < GZ_RB; i += 32) { rbA[i] = 0u; rbB[i] = 0u; }
-				__syncwarp();
-			} else {
-				// ---- CRC of the whole blob
-				uint32_t part = lastIdx != 0xFFFFFFFFu ? d_multmodp(s_xp[(P2 - 1u - lastIdx) * 8u], A) : 0u;   // advance to the last pair
+			// ---- CRC of the whole blob
+			uint32_t part = lastIdx != 0xFFFFFFFFu ? d_multmodp(s_xp[(P2 - 1u - lastIdx) * 8u], A) : 0u;   // advance to the last pair
 #pragma unroll
-				for (int d = 16; d > 0; d >>= 1) part ^= __shfl_xor_sync(0xffffffffu, part, d);
-				uint32_t crc = part;
-				for (uint32_t i = P2 * 8u; i < len; i++) crc = s_T[0][(crc ^ src8[i]) & 0xff] ^ (crc >> 8);
-				crc = ~crc;
-				// ---- tail bytes (< 8), end of block, byte alignment, trailer (CRC32, ISIZE)
-				unsigned long long accA = 0, accB = 0;
-				uint32_t nA = 0, nB = 0;
-				for (uint32_t i = P2 * 8u; i < len; i++) {
-					const uint32_t e = s_lut[src8[i]];
-					if (i < P2 * 8u + 4u) { accA |= (unsigned long long)(e & 0xffffu) << nA; nA += e >> 16; }
-					else { accB |= (unsigned long long)(e & 0xffffu) << nB; nB += e >> 16; }
+			for (int d = 16; d > 0; d >>= 1) part ^= __shfl_xor_sync(0xffffffffu, part, d);
+			uint32_t crc = P2 ? part : 0xFFFFFFFFu;       // fewer than 8 bytes: plain byte-wise CRC from the initial value
+			for (uint32_t i = P2 * 8u; i < len; i++) crc = s_T[0][(crc ^ src8[i]) & 0xff] ^ (crc >> 8);
+			crc = ~crc;
+			// ---- tail bytes (< 8), end of block, byte alignment, trailer (CRC32, ISIZE)
+			unsigned long long accA = 0, accB = 0;
+			uint32_t nA = 0, nB = 0;
+			for (uint32_t i = P2 * 8u; i < len; i++) {
+				const uint32_t e = s_lut[src8[i]];
+				if (i < P2 * 8u + 4u) { accA |= (unsigned long long)(e & 0xffffu) << nA; nA += e >> 16; }
+				else { accB |= (unsigned long long)(e & 0xffffu) << nB; nB += e >> 16; }
+			}
+			{ const uint32_t e = s_lut[256]; accB |= (unsigned long long)(e & 0xffffu) << nB; nB += e >> 16; }   // <= 3 literals + end of block
+			const uint32_t dataEnd = carryBits + nA + nB;
+			const uint32_t trailerAt = (dataEnd + 7u) & ~7u;
+			if (lane == 0) { put_bits(rbA, carryBits, accA, nA); put_bits(rbA, carryBits + nA, accB, nB); }
+			if (lane == 1) put_bits(rbA, trailerAt, (unsigned long long)crc | ((unsigned long long)len << 32), 64);
+			__syncwarp();
+			const uint32_t totalBits = trailerAt + 64u;
+			const uint32_t nw = (totalBits + 31u) >> 5;
+			for (uint32_t i = lane; i < nw; i += 32) { if (outWords + i < pitchWords) dst32[outWords + i] = rbA[i]; rbA[i] = 0u; }
+			outBytes = outWords * 4u + (totalBits >> 3);
+			__syncwarp();
+			if (outBytes > len + (uint32_t)GZ_STORED_EXTRA) {
+				// coding would expand the blob (bytes the table was not fitted to): one stored block, as gz_member_host
+				uint8_t* dst8 = (uint8_t*)dst32;
+				for (uint32_t i = lane; i < len + (uint32_t)GZ_STORED_EXTRA; i += 32) {
+					uint32_t b;
+					if (i < 10u) b = s_prefix[i >> 2] >> (8u * (i & 3u));                        // the gzip header of the coded form
+					else if (i == 10u) b = 1u;                                                  // BFINAL, BTYPE = stored
+					else if (i < 15u) b = (i < 13u ? len : ~len) >> (8u * ((i - 11u) & 1u));   // LEN, NLEN
+					else if (i < 15u + len) b = src8[i - 15u];
+					else b = (i < 19u + len ? crc : len) >> (8u * ((i - 15u - len) & 3u));      // CRC-32, ISIZE
+					dst8[i] = (uint8_t)b;
 				}
-				{ const uint32_t e = s_lut[256]; accB |= (unsigned long long)(e & 0xffffu) << nB; nB += e >> 16; }   // <= 3 literals + end of block
-				const uint32_t dataEnd = carryBits + nA + nB;
-				const uint32_t trailerAt = (dataEnd + 7u) & ~7u;
-				if (lane == 0) { put_bits(rbA, carryBits, accA, nA); put_bits(rbA, carryBits + nA, accB, nB); }
-				if (lane == 1) put_bits(rbA, trailerAt, (unsigned long long)crc | ((unsigned long long)len << 32), 64);
-				__syncwarp();
-				const uint32_t totalBits = trailerAt + 64u;
-				const uint32_t nw = (totalBits + 31u) >> 5;
-				for (uint32_t i = lane; i < nw; i += 32) { dst32[outWords + i] = rbA[i]; rbA[i] = 0u; }
-				outBytes = outWords * 4u + (totalBits >> 3);
+				outBytes = len + (uint32_t)GZ_STORED_EXTRA;
 				__syncwarp();
 			}
-		} else if (len > 0) {
-			if (lane == 0) atomicOr(errorFlags, 8u);
 		}
 		if (lane == 0) {
 			// the two files of a ticket are different jobs: each adds its own half of the packed length (zeroed by the host)
@@ -407,12 +428,12 @@ __global__ void __launch_bounds__(GZ_WARPS * 32) deflate_blobs_kernel(const uint
 
 cudaError_t launch_deflate_blobs(const uint8_t* raw1, const uint8_t* raw2, const unsigned long long* rawLens, int nTiles, uint32_t rawPitch,
                                  uint8_t* gz1, uint8_t* gz2, unsigned long long* gzLens, uint32_t gzPitch, const GzTables* tab,
-                                 unsigned int* errorFlags, int smCount, cudaStream_t stream) {
+                                 int smCount, cudaStream_t stream) {
 	if (nTiles <= 0) return cudaSuccess;
 	int grid = smCount * 6;
 	const int need = (2 * nTiles + GZ_WARPS - 1) / GZ_WARPS;
 	if (grid > need) grid = need;
-	deflate_blobs_kernel<<<grid, GZ_WARPS * 32, 0, stream>>>(raw1, raw2, rawLens, nTiles, rawPitch, gz1, gz2, gzLens, gzPitch, tab, errorFlags);
+	deflate_blobs_kernel<<<grid, GZ_WARPS * 32, 0, stream>>>(raw1, raw2, rawLens, nTiles, rawPitch, gz1, gz2, gzLens, gzPitch, tab);
 	return cudaGetLastError();
 }
 

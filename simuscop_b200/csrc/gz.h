@@ -7,6 +7,9 @@
 namespace ssc {
 
 static constexpr int GZ_PREFIX_WORDS = 96;   // gzip member header + dynamic block header, as a bit stream
+// a stored member: 10-byte gzip header, one stored block (0x01, LEN, NLEN: 5 bytes), the raw bytes, CRC-32 and ISIZE.  A member
+// whose coded form would be longer than the raw bytes plus this is written stored, so no member exceeds it.
+static constexpr int GZ_STORED_EXTRA = 23;
 
 // Built on the host from a byte histogram of the plan's own output, read by the encoder kernel.
 struct GzTables {
@@ -24,6 +27,6 @@ size_t gz_member_host(const GzTables* t, const uint8_t* src, uint32_t len, uint8
 
 cudaError_t launch_deflate_blobs(const uint8_t* raw1, const uint8_t* raw2, const unsigned long long* rawLens, int nTiles, uint32_t rawPitch,
                                  uint8_t* gz1, uint8_t* gz2, unsigned long long* gzLens, uint32_t gzPitch, const GzTables* tab,
-                                 unsigned int* errorFlags, int smCount, cudaStream_t stream);
+                                 int smCount, cudaStream_t stream);
 
 }  // namespace ssc

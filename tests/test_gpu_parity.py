@@ -34,7 +34,7 @@ def test_fastq_bit_exact_vs_instrumented_reference(name, gen, workdir):
 
 # pass 2 of the fast kernel: a stand-alone move after every batch (what GPUs with fewer than 64 SMs run), or the bulk-copy mover;
 # the fast kernel with only the ref == call quality rows in shared memory
-OPTION_MODES = {"standalone_move": ("concurrent_move", 0), "concurrent_move": ("concurrent_move", 8), "fast_qmode2": ("fast_qmode", 2)}
+OPTION_MODES = {"standalone_move": ("concurrent_move", 0), "concurrent_move": ("concurrent_move", 9), "fast_qmode2": ("fast_qmode", 2)}
 
 
 @pytest.mark.parametrize("mode", ["force_generic", "fp64_search", "no_splice", "fast_qmode2", "standalone_move", "concurrent_move"])
@@ -42,7 +42,7 @@ OPTION_MODES = {"standalone_move": ("concurrent_move", 0), "concurrent_move": ("
 def test_fallback_kernels_bit_exact(name, mode, built, workdir):
     """The generic integer kernel, the FP64 linear-search ground-truth kernel, the fast kernel without the spliced indel path,
     with only the ref == call quality rows in shared memory (the rare substituted bases read the full table in global
-    memory), with pass 2 as a stand-alone move after every batch, and with pass 2 on the bulk-copy mover (8 SMs, second
+    memory), with pass 2 as a stand-alone move after every batch, and with pass 2 on the bulk-copy mover (9 SMs, the default, second
     stream, under the next batch's generation) all give the same bytes, and the statistics name the kernel that ran."""
     from simuscop_b200 import cuda_binding
     scn = helpers.build_scenario(name, workdir)

@@ -285,6 +285,49 @@ def test_gzip_member_host_mirror_inflates(built):
     assert gzip.decompress(buf.raw[:m]) == noise
 
 
+def test_gzip_member_host_stores_what_coding_would_expand(built):
+    """A member whose Huffman code (fitted to the sample) would be longer than its bytes + 23 is one stored block: gzip header,
+    0x01, LEN, NLEN, the bytes, CRC-32, ISIZE -- what zlib does, and what the device encoder does too.  Inputs: noise, bytes
+    absent from the sample (codes of 14-15 bits; up to the largest blob, 32 x 612 bytes), and 1..15 bytes (no or one full
+    word pair, less than the block header).  Members that coding does not expand stay coded (BTYPE 2)."""
+    import ctypes as C
+    import random
+    import struct
+    import zlib
+    L = cuda_binding.lib()
+    rnd = random.Random(11)
+    sample = b"".join(b"@normal#chr1#%d#%d/1\n%s\n+\n%s\n" % (rnd.randint(0, 99999), i + 1,
+                                                              bytes(rnd.choice(b"ACGT") for _ in range(151)),
+                                                              bytes(rnd.choice(b"FFF:,") for _ in range(151)))
+                      for i in range(64))
+    absent = bytes(sorted(set(range(256)) - set(sample)))
+    assert len(absent) > 200
+
+    def member(d):
+        buf = C.create_string_buffer(len(d) + 4096)
+        m = L.ssc_gzip_member_host(d, len(d), sample, len(sample), buf, len(buf))
+        assert m > 0
+        return buf.raw[:m]
+
+    def stored(d):
+        n = len(d)
+        return (b"\x1f\x8b\x08\x00\x00\x00\x00\x00\x00\xff" + struct.pack("<BHH", 1, n, n ^ 0xFFFF) + d +
+                struct.pack("<II", zlib.crc32(d), n))
+    expanding = [bytes(rnd.randrange(256) for _ in range(4099)), absent * 3, (absent * 100)[:32 * 612],
+                 b"@" + absent[:63] + b"\n" + bytes(rnd.choice(b"!\"#$%&'()*+,-./0123456") for _ in range(8000)),
+                 absent[:1], absent[:7], bytes(absent[:5]) * 3, sample[:1], sample[100:107]]   # short: a ~60-byte table
+    for d in expanding:
+        z = member(d)
+        assert z == stored(d) and len(z) == len(d) + 23, len(d)
+        assert zlib.decompressobj(wbits=31).decompress(z) == d
+    for d in [sample[:4096], sample[:1001], sample[5:613]]:
+        z = member(d)
+        assert len(z) <= len(d) + 23 and (z[10] >> 1) & 3 == 2 and zlib.decompressobj(wbits=31).decompress(z) == d
+    assert len(member(sample[:4096])) < 4096 // 2
+    buf = C.create_string_buffer(len(expanding[0]) + 22)                      # one byte short of the stored member
+    assert L.ssc_gzip_member_host(expanding[0], len(expanding[0]), sample, len(sample), buf, len(buf)) == 0
+
+
 def test_file_writer_sink_writes_ordered_slabs(built, tmp_path):
     """The output side of the drop-in CLI (ssh_writer_*, the role of SeqWriter::write): slabs handed to the sink in order end
     up back to back in the files, whatever the number of pwrite workers, for paired and single-end layouts."""
