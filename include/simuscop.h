@@ -228,6 +228,38 @@ int ssc_generate(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc_sink_fn si
 int ssc_generate_device(ssc_handle* h, int64_t pair_lo, int64_t pair_hi,
                         uint64_t* bytes1, uint64_t* bytes2, uint64_t* bases, double* device_ms);
 
+/*
+ * Array output: the reads of a pair range written straight into caller-owned device arrays (e.g. torch tensors) for a
+ * consumer on the same GPU -- no FASTQ text, no host copy.  The bytes are the FASTQ record's own; n = capacity in pairs,
+ * M = 1 (SE) or 2 (PE).  Pair i of the range (FASTQ order) is row i.
+ */
+typedef struct ssc_read_arrays {      /* device pointers, caller-owned */
+	uint8_t* reads;    /* [n][M][2][pitch], 16-byte aligned: row 0 = the base characters of the FASTQ record, row 1 = its
+	                      quality characters (phred + 33, as written); every byte past the read's length is 0 */
+	int16_t* length;   /* [n][M]: read length (RL +- indels, as in the FASTQ record) */
+	int64_t* pair_id;  /* [n]: planned pair ID (the Philox address; abandoned pairs are absent, as in the FASTQ) */
+	int32_t* segment;  /* [n]: index into the ssc_segment array of ssc_set_plan: the name prefix "@<popu>#<chr>#" */
+	int32_t* pos;      /* [n]: position field of the read name (pos % segsize) */
+	int32_t* frag;     /* [n]: fragment-counter field of the read name */
+	int64_t capacity;  /* pairs */
+	int32_t pitch;     /* must equal the value ssc_read_shape reports */
+} ssc_read_arrays;
+
+/* Pairs emitted by planned pair IDs [pair_lo, pair_hi), mates per pair, and the slot pitch: RL + 96 (the longest read the
+ * library emits) rounded up to a multiple of 16. */
+int ssc_read_shape(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, int64_t* n_pairs, int32_t* n_mates, int32_t* pitch);
+/* Generates planned pair IDs [pair_lo, pair_hi) into `out` on the fast kernel (kmer 3, read length 33..160; force_generic,
+ * fp64_search and other profiles are refused with SSC_ERR_INVALID; the gzip option does not apply).  `stream` is a
+ * cudaStream_t (0 = the legacy default stream): work queued on it before the call is ordered before the first write.  Returns
+ * once the arrays are complete; *n_pairs (may be NULL) = the pairs written.  Null or misaligned pointers, a capacity below the
+ * range, or a wrong pitch are refused before anything is written.  A read longer than RL + 96 fails with SSC_ERR_OVERFLOW.
+ * ssc_stats counts pairs, reads, bases and launches as for FASTQ output; fastq_bytes is unchanged.  Device memory of the
+ * handle: per-batch bookkeeping only (no FASTQ slab, blob scratch or pinned host buffers). */
+int ssc_generate_reads(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, const ssc_read_arrays* out, void* stream,
+                       int64_t* n_pairs);
+/* The read-name prefix "@<popu>#<chr>#" of a segment, NUL-terminated; cap >= its length + 1. */
+int ssc_segment_name(ssc_handle* h, int32_t segment, char* out, int32_t cap);
+
 /* Host-only diagnostic (no GPU needed): the symbol the integer-threshold table built from
  * `cdf` selects for the 32-bit draw u.  Must equal the reference's
  * randIndx(cdf, n) with r = 2.2204e-16 + (1 - 2.2204e-16) * (u / 2^32) for every u

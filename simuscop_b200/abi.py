@@ -42,7 +42,15 @@ class Stats(C.Structure):
     ]
 
 
-SINK_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_int64, C.c_int64)
+class ReadArrays(C.Structure):
+    _fields_ = [
+        ("reads", C.c_void_p), ("length", C.c_void_p), ("pair_id", C.c_void_p),
+        ("segment", C.c_void_p), ("pos", C.c_void_p), ("frag", C.c_void_p),
+        ("capacity", C.c_int64), ("pitch", C.c_int32),
+    ]
+
+
+SINK_FN =C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_int64, C.c_int64)
 
 BIN_DTYPE = [("hap_base", "<i8"), ("contig_end", "<i8"), ("spos", "<i4"), ("epos", "<i4"),
              ("segsize", "<u4"), ("read_count", "<i4"), ("segment", "<i4"), ("reserved", "<i4")]

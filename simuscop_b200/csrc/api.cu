@@ -141,6 +141,8 @@ struct ssc_handle {
 	DevBuf<int64_t> d_emitBase;
 	DevBuf<uint16_t> d_risky;
 	DevBuf<char> d_names;
+	std::vector<char> names;                         // host copy of the name blob and of the segments' name ranges (ssc_segment_name)
+	std::vector<int32_t> segNameOff, segNameLen;
 	int64_t nDevBins = 0, plannedPairs = 0, emittedPairs = 0;
 	int maxRecBytes = 0;
 
@@ -162,6 +164,12 @@ struct ssc_handle {
 	DevBuf<int32_t> d_cenLens, d_cenGc, d_cenNn;
 	ssc::BatchResult* d_result[2] = {nullptr, nullptr};
 	ssc::BatchResult* h_result[2] = {nullptr, nullptr};
+	// ssc_generate_reads: the bookkeeping of its batches only (no slab, blob scratch or pinned host memory: the caller owns the output);
+	// the batches run back to back on the compute stream and add to one BatchResult
+	DevBuf<int32_t> d_rdTileStart;
+	DevBuf<unsigned int> d_rdTicket;
+	DevBuf<ssc::BatchResult> d_rdResult;
+	cudaEvent_t evCaller = nullptr;                  // the caller's stream at the call: the compute stream waits for it
 
 	// kernel timing of ssc_generate_device: events kev[2 i] and kev[2 i + 1] bracket the i-th timed piece of work of the call,
 	// whose time goes to *kevSum[i] when the call ends (see time_begin)
@@ -320,6 +328,35 @@ int result_to_host(ssc_handle* h, int buf, cudaStream_t after) {
 	return SSC_OK;
 }
 
+// The launch parameters of batch [emitLo, emitHi) every generation kernel reads (tables, plan, Philox keys), and the batch's
+// statistics (one generation launch, its distinct bin records).  qsmem8: the fast kernel with every quality row in shared memory.
+ssc::GenParams batch_params(ssc_handle* h, int64_t emitLo, int64_t emitHi, bool qsmem8) {
+	h->stats.gen_launches += 1;
+	{
+		// distinct bins of the batch (statistics: the algorithmic bin-record bytes of the roofline)
+		const std::vector<int64_t>& eb = h->devEmitBase;
+		const size_t bLo = std::upper_bound(eb.begin(), eb.end(), emitLo) - eb.begin() - 1;
+		const size_t bHi = std::lower_bound(eb.begin(), eb.end(), emitHi) - eb.begin();
+		h->stats.bin_bytes += (uint64_t)(bHi > bLo ? bHi - bLo : 0) * sizeof(ssc::DevBin);
+	}
+	ssc::GenParams P;
+	memset(&P, 0, sizeof(P));
+	P.t = h->dt;
+	P.hap2 = h->d_hap2.p; P.hapN = h->d_hapN.p;
+	P.bins = h->d_bins.p; P.emitBase = h->d_emitBase.p; P.nBins = h->nDevBins;
+	P.riskyAttempt = h->d_risky.p; P.names = h->d_names.p;
+	P.seed = h->seed; P.emitLo = emitLo; P.emitHi = emitHi; P.one = 1; P.noSplice = h->noSplice ? 1 : 0;
+	P.qstride = qsmem8 ? (uint32_t)h->dt.qualBins * 68u : 68u;   // F_QROW of gen_fast.cu (unused by the 16-bit-key mode)
+	P.insLim = h->dt.insEnable ? h->dt.insT + 1u : 0u;
+	P.delLim = h->dt.delEnable ? h->dt.delT + 1u : 0u;
+	P.alwaysSlow = (h->dt.insEnable && h->dt.insT == 0xFFFFFFFFu) || (h->dt.delEnable && h->dt.delT == 0xFFFFFFFFu);
+	for (int r = 0; r < 10; r++) {
+		P.rk[2 * r] = (uint32_t)h->seed + (uint32_t)r * 0x9E3779B9u;
+		P.rk[2 * r + 1] = (uint32_t)(h->seed >> 32) + (uint32_t)r * 0xBB67AE85u;
+	}
+	return P;
+}
+
 // Launches batch [emitLo, emitHi) into buffer set `buf`; evResult[buf] marks its BatchResult in h_result[buf].  Fast kernel,
 // plain output: pass 1 on the compute stream, then the scan of the blob lengths on the mover stream; the blobs are moved to
 // the dense slab d_out[buf] by the mover under the next launch_batch, or by flush_pending (right after the scan when the
@@ -336,29 +373,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 	CK(cudaMemsetAsync(h->d_result[buf], 0, sizeof(ssc::BatchResult), s));
 	CK(ssc::launch_locate(h->d_emitBase.p, h->nDevBins, emitLo, tp, nTiles, h->d_tileStart[buf].p, s));
 	h->stats.launches += 1;
-	h->stats.gen_launches += 1;
-	{
-		// distinct bins of the batch (statistics: the algorithmic bin-record bytes of the roofline)
-		const std::vector<int64_t>& eb = h->devEmitBase;
-		const size_t bLo = std::upper_bound(eb.begin(), eb.end(), emitLo) - eb.begin() - 1;
-		const size_t bHi = std::lower_bound(eb.begin(), eb.end(), emitHi) - eb.begin();
-		h->stats.bin_bytes += (uint64_t)(bHi > bLo ? bHi - bLo : 0) * sizeof(ssc::DevBin);
-	}
-	ssc::GenParams P;
-	memset(&P, 0, sizeof(P));
-	P.t = h->dt;
-	P.hap2 = h->d_hap2.p; P.hapN = h->d_hapN.p;
-	P.bins = h->d_bins.p; P.emitBase = h->d_emitBase.p; P.nBins = h->nDevBins;
-	P.riskyAttempt = h->d_risky.p; P.names = h->d_names.p;
-	P.seed = h->seed; P.emitLo = emitLo; P.emitHi = emitHi; P.one = 1; P.noSplice = h->noSplice ? 1 : 0;
-	P.qstride = (fast && qsmem == 8) ? (uint32_t)h->dt.qualBins * 68u : 68u;   // F_QROW of gen_fast.cu (unused by the 16-bit-key mode)
-	P.insLim = h->dt.insEnable ? h->dt.insT + 1u : 0u;
-	P.delLim = h->dt.delEnable ? h->dt.delT + 1u : 0u;
-	P.alwaysSlow = (h->dt.insEnable && h->dt.insT == 0xFFFFFFFFu) || (h->dt.delEnable && h->dt.delT == 0xFFFFFFFFu);
-	for (int r = 0; r < 10; r++) {
-		P.rk[2 * r] = (uint32_t)h->seed + (uint32_t)r * 0x9E3779B9u;
-		P.rk[2 * r + 1] = (uint32_t)(h->seed >> 32) + (uint32_t)r * 0xBB67AE85u;
-	}
+	ssc::GenParams P = batch_params(h, emitLo, emitHi, fast && qsmem == 8);
 	P.tileStartBin = h->d_tileStart[buf].p; P.nTiles = nTiles;
 	P.tileState = h->d_tileState[buf].p; P.ticket = h->d_ticket[buf].p; P.blobPrefix = h->d_blobPrefix[buf].p;
 	P.out1 = h->d_out[buf][0]; P.out2 = h->d_out[buf][1];
@@ -493,6 +508,7 @@ static int init_handle(ssc_handle* h, int device) {
 	CK(cudaStreamCreateWithFlags(&h->mover, cudaStreamNonBlocking));
 	CK(cudaStreamCreateWithFlags(&h->results, cudaStreamNonBlocking));
 	CK(cudaEventCreateWithFlags(&h->evPre, cudaEventDisableTiming));
+	CK(cudaEventCreateWithFlags(&h->evCaller, cudaEventDisableTiming));
 	CK(cudaEventCreate(&h->evStart));
 	CK(cudaEventCreate(&h->evStop));
 	for (int i = 0; i < 2; i++) {
@@ -578,6 +594,8 @@ int ssc_destroy(ssc_handle* h) {
 	if (h->mover) cudaStreamDestroy(h->mover);
 	if (h->results) cudaStreamDestroy(h->results);
 	if (h->evPre) cudaEventDestroy(h->evPre);
+	if (h->evCaller) cudaEventDestroy(h->evCaller);
+	h->d_rdTileStart.release(); h->d_rdTicket.release(); h->d_rdResult.release();
 	delete h;
 	return SSC_OK;
 }
@@ -1108,7 +1126,7 @@ int ssc_set_plan(ssc_handle* h, uint64_t seed, const ssc_bin* bins, int64_t n_bi
 							d.spos = bins[i].spos; d.epos = bins[i].epos; d.segsize = bins[i].segsize;
 							d.frag_base = (int32_t)fragBase;
 							d.name_off = segs[sIdx].name_offset; d.name_len = segs[sIdx].name_len;
-							d.risky_base = riskyBase[i]; d.pad = 0;
+							d.risky_base = riskyBase[i]; d.segment = (int32_t)sIdx;
 							out[o - o0] = d;
 							devEmitBase[(size_t)o] = eb[i];
 							o++;
@@ -1132,6 +1150,9 @@ int ssc_set_plan(ssc_handle* h, uint64_t seed, const ssc_bin* bins, int64_t n_bi
 	nm.push_back(0);
 	CK(h->d_names.upload(nm, s));
 	CK(cudaStreamSynchronize(s));
+	h->names.swap(nm);
+	h->segNameOff.resize((size_t)n_segs); h->segNameLen.resize((size_t)n_segs);
+	for (int64_t k = 0; k < n_segs; k++) { h->segNameOff[(size_t)k] = segs[k].name_offset; h->segNameLen[(size_t)k] = segs[k].name_len; }
 	h->stats.h2d_bytes += nDev * sizeof(ssc::DevBin) + devEmitBase.size() * 8;
 	// worst-case record bytes per pair per file: header + 2*(RL + 96) + 4
 	h->maxRecBytes = maxName + 10 + 1 + 10 + 3 + 2 * (RL + 96) + 4;
@@ -1278,6 +1299,103 @@ int ssc_generate_device(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, uint64_
 	if (bytes2) *bytes2 = b2;
 	if (bases) *bases = nb;
 	if (device_ms) *device_ms = ms;
+	return SSC_OK;
+}
+
+// bytes between the base rows of two consecutive reads' slots: RL + 96 (the longest read emitted) rounded up to 16
+static int32_t read_pitch(const ssc_handle* h) { return (h->dt.RL + 96 + 15) / 16 * 16; }
+
+int ssc_read_shape(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, int64_t* n_pairs, int32_t* n_mates, int32_t* pitch) {
+	if (!h || !n_pairs || !n_mates || !pitch) return fail(SSC_ERR_INVALID, "null argument");
+	if (!h->havePlan) return fail(SSC_ERR_STATE, "ssc_set_plan must precede ssc_read_shape");
+	if (pair_lo < 0 || pair_hi < pair_lo) return fail(SSC_ERR_INVALID, "bad pair range");
+	*n_pairs = emit_index_of_plan(h, pair_hi) - emit_index_of_plan(h, pair_lo);
+	*n_mates = h->dt.paired ? 2 : 1;
+	*pitch = read_pitch(h);
+	return SSC_OK;
+}
+
+int ssc_segment_name(ssc_handle* h, int32_t segment, char* out, int32_t cap) {
+	if (!h || !out) return fail(SSC_ERR_INVALID, "null argument");
+	if (!h->havePlan) return fail(SSC_ERR_STATE, "ssc_set_plan must precede ssc_segment_name");
+	if (segment < 0 || (size_t)segment >= h->segNameOff.size())
+		return fail(SSC_ERR_INVALID, "segment %d out of range (%zu segments)", segment, h->segNameOff.size());
+	const int32_t len = h->segNameLen[(size_t)segment];
+	if (cap < len + 1) return fail(SSC_ERR_INVALID, "segment name of %d bytes needs a buffer of %d bytes, got %d", len, len + 1, cap);
+	memcpy(out, h->names.data() + h->segNameOff[(size_t)segment], (size_t)len);
+	out[len] = 0;
+	return SSC_OK;
+}
+
+// The batches of ssc_generate_reads, emitted pairs [eLo, eHi), back to back on the compute stream.  Every error return goes
+// through bail() in ssc_generate_reads.
+static int generate_read_batches(ssc_handle* h, int64_t eLo, int64_t eHi, const ssc_read_arrays* out, cudaStream_t caller, int qmode,
+                                 size_t smem) {
+	const int M = h->dt.paired ? 2 : 1;
+	const uint64_t perPair = (uint64_t)M * 2u * (uint64_t)out->pitch;
+	// the kernel addresses a batch's slots with 32-bit offsets
+	const int64_t pairs = std::min<int64_t>({h->batchPairs, eHi - eLo, (int64_t)(((1ull << 32) - 1) / perPair)});
+	const int maxTiles = (int)((pairs + FG_CHUNK - 1) / FG_CHUNK);
+	if (h->d_rdTileStart.n < (size_t)maxTiles) CK(h->d_rdTileStart.alloc((size_t)maxTiles));
+	if (!h->d_rdTicket.p) CK(h->d_rdTicket.alloc(1));
+	if (!h->d_rdResult.p) CK(h->d_rdResult.alloc(1));
+	cudaStream_t s = h->compute;
+	CK(cudaEventRecord(h->evCaller, caller));         // work the caller queued before the call (e.g. on the output arrays) goes first
+	CK(cudaStreamWaitEvent(s, h->evCaller, 0));
+	CK(cudaMemsetAsync(h->d_rdResult.p, 0, sizeof(ssc::BatchResult), s));
+	h->stats.gen_kernel = 1; h->stats.gen_nch = ssc::fast_nch(h->dt.RL); h->stats.gen_qmode = qmode;
+	h->stats.gen_smem_bytes = (int32_t)smem;
+	for (int64_t lo = eLo; lo < eHi; lo += pairs) {
+		const int64_t hi = std::min(eHi, lo + pairs), row = lo - eLo;
+		const int nTiles = (int)((hi - lo + FG_CHUNK - 1) / FG_CHUNK);
+		CK(cudaMemsetAsync(h->d_rdTicket.p, 0, sizeof(unsigned int), s));
+		CK(ssc::launch_locate(h->d_emitBase.p, h->nDevBins, lo, FG_CHUNK, nTiles, h->d_rdTileStart.p, s));
+		ssc::GenParams P = batch_params(h, lo, hi, qmode == 8);
+		P.tileStartBin = h->d_rdTileStart.p; P.nTiles = nTiles; P.ticket = h->d_rdTicket.p; P.result = h->d_rdResult.p;
+		P.out1 = out->reads + (uint64_t)row * perPair;
+		P.rdLength = out->length + row * M; P.rdPairId = out->pair_id + row;
+		P.rdSegment = out->segment + row; P.rdPos = out->pos + row; P.rdFrag = out->frag + row;
+		P.pitch = (uint32_t)out->pitch;
+		// nothing to move: every SM generates
+		int grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount);
+		if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
+		CK(ssc::launch_generate_reads(P, qmode, smem, grid, s));
+		h->stats.launches += 2;
+	}
+	ssc::BatchResult r;
+	CK(cudaMemcpyAsync(&r, h->d_rdResult.p, sizeof(r), cudaMemcpyDeviceToHost, s));
+	CK(cudaStreamSynchronize(s));
+	return check_result(h, r);
+}
+
+int ssc_generate_reads(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, const ssc_read_arrays* out, void* stream, int64_t* n_pairs) {
+	if (!h || !out) return fail(SSC_ERR_INVALID, "null argument");
+	if (!h->havePlan) return fail(SSC_ERR_STATE, "ssc_set_plan must precede ssc_generate_reads");
+	if (pair_lo < 0 || pair_hi < pair_lo) return fail(SSC_ERR_INVALID, "bad pair range");
+	if (!out->reads || !out->length || !out->pair_id || !out->segment || !out->pos || !out->frag)
+		return fail(SSC_ERR_INVALID, "ssc_generate_reads: null array pointer in ssc_read_arrays");
+	if (((uintptr_t)out->reads & 15) || ((uintptr_t)out->length & 1) || ((uintptr_t)out->pair_id & 7) || ((uintptr_t)out->segment & 3) ||
+	    ((uintptr_t)out->pos & 3) || ((uintptr_t)out->frag & 3))
+		return fail(SSC_ERR_INVALID, "ssc_generate_reads: reads must be 16-byte aligned, the other arrays aligned to their element size");
+	if (out->pitch != read_pitch(h))
+		return fail(SSC_ERR_INVALID, "ssc_generate_reads: pitch %d, the plan's read length %d needs %d (ssc_read_shape)", out->pitch, h->dt.RL,
+		            read_pitch(h));
+	const int64_t eLo = emit_index_of_plan(h, pair_lo), eHi = emit_index_of_plan(h, pair_hi);
+	if (out->capacity < eHi - eLo)
+		return fail(SSC_ERR_INVALID, "ssc_generate_reads: capacity %lld pairs, the range emits %lld", (long long)out->capacity,
+		            (long long)(eHi - eLo));
+	if (h->fp64) return fail(SSC_ERR_INVALID, "array output needs the fast kernel; fp64_search selects the FP64 ground-truth kernel");
+	if (h->forceGeneric) return fail(SSC_ERR_INVALID, "array output needs the fast kernel; force_generic selects the generic kernel");
+	int qmode = 0; size_t smem = 0;
+	if (!use_fast(h, &qmode, &smem))
+		return fail(SSC_ERR_INVALID, "array output needs the fast kernel (kmer 3, read length 33..160, tables within shared memory); "
+		            "this profile has kmer %d, read length %d", h->dt.K, h->dt.RL);
+	CK(cudaSetDevice(h->device));
+	if (eHi > eLo) {
+		const int rc = generate_read_batches(h, eLo, eHi, out, (cudaStream_t)stream, qmode, smem);
+		if (rc) return bail(h, rc);
+	}
+	if (n_pairs) *n_pairs = eHi - eLo;
 	return SSC_OK;
 }
 

@@ -15,7 +15,7 @@ struct DevBin {
 	int32_t frag_base;    // emitted pairs in earlier bins of the same segment (fragCount - 1 of ordinal 0)
 	int32_t name_off, name_len;
 	int32_t risky_base;   // index into riskyAttempt of ordinal 0, or -1 when attempt 0 always succeeds
-	int32_t pad;
+	int32_t segment;      // index into the ssc_segment array of the plan (array output: the read-name prefix)
 };
 static_assert(sizeof(DevBin) == 64, "DevBin must be 64 bytes");
 
@@ -86,6 +86,12 @@ struct GenParams {
 	uint8_t* dense1; uint8_t* dense2;   // fast kernel: final slabs (pass 2)
 	unsigned long long cap1, cap2;
 	BatchResult* result;
+	// array output (generate_slots_kernel<NCH, QP, true>): out1 = reads of the batch's first pair, [pair][mate][2][pitch];
+	// the per-pair arrays start at the batch's first pair too
+	int16_t* rdLength;          // [pair][mate]
+	int64_t* rdPairId;
+	int32_t* rdSegment; int32_t* rdPos; int32_t* rdFrag;
+	uint32_t pitch;
 };
 
 }  // namespace ssc

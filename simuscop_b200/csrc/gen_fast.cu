@@ -411,14 +411,15 @@ __device__ __forceinline__ void splice_read(const WarpCtx& w, const IndelPlan& p
 
 // Per-base work of a read of m <= 32 * NCH bases whose source sequence is packed at index dOff (store orientation) of
 // win: the fast path's phase C with the position bins of the post-indel length (Profile.cpp:1671), rolled.
-template <int NCH, int QP>
+// ARRAYS: the qualities lie `pitch` bytes behind the bases (array output) instead of m + 3 (FASTQ record).
+template <int NCH, int QP, bool ARRAYS>
 __device__ __forceinline__ void emit_packed(const WarpCtx& w, const uint32_t* win, int dOff, bool rev, int m, uint32_t lut0, uint32_t lutN,
-                                            uint8_t* stage, int H, const uint32_t (&x2)[NCH], const uint32_t (&x3)[NCH]) {
+                                            uint8_t* stage, int H, uint32_t pitch, const uint32_t (&x2)[NCH], const uint32_t (&x3)[NCH]) {
 	const int lane = w.lane;
 	const uint32_t inv = (m > 1) ? (0xffffffffu / (uint32_t)m + 1u) : 0xffffffffu;
 	const int chunksM = (m + 31) >> 5;
 	uint8_t* pB = stage + H + lane;                 // this lane's base of the current chunk; its quality follows m + 3 bytes later
-	uint8_t* pQ = pB + m + 3;
+	uint8_t* pQ = ARRAYS ? pB + pitch : pB + m + 3;
 	uint32_t a2[NCH], a3[NCH];
 #pragma unroll
 	for (int k = 0; k < NCH; k++) { a2[k] = x2[k]; a3[k] = x3[k]; }
@@ -465,10 +466,10 @@ __device__ __forceinline__ void emit_packed(const WarpCtx& w, const uint32_t* wi
 }
 
 // Step 2b.  x2/x3: the substitution / quality draws of output positions 32c+lane, c < NCH (registers of the caller).
-// Writes bases/quals into stage[H ..].
-template <int NCH, int QP>
+// Writes bases/quals into stage[H ..] (qualities as in emit_packed).
+template <int NCH, int QP, bool ARRAYS>
 __device__ __forceinline__ void emit_mapped(const WarpCtx& w, const IndelPlan& pl, int mate, bool rev, int relFirst,
-                                            uint8_t* stage, int H, const uint32_t (&x2)[NCH], const uint32_t (&x3)[NCH]) {
+                                            uint8_t* stage, int H, uint32_t pitch, const uint32_t (&x2)[NCH], const uint32_t (&x3)[NCH]) {
 	const int RL = w.RL, lane = w.lane, m = pl.m, nEv = pl.nEv;
 	const uint2 e0 = pl.e0;
 	const uint2* evs = (const uint2*)w.ev;
@@ -531,7 +532,8 @@ __device__ __forceinline__ void emit_mapped(const WarpCtx& w, const IndelPlan& p
 				if (n3 & 4u) { ch = 'N'; q = (uint32_t)w.minQ + __umulhi(20u, u3); }   // randomInteger(33, 53), Profile.cpp:1583
 				else lookup16(w, rowIdx, binIdx, u2, u3, n3 != 0u, cur, ch, q);
 				stB[c * 32] = (uint8_t)ch;
-				stB[m + 3 + c * 32] = (uint8_t)q;
+				if (ARRAYS) stB[pitch + c * 32] = (uint8_t)q;
+				else stB[m + 3 + c * 32] = (uint8_t)q;
 				continue;
 			}
 			const uint4 sr = w.sub[rowIdx + binIdx];
@@ -552,7 +554,8 @@ __device__ __forceinline__ void emit_mapped(const WarpCtx& w, const IndelPlan& p
 				ch = __byte_perm(w.baseChars, 0, 0x4440u | (r16 & 3u));
 			}
 			stB[c * 32] = (uint8_t)ch;
-			stB[m + 3 + c * 32] = (uint8_t)q;
+			if (ARRAYS) stB[pitch + c * 32] = (uint8_t)q;
+			else stB[m + 3 + c * 32] = (uint8_t)q;
 		}
 	}
 }
@@ -774,10 +777,24 @@ __global__ void __launch_bounds__(MV_THREADS, 1) move_blobs_tma_kernel(const Gen
 	}
 }
 
+// Array output: zeroes bytes [m, pitch) of a read's base row (row0) and of its quality row (pitch bytes behind).  row0 and
+// pitch are multiples of 16: bytes up to the next 16-byte boundary one lane each, the rest with 16-byte stores.
+__device__ __forceinline__ void clear_rows(uint8_t* row0, int m, uint32_t pitch, int lane) {
+	const int a = (m + 15) & ~15;
+	const int i = m + (lane & 15);
+	if (i < a) row0[(lane >> 4) * pitch + i] = 0;
+	const int nv = ((int)pitch - a) >> 4;
+	for (int v = lane; v < 2 * nv; v += 32) {
+		const int r = v >= nv ? 1 : 0;
+		*(uint4*)(row0 + r * pitch + a + 16 * (v - r * nv)) = make_uint4(0u, 0u, 0u, 0u);
+	}
+}
+
 // ---------------------------------------------------------------------------------------------
-// pass 1: generation into per-ticket blobs
+// pass 1: generation into per-ticket blobs (FASTQ records), or, ARRAYS, into fixed slots of caller-owned arrays: the bases and
+// the qualities of a read at [pair][mate][0 / 1][pitch] without record text, the read-name fields of a pair in arrays of their own
 // ---------------------------------------------------------------------------------------------
-template <int NCH, int QP>
+template <int NCH, int QP, bool ARRAYS>
 __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __grid_constant__ GenParams P) {
 	extern __shared__ __align__(16) uint8_t smem[];
 	const DevTables& t = P.t;
@@ -989,6 +1006,12 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 			k_posmod = posmod; k_frag = fragCount;
 			// name_off (17 bits) | name_len << 17 (7 bits) | digits of posmod << 24 | digits of fragCount << 28
 			k_name = (uint32_t)bin.name_off | ((uint32_t)bin.name_len << 17) | ((uint32_t)f_ndigits(posmod) << 24) | ((uint32_t)f_ndigits(fragCount) << 28);
+			if (ARRAYS && lane < count) {
+				// the read-name fields of pair slot0 + L, one coalesced store per array
+				const uint32_t row = slot0 + (uint32_t)lane;
+				P.rdPairId[row] = (int64_t)pair; P.rdSegment[row] = bin.segment;
+				P.rdPos[row] = (int32_t)posmod; P.rdFrag[row] = (int32_t)fragCount;
+			}
 		}
 
 #pragma unroll 1
@@ -1019,13 +1042,13 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 			if (dc.w) qd = dsrc;
 			const uint32_t dg = qd - 10u * (__umulhi(qd, 0xCCCCCCCDu) >> 3) + '0';
 			const int nameLen = (int)((nameNd >> 17) & 127u), nameOff = (int)(nameNd & 0x1ffffu);
-			const int H = nameLen + nd1 + 1 + nd2 + (t.paired ? 2 : 0) + 1;
+			const int H = ARRAYS ? 0 : nameLen + nd1 + 1 + nd2 + (t.paired ? 2 : 0) + 1;   // array output: no header
 			const int hWords = (H + 31) >> 5;
 			const uint32_t slash = t.paired ? (uint32_t)'/' : (uint32_t)'\n';
 			const int mateAt = t.paired ? H - 2 : -1;
 #pragma unroll
 			for (int r = 0; r < 3; r++) {
-				if (r >= hWords) break;
+				if (ARRAYS || r >= hWords) break;
 				// character i of the header: name | digits of pos % segsize (most significant first) | '#' | digits of the
 				// fragment counter | "/1\n" or "\n" -- selected without branches; the digits come from lanes 0..19 by shuffle
 				const int i = lane + 32 * r;
@@ -1055,7 +1078,9 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 				w.win = s_win;
 				w.mDelta = mOff - dOff;
 				const uint32_t c2cyc = ((uint32_t)mate << 28) | ((uint32_t)STREAM_CYCLE << 24);
-				uint8_t* stage = P.out1 + posA;
+				// array output: the read's slot, (pair * M + mate) * 2 * pitch bytes into the batch (< 2^32, clamped by the host)
+				const uint32_t readIdx = (slot0 + (uint32_t)p) * (uint32_t)nMates + (uint32_t)mate;
+				uint8_t* stage = ARRAYS ? P.out1 + readIdx * 2u * P.pitch : P.out1 + posA;
 				const uint4* subM = s_sub + ((mate == 1 && t.useCdf2) ? t.nRows * subPitch : 0);
 				w.sub = subM;
 				if (QP == 16) {
@@ -1088,7 +1113,7 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 					const uint8_t* lutN = lutB + (rev ? 128 : 0);
 					const uint8_t* subMB = (const uint8_t*)subM;
 					uint8_t* st1 = stage + H + lane;
-					uint8_t* st2 = st1 + RL + 3;
+					uint8_t* st2 = ARRAYS ? st1 + P.pitch : st1 + RL + 3;
 #pragma unroll
 					for (int c = 0; c < NCH; c++) {
 						const uint32_t v6 = __funnelshift_r(dptr[c * dstep], dptr[c * dstep + 1], dsh) & 63u;
@@ -1121,6 +1146,10 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 						if (c < NCH - 1) {
 							st1[c * 32] = (uint8_t)ch;
 							st2[c * 32] = (uint8_t)q;
+						} else if (ARRAYS) {
+							if (jLast >= RL) { ch = 0u; q = 0u; }                  // lanes past the read end zero their bytes
+							st1[c * 32] = (uint8_t)ch;
+							st2[c * 32] = (uint8_t)q;
 						} else if (foldTail) {
 							// "\n+\n" after the bases and the final '\n' ride on the idle lanes of the last chunk
 							if (jLast >= RL) { ch = (jLast == RL + 1) ? '+' : '\n'; q = '\n'; }
@@ -1131,7 +1160,8 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 							st2[c * 32] = (uint8_t)q;
 						}
 					}
-					if (!foldTail && lane == 0) { stage[H + m] = '\n'; stage[H + m + 1] = '+'; stage[H + m + 2] = '\n'; stage[H + 2 * m + 3] = '\n'; }
+					if (ARRAYS) clear_rows(stage, 32 * NCH, P.pitch, lane);
+					else if (!foldTail && lane == 0) { stage[H + m] = '\n'; stage[H + m + 1] = '+'; stage[H + m + 2] = '\n'; stage[H + 2 * m + 3] = '\n'; }
 				} else {
 					uint32_t evbits = 0;
 #pragma unroll
@@ -1142,19 +1172,27 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 						if (ins) evbits |= 1u << (2 * c);
 						else if (del) evbits |= 2u << (2 * c);
 					}
-					const IndelPlan pl = scan_events(w, evbits, mate, &P.result->errorFlags);
+					IndelPlan pl = scan_events(w, evbits, mate, &P.result->errorFlags);
+					if (ARRAYS && pl.m > RL + 96) {
+						// longer than a slot holds (pitch >= RL + 96): flagged as a read that outgrew the scratch, nothing written past the slot
+						if (lane == 0) atomicOr(&P.result->errorFlags, 2u);
+						pl.nEv = 0; pl.m = RL; pl.insTotal = 0;
+					}
 					m = pl.m;
 					// a non-ACGT base in the window, or a read that outgrew the NCH chunks of draws: position-by-position path
 					const bool hasN = __any_sync(0xffffffffu, lane >= 16 && lane < 25 && s_win[lane] != 0u);
 					if (hasN || m > 32 * NCH || P.noSplice) {
 						const int relFirst = rev ? (dOff + RL - 1) : dOff;
-						emit_mapped<NCH, QP>(w, pl, mate, rev, relFirst, stage, H, x2, x3);
+						emit_mapped<NCH, QP, ARRAYS>(w, pl, mate, rev, relFirst, stage, H, P.pitch, x2, x3);
 					} else {
 						if (pl.nEv) splice_read(w, pl, rev, dOff);
-						emit_packed<NCH, QP>(w, pl.nEv ? w.outw : s_win, dOff, rev, m, rev ? lutRev0 : lutFwd0, rev ? 128u : 0u, stage, H, x2, x3);
+						emit_packed<NCH, QP, ARRAYS>(w, pl.nEv ? w.outw : s_win, dOff, rev, m, rev ? lutRev0 : lutFwd0, rev ? 128u : 0u, stage, H,
+						                             P.pitch, x2, x3);
 					}
-					if (lane == 0) { stage[H + m] = '\n'; stage[H + m + 1] = '+'; stage[H + m + 2] = '\n'; stage[H + 2 * m + 3] = '\n'; }
+					if (ARRAYS) clear_rows(stage, m, P.pitch, lane);
+					else if (lane == 0) { stage[H + m] = '\n'; stage[H + m + 1] = '+'; stage[H + m + 2] = '\n'; stage[H + 2 * m + 3] = '\n'; }
 				}
+				if (ARRAYS && lane == 0) P.rdLength[readIdx] = (int16_t)m;
 				posA += (uint32_t)(H + 2 * m + 4);
 				if (nMates == 2) { const uint32_t tswap = posA; posA = posB; posB = tswap; }
 				acc += (uint32_t)m;                                                    // bases of the ticket (<= 2^14)
@@ -1165,11 +1203,11 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 			const uint32_t ticket = (uint32_t)chunk;
 			const uint32_t len1 = posA - blobBase, len2 = nMates == 2 ? posB - blobBase - P.file2Off : 0u;
 			if (lane == 0) {
-				P.tileState[ticket] = ((unsigned long long)len1 << 31) | len2;   // blob lengths, scanned by pass 2
+				if (!ARRAYS) P.tileState[ticket] = ((unsigned long long)len1 << 31) | len2;   // blob lengths, scanned by pass 2
 				const uint32_t nPairs = (uint32_t)count;
 				atomicAdd(&P.result->bases, (unsigned long long)(acc & 0xffffu)); atomicAdd(&P.result->hapBytes, (unsigned long long)(acc >> 16));
 				atomicAdd(&P.result->pairs, (unsigned long long)nPairs); atomicAdd(&P.result->reads, (unsigned long long)(nPairs * nMates));
-				atomicAdd(&P.result->rawBytes, (unsigned long long)len1 + len2);
+				if (!ARRAYS) atomicAdd(&P.result->rawBytes, (unsigned long long)len1 + len2);
 			}
 		}
 	}
@@ -1226,9 +1264,9 @@ bool fast_supported(const DevTables& t, int smemLimit, int* qmode, size_t* smemB
 	return false;
 }
 
-template <int NCH, int QP>
+template <int NCH, int QP, bool ARRAYS>
 static cudaError_t launch_fast_variant(const GenParams& P, size_t smemBytes, int grid, cudaStream_t stream) {
-	auto kern = generate_slots_kernel<NCH, QP>;
+	auto kern = generate_slots_kernel<NCH, QP, ARRAYS>;
 	cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemBytes);
 	if (e != cudaSuccess) return e;
 	kern<<<grid, FG_THREADS, smemBytes, stream>>>(P);
@@ -1238,37 +1276,46 @@ static cudaError_t launch_fast_variant(const GenParams& P, size_t smemBytes, int
 // chunks of 32 cycles of the fast kernel instance for read length RL (33..160): exact, only the last chunk has idle lanes
 int fast_nch(int RL) { return RL <= 64 ? 2 : (RL + 31) / 32; }
 
+template <bool ARRAYS>
+static cudaError_t launch_fast_instance(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream) {
+	const int nch = fast_nch(P.t.RL);
+	if (qmode == 8) {
+		if (nch == 2) return launch_fast_variant<2, 8, ARRAYS>(P, smemBytes, grid, stream);
+		if (nch == 3) return launch_fast_variant<3, 8, ARRAYS>(P, smemBytes, grid, stream);
+		if (nch == 4) return launch_fast_variant<4, 8, ARRAYS>(P, smemBytes, grid, stream);
+		return launch_fast_variant<5, 8, ARRAYS>(P, smemBytes, grid, stream);
+	} else if (qmode == 16) {
+		if (nch == 2) return launch_fast_variant<2, 16, ARRAYS>(P, smemBytes, grid, stream);
+		if (nch == 3) return launch_fast_variant<3, 16, ARRAYS>(P, smemBytes, grid, stream);
+		if (nch == 4) return launch_fast_variant<4, 16, ARRAYS>(P, smemBytes, grid, stream);
+		return launch_fast_variant<5, 16, ARRAYS>(P, smemBytes, grid, stream);
+	} else if (qmode == 2) {
+		if (nch == 2) return launch_fast_variant<2, 2, ARRAYS>(P, smemBytes, grid, stream);
+		if (nch == 3) return launch_fast_variant<3, 2, ARRAYS>(P, smemBytes, grid, stream);
+		if (nch == 4) return launch_fast_variant<4, 2, ARRAYS>(P, smemBytes, grid, stream);
+		return launch_fast_variant<5, 2, ARRAYS>(P, smemBytes, grid, stream);
+	}
+	if (nch == 2) return launch_fast_variant<2, 0, ARRAYS>(P, smemBytes, grid, stream);
+	if (nch == 3) return launch_fast_variant<3, 0, ARRAYS>(P, smemBytes, grid, stream);
+	if (nch == 4) return launch_fast_variant<4, 0, ARRAYS>(P, smemBytes, grid, stream);
+	return launch_fast_variant<5, 0, ARRAYS>(P, smemBytes, grid, stream);
+}
+
 // P.out1/out2 = blob scratch, P.dense1/dense2 = final slabs, P.nTiles = tickets of FG_CHUNK pairs.  Launches pass 1;
 // events e0/e1 (optional) bracket the kernel.
 cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream,
                                  cudaEvent_t e0, cudaEvent_t e1) {
-	const int nch = fast_nch(P.t.RL);
-	cudaError_t e;
 	if (e0) cudaEventRecord(e0, stream);
-	if (qmode == 8) {
-		if (nch == 2) e = launch_fast_variant<2, 8>(P, smemBytes, grid, stream);
-		else if (nch == 3) e = launch_fast_variant<3, 8>(P, smemBytes, grid, stream);
-		else if (nch == 4) e = launch_fast_variant<4, 8>(P, smemBytes, grid, stream);
-		else e = launch_fast_variant<5, 8>(P, smemBytes, grid, stream);
-	} else if (qmode == 16) {
-		if (nch == 2) e = launch_fast_variant<2, 16>(P, smemBytes, grid, stream);
-		else if (nch == 3) e = launch_fast_variant<3, 16>(P, smemBytes, grid, stream);
-		else if (nch == 4) e = launch_fast_variant<4, 16>(P, smemBytes, grid, stream);
-		else e = launch_fast_variant<5, 16>(P, smemBytes, grid, stream);
-	} else if (qmode == 2) {
-		if (nch == 2) e = launch_fast_variant<2, 2>(P, smemBytes, grid, stream);
-		else if (nch == 3) e = launch_fast_variant<3, 2>(P, smemBytes, grid, stream);
-		else if (nch == 4) e = launch_fast_variant<4, 2>(P, smemBytes, grid, stream);
-		else e = launch_fast_variant<5, 2>(P, smemBytes, grid, stream);
-	} else {
-		if (nch == 2) e = launch_fast_variant<2, 0>(P, smemBytes, grid, stream);
-		else if (nch == 3) e = launch_fast_variant<3, 0>(P, smemBytes, grid, stream);
-		else if (nch == 4) e = launch_fast_variant<4, 0>(P, smemBytes, grid, stream);
-		else e = launch_fast_variant<5, 0>(P, smemBytes, grid, stream);
-	}
+	const cudaError_t e = launch_fast_instance<false>(P, qmode, smemBytes, grid, stream);
 	if (e != cudaSuccess) return e;
 	if (e1) cudaEventRecord(e1, stream);
 	return cudaSuccess;
+}
+
+// Array output: P.out1 = reads of the batch's first pair ([pair][mate][2][P.pitch], 16-byte aligned, pairs * M * 2 * pitch < 2^32),
+// P.rdLength / rdPairId / rdSegment / rdPos / rdFrag at the same first pair, P.nTiles = tickets of FG_CHUNK pairs.
+cudaError_t launch_generate_reads(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream) {
+	return launch_fast_instance<true>(P, qmode, smemBytes, grid, stream);
 }
 
 // pass 2a alone: blob lengths P.tileState -> offsets P.blobPrefix, totals in P.result->bytes1/2

@@ -42,6 +42,7 @@ int fast_choose_qbins(int B, int RL);
 int fast_nch(int RL);
 cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream,
                                  cudaEvent_t e0, cudaEvent_t e1);
+cudaError_t launch_generate_reads(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream);
 cudaError_t launch_scan_blobs(const GenParams& P, cudaStream_t stream);
 cudaError_t launch_move_blobs(const GenParams& P, int smCount, cudaStream_t stream);
 cudaError_t launch_move_blobs_tma(const GenParams& P, int ctas, cudaStream_t stream);

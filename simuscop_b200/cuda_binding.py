@@ -12,7 +12,8 @@ from .paths import LIB_CUDA
 
 SYMBOLS = ["ssc_last_error", "ssc_version", "ssc_create", "ssc_destroy", "ssc_set_option", "ssc_set_profile",
            "ssc_genome_reserve", "ssc_genome_append", "ssc_genome_size", "ssc_reference_upload", "ssc_reference_upload_fasta", "ssc_reference_prefetch_fasta", "ssc_reference_adopt_prefetched", "ssc_genome_append_ref", "ssc_genome_poke", "ssc_genome_read", "ssc_gc_census", "ssc_set_plan", "ssc_generate",
-           "ssc_generate_device", "ssc_get_stats", "ssc_reset_stats", "ssc_table_lookup_host", "ssc_sub_lookup_host", "ssc_gzip_member_host", "ssc_issue_floor"]
+           "ssc_generate_device", "ssc_read_shape", "ssc_generate_reads", "ssc_segment_name", "ssc_get_stats", "ssc_reset_stats",
+           "ssc_table_lookup_host", "ssc_sub_lookup_host", "ssc_gzip_member_host", "ssc_issue_floor"]
 
 _lib = None
 
@@ -47,6 +48,11 @@ def lib():
         L.ssc_generate.argtypes = [C.c_void_p, C.c_int64, C.c_int64, abi.SINK_FN, C.c_void_p]
         L.ssc_generate_device.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.POINTER(C.c_uint64),
                                           C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_double)]
+        L.ssc_read_shape.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_int32),
+                                     C.POINTER(C.c_int32)]
+        L.ssc_generate_reads.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.POINTER(abi.ReadArrays), C.c_void_p,
+                                         C.POINTER(C.c_int64)]
+        L.ssc_segment_name.argtypes = [C.c_void_p, C.c_int32, C.c_char_p, C.c_int32]
         L.ssc_get_stats.argtypes = [C.c_void_p, C.POINTER(abi.Stats)]
         L.ssc_reset_stats.argtypes = [C.c_void_p]
         L.ssc_table_lookup_host.argtypes = [C.c_void_p, C.c_int, C.c_uint32]
@@ -63,12 +69,18 @@ def _ck(rc):
         raise SscError("ssc error %d: %s" % (rc, lib().ssc_last_error().decode(errors="replace")))
 
 
+def _read_views(reads, length, pair_id, segment, pos, frag):
+    return dict(reads=reads, seq=reads[:, :, 0], qual=reads[:, :, 1], length=length, pair_id=pair_id, segment=segment, pos=pos,
+                frag=frag)
+
+
 class Generator:
     """One handle on one GPU."""
 
     def __init__(self, device=0):
         self.h = C.c_void_p()
         _ck(lib().ssc_create(device, C.byref(self.h)))
+        self.device = device
         self.planned = 0
         self.emitted = 0
         self._keep = []
@@ -150,6 +162,59 @@ class Generator:
         b1, b2, nb, ms = C.c_uint64(), C.c_uint64(), C.c_uint64(), C.c_double()
         _ck(lib().ssc_generate_device(self.h, lo, hi, C.byref(b1), C.byref(b2), C.byref(nb), C.byref(ms)))
         return dict(bytes1=b1.value, bytes2=b2.value, bases=nb.value, device_ms=ms.value)
+
+    def read_shape(self, lo=0, hi=None):
+        """(pairs the range [lo, hi) emits, mates per pair, slot pitch in bytes) of the array output."""
+        if hi is None:
+            hi = self.planned
+        n, m, p = C.c_int64(), C.c_int32(), C.c_int32()
+        _ck(lib().ssc_read_shape(self.h, lo, hi, C.byref(n), C.byref(m), C.byref(p)))
+        return n.value, m.value, p.value
+
+    def empty_reads(self, n_pairs):
+        """Uninitialised torch arrays for n_pairs pairs of array output on the handle's device (see generate_reads)."""
+        import torch
+        _, mates, pitch = self.read_shape(0, 0)
+        dev = torch.device("cuda", self.device)
+        n = max(int(n_pairs), 1)                     # the library takes no null pointers, also for an empty range
+        reads = torch.empty((n, mates, 2, pitch), dtype=torch.uint8, device=dev)
+        return _read_views(reads, torch.empty((n, mates), dtype=torch.int16, device=dev),
+                           torch.empty(n, dtype=torch.int64, device=dev), torch.empty(n, dtype=torch.int32, device=dev),
+                           torch.empty(n, dtype=torch.int32, device=dev), torch.empty(n, dtype=torch.int32, device=dev))
+
+    def generate_reads(self, lo=0, hi=None, stream=None, out=None):
+        """Pairs [lo, hi) as torch arrays on the handle's device, no FASTQ text and no host copy (ssc_generate_reads).  Returns a
+        dict: reads [n, M, 2, pitch] uint8 (row 0 the bases, row 1 the qualities as FASTQ characters, zero past the length), seq
+        and qual (its two rows), length [n, M] int16, pair_id [n] int64, segment / pos / frag [n] int32 (the read name is
+        segment_name(segment) + pos + '#' + frag + '/mate').  The call is ordered after the work queued on `stream` (default: torch's
+        current stream) and returns when the arrays are complete.  `out`: arrays of an earlier call or of empty_reads, with room
+        for the range, written in place (the result views their first n rows)."""
+        import torch
+        if hi is None:
+            hi = self.planned
+        if out is None:
+            out = self.empty_reads(self.read_shape(lo, hi)[0])
+        a = out
+        for k, dt in (("reads", torch.uint8), ("length", torch.int16), ("pair_id", torch.int64), ("segment", torch.int32),
+                      ("pos", torch.int32), ("frag", torch.int32)):
+            if a[k].dtype != dt or not a[k].is_contiguous() or not a[k].is_cuda:
+                raise ValueError("generate_reads: out[%r] must be a contiguous CUDA tensor of %s" % (k, dt))
+        if stream is None:
+            stream = torch.cuda.current_stream(torch.device("cuda", self.device))
+        st = abi.ReadArrays(a["reads"].data_ptr(), a["length"].data_ptr(), a["pair_id"].data_ptr(), a["segment"].data_ptr(),
+                            a["pos"].data_ptr(), a["frag"].data_ptr(), min(a["reads"].shape[0], a["length"].shape[0],
+                            a["pair_id"].shape[0], a["segment"].shape[0], a["pos"].shape[0], a["frag"].shape[0]),
+                            a["reads"].shape[-1])
+        n = C.c_int64()
+        _ck(lib().ssc_generate_reads(self.h, lo, hi, C.byref(st), C.c_void_p(stream.cuda_stream), C.byref(n)))
+        k = n.value
+        return _read_views(a["reads"][:k], a["length"][:k], a["pair_id"][:k], a["segment"][:k], a["pos"][:k], a["frag"][:k])
+
+    def segment_name(self, i):
+        """Read-name prefix "@<popu>#<chr>#" of segment i of the plan (the `segment` array of generate_reads)."""
+        buf = C.create_string_buffer(80)
+        _ck(lib().ssc_segment_name(self.h, int(i), buf, len(buf)))
+        return buf.value
 
     def issue_floor(self, mode, read_length, n_pairs, reps=3):
         """Mean launch time (ms) of the issue-rate microbenchmark (ssc_issue_floor)."""
