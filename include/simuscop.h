@@ -137,7 +137,9 @@ typedef struct ssc_stats {
  * Sink for finished FASTQ slabs, called in pair order.  buf1/buf2 point to pinned host
  * memory owned by the handle and valid only during the call (SeqWriter::write(char*,char*)
  * semantics, SeqWriter.cpp:49-54: the callee copies or writes synchronously).  In SE
- * layout buf2 == NULL and len2 == 0.  Return 0 to continue.
+ * layout buf2 == NULL and len2 == 0.  With the "interleave" option a PE plan follows the SE
+ * contract too: buf1/len1 hold pair i mate 1, pair i mate 2, ... in pair order, and
+ * buf2 == NULL, len2 == 0.  Return 0 to continue.
  */
 typedef int (*ssc_sink_fn)(void* user, const char* buf1, size_t len1, const char* buf2, size_t len2,
                            int64_t first_pair, int64_t n_pairs);
@@ -153,7 +155,12 @@ int ssc_destroy(ssc_handle* h);
  * handed to the sink hold concatenated gzip members -- a valid .gz stream of the same FASTQ bytes -- compressed on
  * the GPU, one member per 32 pairs, Huffman-coded with a table fitted to the first batch, or stored where that code would
  * expand the member past its bytes + 23, so gzip mode fails only where plain output does; the plain bytes of
- * SeqWriter::write are the default), "concurrent_move" (n > 0: the blobs of batch k are moved by a
+ * SeqWriter::write are the default), "interleave" (0/1: a PE plan writes ONE stream, pair i mate 1 then pair i mate 2 in pair
+ * order, byte for byte the interleave of the _1 / _2 records without the option, "/1" and "/2" suffixes included -- what
+ * `bwa mem -p` and `bowtie2 --interleaved` read; the sink gets it as buf1/len1 with buf2 == NULL, len2 == 0,
+ * ssc_generate_device returns it in *bytes1 with *bytes2 = 0, ssc_stats counts the same fastq_bytes / gz_bytes totals; with
+ * gzip, one member per 32 pairs of both mates; no effect on SE plans and on ssc_generate_reads; like gzip it may be set
+ * between calls and takes effect at the next one), "concurrent_move" (n > 0: the blobs of batch k are moved by a
  * bulk-copy kernel on n SMs, on a second stream, while the generation kernel of batch k+1 runs on the others; default 9 of
  * 148 SMs, 0 below 64 SMs; 0, or n at least the GPU's SM count: a stand-alone kernel after every batch), "max_ctas" (> 0 caps the grid of the generation
  * kernel; 0 = one CTA per SM), "no_splice" (0/1, tests: reads with indel events take the position-by-position path
@@ -224,7 +231,8 @@ int ssc_set_plan(ssc_handle* h, uint64_t seed,
 int ssc_generate(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc_sink_fn sink, void* user);
 
 /* Same work, output left in the handle's device slab (no device->host copy of FASTQ):
- * the device-resident measurement leg.  Any of the out pointers may be NULL. */
+ * the device-resident measurement leg.  Any of the out pointers may be NULL.  Interleaved
+ * PE output: the whole stream in *bytes1, *bytes2 = 0. */
 int ssc_generate_device(ssc_handle* h, int64_t pair_lo, int64_t pair_hi,
                         uint64_t* bytes1, uint64_t* bytes2, uint64_t* bases, double* device_ms);
 

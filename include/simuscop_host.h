@@ -55,10 +55,17 @@ int ssh_selftest_splices(ssh_job* job, int64_t* haplotypes_checked, int64_t* seg
  * workers copy 8 MB chunks into shared mappings of the slab's file ranges (hybrid: beside the two streams). */
 typedef struct ssh_writer ssh_writer;
 int ssh_writer_open(const char* path1, const char* path2, int threads, ssh_writer** out);
+/* A single-stream writer on a descriptor the caller opened and closes (standard output, a pipe to an aligner): slabs are
+ * written in order with write() from the calling thread, so descriptors that cannot seek work.  buf2 must be NULL (SE or
+ * interleaved PE).  A failed write (EPIPE once the reader has gone, with SIGPIPE ignored) makes the sink return non-zero. */
+int ssh_writer_open_fd(int fd, ssh_writer** out);
 ssc_sink_fn ssh_writer_sink(void);
 int ssh_writer_close(ssh_writer* w, uint64_t* bytes1, uint64_t* bytes2);
 
-/* The whole drop-in run: every sample -> FASTQ files in the output directory, on `device`. */
+/* The whole drop-in run: every sample -> FASTQ files in the output directory, on `device`.  Environment:
+ * SIMUSCOP_INTERLEAVE=1 writes a PE sample to <output>/<stem>.fq (.fq.gz with SIMUSCOP_GZIP=1), mate 1 and mate 2 of each pair
+ * in turn, instead of <stem>_1 / <stem>_2; SIMUSCOP_STDOUT=1 writes the reads (PE interleaved) to standard output and no
+ * FASTQ file, and refuses a configuration with more than one sample. */
 int ssh_run(ssh_job* job, int device);
 
 #ifdef __cplusplus

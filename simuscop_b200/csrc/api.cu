@@ -87,6 +87,8 @@ struct ssc_handle {
 	cudaEvent_t evResult[2] = {nullptr, nullptr};    // batch of buffer set b: its BatchResult in h_result[b]
 	int fastQmode = -1;           // "fast_qmode": -1 automatic, else the only quality-table mode the fast kernel may use (tests)
 	bool gzip = false;            // slabs hold gzip members (one per ticket blob) instead of plain FASTQ
+	bool interleave = false;      // "interleave": a PE plan's mates go to one stream, mate 1 and mate 2 of each pair in turn
+	size_t gzBlobBytes = 0;       // allocation of d_gzBlobs[0] (interleaved: both mates per ticket)
 	bool haveGz = false;          // Huffman / CRC tables of the current plan are on the device
 	ssc::GzTables* d_gzTab = nullptr;
 	uint8_t* d_gzBlobs[2] = {nullptr, nullptr};
@@ -149,6 +151,7 @@ struct ssc_handle {
 	// batch resources
 	int64_t slabPairs = 0;
 	uint64_t slabCap = 0;
+	int slabFiles = 0;                             // output streams the slabs were allocated for (out_files)
 	uint8_t* d_out[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};   // [buffer][file]
 	uint8_t* h_out[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};
 	DevBuf<int32_t> d_tileStart[2];
@@ -188,13 +191,22 @@ bool use_fast(const ssc_handle* h, int* qmode, size_t* smemBytes) {
 	return ssc::fast_supported(h->dt, h->smemLimit, qmode, smemBytes);
 }
 
+// PE plan with the "interleave" option: one output stream holding both mates (the option has no effect on SE plans)
+bool interleaved(const ssc_handle* h) { return h->interleave && h->dt.paired; }
+
+// output streams of ssc_generate / ssc_generate_device: 2 for two-file PE, 1 for SE and interleaved PE
+int out_files(const ssc_handle* h) { return h->dt.paired && !h->interleave ? 2 : 1; }
+
 
 int ensure_batch_resources(ssc_handle* h, bool needHost) {
 	int64_t pairs = std::min<int64_t>(h->batchPairs, std::max<int64_t>(h->emittedPairs, 1));
 	pairs = ((pairs + GEN_TILE_PAIRS - 1) / GEN_TILE_PAIRS) * GEN_TILE_PAIRS;   // multiple of both tile sizes
-	// gzip mode: a member is at most its blob plus the bytes of a stored block (gz.cu), and there is one member per ticket
-	const uint64_t perPair = (uint64_t)h->maxRecBytes + (h->gzip ? 1 : 0);
-	auto slab_cap = [&](int64_t n) { return (uint64_t)n * (uint64_t)h->maxRecBytes + 4096 + (h->gzip ? (uint64_t)(n / FG_CHUNK) * ssc::GZ_STORED_EXTRA : 0); };
+	// gzip mode: a member is at most its blob plus the bytes of a stored block (gz.cu), and there is one member per ticket.
+	// Interleaved output: a slab holds both mates of a pair.  The scan packs a slab length into 31 bits, so the slab bound stays
+	// below 2^31 in every mode.
+	const uint64_t recBytes = (uint64_t)h->maxRecBytes * (interleaved(h) ? 2u : 1u);
+	const uint64_t perPair = recBytes + (h->gzip ? 1 : 0);
+	auto slab_cap = [&](int64_t n) { return (uint64_t)n * recBytes + 4096 + (h->gzip ? (uint64_t)(n / FG_CHUNK) * ssc::GZ_STORED_EXTRA : 0); };
 	uint64_t cap = slab_cap(pairs);
 	if (cap >= (1ull << 31)) {
 		pairs = (int64_t)(((1ull << 31) - 8192) / perPair);
@@ -202,16 +214,17 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 		if (pairs <= 0) return fail(SSC_ERR_INVALID, "record size too large");
 		cap = slab_cap(pairs);
 	}
-	int nFiles = h->dt.paired ? 2 : 1;
+	int nFiles = h->dt.paired ? 2 : 1;             // halves of the blob scratch (interleaved: one blob of both mates across both)
+	const int slabFiles = out_files(h);
 	{
-		// the fast kernel addresses its blob scratch (FG_SLOT bytes per record, both files) with 32-bit offsets
+		// the fast kernel addresses its blob scratch (FG_SLOT bytes per record, both mates) with 32-bit offsets
 		const int64_t maxFast = (int64_t)(((1ull << 32) - (1ull << 20)) / ((uint64_t)FG_SLOT * (uint64_t)nFiles));
 		if (pairs > maxFast) {
 			pairs = (maxFast / GEN_TILE_PAIRS) * GEN_TILE_PAIRS;
 			cap = slab_cap(pairs);
 		}
 	}
-	if (pairs != h->slabPairs || cap != h->slabCap) {
+	if (pairs != h->slabPairs || cap != h->slabCap || slabFiles != h->slabFiles) {
 		for (int b = 0; b < 2; b++)
 			for (int f = 0; f < 2; f++) {
 				if (h->d_out[b][f]) cudaFree(h->d_out[b][f]);
@@ -219,7 +232,7 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 				h->d_out[b][f] = nullptr; h->h_out[b][f] = nullptr;
 			}
 		for (int b = 0; b < 2; b++) { if (h->d_slots[b][0]) cudaFree(h->d_slots[b][0]); h->d_slots[b][0] = h->d_slots[b][1] = nullptr; }
-		h->slabPairs = 0; h->slabCap = 0;          // committed below, once every allocation has succeeded
+		h->slabPairs = 0; h->slabCap = 0; h->slabFiles = 0;   // committed below, once every allocation has succeeded
 		h->pending.valid = false;
 		for (int b = 0; b < 2; b++) {
 			// file 2's blobs behind file 1's: the kernel addresses both from one base pointer with 32-bit cursors
@@ -228,23 +241,29 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 			CK(h->d_blobPrefix[b].alloc((size_t)(pairs / 16) + 2));
 		}
 		for (int f = 0; f < 2; f++) { if (h->d_gzBlobs[f]) cudaFree(h->d_gzBlobs[f]); h->d_gzBlobs[f] = nullptr; }
+		h->gzBlobBytes = 0;
 		int nTiles = (int)(pairs / 16) + 2;   // enough for every kernel's tile size
 		for (int b = 0; b < 2; b++) {
-			for (int f = 0; f < nFiles; f++) CK(cudaMalloc((void**)&h->d_out[b][f], cap));
+			for (int f = 0; f < slabFiles; f++) CK(cudaMalloc((void**)&h->d_out[b][f], cap));
 			CK(h->d_tileStart[b].alloc(nTiles));
 			CK(h->d_tileState[b].alloc(nTiles));
 			CK(h->d_ticket[b].alloc(1));
 		}
-		h->slabPairs = pairs; h->slabCap = cap;
+		h->slabPairs = pairs; h->slabCap = cap; h->slabFiles = slabFiles;
 	}
-	if (h->gzip && !h->d_gzBlobs[0]) {
-		for (int f = 0; f < 2; f++) CK(cudaMalloc((void**)&h->d_gzBlobs[f], (size_t)h->slabPairs * FG_SLOT + 64));
+	// gzip members: one per ticket blob, at the blob's pitch (interleaved: twice the per-file pitch, one file)
+	const size_t gzBytes = (size_t)h->slabPairs * FG_SLOT * (interleaved(h) ? 2 : 1) + 64;
+	if (h->gzip && h->gzBlobBytes != gzBytes) {
+		for (int f = 0; f < 2; f++) { if (h->d_gzBlobs[f]) cudaFree(h->d_gzBlobs[f]); h->d_gzBlobs[f] = nullptr; }
+		h->gzBlobBytes = 0;
+		for (int f = 0; f < (interleaved(h) ? 1 : 2); f++) CK(cudaMalloc((void**)&h->d_gzBlobs[f], gzBytes));
+		h->gzBlobBytes = gzBytes;
 		CK(h->d_gzLens.alloc((size_t)(h->slabPairs / 16) + 2));
 		if (!h->d_gzTab) CK(cudaMalloc((void**)&h->d_gzTab, sizeof(ssc::GzTables)));
 	}
 	if (needHost)
 		for (int b = 0; b < 2; b++)
-			for (int f = 0; f < nFiles; f++)
+			for (int f = 0; f < slabFiles; f++)
 				if (!h->h_out[b][f]) CK(cudaMallocHost((void**)&h->h_out[b][f], h->slabCap));
 	return SSC_OK;
 }
@@ -269,7 +288,7 @@ int build_gz_tables(ssc_handle* h, const ssc::GenParams& P, int nTiles) {
 	memset(hist, 0, sizeof(hist));
 	CK(cudaStreamSynchronize(h->compute));
 	CK(cudaMemcpy(lens.data(), P.tileState, lens.size() * 8, cudaMemcpyDeviceToHost));
-	for (int f = 0; f < (h->dt.paired ? 2 : 1); f++) {
+	for (int f = 0; f < out_files(h); f++) {
 		CK(cudaMemcpy(blob.data(), f ? P.out2 : P.out1, blob.size(), cudaMemcpyDeviceToHost));
 		for (int j = 0; j < sample; j++) {
 			const size_t n = f ? (size_t)(lens[j] & 0x7fffffffull) : (size_t)(lens[j] >> 31);
@@ -386,7 +405,9 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 		// pass 1 writes one blob per ticket and file into the scratch, pass 2 (scan of the blob lengths + one move per blob) the dense slab
 		P.dense1 = P.out1; P.dense2 = P.out2;
 		P.out1 = h->d_slots[buf][0]; P.out2 = h->d_slots[buf][1];
-		P.blobPitch = (uint32_t)(FG_CHUNK * FG_SLOT);
+		// interleaved: one blob per ticket over both halves of the scratch, so twice the per-file pitch
+		const bool ilv = interleaved(h);
+		P.blobPitch = (uint32_t)(FG_CHUNK * FG_SLOT * (ilv ? 2 : 1));
 		P.file2Off = (uint32_t)(h->d_slots[buf][1] ? h->d_slots[buf][1] - h->d_slots[buf][0] : 0);
 		cudaEvent_t te;
 		if (!h->gzip) {
@@ -408,7 +429,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 			grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount - (movedBuf >= 0 ? h->moverCtas : 0));
 			if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
 			CK(time_begin(h, s, &h->stats.gen_kernel_ms, &te));
-			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, nullptr, te));
+			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, nullptr, te, ilv));
 			// pass 2a on the mover stream, behind the previous batch's move: only the moves and the host need its offsets and
 			// totals, so the compute stream goes straight on to the next batch
 			CK(cudaEventRecord(h->evPre, s));
@@ -431,14 +452,14 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 			grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount);
 			if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
 			CK(time_begin(h, s, &h->stats.gen_kernel_ms, &te));
-			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, nullptr, te));
+			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, nullptr, te, ilv));
 			CK(time_begin(h, s, &h->stats.compact_kernel_ms, &te));
 			if (!h->haveGz) { rc = build_gz_tables(h, P, nTiles); if (rc) return rc; }
 			CK(cudaMemsetAsync(h->d_gzLens.p, 0, sizeof(unsigned long long) * nTiles, s));
 			CK(ssc::launch_deflate_blobs(P.out1, P.out2, P.tileState, nTiles, P.blobPitch, h->d_gzBlobs[0], h->d_gzBlobs[1], h->d_gzLens.p,
-			                             FG_CHUNK * FG_SLOT, h->d_gzTab, h->smCount, s));
+			                             P.blobPitch, h->d_gzTab, h->smCount, s));
 			ssc::GenParams P2 = P;
-			P2.out1 = h->d_gzBlobs[0]; P2.out2 = h->d_gzBlobs[1]; P2.tileState = h->d_gzLens.p; P2.blobPitch = FG_CHUNK * FG_SLOT;
+			P2.out1 = h->d_gzBlobs[0]; P2.out2 = h->d_gzBlobs[1]; P2.tileState = h->d_gzLens.p; P2.blobPitch = P.blobPitch;
 			CK(ssc::launch_pass2(P2, h->smCount, s));
 			if (te) CK(cudaEventRecord(te, s));
 			h->stats.launches += 4;
@@ -451,7 +472,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 		if (!v.ok) return fail(SSC_ERR_INVALID, "no kernel variant for read length %d / kmer %d", h->dt.RL, h->dt.K);
 		h->stats.gen_kernel = v.fp64 ? 4 : v.k3 ? 2 : 3; h->stats.gen_nch = v.nch; h->stats.gen_qmode = -1;
 		h->stats.gen_smem_bytes = (int32_t)v.smemBytes;
-		CK(ssc::launch_generate(P, v, grid, s));
+		CK(ssc::launch_generate(P, v, grid, s, interleaved(h)));
 		h->stats.launches += 1;
 	}
 	return result_to_host(h, buf, s);
@@ -608,6 +629,7 @@ int ssc_set_option(ssc_handle* h, const char* key, int64_t value) {
 		return SSC_OK;
 	}
 	if (!strcmp(key, "gzip")) { h->gzip = value != 0; return SSC_OK; }
+	if (!strcmp(key, "interleave")) { h->interleave = value != 0; return SSC_OK; }   // slabs re-sized at the next call if they must
 	if (!strcmp(key, "concurrent_move")) {
 		if (value < 0 || value > 64) return fail(SSC_ERR_INVALID, "concurrent_move: 0 (off) .. 64 SMs");
 		h->moverCtas = value < h->smCount ? (int)value : 0;     // the generation kernel needs SMs beside the mover
@@ -1168,7 +1190,7 @@ static int generate_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc
 	if (rc) return rc;
 	const int64_t eLo = emit_index_of_plan(h, pair_lo), eHi = emit_index_of_plan(h, pair_hi);
 	if (eHi <= eLo) return SSC_OK;
-	const int nFiles = h->dt.paired ? 2 : 1;
+	const int nFiles = out_files(h);
 	struct Batch { int64_t lo, hi; };
 	std::vector<Batch> batches;
 	for (int64_t e = eLo; e < eHi; e += h->slabPairs) batches.push_back({e, std::min(eHi, e + h->slabPairs)});

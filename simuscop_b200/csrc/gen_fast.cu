@@ -791,11 +791,19 @@ __device__ __forceinline__ void clear_rows(uint8_t* row0, int m, uint32_t pitch,
 }
 
 // ---------------------------------------------------------------------------------------------
-// pass 1: generation into per-ticket blobs (FASTQ records), or, ARRAYS, into fixed slots of caller-owned arrays: the bases and
-// the qualities of a read at [pair][mate][0 / 1][pitch] without record text, the read-name fields of a pair in arrays of their own
+// pass 1: generation into per-ticket blobs (FASTQ records), or, OUT_ARRAYS, into fixed slots of caller-owned arrays: the bases
+// and the qualities of a read at [pair][mate][0 / 1][pitch] without record text, the read-name fields of a pair in arrays of
+// their own.  OUT_FASTQ: one blob per ticket and file (PE: file 2's blob P.file2Off bytes behind file 1's); OUT_INTERLEAVED
+// (PE only): one blob per ticket holding mate 1, mate 2 of every pair in turn, at pitch 2 x FG_CHUNK x FG_SLOT over both halves
+// of the scratch.  Mate 2's header is written at the cursor behind mate 1's record, which is known once mate 1's indel scan
+// has fixed its length.
 // ---------------------------------------------------------------------------------------------
-template <int NCH, int QP, bool ARRAYS>
+enum { OUT_FASTQ = 0, OUT_ARRAYS = 1, OUT_INTERLEAVED = 2 };
+
+template <int NCH, int QP, int OUT>
 __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __grid_constant__ GenParams P) {
+	constexpr bool ARRAYS = OUT == OUT_ARRAYS;
+	constexpr bool ILV = OUT == OUT_INTERLEAVED;
 	extern __shared__ __align__(16) uint8_t smem[];
 	const DevTables& t = P.t;
 	const int lane = threadIdx.x & 31;
@@ -952,7 +960,8 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 		uint32_t acc = 0;                                // bases | haplotype bytes << 16 of this ticket
 		// next free byte of this ticket's two blobs, relative to P.out1 (file 2's blobs lie P.file2Off bytes behind file 1's in the
 		// same allocation; scratch < 2^32 bytes).
-		// posA belongs to the file of the current mate: the two cursors change places after every mate of a pair.
+		// posA belongs to the file of the current mate: the two cursors change places after every mate of a pair (interleaved
+		// output: posA is the one cursor of the ticket's blob, posB is not used).
 		const uint32_t blobBase = (uint32_t)chunk * P.blobPitch;
 		uint32_t posA = blobBase, posB = blobBase + P.file2Off;
 
@@ -1046,6 +1055,7 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 			const int hWords = (H + 31) >> 5;
 			const uint32_t slash = t.paired ? (uint32_t)'/' : (uint32_t)'\n';
 			const int mateAt = t.paired ? H - 2 : -1;
+			uint32_t hdr = 0;                                                        // interleaved: this lane's header characters, byte r
 #pragma unroll
 			for (int r = 0; r < 3; r++) {
 				if (ARRAYS || r >= hWords) break;
@@ -1064,8 +1074,9 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 				if (i < H) {
 					const bool mateDigit = i == mateAt;
 					P.out1[posA + i] = (uint8_t)(mateDigit ? (uint32_t)'1' : ch);
-					if (t.paired) P.out1[posB + i] = (uint8_t)(mateDigit ? (uint32_t)'2' : ch);
+					if (t.paired && !ILV) P.out1[posB + i] = (uint8_t)(mateDigit ? (uint32_t)'2' : ch);
 				}
+				if (ILV) hdr |= (ch & 0xffu) << (8 * r);                               // mate 2's header, written behind mate 1's record
 			}
 
 #pragma unroll 1
@@ -1194,14 +1205,22 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 				}
 				if (ARRAYS && lane == 0) P.rdLength[readIdx] = (int16_t)m;
 				posA += (uint32_t)(H + 2 * m + 4);
-				if (nMates == 2) { const uint32_t tswap = posA; posA = posB; posB = tswap; }
+				if (ILV) {
+					if (mate == 0) {
+#pragma unroll
+						for (int r = 0; r < 3; r++) {
+							const int i = lane + 32 * r;
+							if (i < H) P.out1[posA + i] = (uint8_t)(i == mateAt ? (uint32_t)'2' : (hdr >> (8 * r)) & 0xffu);
+						}
+					}
+				} else if (nMates == 2) { const uint32_t tswap = posA; posA = posB; posB = tswap; }
 				acc += (uint32_t)m;                                                    // bases of the ticket (<= 2^14)
 				__syncwarp();
 			}
 		}
 		{
 			const uint32_t ticket = (uint32_t)chunk;
-			const uint32_t len1 = posA - blobBase, len2 = nMates == 2 ? posB - blobBase - P.file2Off : 0u;
+			const uint32_t len1 = posA - blobBase, len2 = (nMates == 2 && !ILV) ? posB - blobBase - P.file2Off : 0u;
 			if (lane == 0) {
 				if (!ARRAYS) P.tileState[ticket] = ((unsigned long long)len1 << 31) | len2;   // blob lengths, scanned by pass 2
 				const uint32_t nPairs = (uint32_t)count;
@@ -1264,9 +1283,9 @@ bool fast_supported(const DevTables& t, int smemLimit, int* qmode, size_t* smemB
 	return false;
 }
 
-template <int NCH, int QP, bool ARRAYS>
+template <int NCH, int QP, int OUT>
 static cudaError_t launch_fast_variant(const GenParams& P, size_t smemBytes, int grid, cudaStream_t stream) {
-	auto kern = generate_slots_kernel<NCH, QP, ARRAYS>;
+	auto kern = generate_slots_kernel<NCH, QP, OUT>;
 	cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemBytes);
 	if (e != cudaSuccess) return e;
 	kern<<<grid, FG_THREADS, smemBytes, stream>>>(P);
@@ -1276,37 +1295,38 @@ static cudaError_t launch_fast_variant(const GenParams& P, size_t smemBytes, int
 // chunks of 32 cycles of the fast kernel instance for read length RL (33..160): exact, only the last chunk has idle lanes
 int fast_nch(int RL) { return RL <= 64 ? 2 : (RL + 31) / 32; }
 
-template <bool ARRAYS>
+template <int OUT>
 static cudaError_t launch_fast_instance(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream) {
 	const int nch = fast_nch(P.t.RL);
 	if (qmode == 8) {
-		if (nch == 2) return launch_fast_variant<2, 8, ARRAYS>(P, smemBytes, grid, stream);
-		if (nch == 3) return launch_fast_variant<3, 8, ARRAYS>(P, smemBytes, grid, stream);
-		if (nch == 4) return launch_fast_variant<4, 8, ARRAYS>(P, smemBytes, grid, stream);
-		return launch_fast_variant<5, 8, ARRAYS>(P, smemBytes, grid, stream);
+		if (nch == 2) return launch_fast_variant<2, 8, OUT>(P, smemBytes, grid, stream);
+		if (nch == 3) return launch_fast_variant<3, 8, OUT>(P, smemBytes, grid, stream);
+		if (nch == 4) return launch_fast_variant<4, 8, OUT>(P, smemBytes, grid, stream);
+		return launch_fast_variant<5, 8, OUT>(P, smemBytes, grid, stream);
 	} else if (qmode == 16) {
-		if (nch == 2) return launch_fast_variant<2, 16, ARRAYS>(P, smemBytes, grid, stream);
-		if (nch == 3) return launch_fast_variant<3, 16, ARRAYS>(P, smemBytes, grid, stream);
-		if (nch == 4) return launch_fast_variant<4, 16, ARRAYS>(P, smemBytes, grid, stream);
-		return launch_fast_variant<5, 16, ARRAYS>(P, smemBytes, grid, stream);
+		if (nch == 2) return launch_fast_variant<2, 16, OUT>(P, smemBytes, grid, stream);
+		if (nch == 3) return launch_fast_variant<3, 16, OUT>(P, smemBytes, grid, stream);
+		if (nch == 4) return launch_fast_variant<4, 16, OUT>(P, smemBytes, grid, stream);
+		return launch_fast_variant<5, 16, OUT>(P, smemBytes, grid, stream);
 	} else if (qmode == 2) {
-		if (nch == 2) return launch_fast_variant<2, 2, ARRAYS>(P, smemBytes, grid, stream);
-		if (nch == 3) return launch_fast_variant<3, 2, ARRAYS>(P, smemBytes, grid, stream);
-		if (nch == 4) return launch_fast_variant<4, 2, ARRAYS>(P, smemBytes, grid, stream);
-		return launch_fast_variant<5, 2, ARRAYS>(P, smemBytes, grid, stream);
+		if (nch == 2) return launch_fast_variant<2, 2, OUT>(P, smemBytes, grid, stream);
+		if (nch == 3) return launch_fast_variant<3, 2, OUT>(P, smemBytes, grid, stream);
+		if (nch == 4) return launch_fast_variant<4, 2, OUT>(P, smemBytes, grid, stream);
+		return launch_fast_variant<5, 2, OUT>(P, smemBytes, grid, stream);
 	}
-	if (nch == 2) return launch_fast_variant<2, 0, ARRAYS>(P, smemBytes, grid, stream);
-	if (nch == 3) return launch_fast_variant<3, 0, ARRAYS>(P, smemBytes, grid, stream);
-	if (nch == 4) return launch_fast_variant<4, 0, ARRAYS>(P, smemBytes, grid, stream);
-	return launch_fast_variant<5, 0, ARRAYS>(P, smemBytes, grid, stream);
+	if (nch == 2) return launch_fast_variant<2, 0, OUT>(P, smemBytes, grid, stream);
+	if (nch == 3) return launch_fast_variant<3, 0, OUT>(P, smemBytes, grid, stream);
+	if (nch == 4) return launch_fast_variant<4, 0, OUT>(P, smemBytes, grid, stream);
+	return launch_fast_variant<5, 0, OUT>(P, smemBytes, grid, stream);
 }
 
 // P.out1/out2 = blob scratch, P.dense1/dense2 = final slabs, P.nTiles = tickets of FG_CHUNK pairs.  Launches pass 1;
-// events e0/e1 (optional) bracket the kernel.
+// events e0/e1 (optional) bracket the kernel.  interleaved (PE): one blob per ticket, P.blobPitch = 2 x FG_CHUNK x FG_SLOT.
 cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream,
-                                 cudaEvent_t e0, cudaEvent_t e1) {
+                                 cudaEvent_t e0, cudaEvent_t e1, bool interleaved) {
 	if (e0) cudaEventRecord(e0, stream);
-	const cudaError_t e = launch_fast_instance<false>(P, qmode, smemBytes, grid, stream);
+	const cudaError_t e = interleaved ? launch_fast_instance<OUT_INTERLEAVED>(P, qmode, smemBytes, grid, stream)
+	                                  : launch_fast_instance<OUT_FASTQ>(P, qmode, smemBytes, grid, stream);
 	if (e != cudaSuccess) return e;
 	if (e1) cudaEventRecord(e1, stream);
 	return cudaSuccess;
@@ -1315,7 +1335,7 @@ cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes
 // Array output: P.out1 = reads of the batch's first pair ([pair][mate][2][P.pitch], 16-byte aligned, pairs * M * 2 * pitch < 2^32),
 // P.rdLength / rdPairId / rdSegment / rdPos / rdFrag at the same first pair, P.nTiles = tickets of FG_CHUNK pairs.
 cudaError_t launch_generate_reads(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream) {
-	return launch_fast_instance<true>(P, qmode, smemBytes, grid, stream);
+	return launch_fast_instance<OUT_ARRAYS>(P, qmode, smemBytes, grid, stream);
 }
 
 // pass 2a alone: blob lengths P.tileState -> offsets P.blobPrefix, totals in P.result->bytes1/2

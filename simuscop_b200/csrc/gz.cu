@@ -8,9 +8,10 @@
 // Bytes absent from the sample still get codes, of 14-15 bits: a later blob full of them (a 64-byte name that is not in
 // the sample, N-run qualities) can code to nearly twice its size.  So, as zlib does, a member whose coded form would be
 // longer than its raw bytes + 23 is written as one stored block instead (gzip header, 0x01, LEN, NLEN, the raw bytes,
-// CRC-32, ISIZE): no member exceeds its blob + 23 bytes (a blob is at most 32 x 612 = 19 584 bytes, its scratch 20 480).
+// CRC-32, ISIZE): no member exceeds its blob + 23 bytes (a blob is at most 32 x 612 = 19 584 bytes, its scratch 20 480; an
+// interleaved blob of both mates at most 39 168, its scratch 40 960: still within the 16-bit LEN of one stored block).
 //
-// Kernel: one warp per (ticket, file).  A round takes 256 bytes (two 32-bit words per lane): LUT -> up to 2 x 60 bits
+// Kernel: one warp per (ticket, file); interleaved output is one file (the second file's jobs have length 0).  A round takes 256 bytes (two 32-bit words per lane): LUT -> up to 2 x 60 bits
 // per lane, warp scan of the bit counts, OR into a shared-memory round buffer (two buffers in turn: the one just
 // written out is zeroed word by word as it is stored), coalesced store of the completed words.  CRC-32 (the gzip
 // trailer) is computed on the fly without a second pass: lane l keeps the pure remainder of its strided word pairs

@@ -342,7 +342,10 @@ __device__ __forceinline__ void copy_out(const uint8_t* sm, int len, uint8_t* g,
 	if (lane < len - t0) g[t0 + lane] = sm[t0 + lane];
 }
 
-template <int NCH, bool K3, bool QSMEM, bool FP64>
+// ILV (interleaved output, PE): mate 2's record goes right behind mate 1's in the warp's first stage buffer, whose neighbour is
+// its second one (2 x STAGE_CAP hold both mates of GEN_PPW pairs), and the one slab P.out1 receives mate 1, mate 2 of every
+// pair in turn; off2, the second length of the look-back and P.out2 stay unused.
+template <int NCH, bool K3, bool QSMEM, bool FP64, bool ILV>
 __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParams P) {
 	extern __shared__ __align__(16) uint8_t smem[];
 	using Cfg = GenCfg<NCH>;
@@ -555,7 +558,7 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 				__syncwarp();
 
 				// ---- record header
-				uint8_t* stage = (mate == 0) ? s_stage1 + off1 : s_stage2 + off2;
+				uint8_t* stage = (mate == 0 || ILV) ? s_stage1 + off1 : s_stage2 + off2;
 				const int H = write_header(stage, P.names + bin.name_off, bin.name_len, posmod, fragCount,
 				                           t.paired ? (mate + 1) : 0, lane);
 				if (lane == 0) { stage[H + m] = '\n'; stage[H + m + 1] = '+'; stage[H + m + 2] = '\n'; stage[H + 2 * m + 3] = '\n'; }
@@ -616,7 +619,7 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 					const int j = c * 32 + lane;
 					if (j < m) { u32x4 blk = draw_block(P.seed, pair, mate, STREAM_CYCLE, 0, (uint32_t)j); emit(j, blk.z, blk.w); }
 				}
-				if (mate == 0) off1 += H + 2 * m + 4; else off2 += H + 2 * m + 4;
+				if (mate == 0 || ILV) off1 += H + 2 * m + 4; else off2 += H + 2 * m + 4;
 				accBases += (unsigned long long)m;
 				accReads += 1;
 				__syncwarp();
@@ -681,7 +684,7 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 				if (lane == 0) atomicOr(&P.result->errorFlags, 1u);
 			} else {
 				copy_out(s_stage1, off1, P.out1 + g1, lane);
-				if (t.paired) copy_out(s_stage2, off2, P.out2 + g2, lane);
+				if (t.paired && !ILV) copy_out(s_stage2, off2, P.out2 + g2, lane);
 			}
 		}
 	}
@@ -701,9 +704,9 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 // ----------------------------------------------------------------------------------------
 // host-side launchers
 // ----------------------------------------------------------------------------------------
-template <int NCH, bool K3, bool QSMEM, bool FP64>
+template <int NCH, bool K3, bool QSMEM, bool FP64, bool ILV>
 static cudaError_t launch_variant(const GenParams& P, int grid, size_t smemBytes, cudaStream_t stream) {
-	auto kern = generate_kernel<NCH, K3, QSMEM, FP64>;
+	auto kern = generate_kernel<NCH, K3, QSMEM, FP64, ILV>;
 	cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemBytes);
 	if (e != cudaSuccess) return e;
 	kern<<<grid, GEN_THREADS, smemBytes, stream>>>(P);
@@ -732,10 +735,15 @@ GenVariant choose_variant(const DevTables& t, bool fp64, int smemLimit) {
 	return v;
 }
 
-cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream) {
-	if (v.fp64) return launch_variant<10, false, false, true>(P, grid, v.smemBytes, stream);
-	if (v.k3) return launch_variant<10, true, false, false>(P, grid, v.smemBytes, stream);
-	return launch_variant<10, false, false, false>(P, grid, v.smemBytes, stream);
+cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream, bool interleaved) {
+	if (interleaved) {
+		if (v.fp64) return launch_variant<10, false, false, true, true>(P, grid, v.smemBytes, stream);
+		if (v.k3) return launch_variant<10, true, false, false, true>(P, grid, v.smemBytes, stream);
+		return launch_variant<10, false, false, false, true>(P, grid, v.smemBytes, stream);
+	}
+	if (v.fp64) return launch_variant<10, false, false, true, false>(P, grid, v.smemBytes, stream);
+	if (v.k3) return launch_variant<10, true, false, false, false>(P, grid, v.smemBytes, stream);
+	return launch_variant<10, false, false, false, false>(P, grid, v.smemBytes, stream);
 }
 
 // ----------------------------------------------------------------------------------------

@@ -35,19 +35,22 @@ struct ssh_job {
 //   * in the modes with mappings the other threads, and a stream thread whose file is finished, copy chunks into a
 //     MAP_SHARED mapping of the slab's file range, back to front, in whichever file has more left.
 // SIMUSCOP_WRITER_MODE = pwrite (streams only) | mmap (mappings only) | hybrid (both; needs more than two threads).
+// A writer on a descriptor the caller opened (ssh_writer_open_fd: standard output, a pipe to an aligner) writes one stream with
+// write() from the caller's thread: a pipe has no offsets for pwrite() and no pages to map.
 // ------------------------------------------------------------------------------------------------
 struct ssh_writer {
 	enum Mode { PWRITE = 0, MMAP = 1, HYBRID = 2 };
 	static const size_t CH = 8u << 20;
 	int fd[2] = {-1, -1};
 	uint64_t off[2] = {0, 0};
+	bool seq = false;             // ssh_writer_open_fd: sequential write() on fd[0], which the writer does not close
 	int nThreads = 1;
 	int mode = PWRITE;
 	std::vector<std::thread> pool;
 	std::mutex mu;
 	std::condition_variable cvWork, cvDone;
 	// the slab of one file in flight: chunks [front, back) are still to be taken
-	struct FileJob { int fd = -1; const char* p = nullptr; size_t len = 0; uint64_t off = 0; char* base = nullptr; size_t front = 0, back = 0; };
+	struct FileJob { int fd = -1; const char* p = nullptr; size_t len = 0; uint64_t off = 0; char* base = nullptr; size_t front = 0, back = 0; bool seq = false; };
 	FileJob job[2];
 	size_t inFlight = 0;
 	bool stop = false, noMap = false;
@@ -65,8 +68,18 @@ struct ssh_writer {
 		}
 		return 0;
 	}
+	// EPIPE when the reader has gone (the process ignores SIGPIPE): the sink fails and the run ends with SSC_ERR_SINK
+	static int write_all(int fd, const char* p, size_t n) {
+		while (n > 0) {
+			ssize_t w = write(fd, p, n);
+			if (w < 0) { if (errno == EINTR) continue; return errno ? errno : EIO; }
+			p += w; n -= (size_t)w;
+		}
+		return 0;
+	}
 	static int put(const FileJob& j, size_t chunk, bool mapped) {
 		const size_t o = chunk * CH, n = std::min(CH, j.len - o);
+		if (j.seq) return write_all(j.fd, j.p + o, n);
 		if (!mapped) return pwrite_all(j.fd, j.p + o, n, j.off + o);
 		char* dst = j.base + o;
 #ifdef MADV_POPULATE_WRITE
@@ -114,12 +127,13 @@ struct ssh_writer {
 	// Both slabs to their files at the running offsets; returns when written.
 	int write_slabs(const char* b1, size_t l1, const char* b2, size_t l2) {
 		std::unique_lock<std::mutex> lk(mu);
+		if (seq && err) return err;   // a stream that failed once (the reader of the pipe has gone) takes no more bytes
 		const char* bufs[2] = {b1, b2}; const size_t lens[2] = {l1, fd[1] >= 0 ? l2 : 0};
 		void* maps[2] = {nullptr, nullptr}; size_t mapLen[2] = {0, 0};
 		for (int f = 0; f < 2; f++) {
 			job[f] = FileJob();
 			if (!lens[f]) continue;
-			job[f].fd = fd[f]; job[f].p = bufs[f]; job[f].len = lens[f]; job[f].off = off[f];
+			job[f].fd = fd[f]; job[f].p = bufs[f]; job[f].len = lens[f]; job[f].off = off[f]; job[f].seq = seq;
 			job[f].back = (lens[f] + CH - 1) / CH;
 			const bool wantMap = !pool.empty() && !noMap && (mode == MMAP || (mode == HYBRID && nThreads > 2));
 			if (wantMap) {
@@ -133,7 +147,7 @@ struct ssh_writer {
 			off[f] += lens[f];
 		}
 		if (!left()) return err;
-		if (pool.empty()) {           // single-threaded: write here
+		if (pool.empty()) {           // single-threaded (and the sequential stream): write here
 			for (int f = 0; f < 2; f++) {
 				for (size_t c = job[f].front; c < job[f].back; c++) { const int e = put(job[f], c, false); if (e && !err) err = e; }
 				job[f] = FileJob();
@@ -277,6 +291,15 @@ int ssh_writer_open(const char* path1, const char* path2, int threads, ssh_write
 	return SSC_OK;
 }
 
+int ssh_writer_open_fd(int fd, ssh_writer** out) {
+	if (fd < 0 || !out) return SSC_ERR_INVALID;
+	ssh_writer* w = new ssh_writer();
+	w->fd[0] = fd;
+	w->seq = true;
+	*out = w;
+	return SSC_OK;
+}
+
 ssc_sink_fn ssh_writer_sink(void) { return writer_sink; }
 
 int ssh_writer_close(ssh_writer* w, uint64_t* bytes1, uint64_t* bytes2) {
@@ -288,7 +311,8 @@ int ssh_writer_close(ssh_writer* w, uint64_t* bytes1, uint64_t* bytes2) {
 	w->cvWork.notify_all();
 	for (auto& t : w->pool) t.join();
 	int rc = w->err ? SSC_ERR_SINK : SSC_OK;
-	for (int f = 0; f < 2; f++) if (w->fd[f] >= 0 && close(w->fd[f]) != 0) rc = SSC_ERR_SINK;
+	if (!w->seq)
+		for (int f = 0; f < 2; f++) if (w->fd[f] >= 0 && close(w->fd[f]) != 0) rc = SSC_ERR_SINK;
 	if (bytes1) *bytes1 = w->off[0];
 	if (bytes2) *bytes2 = w->off[1];
 	delete w;
@@ -315,6 +339,18 @@ int ssh_run(ssh_job* job, int device) {
 		for (const std::string& t : sschost::split(dl, ',')) if (!sschost::trim(t).empty()) devIds.push_back(atoi(t.c_str()));
 	}
 	if (devIds.empty()) devIds.push_back(device);
+	sschost::Job& J = job->job;
+	// SIMUSCOP_STDOUT=1: the reads of the one sample go to standard output (PE interleaved) and no FASTQ file is written;
+	// SIMUSCOP_INTERLEAVE=1: a PE sample is written to <output>/<stem>.fq[.gz], mate 1 and mate 2 of each pair in turn
+	const char* soEnv = getenv("SIMUSCOP_STDOUT");
+	const bool toStdout = soEnv && atoi(soEnv) != 0;
+	const char* ilEnv = getenv("SIMUSCOP_INTERLEAVE");
+	const bool interleave = J.cfg.paired() && (toStdout || (ilEnv && atoi(ilEnv) != 0));
+	if (toStdout && J.samples.size() > 1) {
+		std::cerr << "Error: SIMUSCOP_STDOUT=1 writes one sample, this configuration yields " << J.samples.size()
+		          << " (one per row of the abundance file); write them to files instead" << std::endl;
+		return 1;
+	}
 	std::vector<ssc_handle*> devs;
 	int rc = 0;
 	for (int id : devIds) {
@@ -329,14 +365,15 @@ int ssh_run(ssh_job* job, int device) {
 	const char* gzEnv = getenv("SIMUSCOP_GZIP");
 	const bool gz = gzEnv && atoi(gzEnv) != 0;
 	if (gz) for (auto* d : devs) ssc_set_option(d, "gzip", 1);
-	sschost::Job& J = job->job;
+	if (interleave) for (auto* d : devs) ssc_set_option(d, "interleave", 1);
 	const int G = (int)devs.size();
 	for (int s = 0; s < (int)J.samples.size() && !rc; s++) {
 		const std::string prefix = J.cfg.str["output"] + "/" + J.samples[s].stem;
 		const bool paired = J.cfg.paired();
 		const std::string ext = gz ? ".fq.gz" : ".fq";
-		const std::string f1 = paired ? prefix + "_1" + ext : prefix + ext;
-		const std::string f2 = paired ? prefix + "_2" + ext : "";
+		const bool twoFiles = paired && !interleave;
+		const std::string f1 = toStdout ? "<standard output>" : (twoFiles ? prefix + "_1" + ext : prefix + ext);
+		const std::string f2 = twoFiles ? prefix + "_2" + ext : "";
 		std::string dump;
 		if (dumpPrefix) dump = std::string(dumpPrefix) + "." + std::to_string(s) + ".plan";
 		int64_t planned = 0, emitted = 0;
@@ -351,7 +388,7 @@ int ssh_run(ssh_job* job, int device) {
 		ssh_writer* w = nullptr;
 		int wthreads = 4;
 		if (const char* wt = getenv("SIMUSCOP_WRITER_THREADS")) wthreads = atoi(wt);
-		if (ssh_writer_open(f1.c_str(), paired ? f2.c_str() : nullptr, wthreads, &w))
+		if (toStdout ? ssh_writer_open_fd(1, &w) : ssh_writer_open(f1.c_str(), twoFiles ? f2.c_str() : nullptr, wthreads, &w))
 			sschost::die(-1, "Error: can not open fastq file to save results:\n" + f1);
 		if (G == 1) {
 			rc = ssc_generate(devs[0], 0, planned, writer_sink, w);

@@ -1,7 +1,11 @@
 // main.cpp -- drop-in `simuReads <configuration file>` (reference src/simuReads.cpp:24-97).
 // New knobs come from the environment only, so existing configuration files stay valid:
 //   SIMUSCOP_SEED (default: wall clock, like the reference), SIMUSCOP_DEVICE (default 0),
-//   SIMUSCOP_DUMP_PLAN=<prefix>, SIMUSCOP_BATCH_PAIRS, SIMUSCOP_GZIP=1 (<name>.fq.gz, compressed on the GPU).
+//   SIMUSCOP_DUMP_PLAN=<prefix>, SIMUSCOP_BATCH_PAIRS, SIMUSCOP_GZIP=1 (<name>.fq.gz, compressed on the GPU),
+//   SIMUSCOP_INTERLEAVE=1 (PE: one <name>.fq, mates in turn), SIMUSCOP_STDOUT=1 (the reads to standard output, e.g.
+//   `simuReads config | bwa mem -p ref.fa -`).  Every message goes to stderr, so stdout carries FASTQ bytes only.
+#include <signal.h>
+
 #include <chrono>
 #include <cstdlib>
 #include <ctime>
@@ -22,6 +26,10 @@ int main(int argc, char* argv[]) {
 	const char* s = getenv("SIMUSCOP_SEED");
 	uint64_t seed = s ? strtoull(s, NULL, 10) : (uint64_t)std::chrono::system_clock::now().time_since_epoch().count();
 	const char* d = getenv("SIMUSCOP_DEVICE");
+	// a reader that closes the pipe early makes the next write fail with EPIPE instead of killing the process: the run ends
+	// with an error message and exit code 1
+	const char* so = getenv("SIMUSCOP_STDOUT");
+	if (so && atoi(so) != 0) signal(SIGPIPE, SIG_IGN);
 	ssh_job* job = nullptr;
 	if (ssh_open(argv[1], seed, &job)) return 1;
 	int rc = ssh_run(job, d ? atoi(d) : 0);
