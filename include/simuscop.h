@@ -121,7 +121,7 @@ typedef struct ssc_stats {
 	double   gen_kernel_ms;    /* CUDA-event time of the generation kernel alone (ssc_generate_device) */
 	double   compact_kernel_ms;/* CUDA-event time of the compaction kernel alone (ssc_generate_device) */
 	uint64_t timed_batches;    /* launches covered by gen_kernel_ms */
-	uint64_t gz_bytes;         /* gzip mode: compressed bytes written to the slabs (fastq_bytes stays the plain size) */
+	uint64_t gz_bytes;         /* gzip mode: compressed bytes written to the slabs, BGZF blocks with "bgzf" (fastq_bytes stays the plain size) */
 	uint64_t bin_bytes;        /* algorithmic bin-record bytes read: 64 bytes per distinct bin of every generated batch */
 	double   mover_kernel_ms;  /* CUDA-event time of the concurrent blob mover (concurrent_move > 0) on its own stream, under the
 	                              generation kernel of the next batch (ssc_generate_device) */
@@ -155,7 +155,14 @@ int ssc_destroy(ssc_handle* h);
  * handed to the sink hold concatenated gzip members -- a valid .gz stream of the same FASTQ bytes -- compressed on
  * the GPU, one member per 32 pairs, Huffman-coded with a table fitted to the first batch, or stored where that code would
  * expand the member past its bytes + 23, so gzip mode fails only where plain output does; the plain bytes of
- * SeqWriter::write are the default), "interleave" (0/1: a PE plan writes ONE stream, pair i mate 1 then pair i mate 2 in pair
+ * SeqWriter::write are the default), "bgzf" (0/1, default 0; no effect without gzip: every gzip member is written as a BGZF
+ * block -- FLG = FEXTRA and the 8 bytes 06 00 'B' 'C' 02 00 BSIZE(2, = block length - 1) after the 10-byte header, the
+ * DEFLATE data unchanged, a stored block raw + 31 bytes -- so bgzip, samtools and other htslib readers can decompress in
+ * parallel and seek.  A block holds the records of 32 pairs (interleaved: of both mates), at most 39 199 bytes; in PE output
+ * block k of file 1 and block k of file 2 hold the same pairs.  The slabs and ssc_generate_device hold whole blocks, gz_bytes
+ * counts them.  The library does not write the 28-byte BGZF end-of-file block, since it cannot know which call is the last:
+ * the writer appends 1f 8b 08 04 00 00 00 00 00 ff 06 00 42 43 02 00 1b 00 03 00 00 00 00 00 00 00 00 00 (ssh_writer_bgzf
+ * does it).  Like gzip it may be set between calls and takes effect at the next one), "interleave" (0/1: a PE plan writes ONE stream, pair i mate 1 then pair i mate 2 in pair
  * order, byte for byte the interleave of the _1 / _2 records without the option, "/1" and "/2" suffixes included -- what
  * `bwa mem -p` and `bowtie2 --interleaved` read; the sink gets it as buf1/len1 with buf2 == NULL, len2 == 0,
  * ssc_generate_device returns it in *bytes1 with *bytes2 = 0, ssc_stats counts the same fastq_bytes / gz_bytes totals; with

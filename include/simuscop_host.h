@@ -59,13 +59,24 @@ int ssh_writer_open(const char* path1, const char* path2, int threads, ssh_write
  * written in order with write() from the calling thread, so descriptors that cannot seek work.  buf2 must be NULL (SE or
  * interleaved PE).  A failed write (EPIPE once the reader has gone, with SIGPIPE ignored) makes the sink return non-zero. */
 int ssh_writer_open_fd(int fd, ssh_writer** out);
+/* BGZF output (the handles' "gzip" and "bgzf" options): call after ssh_writer_open / ssh_writer_open_fd and before the first
+ * slab.  From then on every slab must be a whole number of well-formed BGZF blocks (else the sink returns non-zero, takes no
+ * more slabs, and ssh_writer_close reports SSC_ERR_SINK); ssh_writer_close appends the 28-byte BGZF EOF block to each stream
+ * (also on a descriptor) unless a write failed.  index1 / index2 (either may be NULL; index2 needs a second file): a .gzi block
+ * index of stream 1 / 2 in the layout of htslib's bgzf_index_dump -- uint64 entry count, then one (compressed offset,
+ * uncompressed offset) uint64 pair per data block after the first (block 0 at (0, 0) is implicit, the EOF block has none), all
+ * little-endian.  Entries are written as the slabs arrive and the count at close: 16 bytes per block of 32 pairs, ~150 MB per
+ * file of a 3 Gb x 30x PE run.  Returns SSC_ERR_STATE after the first slab or a second call, SSC_ERR_SINK when an index
+ * cannot be created. */
+int ssh_writer_bgzf(ssh_writer* w, const char* index1, const char* index2);
 ssc_sink_fn ssh_writer_sink(void);
 int ssh_writer_close(ssh_writer* w, uint64_t* bytes1, uint64_t* bytes2);
 
 /* The whole drop-in run: every sample -> FASTQ files in the output directory, on `device`.  Environment:
  * SIMUSCOP_INTERLEAVE=1 writes a PE sample to <output>/<stem>.fq (.fq.gz with SIMUSCOP_GZIP=1), mate 1 and mate 2 of each pair
  * in turn, instead of <stem>_1 / <stem>_2; SIMUSCOP_STDOUT=1 writes the reads (PE interleaved) to standard output and no
- * FASTQ file, and refuses a configuration with more than one sample. */
+ * FASTQ file, and refuses a configuration with more than one sample; SIMUSCOP_BGZF=1 (implies SIMUSCOP_GZIP=1) writes every
+ * .fq.gz as BGZF, ended by the EOF block, with its block index <name>.fq.gz.gzi beside it (standard output: no index). */
 int ssh_run(ssh_job* job, int device);
 
 #ifdef __cplusplus

@@ -87,10 +87,11 @@ struct ssc_handle {
 	cudaEvent_t evResult[2] = {nullptr, nullptr};    // batch of buffer set b: its BatchResult in h_result[b]
 	int fastQmode = -1;           // "fast_qmode": -1 automatic, else the only quality-table mode the fast kernel may use (tests)
 	bool gzip = false;            // slabs hold gzip members (one per ticket blob) instead of plain FASTQ
+	bool bgzf = false;            // "bgzf": with gzip, every member is a BGZF block (no effect without gzip)
 	bool interleave = false;      // "interleave": a PE plan's mates go to one stream, mate 1 and mate 2 of each pair in turn
 	size_t gzBlobBytes = 0;       // allocation of d_gzBlobs[0] (interleaved: both mates per ticket)
 	bool haveGz = false;          // Huffman / CRC tables of the current plan are on the device
-	ssc::GzTables* d_gzTab = nullptr;
+	ssc::GzTables* d_gzTab = nullptr;   // [0] gzip members, [1] BGZF blocks: one Huffman table, two member headers
 	uint8_t* d_gzBlobs[2] = {nullptr, nullptr};
 	DevBuf<unsigned long long> d_gzLens;
 
@@ -201,12 +202,13 @@ int out_files(const ssc_handle* h) { return h->dt.paired && !h->interleave ? 2 :
 int ensure_batch_resources(ssc_handle* h, bool needHost) {
 	int64_t pairs = std::min<int64_t>(h->batchPairs, std::max<int64_t>(h->emittedPairs, 1));
 	pairs = ((pairs + GEN_TILE_PAIRS - 1) / GEN_TILE_PAIRS) * GEN_TILE_PAIRS;   // multiple of both tile sizes
-	// gzip mode: a member is at most its blob plus the bytes of a stored block (gz.cu), and there is one member per ticket.
-	// Interleaved output: a slab holds both mates of a pair.  The scan packs a slab length into 31 bits, so the slab bound stays
-	// below 2^31 in every mode.
+	// gzip mode: a member is at most its blob plus the bytes of a stored block (gz.cu: 23, a BGZF block 31), and there is one
+	// member per ticket.  Interleaved output: a slab holds both mates of a pair.  The scan packs a slab length into 31 bits, so
+	// the slab bound stays below 2^31 in every mode: the clamp budgets the stored-block bytes as ceil(extra / 32) = 1 per pair.
 	const uint64_t recBytes = (uint64_t)h->maxRecBytes * (interleaved(h) ? 2u : 1u);
-	const uint64_t perPair = recBytes + (h->gzip ? 1 : 0);
-	auto slab_cap = [&](int64_t n) { return (uint64_t)n * recBytes + 4096 + (h->gzip ? (uint64_t)(n / FG_CHUNK) * ssc::GZ_STORED_EXTRA : 0); };
+	const uint64_t gzExtra = h->gzip ? (uint64_t)(h->bgzf ? ssc::GZ_BGZF_STORED_EXTRA : ssc::GZ_STORED_EXTRA) : 0;
+	const uint64_t perPair = recBytes + (gzExtra + FG_CHUNK - 1) / FG_CHUNK;
+	auto slab_cap = [&](int64_t n) { return (uint64_t)n * recBytes + 4096 + (uint64_t)(n / FG_CHUNK) * gzExtra; };
 	uint64_t cap = slab_cap(pairs);
 	if (cap >= (1ull << 31)) {
 		pairs = (int64_t)(((1ull << 31) - 8192) / perPair);
@@ -251,7 +253,9 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 		}
 		h->slabPairs = pairs; h->slabCap = cap; h->slabFiles = slabFiles;
 	}
-	// gzip members: one per ticket blob, at the blob's pitch (interleaved: twice the per-file pitch, one file)
+	// gzip members: one per ticket blob, at the blob's pitch (interleaved: twice the per-file pitch, one file).  A BGZF block is
+	// at most 19 584 + 31 bytes (interleaved 39 168 + 31) in a pitch of 20 480 (40 960)
+	static_assert(FG_SLOT * FG_CHUNK >= 19584 + ssc::GZ_BGZF_STORED_EXTRA, "a BGZF block fits its ticket's member pitch");
 	const size_t gzBytes = (size_t)h->slabPairs * FG_SLOT * (interleaved(h) ? 2 : 1) + 64;
 	if (h->gzip && h->gzBlobBytes != gzBytes) {
 		for (int f = 0; f < 2; f++) { if (h->d_gzBlobs[f]) cudaFree(h->d_gzBlobs[f]); h->d_gzBlobs[f] = nullptr; }
@@ -259,7 +263,7 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 		for (int f = 0; f < (interleaved(h) ? 1 : 2); f++) CK(cudaMalloc((void**)&h->d_gzBlobs[f], gzBytes));
 		h->gzBlobBytes = gzBytes;
 		CK(h->d_gzLens.alloc((size_t)(h->slabPairs / 16) + 2));
-		if (!h->d_gzTab) CK(cudaMalloc((void**)&h->d_gzTab, sizeof(ssc::GzTables)));
+		if (!h->d_gzTab) CK(cudaMalloc((void**)&h->d_gzTab, 2 * sizeof(ssc::GzTables)));
 	}
 	if (needHost)
 		for (int b = 0; b < 2; b++)
@@ -296,11 +300,15 @@ int build_gz_tables(ssc_handle* h, const ssc::GenParams& P, int nTiles) {
 			for (size_t i = 0; i < n; i++) hist[p[i]]++;
 		}
 	}
-	ssc::GzTables tab;
-	const char* err = ssc::gz_build_tables(hist, &tab);
-	if (err[0]) return fail(SSC_ERR_INVALID, "gzip tables: %s", err);
-	CK(cudaMemcpyAsync(h->d_gzTab, &tab, sizeof(tab), cudaMemcpyHostToDevice, h->compute));   // stream order with the deflate kernel
-	CK(cudaStreamSynchronize(h->compute));          // tab lives on this stack frame
+	// the gzip and the BGZF tables from the one fit, so that "bgzf" may change between calls and each block is its gzip member
+	// with the BC field inserted
+	std::vector<ssc::GzTables> tab(2);
+	for (int b = 0; b < 2; b++) {
+		const char* err = ssc::gz_build_tables(hist, &tab[b], b == 1);
+		if (err[0]) return fail(SSC_ERR_INVALID, "gzip tables: %s", err);
+	}
+	CK(cudaMemcpyAsync(h->d_gzTab, tab.data(), 2 * sizeof(ssc::GzTables), cudaMemcpyHostToDevice, h->compute));   // stream order with the deflate kernel
+	CK(cudaStreamSynchronize(h->compute));          // tab is freed on return
 	h->haveGz = true;
 	return SSC_OK;
 }
@@ -457,7 +465,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 			if (!h->haveGz) { rc = build_gz_tables(h, P, nTiles); if (rc) return rc; }
 			CK(cudaMemsetAsync(h->d_gzLens.p, 0, sizeof(unsigned long long) * nTiles, s));
 			CK(ssc::launch_deflate_blobs(P.out1, P.out2, P.tileState, nTiles, P.blobPitch, h->d_gzBlobs[0], h->d_gzBlobs[1], h->d_gzLens.p,
-			                             P.blobPitch, h->d_gzTab, h->smCount, s));
+			                             P.blobPitch, h->d_gzTab + (h->bgzf ? 1 : 0), h->smCount, s));
 			ssc::GenParams P2 = P;
 			P2.out1 = h->d_gzBlobs[0]; P2.out2 = h->d_gzBlobs[1]; P2.tileState = h->d_gzLens.p; P2.blobPitch = P.blobPitch;
 			CK(ssc::launch_pass2(P2, h->smCount, s));
@@ -629,6 +637,7 @@ int ssc_set_option(ssc_handle* h, const char* key, int64_t value) {
 		return SSC_OK;
 	}
 	if (!strcmp(key, "gzip")) { h->gzip = value != 0; return SSC_OK; }
+	if (!strcmp(key, "bgzf")) { h->bgzf = value != 0; return SSC_OK; }        // takes effect with gzip, at the next call
 	if (!strcmp(key, "interleave")) { h->interleave = value != 0; return SSC_OK; }   // slabs re-sized at the next call if they must
 	if (!strcmp(key, "concurrent_move")) {
 		if (value < 0 || value > 64) return fail(SSC_ERR_INVALID, "concurrent_move: 0 (off) .. 64 SMs");

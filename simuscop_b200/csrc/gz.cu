@@ -10,6 +10,9 @@
 // longer than its raw bytes + 23 is written as one stored block instead (gzip header, 0x01, LEN, NLEN, the raw bytes,
 // CRC-32, ISIZE): no member exceeds its blob + 23 bytes (a blob is at most 32 x 612 = 19 584 bytes, its scratch 20 480; an
 // interleaved blob of both mates at most 39 168, its scratch 40 960: still within the 16-bit LEN of one stored block).
+// BGZF (the "bgzf" option, DESIGN 13): the same member with FLG = FEXTRA and the 8-byte BC field after the 10-byte header, so
+// the tables carry an 18-byte header in the prefix and the DEFLATE bits follow 64 bits later; the warp writes BSIZE (member
+// length - 1) once the length is known.  A stored member is then raw + 31 bytes, and no block exceeds 39 199 bytes (< 65 536).
 //
 // Kernel: one warp per (ticket, file); interleaved output is one file (the second file's jobs have length 0).  A round takes 256 bytes (two 32-bit words per lane): LUT -> up to 2 x 60 bits
 // per lane, warp scan of the bit counts, OR into a shared-memory round buffer (two buffers in turn: the one just
@@ -141,7 +144,7 @@ struct BitWriter {
 
 }  // namespace
 
-const char* gz_build_tables(const uint64_t hist[256], GzTables* t) {
+const char* gz_build_tables(const uint64_t hist[256], GzTables* t, bool bgzf) {
 	memset(t, 0, sizeof(*t));
 	// ---- literal/length code: all 256 byte values stay encodable (a population name may hold any byte), + end of block
 	std::vector<uint64_t> freq(257);
@@ -155,8 +158,11 @@ const char* gz_build_tables(const uint64_t hist[256], GzTables* t) {
 
 	// ---- gzip member header (RFC 1952) + dynamic block header (RFC 1951 3.2.7)
 	BitWriter bw;
-	const uint8_t gzh[10] = {0x1f, 0x8b, 8, 0, 0, 0, 0, 0, 0, 0xff};
-	for (int i = 0; i < 10; i++) bw.put(gzh[i], 8);
+	// BGZF: FLG = FEXTRA and the 8-byte extra field (XLEN 6, SI1 'B', SI2 'C', SLEN 2, BSIZE) after the 10 bytes; the encoder
+	// writes BSIZE (block length - 1) once it knows the length
+	const uint8_t gzh[18] = {0x1f, 0x8b, 8, (uint8_t)(bgzf ? 4 : 0), 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, 0, 0};
+	t->headerBytes = bgzf ? 18 : 10;
+	for (uint32_t i = 0; i < t->headerBytes; i++) bw.put(gzh[i], 8);
 	bw.put(1, 1);                          // BFINAL
 	bw.put(2, 2);                          // BTYPE = dynamic Huffman
 	// code length sequence: 257 literal/length lengths + 2 distance lengths of 1 (never used: the block is all literals;
@@ -219,6 +225,9 @@ const char* gz_build_tables(const uint64_t hist[256], GzTables* t) {
 // without a GPU, and the kernel's members byte for byte.  Returns the member size, or 0 when it does not fit cap.
 size_t gz_member_host(const GzTables* t, const uint8_t* src, uint32_t len, uint8_t* dst, size_t cap) {
 	if (len == 0 || len > 0xFFFFu) return 0;
+	const uint32_t hb = t->headerBytes;                   // 10, or 18 for a BGZF block
+	const size_t storedExtra = hb + 13;                   // GZ_STORED_EXTRA or GZ_BGZF_STORED_EXTRA
+	if (hb > 10 && (size_t)len + storedExtra > (size_t)GZ_BGZF_MAX_BLOCK) return 0;   // a block might not fit its 16-bit BSIZE
 	std::vector<uint32_t> out(t->prefix, t->prefix + ((t->prefixBits + 31) >> 5));
 	uint64_t bits = t->prefixBits;
 	auto put = [&](uint64_t v, uint32_t n) {
@@ -250,18 +259,20 @@ size_t gz_member_host(const GzTables* t, const uint8_t* src, uint32_t len, uint8
 	put(t->lut[256] & 0xffffu, t->lut[256] >> 16);
 	while (bits & 7) put(0, 1);
 	put(crc, 32); put(len, 32);
-	const size_t n = (size_t)(bits >> 3);
-	if (n > (size_t)len + GZ_STORED_EXTRA) {              // coding would expand the blob: one stored block
-		if ((size_t)len + GZ_STORED_EXTRA > cap) return 0;
-		memcpy(dst, out.data(), 10);                      // the gzip header of the coded form
+	size_t n = (size_t)(bits >> 3);
+	if (n > (size_t)len + storedExtra) {                  // coding would expand the blob: one stored block
+		if ((size_t)len + storedExtra > cap) return 0;
+		memcpy(dst, out.data(), hb);                      // the gzip header of the coded form
 		const uint8_t blk[5] = {0x01, (uint8_t)len, (uint8_t)(len >> 8), (uint8_t)~len, (uint8_t)(~len >> 8)};
-		memcpy(dst + 10, blk, 5);
-		memcpy(dst + 15, src, len);
-		for (int k = 0; k < 4; k++) { dst[15 + len + k] = (uint8_t)(crc >> (8 * k)); dst[19 + len + k] = (uint8_t)(len >> (8 * k)); }
-		return (size_t)len + GZ_STORED_EXTRA;
+		memcpy(dst + hb, blk, 5);
+		memcpy(dst + hb + 5, src, len);
+		for (int k = 0; k < 4; k++) { dst[hb + 5 + len + k] = (uint8_t)(crc >> (8 * k)); dst[hb + 9 + len + k] = (uint8_t)(len >> (8 * k)); }
+		n = (size_t)len + storedExtra;
+	} else {
+		if (n > cap) return 0;
+		memcpy(dst, out.data(), n);
 	}
-	if (n > cap) return 0;
-	memcpy(dst, out.data(), n);
+	if (hb > 10) { dst[16] = (uint8_t)(n - 1); dst[17] = (uint8_t)((n - 1) >> 8); }   // BSIZE
 	return n;
 }
 
@@ -312,6 +323,8 @@ __global__ void __launch_bounds__(GZ_WARPS * 32) deflate_blobs_kernel(const uint
 	uint32_t* rbA = s_rb[warp][0];              // buffer of the current round: all zero except its first word (the carry)
 	uint32_t* rbB = s_rb[warp][1];              // all zero
 	const uint32_t prefixBits = tab->prefixBits;
+	const uint32_t hdrBytes = tab->headerBytes;          // 10, or 18 for a BGZF block
+	const uint32_t storedExtra = hdrBytes + 13u;         // GZ_STORED_EXTRA or GZ_BGZF_STORED_EXTRA
 	const int nWarps = gridDim.x * GZ_WARPS;
 	auto crc_step = [&](uint32_t c) { return s_T[3][c & 0xff] ^ s_T[2][(c >> 8) & 0xff] ^ s_T[1][(c >> 16) & 0xff] ^ s_T[0][c >> 24]; };
 	for (int job = blockIdx.x * GZ_WARPS + warp; job < 2 * nTiles; job += nWarps) {
@@ -404,20 +417,27 @@ __global__ void __launch_bounds__(GZ_WARPS * 32) deflate_blobs_kernel(const uint
 			for (uint32_t i = lane; i < nw; i += 32) { if (outWords + i < pitchWords) dst32[outWords + i] = rbA[i]; rbA[i] = 0u; }
 			outBytes = outWords * 4u + (totalBits >> 3);
 			__syncwarp();
-			if (outBytes > len + (uint32_t)GZ_STORED_EXTRA) {
+			if (outBytes > len + storedExtra) {
 				// coding would expand the blob (bytes the table was not fitted to): one stored block, as gz_member_host
 				uint8_t* dst8 = (uint8_t*)dst32;
-				for (uint32_t i = lane; i < len + (uint32_t)GZ_STORED_EXTRA; i += 32) {
+				const uint32_t h = hdrBytes;
+				for (uint32_t i = lane; i < len + storedExtra; i += 32) {
 					uint32_t b;
-					if (i < 10u) b = s_prefix[i >> 2] >> (8u * (i & 3u));                        // the gzip header of the coded form
-					else if (i == 10u) b = 1u;                                                  // BFINAL, BTYPE = stored
-					else if (i < 15u) b = (i < 13u ? len : ~len) >> (8u * ((i - 11u) & 1u));   // LEN, NLEN
-					else if (i < 15u + len) b = src8[i - 15u];
-					else b = (i < 19u + len ? crc : len) >> (8u * ((i - 15u - len) & 3u));      // CRC-32, ISIZE
+					if (i < h) b = s_prefix[i >> 2] >> (8u * (i & 3u));                              // the gzip header of the coded form
+					else if (i == h) b = 1u;                                                      // BFINAL, BTYPE = stored
+					else if (i < h + 5u) b = (i < h + 3u ? len : ~len) >> (8u * ((i - h - 1u) & 1u));   // LEN, NLEN
+					else if (i < h + 5u + len) b = src8[i - h - 5u];
+					else b = (i < h + 9u + len ? crc : len) >> (8u * ((i - h - 5u - len) & 3u));  // CRC-32, ISIZE
 					dst8[i] = (uint8_t)b;
 				}
-				outBytes = len + (uint32_t)GZ_STORED_EXTRA;
+				outBytes = len + storedExtra;
 				__syncwarp();
+			}
+			if (hdrBytes > 10u && lane == 0) {
+				// BGZF: BSIZE = block length - 1, over the 0 of the prefix (its word was stored before the last __syncwarp)
+				uint8_t* dst8 = (uint8_t*)dst32;
+				dst8[16] = (uint8_t)(outBytes - 1u);
+				dst8[17] = (uint8_t)((outBytes - 1u) >> 8);
 			}
 		}
 		if (lane == 0) {

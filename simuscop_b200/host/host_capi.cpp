@@ -59,6 +59,15 @@ struct ssh_writer {
 	// batch before it has been
 	int64_t turn = 0;
 	std::condition_variable cvTurn;
+	// ssh_writer_bgzf: every slab is whole BGZF blocks.  Their starts go to a .gzi per stream as the slabs arrive (the layout of
+	// htslib's bgzf_index_dump: uint64 count, then (compressed, uncompressed) offset pairs of every block after the first, all
+	// little-endian; the count is patched at close), and the EOF block is appended at close
+	bool bgzf = false;
+	int gzi[2] = {-1, -1};
+	uint64_t gziEntries[2] = {0, 0};
+	uint64_t blocks[2] = {0, 0};      // data blocks so far
+	uint64_t uoff[2] = {0, 0};        // uncompressed bytes so far (the running sum of ISIZE)
+	static constexpr uint8_t BGZF_EOF[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
 
 	static int pwrite_all(int fd, const char* p, size_t n, uint64_t off) {
 		while (n > 0) {
@@ -91,6 +100,60 @@ struct ssh_writer {
 #endif
 		memcpy(dst, j.p + o, n);
 		return 0;
+	}
+	static void put_le64(std::vector<uint8_t>& v, uint64_t x) { for (int k = 0; k < 8; k++) v.push_back((uint8_t)(x >> (8 * k))); }
+	// Walks the BGZF blocks of a slab of stream f that starts at compressed offset off[f]: the index entries of the blocks in *e
+	// and the stream's counts after it in *nb / *u.  EINVAL unless the slab is a whole number of well-formed blocks (the header
+	// checks of htslib's reader, a BSIZE within the slab, at least the 28 bytes of an empty block, ISIZE <= 64 KiB).
+	int walk_bgzf(int f, const char* p, size_t n, std::vector<uint8_t>* e, uint64_t* nb, uint64_t* u) const {
+		*nb = blocks[f]; *u = uoff[f];
+		uint64_t c = off[f];
+		for (size_t at = 0; at < n;) {
+			const uint8_t* b = (const uint8_t*)p + at;
+			if (n - at < 18 || b[0] != 0x1f || b[1] != 0x8b || b[2] != 8 || !(b[3] & 4) || b[10] != 6 || b[11] != 0 || b[12] != 'B' ||
+			    b[13] != 'C' || b[14] != 2 || b[15] != 0)
+				return EINVAL;
+			const size_t bs = (size_t)(b[16] | b[17] << 8) + 1;
+			if (bs < 28 || bs > n - at) return EINVAL;
+			const uint32_t isize = b[bs - 4] | b[bs - 3] << 8 | b[bs - 2] << 16 | (uint32_t)b[bs - 1] << 24;
+			if (isize > 65536) return EINVAL;
+			if (*nb > 0 && gzi[f] >= 0) { put_le64(*e, c); put_le64(*e, *u); }   // block 0 at (0, 0) has no entry
+			++*nb; c += bs; *u += isize; at += bs;
+		}
+		return 0;
+	}
+	// The index entries of both slabs of a write_slabs call, or EINVAL (and nothing written) if either is not BGZF blocks.
+	int index_slabs(const char* const* bufs, const size_t* lens) {
+		std::vector<uint8_t> e[2];
+		uint64_t nb[2], u[2];
+		for (int f = 0; f < 2; f++) {
+			const int r = walk_bgzf(f, bufs[f], lens[f], &e[f], &nb[f], &u[f]);
+			if (r) return r;
+		}
+		for (int f = 0; f < 2; f++) {
+			if (!e[f].empty()) {
+				const int r = pwrite_all(gzi[f], (const char*)e[f].data(), e[f].size(), 8 + gziEntries[f] * 16);
+				if (r) return r;
+				gziEntries[f] += e[f].size() / 16;
+			}
+			blocks[f] = nb[f]; uoff[f] = u[f];
+		}
+		return 0;
+	}
+	// close: the EOF block behind each stream, and the entry count at the head of each index
+	int finish_bgzf() {
+		int r = 0;
+		for (int f = 0; f < 2 && !r; f++) {
+			if (fd[f] < 0) continue;
+			r = seq ? write_all(fd[f], (const char*)BGZF_EOF, 28) : pwrite_all(fd[f], (const char*)BGZF_EOF, 28, off[f]);
+			if (!r) off[f] += 28;
+			if (!r && gzi[f] >= 0) {
+				std::vector<uint8_t> cnt;
+				put_le64(cnt, gziEntries[f]);
+				r = pwrite_all(gzi[f], (const char*)cnt.data(), 8, 0);
+			}
+		}
+		return r;
 	}
 	bool left() const { return job[0].front < job[0].back || job[1].front < job[1].back; }
 	// the next chunk for pool thread `id` (called with mu held): false when there is nothing this thread may take
@@ -127,8 +190,14 @@ struct ssh_writer {
 	// Both slabs to their files at the running offsets; returns when written.
 	int write_slabs(const char* b1, size_t l1, const char* b2, size_t l2) {
 		std::unique_lock<std::mutex> lk(mu);
-		if (seq && err) return err;   // a stream that failed once (the reader of the pipe has gone) takes no more bytes
+		// a stream that failed once (the reader of the pipe has gone) takes no more bytes; nor does a BGZF stream (its index
+		// would no longer match the file)
+		if ((seq || bgzf) && err) return err;
 		const char* bufs[2] = {b1, b2}; const size_t lens[2] = {l1, fd[1] >= 0 ? l2 : 0};
+		if (bgzf) {
+			const int e = index_slabs(bufs, lens);
+			if (e) { if (!err) err = e; return err; }
+		}
 		void* maps[2] = {nullptr, nullptr}; size_t mapLen[2] = {0, 0};
 		for (int f = 0; f < 2; f++) {
 			job[f] = FileJob();
@@ -300,6 +369,24 @@ int ssh_writer_open_fd(int fd, ssh_writer** out) {
 	return SSC_OK;
 }
 
+int ssh_writer_bgzf(ssh_writer* w, const char* index1, const char* index2) {
+	if (!w) return SSC_ERR_INVALID;
+	if (w->bgzf || w->off[0] || w->off[1]) return SSC_ERR_STATE;
+	if (index2 && w->fd[1] < 0) return SSC_ERR_INVALID;
+	const char* idx[2] = {index1, index2};
+	for (int f = 0; f < 2; f++) {
+		if (!idx[f]) continue;
+		const uint8_t zero[8] = {0, 0, 0, 0, 0, 0, 0, 0};         // the entry count, patched at close
+		w->gzi[f] = open(idx[f], O_WRONLY | O_CREAT | O_TRUNC, 0644);
+		if (w->gzi[f] < 0 || ssh_writer::pwrite_all(w->gzi[f], (const char*)zero, 8, 0)) {
+			for (int k = 0; k <= f; k++) if (w->gzi[k] >= 0) { close(w->gzi[k]); w->gzi[k] = -1; }
+			return SSC_ERR_SINK;
+		}
+	}
+	w->bgzf = true;
+	return SSC_OK;
+}
+
 ssc_sink_fn ssh_writer_sink(void) { return writer_sink; }
 
 int ssh_writer_close(ssh_writer* w, uint64_t* bytes1, uint64_t* bytes2) {
@@ -310,7 +397,10 @@ int ssh_writer_close(ssh_writer* w, uint64_t* bytes1, uint64_t* bytes2) {
 	}
 	w->cvWork.notify_all();
 	for (auto& t : w->pool) t.join();
+	// a BGZF stream that failed gets no EOF block: a reader then sees it is truncated
+	if (w->bgzf && !w->err) w->err = w->finish_bgzf();
 	int rc = w->err ? SSC_ERR_SINK : SSC_OK;
+	for (int f = 0; f < 2; f++) if (w->gzi[f] >= 0 && close(w->gzi[f]) != 0) rc = SSC_ERR_SINK;
 	if (!w->seq)
 		for (int f = 0; f < 2; f++) if (w->fd[f] >= 0 && close(w->fd[f]) != 0) rc = SSC_ERR_SINK;
 	if (bytes1) *bytes1 = w->off[0];
@@ -362,9 +452,14 @@ int ssh_run(ssh_job* job, int device) {
 	const char* dumpPrefix = getenv("SIMUSCOP_DUMP_PLAN");
 	if (const char* bp = getenv("SIMUSCOP_BATCH_PAIRS")) for (auto* d : devs) ssc_set_option(d, "batch_pairs", atoll(bp));
 	// SIMUSCOP_GZIP=1: the same FASTQ, compressed on the GPU, written as <name>.fq.gz (concatenated gzip members)
+	// SIMUSCOP_BGZF=1: the same, each member a BGZF block, the file ended by the BGZF EOF block, and <name>.fq.gz.gzi beside it
+	// (the block index `bgzip -i` writes; none on standard output); implies SIMUSCOP_GZIP=1
 	const char* gzEnv = getenv("SIMUSCOP_GZIP");
-	const bool gz = gzEnv && atoi(gzEnv) != 0;
+	const char* bgzfEnv = getenv("SIMUSCOP_BGZF");
+	const bool bgzf = bgzfEnv && atoi(bgzfEnv) != 0;
+	const bool gz = bgzf || (gzEnv && atoi(gzEnv) != 0);
 	if (gz) for (auto* d : devs) ssc_set_option(d, "gzip", 1);
+	if (bgzf) for (auto* d : devs) ssc_set_option(d, "bgzf", 1);
 	if (interleave) for (auto* d : devs) ssc_set_option(d, "interleave", 1);
 	const int G = (int)devs.size();
 	for (int s = 0; s < (int)J.samples.size() && !rc; s++) {
@@ -390,6 +485,11 @@ int ssh_run(ssh_job* job, int device) {
 		if (const char* wt = getenv("SIMUSCOP_WRITER_THREADS")) wthreads = atoi(wt);
 		if (toStdout ? ssh_writer_open_fd(1, &w) : ssh_writer_open(f1.c_str(), twoFiles ? f2.c_str() : nullptr, wthreads, &w))
 			sschost::die(-1, "Error: can not open fastq file to save results:\n" + f1);
+		if (bgzf) {
+			const std::string i1 = f1 + ".gzi", i2 = f2 + ".gzi";
+			if (ssh_writer_bgzf(w, toStdout ? nullptr : i1.c_str(), twoFiles ? i2.c_str() : nullptr))
+				sschost::die(-1, "Error: can not open the BGZF index file of:\n" + f1);
+		}
 		if (G == 1) {
 			rc = ssc_generate(devs[0], 0, planned, writer_sink, w);
 			if (rc) std::cerr << "Error: " << ssc_last_error() << std::endl;
