@@ -42,21 +42,67 @@ int fail(int code, const char* fmt, ...) {
 			return fail(SSC_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e__), __FILE__, __LINE__); \
 	} while (0)
 
-template <class T> struct DevBuf {
+// n elements of T in device memory, or in pinned host memory (Pinned); freed when the buffer is re-allocated or destroyed
+template <class T, bool Pinned> struct Buffer {
 	T* p = nullptr;
 	size_t n = 0;
+	Buffer() = default;
+	Buffer(Buffer&& o) noexcept : p(o.p), n(o.n) { o.p = nullptr; o.n = 0; }
+	Buffer& operator=(Buffer&& o) noexcept { std::swap(p, o.p); std::swap(n, o.n); return *this; }
+	~Buffer() { release(); }
 	cudaError_t alloc(size_t count) {
 		release();
-		n = count;
 		if (count == 0) return cudaSuccess;
-		return cudaMalloc((void**)&p, count * sizeof(T));
+		const cudaError_t e = Pinned ? cudaMallocHost((void**)&p, count * sizeof(T)) : cudaMalloc((void**)&p, count * sizeof(T));
+		if (e == cudaSuccess) n = count;
+		return e;
 	}
 	cudaError_t upload(const std::vector<T>& v, cudaStream_t s) {
 		cudaError_t e = alloc(v.size());
 		if (e != cudaSuccess || v.empty()) return e;
 		return cudaMemcpyAsync(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, s);
 	}
-	void release() { if (p) cudaFree(p); p = nullptr; n = 0; }
+	void release() {
+		if (p) { if (Pinned) cudaFreeHost(p); else cudaFree(p); }
+		p = nullptr; n = 0;
+	}
+};
+template <class T> using DevBuf = Buffer<T, false>;
+template <class T> using HostBuf = Buffer<T, true>;
+
+// A stream or event that is destroyed with its owner; it converts to the raw handle for the runtime calls
+template <class H, cudaError_t (*Destroy)(H)> struct Owned {
+	H h = nullptr;
+	Owned() = default;
+	Owned(Owned&& o) noexcept : h(o.h) { o.h = nullptr; }
+	Owned& operator=(Owned&& o) noexcept { std::swap(h, o.h); return *this; }
+	~Owned() { if (h) Destroy(h); }
+	operator H() const { return h; }
+};
+using Stream = Owned<cudaStream_t, cudaStreamDestroy>;
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
+
+cudaError_t create(Stream& s) { return cudaStreamCreateWithFlags(&s.h, cudaStreamNonBlocking); }
+cudaError_t create(Event& e, unsigned flags = cudaEventDisableTiming) { return cudaEventCreateWithFlags(&e.h, flags); }
+
+// Everything a batch in flight owns.  The handle has two sets: batch k+1 is generated into one while the blobs of batch k are
+// moved and its slabs copied out of the other.
+struct BufferSet {
+	DevBuf<uint8_t> d_out[2];                   // [file] dense slabs
+	HostBuf<uint8_t> h_out[2];                  // their host copies (ssc_generate)
+	DevBuf<uint8_t> d_slots;                    // pass-1 blob scratch of the fast kernel, FG_SLOT bytes per record
+	size_t file2Off = 0;                        // file 2's blobs start this many bytes into d_slots (0: one file)
+	DevBuf<unsigned long long> d_blobPrefix;
+	DevBuf<int32_t> d_tileStart;
+	DevBuf<unsigned long long> d_tileState;
+	DevBuf<unsigned int> d_ticket;
+	DevBuf<ssc::BatchResult> d_result;
+	HostBuf<ssc::BatchResult> h_result;
+	Event evDense;                              // the dense slabs are complete in the compute stream
+	Event evScanned;                            // the batch's last kernel (fast kernel, plain output: the scan) done
+	Event evResult;                             // the BatchResult is in h_result
+	Event evMoved;                              // the mover has moved the blobs
+	Event evCopy, evCopy2;                      // the device->host copies of file 1 / file 2 are done
 };
 
 }  // namespace
@@ -65,8 +111,8 @@ struct ssc_handle {
 	int device = 0;
 	int smCount = 0;
 	int smemLimit = 0;
-	cudaStream_t compute = nullptr, copy = nullptr, copy2 = nullptr;   // copy/copy2: device->host of file 1 / file 2 (two copy engines)
-	cudaEvent_t evStart = nullptr, evStop = nullptr, evCopy[2] = {nullptr, nullptr}, evCopy2[2] = {nullptr, nullptr};
+	Stream compute, copy, copy2;                  // copy/copy2: device->host of file 1 / file 2 (two copy engines)
+	Event evStart, evStop;
 
 	// options
 	int64_t batchPairs = 1 << 20;
@@ -77,22 +123,19 @@ struct ssc_handle {
 	int moverCtas = 0;            // "concurrent_move": pass 2b of batch k runs on that many SMs (bulk-copy mover, second stream) under the
 	                              // generation kernel of batch k+1, which leaves them free; 0 or [1, smCount), 0 = a stand-alone move
 	                              // after every batch.  Default: init_handle
-	cudaStream_t mover = nullptr; // pass 2 of the fast kernel's plain output: the scans and the concurrent moves
-	cudaEvent_t evPre = nullptr;  // a point of the compute stream the mover stream waits for (recorded anew for every wait)
-	cudaEvent_t evScanned[2] = {nullptr, nullptr};   // batch of buffer set b: its last kernel (fast kernel, plain output: the scan) done
-	cudaEvent_t evMoved[2] = {nullptr, nullptr};
+	Stream mover;                 // pass 2 of the fast kernel's plain output: the scans and the concurrent moves
+	Event evPre;                  // a point of the compute stream the mover stream waits for (recorded anew for every wait)
 	// the device->host copy of a batch's BatchResult: on a stream of its own, because the copy engines may be busy with the
 	// FASTQ slabs of ssc_generate for milliseconds, and no kernel must queue behind it
-	cudaStream_t results = nullptr;
-	cudaEvent_t evResult[2] = {nullptr, nullptr};    // batch of buffer set b: its BatchResult in h_result[b]
+	Stream results;
 	int fastQmode = -1;           // "fast_qmode": -1 automatic, else the only quality-table mode the fast kernel may use (tests)
 	bool gzip = false;            // slabs hold gzip members (one per ticket blob) instead of plain FASTQ
 	bool bgzf = false;            // "bgzf": with gzip, every member is a BGZF block (no effect without gzip)
 	bool interleave = false;      // "interleave": a PE plan's mates go to one stream, mate 1 and mate 2 of each pair in turn
 	size_t gzBlobBytes = 0;       // allocation of d_gzBlobs[0] (interleaved: both mates per ticket)
 	bool haveGz = false;          // Huffman / CRC tables of the current plan are on the device
-	ssc::GzTables* d_gzTab = nullptr;   // [0] gzip members, [1] BGZF blocks: one Huffman table, two member headers
-	uint8_t* d_gzBlobs[2] = {nullptr, nullptr};
+	DevBuf<ssc::GzTables> d_gzTab;      // [0] gzip members, [1] BGZF blocks: one Huffman table, two member headers
+	DevBuf<uint8_t> d_gzBlobs[2];
 	DevBuf<unsigned long long> d_gzLens;
 
 	// profile
@@ -117,21 +160,21 @@ struct ssc_handle {
 	// on its own stream while the caller works with the current reference; ssc_reference_adopt_prefetched swaps the sets
 	DevBuf<uint8_t> d_ref2, d_raw2;
 	DevBuf<unsigned long long> d_other2;
-	cudaStream_t upload = nullptr;
-	cudaEvent_t evRefFree = nullptr;
+	Stream upload;
+	Event evRefFree;
 	std::thread prefetchThread;
 	bool prefetching = false;
 	int prefetchRc = 0;
 	std::string prefetchErr;
 	uint64_t prefetchBases = 0, prefetchRaw = 0, prefetchOther = 0;
 	uint64_t refSize = 0;
-	uint8_t* h_stage[2] = {nullptr, nullptr};   // pinned upload staging
-	uint8_t* d_stage[2] = {nullptr, nullptr};
-	cudaEvent_t evStage[2] = {nullptr, nullptr};
+	HostBuf<uint8_t> h_stage[2];                  // pinned upload staging
+	DevBuf<uint8_t> d_stage[2];
+	Event evStage[2];
 	static constexpr int FA_READERS = 2;          // ssc_reference_upload_fasta: reader threads, one pinned buffer each (four readers
 	                                              // of 16 MB chunks were slower on the 16-vCPU boxes: 0.69 vs 0.28-0.31 s for the 3 Gb FASTA)
-	uint8_t* h_fa[2 * FA_READERS] = {nullptr, nullptr, nullptr, nullptr};       // [0, FA_READERS): foreground, the rest: prefetch
-	cudaEvent_t evFa[2 * FA_READERS] = {nullptr, nullptr, nullptr, nullptr};
+	HostBuf<uint8_t> h_fa[2 * FA_READERS];        // [0, FA_READERS): foreground, the rest: prefetch
+	Event evFa[2 * FA_READERS];
 	size_t faBytes = 32u << 20;
 	size_t stageBytes = 32u << 20;
 
@@ -153,31 +196,20 @@ struct ssc_handle {
 	int64_t slabPairs = 0;
 	uint64_t slabCap = 0;
 	int slabFiles = 0;                             // output streams the slabs were allocated for (out_files)
-	uint8_t* d_out[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};   // [buffer][file]
-	uint8_t* h_out[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};
-	DevBuf<int32_t> d_tileStart[2];
-	DevBuf<unsigned long long> d_tileState[2];
-	DevBuf<unsigned int> d_ticket[2];
-	uint8_t* d_slots[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};   // [buffer][file] pass-1 blob scratch of the fast kernel; file 2 lies
-	                                                                     // behind file 1 in the same allocation.  Two buffers: the mover moves
-	                                                                     // the blobs of batch k while batch k+1 is generated
-	DevBuf<unsigned long long> d_blobPrefix[2];
+	BufferSet set[2];
 	struct { bool valid = false; int buf = 0; ssc::GenParams P; } pending;   // generated (scan queued), blobs not yet moved
-	cudaEvent_t evDense[2] = {nullptr, nullptr};
 	DevBuf<int64_t> d_cenStarts;                  // ssc_gc_census scratch (grow-only)
 	DevBuf<int32_t> d_cenLens, d_cenGc, d_cenNn;
-	ssc::BatchResult* d_result[2] = {nullptr, nullptr};
-	ssc::BatchResult* h_result[2] = {nullptr, nullptr};
 	// ssc_generate_reads: the bookkeeping of its batches only (no slab, blob scratch or pinned host memory: the caller owns the output);
 	// the batches run back to back on the compute stream and add to one BatchResult
 	DevBuf<int32_t> d_rdTileStart;
 	DevBuf<unsigned int> d_rdTicket;
 	DevBuf<ssc::BatchResult> d_rdResult;
-	cudaEvent_t evCaller = nullptr;                  // the caller's stream at the call: the compute stream waits for it
+	Event evCaller;                                  // the caller's stream at the call: the compute stream waits for it
 
 	// kernel timing of ssc_generate_device: events kev[2 i] and kev[2 i + 1] bracket the i-th timed piece of work of the call,
 	// whose time goes to *kevSum[i] when the call ends (see time_begin)
-	std::vector<cudaEvent_t> kev;
+	std::vector<Event> kev;
 	std::vector<double*> kevSum;
 	int kevUsed = 0;
 	bool timeKernels = false;
@@ -227,29 +259,24 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 		}
 	}
 	if (pairs != h->slabPairs || cap != h->slabCap || slabFiles != h->slabFiles) {
-		for (int b = 0; b < 2; b++)
-			for (int f = 0; f < 2; f++) {
-				if (h->d_out[b][f]) cudaFree(h->d_out[b][f]);
-				if (h->h_out[b][f]) cudaFreeHost(h->h_out[b][f]);
-				h->d_out[b][f] = nullptr; h->h_out[b][f] = nullptr;
-			}
-		for (int b = 0; b < 2; b++) { if (h->d_slots[b][0]) cudaFree(h->d_slots[b][0]); h->d_slots[b][0] = h->d_slots[b][1] = nullptr; }
 		h->slabPairs = 0; h->slabCap = 0; h->slabFiles = 0;   // committed below, once every allocation has succeeded
 		h->pending.valid = false;
-		for (int b = 0; b < 2; b++) {
-			// file 2's blobs behind file 1's: the kernel addresses both from one base pointer with 32-bit cursors
-			CK(cudaMalloc((void**)&h->d_slots[b][0], ((size_t)pairs * FG_SLOT + 256) * nFiles));
-			h->d_slots[b][1] = nFiles == 2 ? h->d_slots[b][0] + ((size_t)pairs * FG_SLOT + 256) : nullptr;
-			CK(h->d_blobPrefix[b].alloc((size_t)(pairs / 16) + 2));
-		}
-		for (int f = 0; f < 2; f++) { if (h->d_gzBlobs[f]) cudaFree(h->d_gzBlobs[f]); h->d_gzBlobs[f] = nullptr; }
+		h->d_gzBlobs[0].release(); h->d_gzBlobs[1].release();   // sized by the slabs: allocated below when gzip is on
 		h->gzBlobBytes = 0;
 		int nTiles = (int)(pairs / 16) + 2;   // enough for every kernel's tile size
-		for (int b = 0; b < 2; b++) {
-			for (int f = 0; f < slabFiles; f++) CK(cudaMalloc((void**)&h->d_out[b][f], cap));
-			CK(h->d_tileStart[b].alloc(nTiles));
-			CK(h->d_tileState[b].alloc(nTiles));
-			CK(h->d_ticket[b].alloc(1));
+		for (BufferSet& S : h->set) {
+			// file 2's blobs behind file 1's: the kernel addresses both from one base pointer with 32-bit cursors
+			const size_t fileBytes = (size_t)pairs * FG_SLOT + 256;
+			CK(S.d_slots.alloc(fileBytes * nFiles));
+			S.file2Off = nFiles == 2 ? fileBytes : 0;
+			CK(S.d_blobPrefix.alloc(nTiles));
+			for (int f = 0; f < 2; f++) {
+				S.h_out[f].release();                   // allocated below when the call copies to the host
+				CK(S.d_out[f].alloc(f < slabFiles ? cap : 0));
+			}
+			CK(S.d_tileStart.alloc(nTiles));
+			CK(S.d_tileState.alloc(nTiles));
+			CK(S.d_ticket.alloc(1));
 		}
 		h->slabPairs = pairs; h->slabCap = cap; h->slabFiles = slabFiles;
 	}
@@ -258,17 +285,16 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 	static_assert(FG_SLOT * FG_CHUNK >= 19584 + ssc::GZ_BGZF_STORED_EXTRA, "a BGZF block fits its ticket's member pitch");
 	const size_t gzBytes = (size_t)h->slabPairs * FG_SLOT * (interleaved(h) ? 2 : 1) + 64;
 	if (h->gzip && h->gzBlobBytes != gzBytes) {
-		for (int f = 0; f < 2; f++) { if (h->d_gzBlobs[f]) cudaFree(h->d_gzBlobs[f]); h->d_gzBlobs[f] = nullptr; }
 		h->gzBlobBytes = 0;
-		for (int f = 0; f < (interleaved(h) ? 1 : 2); f++) CK(cudaMalloc((void**)&h->d_gzBlobs[f], gzBytes));
+		for (int f = 0; f < 2; f++) CK(h->d_gzBlobs[f].alloc(f < (interleaved(h) ? 1 : 2) ? gzBytes : 0));
 		h->gzBlobBytes = gzBytes;
 		CK(h->d_gzLens.alloc((size_t)(h->slabPairs / 16) + 2));
-		if (!h->d_gzTab) CK(cudaMalloc((void**)&h->d_gzTab, 2 * sizeof(ssc::GzTables)));
+		if (!h->d_gzTab.p) CK(h->d_gzTab.alloc(2));
 	}
 	if (needHost)
-		for (int b = 0; b < 2; b++)
+		for (BufferSet& S : h->set)
 			for (int f = 0; f < slabFiles; f++)
-				if (!h->h_out[b][f]) CK(cudaMallocHost((void**)&h->h_out[b][f], h->slabCap));
+				if (!S.h_out[f].p) CK(S.h_out[f].alloc(h->slabCap));
 	return SSC_OK;
 }
 
@@ -307,7 +333,7 @@ int build_gz_tables(ssc_handle* h, const ssc::GenParams& P, int nTiles) {
 		const char* err = ssc::gz_build_tables(hist, &tab[b], b == 1);
 		if (err[0]) return fail(SSC_ERR_INVALID, "gzip tables: %s", err);
 	}
-	CK(cudaMemcpyAsync(h->d_gzTab, tab.data(), 2 * sizeof(ssc::GzTables), cudaMemcpyHostToDevice, h->compute));   // stream order with the deflate kernel
+	CK(cudaMemcpyAsync(h->d_gzTab.p, tab.data(), 2 * sizeof(ssc::GzTables), cudaMemcpyHostToDevice, h->compute));   // stream order with the deflate kernel
 	CK(cudaStreamSynchronize(h->compute));          // tab is freed on return
 	h->haveGz = true;
 	return SSC_OK;
@@ -320,10 +346,10 @@ cudaError_t time_begin(ssc_handle* h, cudaStream_t s, double* sum, cudaEvent_t* 
 	*end = nullptr;
 	if (!h->timeKernels) return cudaSuccess;
 	while (h->kev.size() < 2 * (size_t)(h->kevUsed + 1)) {
-		cudaEvent_t e;
-		const cudaError_t err = cudaEventCreate(&e);
+		Event e;
+		const cudaError_t err = create(e, cudaEventDefault);
 		if (err != cudaSuccess) return err;
-		h->kev.push_back(e);
+		h->kev.push_back(std::move(e));
 	}
 	h->kevSum.resize((size_t)h->kevUsed + 1);
 	h->kevSum[h->kevUsed] = sum;
@@ -336,7 +362,7 @@ cudaError_t time_begin(ssc_handle* h, cudaStream_t s, double* sum, cudaEvent_t* 
 int flush_pending(ssc_handle* h) {
 	if (!h->pending.valid) return SSC_OK;
 	h->pending.valid = false;
-	CK(cudaStreamWaitEvent(h->compute, h->evScanned[h->pending.buf], 0));    // the blob offsets, scanned on the mover stream
+	CK(cudaStreamWaitEvent(h->compute, h->set[h->pending.buf].evScanned, 0));    // the blob offsets, scanned on the mover stream
 	cudaEvent_t te;
 	CK(time_begin(h, h->compute, &h->stats.compact_kernel_ms, &te));
 	CK(ssc::launch_move_blobs(h->pending.P, h->smCount, h->compute));
@@ -345,13 +371,13 @@ int flush_pending(ssc_handle* h) {
 	return SSC_OK;
 }
 
-// Copies the BatchResult of buffer set `buf` to h_result[buf] (evResult[buf]) once the work queued on stream `after`, which
-// writes it last, is done (evScanned[buf]).
+// Copies the BatchResult of buffer set `buf` to its h_result (evResult) once the work queued on stream `after`, which writes it
+// last, is done (evScanned).
 int result_to_host(ssc_handle* h, int buf, cudaStream_t after) {
-	CK(cudaEventRecord(h->evScanned[buf], after));
-	CK(cudaStreamWaitEvent(h->results, h->evScanned[buf], 0));
-	CK(cudaMemcpyAsync(h->h_result[buf], h->d_result[buf], sizeof(ssc::BatchResult), cudaMemcpyDeviceToHost, h->results));
-	CK(cudaEventRecord(h->evResult[buf], h->results));
+	CK(cudaEventRecord(h->set[buf].evScanned, after));
+	CK(cudaStreamWaitEvent(h->results, h->set[buf].evScanned, 0));
+	CK(cudaMemcpyAsync(h->set[buf].h_result.p, h->set[buf].d_result.p, sizeof(ssc::BatchResult), cudaMemcpyDeviceToHost, h->results));
+	CK(cudaEventRecord(h->set[buf].evResult, h->results));
 	return SSC_OK;
 }
 
@@ -384,39 +410,40 @@ ssc::GenParams batch_params(ssc_handle* h, int64_t emitLo, int64_t emitHi, bool 
 	return P;
 }
 
-// Launches batch [emitLo, emitHi) into buffer set `buf`; evResult[buf] marks its BatchResult in h_result[buf].  Fast kernel,
+// Launches batch [emitLo, emitHi) into buffer set `buf`; its evResult marks the BatchResult in its h_result.  Fast kernel,
 // plain output: pass 1 on the compute stream, then the scan of the blob lengths on the mover stream; the blobs are moved to
-// the dense slab d_out[buf] by the mover under the next launch_batch, or by flush_pending (right after the scan when the
-// mover is off).  Every other mode leaves the finished slab in d_out[buf] when its kernels have run on the compute stream.
+// the set's dense slabs d_out by the mover under the next launch_batch, or by flush_pending (right after the scan when the
+// mover is off).  Every other mode leaves the finished slabs in d_out when its kernels have run on the compute stream.
 int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 	int qsmem = 0; size_t fastSmem = 0;
 	const bool fast = use_fast(h, &qsmem, &fastSmem);
 	const int tp = fast ? FG_CHUNK : GEN_TILE_PAIRS;
 	int nTiles = (int)((emitHi - emitLo + tp - 1) / tp);
 	cudaStream_t s = h->compute;
-	CK(cudaStreamWaitEvent(s, h->evResult[buf], 0));          // the copy of the BatchResult this buffer set held before
-	CK(cudaMemsetAsync(h->d_tileState[buf].p, 0, sizeof(unsigned long long) * nTiles, s));
-	CK(cudaMemsetAsync(h->d_ticket[buf].p, 0, sizeof(unsigned int), s));
-	CK(cudaMemsetAsync(h->d_result[buf], 0, sizeof(ssc::BatchResult), s));
-	CK(ssc::launch_locate(h->d_emitBase.p, h->nDevBins, emitLo, tp, nTiles, h->d_tileStart[buf].p, s));
+	BufferSet& S = h->set[buf];
+	CK(cudaStreamWaitEvent(s, S.evResult, 0));                // the copy of the BatchResult this buffer set held before
+	CK(cudaMemsetAsync(S.d_tileState.p, 0, sizeof(unsigned long long) * nTiles, s));
+	CK(cudaMemsetAsync(S.d_ticket.p, 0, sizeof(unsigned int), s));
+	CK(cudaMemsetAsync(S.d_result.p, 0, sizeof(ssc::BatchResult), s));
+	CK(ssc::launch_locate(h->d_emitBase.p, h->nDevBins, emitLo, tp, nTiles, S.d_tileStart.p, s));
 	h->stats.launches += 1;
 	ssc::GenParams P = batch_params(h, emitLo, emitHi, fast && qsmem == 8);
-	P.tileStartBin = h->d_tileStart[buf].p; P.nTiles = nTiles;
-	P.tileState = h->d_tileState[buf].p; P.ticket = h->d_ticket[buf].p; P.blobPrefix = h->d_blobPrefix[buf].p;
-	P.out1 = h->d_out[buf][0]; P.out2 = h->d_out[buf][1];
+	P.tileStartBin = S.d_tileStart.p; P.nTiles = nTiles;
+	P.tileState = S.d_tileState.p; P.ticket = S.d_ticket.p; P.blobPrefix = S.d_blobPrefix.p;
+	P.out1 = S.d_out[0].p; P.out2 = S.d_out[1].p;
 	P.cap1 = h->slabCap; P.cap2 = h->slabCap;
-	P.result = h->d_result[buf];
+	P.result = S.d_result.p;
 	int grid = std::min(nTiles, h->smCount);
 	if (fast) {
 		h->stats.gen_kernel = 1; h->stats.gen_nch = ssc::fast_nch(h->dt.RL); h->stats.gen_qmode = qsmem;
 		h->stats.gen_smem_bytes = (int32_t)fastSmem;
 		// pass 1 writes one blob per ticket and file into the scratch, pass 2 (scan of the blob lengths + one move per blob) the dense slab
 		P.dense1 = P.out1; P.dense2 = P.out2;
-		P.out1 = h->d_slots[buf][0]; P.out2 = h->d_slots[buf][1];
+		P.out1 = S.d_slots.p; P.out2 = S.file2Off ? S.d_slots.p + S.file2Off : nullptr;
 		// interleaved: one blob per ticket over both halves of the scratch, so twice the per-file pitch
 		const bool ilv = interleaved(h);
 		P.blobPitch = (uint32_t)(FG_CHUNK * FG_SLOT * (ilv ? 2 : 1));
-		P.file2Off = (uint32_t)(h->d_slots[buf][1] ? h->d_slots[buf][1] - h->d_slots[buf][0] : 0);
+		P.file2Off = (uint32_t)S.file2Off;
 		cudaEvent_t te;
 		if (!h->gzip) {
 			int movedBuf = -1;
@@ -430,14 +457,15 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 				CK(time_begin(h, h->mover, &h->stats.mover_kernel_ms, &te));
 				CK(ssc::launch_move_blobs_tma(Q, h->moverCtas, h->mover));
 				if (te) CK(cudaEventRecord(te, h->mover));
-				CK(cudaEventRecord(h->evMoved[movedBuf], h->mover));
+				CK(cudaEventRecord(h->set[movedBuf].evMoved, h->mover));
 				h->pending.valid = false;
 				h->stats.launches += 1;
 			}
 			grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount - (movedBuf >= 0 ? h->moverCtas : 0));
 			if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
 			CK(time_begin(h, s, &h->stats.gen_kernel_ms, &te));
-			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, nullptr, te, ilv));
+			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, ilv));
+			if (te) CK(cudaEventRecord(te, s));
 			// pass 2a on the mover stream, behind the previous batch's move: only the moves and the host need its offsets and
 			// totals, so the compute stream goes straight on to the next batch
 			CK(cudaEventRecord(h->evPre, s));
@@ -451,7 +479,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 			h->stats.launches += 2;
 			if (h->moverCtas == 0) return flush_pending(h);              // stand-alone move right after the scan
 			// later work on this stream (the next launch reuses the blob scratch, copies read the dense slab) comes after the mover
-			if (movedBuf >= 0) CK(cudaStreamWaitEvent(s, h->evMoved[movedBuf], 0));
+			if (movedBuf >= 0) CK(cudaStreamWaitEvent(s, h->set[movedBuf].evMoved, 0));
 			return SSC_OK;
 		} else {
 			// gzip mode: blobs -> (first batch of a plan: fit the Huffman table to a sample) -> one gzip member per blob -> pass 2 on the members
@@ -460,14 +488,15 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 			grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount);
 			if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
 			CK(time_begin(h, s, &h->stats.gen_kernel_ms, &te));
-			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, nullptr, te, ilv));
+			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, ilv));
+			if (te) CK(cudaEventRecord(te, s));
 			CK(time_begin(h, s, &h->stats.compact_kernel_ms, &te));
 			if (!h->haveGz) { rc = build_gz_tables(h, P, nTiles); if (rc) return rc; }
 			CK(cudaMemsetAsync(h->d_gzLens.p, 0, sizeof(unsigned long long) * nTiles, s));
-			CK(ssc::launch_deflate_blobs(P.out1, P.out2, P.tileState, nTiles, P.blobPitch, h->d_gzBlobs[0], h->d_gzBlobs[1], h->d_gzLens.p,
-			                             P.blobPitch, h->d_gzTab + (h->bgzf ? 1 : 0), h->smCount, s));
+			CK(ssc::launch_deflate_blobs(P.out1, P.out2, P.tileState, nTiles, P.blobPitch, h->d_gzBlobs[0].p, h->d_gzBlobs[1].p, h->d_gzLens.p,
+			                             P.blobPitch, h->d_gzTab.p + (h->bgzf ? 1 : 0), h->smCount, s));
 			ssc::GenParams P2 = P;
-			P2.out1 = h->d_gzBlobs[0]; P2.out2 = h->d_gzBlobs[1]; P2.tileState = h->d_gzLens.p; P2.blobPitch = P.blobPitch;
+			P2.out1 = h->d_gzBlobs[0].p; P2.out2 = h->d_gzBlobs[1].p; P2.tileState = h->d_gzLens.p;
 			CK(ssc::launch_pass2(P2, h->smCount, s));
 			if (te) CK(cudaEventRecord(te, s));
 			h->stats.launches += 4;
@@ -478,7 +507,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 		if (rc) return rc;
 		ssc::GenVariant v = ssc::choose_variant(h->dt, h->fp64, h->smemLimit);
 		if (!v.ok) return fail(SSC_ERR_INVALID, "no kernel variant for read length %d / kmer %d", h->dt.RL, h->dt.K);
-		h->stats.gen_kernel = v.fp64 ? 4 : v.k3 ? 2 : 3; h->stats.gen_nch = v.nch; h->stats.gen_qmode = -1;
+		h->stats.gen_kernel = v.fp64 ? 4 : v.k3 ? 2 : 3; h->stats.gen_nch = GEN_NCH; h->stats.gen_qmode = -1;
 		h->stats.gen_smem_bytes = (int32_t)v.smemBytes;
 		CK(ssc::launch_generate(P, v, grid, s, interleaved(h)));
 		h->stats.launches += 1;
@@ -531,25 +560,14 @@ static int init_handle(ssc_handle* h, int device) {
 	// too few costs 4-6 % (the mover sets the step) where one too many costs 0.5-0.7 %: every profile gets the count XTen needs.
 	h->moverCtas = h->smCount >= 64 ? (h->smCount * 9 + 74) / 148 : 0;   // < smCount
 	h->smemLimit = (int)prop.sharedMemPerBlockOptin - 1024;
-	CK(cudaStreamCreateWithFlags(&h->compute, cudaStreamNonBlocking));
-	CK(cudaStreamCreateWithFlags(&h->copy, cudaStreamNonBlocking));
-	CK(cudaStreamCreateWithFlags(&h->copy2, cudaStreamNonBlocking));
-	CK(cudaStreamCreateWithFlags(&h->mover, cudaStreamNonBlocking));
-	CK(cudaStreamCreateWithFlags(&h->results, cudaStreamNonBlocking));
-	CK(cudaEventCreateWithFlags(&h->evPre, cudaEventDisableTiming));
-	CK(cudaEventCreateWithFlags(&h->evCaller, cudaEventDisableTiming));
-	CK(cudaEventCreate(&h->evStart));
-	CK(cudaEventCreate(&h->evStop));
-	for (int i = 0; i < 2; i++) {
-		CK(cudaEventCreateWithFlags(&h->evCopy[i], cudaEventDisableTiming));
-		CK(cudaEventCreateWithFlags(&h->evCopy2[i], cudaEventDisableTiming));
-		CK(cudaEventCreateWithFlags(&h->evStage[i], cudaEventDisableTiming));
-		CK(cudaEventCreateWithFlags(&h->evDense[i], cudaEventDisableTiming));
-		CK(cudaEventCreateWithFlags(&h->evScanned[i], cudaEventDisableTiming));
-		CK(cudaEventCreateWithFlags(&h->evResult[i], cudaEventDisableTiming));
-		CK(cudaEventCreateWithFlags(&h->evMoved[i], cudaEventDisableTiming));
-		CK(cudaMalloc((void**)&h->d_result[i], sizeof(ssc::BatchResult)));
-		CK(cudaMallocHost((void**)&h->h_result[i], sizeof(ssc::BatchResult)));
+	CK(create(h->compute)); CK(create(h->copy)); CK(create(h->copy2)); CK(create(h->mover)); CK(create(h->results));
+	CK(create(h->evPre)); CK(create(h->evCaller));
+	CK(create(h->evStart, cudaEventDefault)); CK(create(h->evStop, cudaEventDefault));
+	for (Event& e : h->evStage) CK(create(e));
+	for (BufferSet& S : h->set) {
+		for (Event* e : {&S.evDense, &S.evScanned, &S.evResult, &S.evMoved, &S.evCopy, &S.evCopy2}) CK(create(*e));
+		CK(S.d_result.alloc(1));
+		CK(S.h_result.alloc(1));
 	}
 	return SSC_OK;
 }
@@ -574,57 +592,10 @@ int ssc_create(int device, ssc_handle** out) {
 int ssc_destroy(ssc_handle* h) {
 	if (!h) return SSC_OK;
 	if (h->prefetchThread.joinable()) h->prefetchThread.join();
+	// the members free their memory, streams and events as they are destroyed: with the handle's device current, and only
+	// once nothing queued on it can still use them
 	cudaSetDevice(h->device);
 	cudaDeviceSynchronize();
-	for (int b = 0; b < 2; b++) {
-		for (int f = 0; f < 2; f++) {
-			if (h->d_out[b][f]) cudaFree(h->d_out[b][f]);
-			if (h->h_out[b][f]) cudaFreeHost(h->h_out[b][f]);
-		}
-		if (h->h_stage[b]) cudaFreeHost(h->h_stage[b]);
-		if (h->d_stage[b]) cudaFree(h->d_stage[b]);
-		for (int r = b; r < 2 * ssc_handle::FA_READERS; r += 2) {
-			if (h->h_fa[r]) cudaFreeHost(h->h_fa[r]);
-			if (h->evFa[r]) cudaEventDestroy(h->evFa[r]);
-		}
-		if (h->d_slots[b][0]) cudaFree(h->d_slots[b][0]);       // d_slots[b][1] points into the same allocation
-		h->d_blobPrefix[b].release();
-		if (h->evDense[b]) cudaEventDestroy(h->evDense[b]);
-		if (h->evScanned[b]) cudaEventDestroy(h->evScanned[b]);
-		if (h->evResult[b]) cudaEventDestroy(h->evResult[b]);
-		if (h->evMoved[b]) cudaEventDestroy(h->evMoved[b]);
-		if (h->d_result[b]) cudaFree(h->d_result[b]);
-		if (h->h_result[b]) cudaFreeHost(h->h_result[b]);
-		h->d_tileStart[b].release(); h->d_tileState[b].release(); h->d_ticket[b].release();
-		if (h->evCopy[b]) cudaEventDestroy(h->evCopy[b]);
-		if (h->evCopy2[b]) cudaEventDestroy(h->evCopy2[b]);
-		if (h->evStage[b]) cudaEventDestroy(h->evStage[b]);
-	}
-	h->d_isizeT.release(); h->d_insT.release(); h->d_delT.release(); h->d_qualT.release();
-	h->d_qualDiagT.release(); h->d_qualDiagSym.release();
-	h->d_isizeSym.release(); h->d_insSym.release(); h->d_delSym.release(); h->d_qualSym.release();
-	h->d_sub.release(); h->d_fIsize.release(); h->d_fIns.release(); h->d_fDel.release();
-	h->d_fSub1.release(); h->d_fSub2.release(); h->d_fQual.release(); h->d_lut.release();
-	h->d_hap2.release(); h->d_hapN.release(); h->d_ref.release(); h->d_raw.release(); h->d_other.release();
-	h->d_ref2.release(); h->d_raw2.release(); h->d_other2.release();
-	if (h->upload) cudaStreamDestroy(h->upload);
-	if (h->evRefFree) cudaEventDestroy(h->evRefFree);
-	h->d_gzLens.release();
-	for (int f = 0; f < 2; f++) if (h->d_gzBlobs[f]) cudaFree(h->d_gzBlobs[f]);
-	if (h->d_gzTab) cudaFree(h->d_gzTab);
-	h->d_cenStarts.release(); h->d_cenLens.release(); h->d_cenGc.release(); h->d_cenNn.release();
-	h->d_bins.release(); h->d_emitBase.release(); h->d_risky.release(); h->d_names.release();
-	for (cudaEvent_t e : h->kev) cudaEventDestroy(e);
-	if (h->evStart) cudaEventDestroy(h->evStart);
-	if (h->evStop) cudaEventDestroy(h->evStop);
-	if (h->compute) cudaStreamDestroy(h->compute);
-	if (h->copy) cudaStreamDestroy(h->copy);
-	if (h->copy2) cudaStreamDestroy(h->copy2);
-	if (h->mover) cudaStreamDestroy(h->mover);
-	if (h->results) cudaStreamDestroy(h->results);
-	if (h->evPre) cudaEventDestroy(h->evPre);
-	if (h->evCaller) cudaEventDestroy(h->evCaller);
-	h->d_rdTileStart.release(); h->d_rdTicket.release(); h->d_rdResult.release();
 	delete h;
 	return SSC_OK;
 }
@@ -741,8 +712,8 @@ int ssc_genome_reserve(ssc_handle* h, uint64_t total_bases) {
 	CK(cudaMemsetAsync(h->d_hap2.p, 0, (groups * 2 + 64) * 4, h->compute));
 	CK(cudaMemsetAsync(h->d_hapN.p, 0, (groups + 64) * 4, h->compute));
 	for (int i = 0; i < 2; i++) {
-		if (!h->h_stage[i]) CK(cudaMallocHost((void**)&h->h_stage[i], h->stageBytes));
-		if (!h->d_stage[i]) CK(cudaMalloc((void**)&h->d_stage[i], h->stageBytes));
+		if (!h->h_stage[i].p) CK(h->h_stage[i].alloc(h->stageBytes));
+		if (!h->d_stage[i].p) CK(h->d_stage[i].alloc(h->stageBytes));
 	}
 	h->genomeCap = total_bases;
 	h->genomeSize = 0;
@@ -760,9 +731,9 @@ int ssc_genome_append(ssc_handle* h, const char* ascii, uint64_t n, uint64_t* fi
 	while (done < n) {
 		uint64_t chunk = std::min<uint64_t>(h->stageBytes, n - done);
 		CK(cudaEventSynchronize(h->evStage[k]));           // staging buffer k free again
-		memcpy(h->h_stage[k], ascii + done, chunk);
-		CK(cudaMemcpyAsync(h->d_stage[k], h->h_stage[k], chunk, cudaMemcpyHostToDevice, h->compute));
-		CK(ssc::launch_pack(h->d_stage[k], chunk, SSC_GPAD + h->genomeSize + done, h->d_hap2.p, h->d_hapN.p, h->d_lut.p, h->compute));
+		memcpy(h->h_stage[k].p, ascii + done, chunk);
+		CK(cudaMemcpyAsync(h->d_stage[k].p, h->h_stage[k].p, chunk, cudaMemcpyHostToDevice, h->compute));
+		CK(ssc::launch_pack(h->d_stage[k].p, chunk, SSC_GPAD + h->genomeSize + done, h->d_hap2.p, h->d_hapN.p, h->d_lut.p, h->compute));
 		CK(cudaEventRecord(h->evStage[k], h->compute));
 		h->stats.launches += 1;
 		h->stats.h2d_bytes += chunk;
@@ -802,8 +773,8 @@ int upload_fasta_record(ssc_handle* h, int slot, cudaStream_t s, DevBuf<uint8_t>
 	if (!otherBuf.p) CK(otherBuf.alloc(1));
 	const int NR = ssc_handle::FA_READERS, b0 = slot * NR;
 	for (int i = b0; i < b0 + NR; i++) {
-		if (!h->h_fa[i]) CK(cudaMallocHost((void**)&h->h_fa[i], h->faBytes));
-		if (!h->evFa[i]) CK(cudaEventCreateWithFlags(&h->evFa[i], cudaEventDisableTiming));
+		if (!h->h_fa[i].p) CK(h->h_fa[i].alloc(h->faBytes));
+		if (!h->evFa[i]) CK(create(h->evFa[i]));
 	}
 	if (waitFor) CK(cudaStreamWaitEvent(s, waitFor, 0));         // earlier readers of `ref` (pack kernels of the record before the last)
 	CK(cudaMemsetAsync(otherBuf.p, 0, 8, s));
@@ -814,7 +785,7 @@ int upload_fasta_record(ssc_handle* h, int slot, cudaStream_t s, DevBuf<uint8_t>
 	std::string errMsg[ssc_handle::FA_READERS];
 	auto feed = [&](int k) {
 		if (cudaSetDevice(h->device) != cudaSuccess) { rcs[k] = SSC_ERR_CUDA; errMsg[k] = "cudaSetDevice failed"; return; }
-		uint8_t* buf = h->h_fa[b0 + k];
+		uint8_t* buf = h->h_fa[b0 + k].p;
 		cudaEvent_t ev = h->evFa[b0 + k];
 		for (uint64_t c = (uint64_t)k; c < nChunks; c += NR) {
 			const uint64_t done = c * h->faBytes;
@@ -879,8 +850,8 @@ int ssc_reference_prefetch_fasta(ssc_handle* h, int fd, uint64_t file_offset, ui
 	int rc = check_fasta_geometry(n_bases, line_bases, line_width);
 	if (rc) return rc;
 	CK(cudaSetDevice(h->device));
-	if (!h->upload) CK(cudaStreamCreateWithFlags(&h->upload, cudaStreamNonBlocking));
-	if (!h->evRefFree) CK(cudaEventCreateWithFlags(&h->evRefFree, cudaEventDisableTiming));
+	if (!h->upload) CK(create(h->upload));
+	if (!h->evRefFree) CK(create(h->evRefFree));
 	// the second buffer set was the current reference until the last adoption: its readers are in the compute stream by now
 	CK(cudaEventRecord(h->evRefFree, h->compute));
 	h->prefetching = true;
@@ -934,7 +905,6 @@ int ssc_genome_poke(ssc_handle* h, const int64_t* store_pos, const char* chars, 
 	CK(cudaMemcpyAsync(d_ch.p, chars, (size_t)n, cudaMemcpyHostToDevice, h->compute));
 	CK(ssc::launch_poke(h->d_hap2.p, h->d_hapN.p, d_pos.p, d_ch.p, n, h->d_lut.p, h->compute));
 	CK(cudaStreamSynchronize(h->compute));
-	d_pos.release(); d_ch.release();
 	h->stats.launches += 1;
 	return SSC_OK;
 }
@@ -949,7 +919,6 @@ int ssc_genome_read(ssc_handle* h, uint64_t start, uint64_t n, char* out) {
 	CK(ssc::launch_unpack(h->d_hap2.p, h->d_hapN.p, SSC_GPAD + start, n, h->dt.baseChars, d_out.p, h->compute));
 	CK(cudaMemcpyAsync(out, d_out.p, (size_t)n, cudaMemcpyDeviceToHost, h->compute));
 	CK(cudaStreamSynchronize(h->compute));
-	d_out.release();
 	h->stats.launches += 1;
 	return SSC_OK;
 }
@@ -1097,7 +1066,6 @@ int ssc_set_plan(ssc_handle* h, uint64_t seed, const ssc_bin* bins, int64_t n_bi
 		CK(cudaStreamSynchronize(s));
 		h->stats.launches += 1;
 		for (size_t k = 0; k < census.size(); k++) emit[censusOf[k]] = em[k];
-		d_census.release(); d_emitted.release();
 	}
 
 	// ---- prefix sums, compaction
@@ -1132,7 +1100,7 @@ int ssc_set_plan(ssc_handle* h, uint64_t seed, const ssc_bin* bins, int64_t n_bi
 	// The device bins (64 bytes each, 384 MB for a 3 Gb diploid plan) are formatted straight into the two pinned staging
 	// buffers, a run of whole segments at a time, and copied from there: no pageable image of the table is ever built.
 	for (int i = 0; i < 2; i++) {
-		if (!h->h_stage[i]) CK(cudaMallocHost((void**)&h->h_stage[i], h->stageBytes));
+		if (!h->h_stage[i].p) CK(h->h_stage[i].alloc(h->stageBytes));
 		CK(cudaEventSynchronize(h->evStage[i]));
 	}
 	CK(h->d_bins.alloc(std::max<size_t>(nDev, 1)));
@@ -1145,7 +1113,7 @@ int ssc_set_plan(ssc_handle* h, uint64_t seed, const ssc_bin* bins, int64_t n_bi
 		const int64_t o0 = segOff[s0], cnt = segOff[s1] - o0;
 		if (cnt > 0) {
 			CK(cudaEventSynchronize(h->evStage[stage]));
-			ssc::DevBin* out = (ssc::DevBin*)h->h_stage[stage];
+			ssc::DevBin* out = (ssc::DevBin*)h->h_stage[stage].p;
 			parallel(s1 - s0, [&](int64_t lo, int64_t hi, unsigned) {
 				for (int64_t sIdx = s0 + lo; sIdx < s0 + hi; sIdx++) {
 					int64_t fragBase = 0, o = segOff[sIdx];
@@ -1213,11 +1181,11 @@ static int generate_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc
 		// the dense slab this launch writes: d_out[(k-1) & 1] when the mover completes the previous batch under it, else
 		// d_out[k & 1]; its last reader is the copy of the batch two before the one that now lands there
 		const int target = moverCompletes ? (k + 1) & 1 : k & 1;
-		CK(cudaStreamWaitEvent(h->compute, h->evCopy[target], 0));
-		CK(cudaStreamWaitEvent(h->compute, h->evCopy2[target], 0));
+		CK(cudaStreamWaitEvent(h->compute, h->set[target].evCopy, 0));
+		CK(cudaStreamWaitEvent(h->compute, h->set[target].evCopy2, 0));
 		int r = launch_batch(h, k & 1, batches[k].lo, batches[k].hi);
 		if (r) return r;
-		if (!moverCompletes) CK(cudaEventRecord(h->evDense[k & 1], h->compute));     // the dense slab of batch k is complete with its own launch
+		if (!moverCompletes) CK(cudaEventRecord(h->set[k & 1].evDense, h->compute));     // the dense slab of batch k is complete with its own launch
 		return SSC_OK;
 	};
 	rc = launch(0);
@@ -1227,34 +1195,34 @@ static int generate_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc
 		const int buf = k & 1;
 		rc = k + 1 < nb ? launch(k + 1) : flush_pending(h);         // after this the dense slab of batch k is in the stream
 		if (rc) return rc;
-		if (moverCompletes) CK(cudaEventRecord(h->evDense[buf], h->compute));    // (its pass 2b came with the launch of batch k+1)
-		CK(cudaEventSynchronize(h->evResult[buf]));
-		res[buf] = *h->h_result[buf];
+		if (moverCompletes) CK(cudaEventRecord(h->set[buf].evDense, h->compute));    // (its pass 2b came with the launch of batch k+1)
+		CK(cudaEventSynchronize(h->set[buf].evResult));
+		res[buf] = *h->set[buf].h_result.p;
 		rc = check_result(h, res[buf]);
 		if (rc) return rc;
-		CK(cudaStreamWaitEvent(h->copy, h->evDense[buf], 0));
-		CK(cudaMemcpyAsync(h->h_out[buf][0], h->d_out[buf][0], res[buf].bytes1, cudaMemcpyDeviceToHost, h->copy));
-		CK(cudaEventRecord(h->evCopy[buf], h->copy));
+		CK(cudaStreamWaitEvent(h->copy, h->set[buf].evDense, 0));
+		CK(cudaMemcpyAsync(h->set[buf].h_out[0].p, h->set[buf].d_out[0].p, res[buf].bytes1, cudaMemcpyDeviceToHost, h->copy));
+		CK(cudaEventRecord(h->set[buf].evCopy, h->copy));
 		if (nFiles == 2) {
-			CK(cudaStreamWaitEvent(h->copy2, h->evDense[buf], 0));
-			CK(cudaMemcpyAsync(h->h_out[buf][1], h->d_out[buf][1], res[buf].bytes2, cudaMemcpyDeviceToHost, h->copy2));
+			CK(cudaStreamWaitEvent(h->copy2, h->set[buf].evDense, 0));
+			CK(cudaMemcpyAsync(h->set[buf].h_out[1].p, h->set[buf].d_out[1].p, res[buf].bytes2, cudaMemcpyDeviceToHost, h->copy2));
 		}
-		CK(cudaEventRecord(h->evCopy2[buf], h->copy2));
+		CK(cudaEventRecord(h->set[buf].evCopy2, h->copy2));
 		h->stats.d2h_bytes += res[buf].bytes1 + res[buf].bytes2;
 		if (k >= 1) {
 			const int pb = (k - 1) & 1;
-			CK(cudaEventSynchronize(h->evCopy[pb]));
-			CK(cudaEventSynchronize(h->evCopy2[pb]));
-			int src = sink(user, (const char*)h->h_out[pb][0], res[pb].bytes1, nFiles == 2 ? (const char*)h->h_out[pb][1] : nullptr,
+			CK(cudaEventSynchronize(h->set[pb].evCopy));
+			CK(cudaEventSynchronize(h->set[pb].evCopy2));
+			int src = sink(user, (const char*)h->set[pb].h_out[0].p, res[pb].bytes1, nFiles == 2 ? (const char*)h->set[pb].h_out[1].p : nullptr,
 			               nFiles == 2 ? res[pb].bytes2 : 0, batches[k - 1].lo, batches[k - 1].hi - batches[k - 1].lo);
 			if (src) return fail(SSC_ERR_SINK, "sink returned %d", src);
 		}
 	}
 	{
 		const int pb = (nb - 1) & 1;
-		CK(cudaEventSynchronize(h->evCopy[pb]));
-		CK(cudaEventSynchronize(h->evCopy2[pb]));
-		int src = sink(user, (const char*)h->h_out[pb][0], res[pb].bytes1, nFiles == 2 ? (const char*)h->h_out[pb][1] : nullptr,
+		CK(cudaEventSynchronize(h->set[pb].evCopy));
+		CK(cudaEventSynchronize(h->set[pb].evCopy2));
+		int src = sink(user, (const char*)h->set[pb].h_out[0].p, res[pb].bytes1, nFiles == 2 ? (const char*)h->set[pb].h_out[1].p : nullptr,
 		               nFiles == 2 ? res[pb].bytes2 : 0, batches[nb - 1].lo, batches[nb - 1].hi - batches[nb - 1].lo);
 		if (src) return fail(SSC_ERR_SINK, "sink returned %d", src);
 	}
@@ -1284,8 +1252,8 @@ static int generate_device_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_
 	for (int64_t e = eLo; e < eHi; e += h->slabPairs, k++) {
 		const int buf = k & 1;
 		if (k >= 2) {
-			CK(cudaEventSynchronize(h->evResult[buf]));
-			ssc::BatchResult r = *h->h_result[buf];
+			CK(cudaEventSynchronize(h->set[buf].evResult));
+			ssc::BatchResult r = *h->set[buf].h_result.p;
 			rc = check_result(h, r);
 			if (rc) return rc;
 			*b1 += r.bytes1; *b2 += r.bytes2; *nb += r.bases;
@@ -1298,8 +1266,8 @@ static int generate_device_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_
 	CK(cudaEventRecord(h->evStop, h->compute));    // the compute stream has waited for the mover stream's last work
 	CK(cudaEventSynchronize(h->evStop));
 	for (int j = std::max(0, k - 2); j < k; j++) {
-		CK(cudaEventSynchronize(h->evResult[j & 1]));
-		ssc::BatchResult r = *h->h_result[j & 1];
+		CK(cudaEventSynchronize(h->set[j & 1].evResult));
+		ssc::BatchResult r = *h->set[j & 1].h_result.p;
 		rc = check_result(h, r);
 		if (rc) return rc;
 		*b1 += r.bytes1; *b2 += r.bytes2; *nb += r.bases;
@@ -1481,7 +1449,6 @@ int ssc_issue_floor(ssc_handle* h, int mode, int read_length, int64_t n_pairs, i
 	CK(cudaEventElapsedTime(&ms, h->evStart, h->evStop));
 	*ms_per_launch = (double)ms / reps;
 	h->stats.launches += (uint64_t)reps + 1;
-	scratch.release(); blobs.release();
 	return SSC_OK;
 }
 

@@ -39,10 +39,6 @@
 
 namespace ssc {
 
-#define ST_A (1ull << 62)
-#define ST_P (2ull << 62)
-#define ST_MASK (3ull << 62)
-
 static constexpr int F_SRC_CAP = 256;           // longest read after indels
 static constexpr int F_EV_MAX = 32;
 static constexpr int F_INS_CAP = 128;
@@ -1320,16 +1316,11 @@ static cudaError_t launch_fast_instance(const GenParams& P, int qmode, size_t sm
 	return launch_fast_variant<5, 0, OUT>(P, smemBytes, grid, stream);
 }
 
-// P.out1/out2 = blob scratch, P.dense1/dense2 = final slabs, P.nTiles = tickets of FG_CHUNK pairs.  Launches pass 1;
-// events e0/e1 (optional) bracket the kernel.  interleaved (PE): one blob per ticket, P.blobPitch = 2 x FG_CHUNK x FG_SLOT.
-cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream,
-                                 cudaEvent_t e0, cudaEvent_t e1, bool interleaved) {
-	if (e0) cudaEventRecord(e0, stream);
-	const cudaError_t e = interleaved ? launch_fast_instance<OUT_INTERLEAVED>(P, qmode, smemBytes, grid, stream)
-	                                  : launch_fast_instance<OUT_FASTQ>(P, qmode, smemBytes, grid, stream);
-	if (e != cudaSuccess) return e;
-	if (e1) cudaEventRecord(e1, stream);
-	return cudaSuccess;
+// P.out1/out2 = blob scratch, P.dense1/dense2 = final slabs, P.nTiles = tickets of FG_CHUNK pairs.  Launches pass 1.
+// interleaved (PE): one blob per ticket, P.blobPitch = 2 x FG_CHUNK x FG_SLOT.
+cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream, bool interleaved) {
+	return interleaved ? launch_fast_instance<OUT_INTERLEAVED>(P, qmode, smemBytes, grid, stream)
+	                   : launch_fast_instance<OUT_FASTQ>(P, qmode, smemBytes, grid, stream);
 }
 
 // Array output: P.out1 = reads of the batch's first pair ([pair][mate][2][P.pitch], 16-byte aligned, pairs * M * 2 * pitch < 2^32),

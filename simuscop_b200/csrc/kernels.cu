@@ -238,33 +238,30 @@ static constexpr int EV_MAX = 32;     // indel events per read
 #define ST_P (2ull << 62)
 #define ST_MASK (3ull << 62)
 
-template <int NCH> struct GenCfg {
-	static constexpr int SRC_CAP = NCH * 32 + 96;                       // longest read the scratch holds
+struct GenCfg {
+	static constexpr int SRC_CAP = GEN_NCH * 32 + 96;                   // longest read the scratch holds
 	static constexpr int REC_CAP = HDR_MAX + 2 * SRC_CAP + 8;
 	static constexpr int STAGE_CAP = ((GEN_PPW * REC_CAP + 15) / 16) * 16 + 16;
 };
 
 struct SmemLayout {
-	int sub, qualT, qualSym, isizeT, isizeSym, insT, insSym, delT, delSym, src, ev, insb, stage, total;
+	int sub, isizeT, isizeSym, insT, insSym, delT, delSym, src, ev, insb, stage, total;
 };
 
-template <int NCH>
-__host__ __device__ inline SmemLayout smem_layout(int nSubTotal, int nQual /*rows*pitch or 0*/, int nIsize, int nIns, int nDel) {
+__host__ __device__ inline SmemLayout smem_layout(int nSubTotal, int nIsize, int nIns, int nDel) {
 	SmemLayout L;
 	int o = 0;
 	L.sub = o; o += nSubTotal * 16;
-	L.qualT = o; o += nQual * 4;
-	L.qualSym = o; o += (nQual + 15) / 16 * 16;
 	L.isizeT = o; o += (nIsize * 4 + 15) / 16 * 16;
 	L.isizeSym = o; o += (nIsize * 2 + 15) / 16 * 16;
 	L.insT = o; o += (nIns * 4 + 15) / 16 * 16;
 	L.insSym = o; o += (nIns * 2 + 15) / 16 * 16;
 	L.delT = o; o += (nDel * 4 + 15) / 16 * 16;
 	L.delSym = o; o += (nDel * 2 + 15) / 16 * 16;
-	L.src = o; o += GEN_WARPS * GenCfg<NCH>::SRC_CAP;
+	L.src = o; o += GEN_WARPS * GenCfg::SRC_CAP;
 	L.ev = o; o += GEN_WARPS * EV_MAX * 4;
 	L.insb = o; o += GEN_WARPS * 128;
-	L.stage = o; o += GEN_WARPS * 2 * GenCfg<NCH>::STAGE_CAP;
+	L.stage = o; o += GEN_WARPS * 2 * GenCfg::STAGE_CAP;
 	L.total = o;
 	return L;
 }
@@ -345,31 +342,27 @@ __device__ __forceinline__ void copy_out(const uint8_t* sm, int len, uint8_t* g,
 // ILV (interleaved output, PE): mate 2's record goes right behind mate 1's in the warp's first stage buffer, whose neighbour is
 // its second one (2 x STAGE_CAP hold both mates of GEN_PPW pairs), and the one slab P.out1 receives mate 1, mate 2 of every
 // pair in turn; off2, the second length of the look-back and P.out2 stay unused.
-template <int NCH, bool K3, bool QSMEM, bool FP64, bool ILV>
+template <bool K3, bool FP64, bool ILV>
 __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParams P) {
 	extern __shared__ __align__(16) uint8_t smem[];
-	using Cfg = GenCfg<NCH>;
 	const DevTables& t = P.t;
 	const int lane = threadIdx.x & 31;
 	const int warp = threadIdx.x >> 5;
 	const int subSmemRows = (K3 && !FP64) ? t.nSub * (t.useCdf2 ? 2 : 1) : 0;
-	const int qualSmem = (QSMEM && !FP64) ? t.nQualRows * t.qualPitch : 0;
-	const SmemLayout L = smem_layout<NCH>(subSmemRows, qualSmem, FP64 ? 0 : t.nIsize, FP64 ? 0 : t.nInsLen, FP64 ? 0 : t.nDelLen);
+	const SmemLayout L = smem_layout(subSmemRows, FP64 ? 0 : t.nIsize, FP64 ? 0 : t.nInsLen, FP64 ? 0 : t.nDelLen);
 
 	uint4* s_sub = (uint4*)(smem + L.sub);
-	uint32_t* s_qualT = (uint32_t*)(smem + L.qualT);
-	uint8_t* s_qualSym = smem + L.qualSym;
 	uint32_t* s_isizeT = (uint32_t*)(smem + L.isizeT);
 	uint16_t* s_isizeSym = (uint16_t*)(smem + L.isizeSym);
 	uint32_t* s_insT = (uint32_t*)(smem + L.insT);
 	uint16_t* s_insSym = (uint16_t*)(smem + L.insSym);
 	uint32_t* s_delT = (uint32_t*)(smem + L.delT);
 	uint16_t* s_delSym = (uint16_t*)(smem + L.delSym);
-	uint8_t* s_src = smem + L.src + warp * Cfg::SRC_CAP;
+	uint8_t* s_src = smem + L.src + warp * GenCfg::SRC_CAP;
 	uint32_t* s_ev = (uint32_t*)(smem + L.ev) + warp * EV_MAX;
 	uint8_t* s_insb = smem + L.insb + warp * 128;
-	uint8_t* s_stage1 = smem + L.stage + (warp * 2 + 0) * Cfg::STAGE_CAP;
-	uint8_t* s_stage2 = smem + L.stage + (warp * 2 + 1) * Cfg::STAGE_CAP;
+	uint8_t* s_stage1 = smem + L.stage + (warp * 2 + 0) * GenCfg::STAGE_CAP;
+	uint8_t* s_stage2 = smem + L.stage + (warp * 2 + 1) * GenCfg::STAGE_CAP;
 
 	__shared__ unsigned long long s_warpLen[GEN_WARPS];   // len1 << 32 | len2
 	__shared__ unsigned long long s_warpOff[GEN_WARPS];
@@ -380,15 +373,14 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 	// ---- stage the tables
 	if (!FP64) {
 		for (int i = threadIdx.x; i < subSmemRows; i += GEN_THREADS) s_sub[i] = t.sub[i];
-		for (int i = threadIdx.x; i < qualSmem; i += GEN_THREADS) { s_qualT[i] = t.qualT[i]; s_qualSym[i] = t.qualSym[i]; }
 		for (int i = threadIdx.x; i < t.nIsize; i += GEN_THREADS) { s_isizeT[i] = t.isizeT[i]; s_isizeSym[i] = t.isizeSym[i]; }
 		for (int i = threadIdx.x; i < t.nInsLen; i += GEN_THREADS) { s_insT[i] = t.insLenT[i]; s_insSym[i] = t.insLenSym[i]; }
 		for (int i = threadIdx.x; i < t.nDelLen; i += GEN_THREADS) { s_delT[i] = t.delLenT[i]; s_delSym[i] = t.delLenSym[i]; }
 	}
 	if (threadIdx.x < 4) s_stats[threadIdx.x] = 0;
 	const uint4* subTab = (K3 && !FP64) ? s_sub : t.sub;
-	const uint32_t* qualT = (QSMEM && !FP64) ? s_qualT : t.qualT;
-	const uint8_t* qualSym = (QSMEM && !FP64) ? s_qualSym : t.qualSym;
+	const uint32_t* qualT = t.qualT;
+	const uint8_t* qualSym = t.qualSym;
 
 	const int RL = t.RL, B = t.B, K = t.K;
 	const int nMates = t.paired ? 2 : 1;
@@ -438,11 +430,11 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 				if (lane <= (int)(((g0 + RL - 1) >> 5) - m0)) maskW = __ldg(P.hapN + m0 + lane);
 
 				// ---- phase A: one Philox block per cycle; indel tests at reference position j
-				uint32_t x2[NCH], x3[NCH], insMask[NCH], delMask[NCH];
+				uint32_t x2[GEN_NCH], x3[GEN_NCH], insMask[GEN_NCH], delMask[GEN_NCH];
 				uint32_t tcode = 0;   // 3 bits per chunk
 				uint32_t anyEv = 0;
 #pragma unroll
-				for (int c = 0; c < NCH; c++) {
+				for (int c = 0; c < GEN_NCH; c++) {
 					insMask[c] = 0; delMask[c] = 0; x2[c] = 0; x3[c] = 0;
 					if (c < chunksRL) {
 						const int j = c * 32 + lane;
@@ -479,7 +471,7 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 				int m = RL;
 				if (anyEv == 0) {
 #pragma unroll
-					for (int c = 0; c < NCH; c++) {
+					for (int c = 0; c < GEN_NCH; c++) {
 						const int j = c * 32 + lane;
 						if (c < chunksRL && j < RL) s_src[j] = (uint8_t)((tcode >> (3 * c)) & 7u);
 					}
@@ -487,7 +479,7 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 					int nEv = 0, insTotal = 0, indelLength = 0, skipUntil = 0;
 					bool tooMany = false;
 #pragma unroll
-					for (int c = 0; c < NCH; c++) {
+					for (int c = 0; c < GEN_NCH; c++) {
 						uint32_t mask = insMask[c] | delMask[c];
 						while (mask) {
 							const int bit = __ffs(mask) - 1;
@@ -523,14 +515,14 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 					}
 					if (RL + indelLength < 50) { nEv = 0; indelLength = 0; }   // Profile.cpp:1627-1634
 					m = RL + indelLength;
-					if (tooMany || m > Cfg::SRC_CAP) {
+					if (tooMany || m > GenCfg::SRC_CAP) {
 						if (lane == 0) atomicOr(&P.result->errorFlags, tooMany ? 4u : 2u);
 						nEv = 0; m = RL;
 					}
 					__syncwarp();
 					// template bases to their output positions
 #pragma unroll
-					for (int c = 0; c < NCH; c++) {
+					for (int c = 0; c < GEN_NCH; c++) {
 						const int j = c * 32 + lane;
 						if (c < chunksRL && j < RL) {
 							int shift = 0; bool dropped = false;
@@ -608,14 +600,14 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 					stage[H + m + 3 + j] = q;
 				};
 #pragma unroll
-				for (int c = 0; c < NCH; c++) {
+				for (int c = 0; c < GEN_NCH; c++) {
 					const int j = c * 32 + lane;
 					if (c < chunksM && j < m) {
 						if (c < chunksRL) emit(j, x2[c], x3[c]);
 						else { u32x4 blk = draw_block(P.seed, pair, mate, STREAM_CYCLE, 0, (uint32_t)j); emit(j, blk.z, blk.w); }
 					}
 				}
-				for (int c = NCH; c < chunksM; c++) {
+				for (int c = GEN_NCH; c < chunksM; c++) {
 					const int j = c * 32 + lane;
 					if (j < m) { u32x4 blk = draw_block(P.seed, pair, mate, STREAM_CYCLE, 0, (uint32_t)j); emit(j, blk.z, blk.w); }
 				}
@@ -704,9 +696,9 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 // ----------------------------------------------------------------------------------------
 // host-side launchers
 // ----------------------------------------------------------------------------------------
-template <int NCH, bool K3, bool QSMEM, bool FP64, bool ILV>
+template <bool K3, bool FP64, bool ILV>
 static cudaError_t launch_variant(const GenParams& P, int grid, size_t smemBytes, cudaStream_t stream) {
-	auto kern = generate_kernel<NCH, K3, QSMEM, FP64, ILV>;
+	auto kern = generate_kernel<K3, FP64, ILV>;
 	cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemBytes);
 	if (e != cudaSuccess) return e;
 	kern<<<grid, GEN_THREADS, smemBytes, stream>>>(P);
@@ -715,35 +707,32 @@ static cudaError_t launch_variant(const GenParams& P, int grid, size_t smemBytes
 
 GenVariant choose_variant(const DevTables& t, bool fp64, int smemLimit) {
 	GenVariant v;
-	v.nch = 10;
 	v.fp64 = fp64;
 	v.k3 = (t.K == 3) && !fp64;
-	v.qsmem = false;
 	v.smemBytes = 0;
-	v.ok = t.RL <= 320;
-	auto size = [&](bool k3, bool qs) {
+	v.ok = t.RL <= GEN_NCH * 32;
+	auto size = [&](bool k3) {
 		int nSub = k3 ? t.nSub * (t.useCdf2 ? 2 : 1) : 0;
-		int nQ = qs ? t.nQualRows * t.qualPitch : 0;
 		int a = fp64 ? 0 : t.nIsize, b = fp64 ? 0 : t.nInsLen, c = fp64 ? 0 : t.nDelLen;
-		return smem_layout<10>(nSub, nQ, a, b, c).total;
+		return smem_layout(nSub, a, b, c).total;
 	};
-	if (fp64) { v.smemBytes = size(false, false); return v; }
-	if (v.k3 && size(true, false) <= smemLimit) { v.smemBytes = size(true, false); return v; }
+	if (fp64) { v.smemBytes = size(false); return v; }
+	if (v.k3 && size(true) <= smemLimit) { v.smemBytes = size(true); return v; }
 	v.k3 = false;
-	v.smemBytes = size(false, false);
+	v.smemBytes = size(false);
 	if ((int)v.smemBytes > smemLimit) v.ok = false;
 	return v;
 }
 
 cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream, bool interleaved) {
 	if (interleaved) {
-		if (v.fp64) return launch_variant<10, false, false, true, true>(P, grid, v.smemBytes, stream);
-		if (v.k3) return launch_variant<10, true, false, false, true>(P, grid, v.smemBytes, stream);
-		return launch_variant<10, false, false, false, true>(P, grid, v.smemBytes, stream);
+		if (v.fp64) return launch_variant<false, true, true>(P, grid, v.smemBytes, stream);
+		if (v.k3) return launch_variant<true, false, true>(P, grid, v.smemBytes, stream);
+		return launch_variant<false, false, true>(P, grid, v.smemBytes, stream);
 	}
-	if (v.fp64) return launch_variant<10, false, false, true, false>(P, grid, v.smemBytes, stream);
-	if (v.k3) return launch_variant<10, true, false, false, false>(P, grid, v.smemBytes, stream);
-	return launch_variant<10, false, false, false, false>(P, grid, v.smemBytes, stream);
+	if (v.fp64) return launch_variant<false, true, false>(P, grid, v.smemBytes, stream);
+	if (v.k3) return launch_variant<true, false, false>(P, grid, v.smemBytes, stream);
+	return launch_variant<false, false, false>(P, grid, v.smemBytes, stream);
 }
 
 // ----------------------------------------------------------------------------------------

@@ -9,6 +9,7 @@
 #define GEN_THREADS (GEN_WARPS * 32)
 #define GEN_PPW 2                                 /* pairs per warp per tile */
 #define GEN_TILE_PAIRS (GEN_WARPS * GEN_PPW)
+#define GEN_NCH 10                                /* chunks of 32 cycles the generic kernel holds in registers (RL <= 320) */
 
 #ifndef FG_WORKERS
 #define FG_WORKERS 32                             /* warps per CTA of the fast kernel */
@@ -27,9 +28,7 @@
 namespace ssc {
 
 struct GenVariant {
-	int nch;        // chunks of 32 cycles held in registers (5: RL <= 160, 10: RL <= 320)
 	bool k3;        // K == 3 fast context indexing with the substitution tables in shared memory
-	bool qsmem;     // quality tables in shared memory
 	bool fp64;      // FP64 linear-search ground truth
 	size_t smemBytes;
 	bool ok;
@@ -40,8 +39,7 @@ cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, c
 bool fast_supported(const DevTables& t, int smemLimit, int* qmode, size_t* smemBytes);   // qmode: 8 / 16 / 2 / 0, see gen_fast.cu
 int fast_choose_qbins(int B, int RL);
 int fast_nch(int RL);
-cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream,
-                                 cudaEvent_t e0, cudaEvent_t e1, bool interleaved);
+cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream, bool interleaved);
 cudaError_t launch_generate_reads(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream);
 cudaError_t launch_scan_blobs(const GenParams& P, cudaStream_t stream);
 cudaError_t launch_move_blobs(const GenParams& P, int smCount, cudaStream_t stream);
