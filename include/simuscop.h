@@ -154,11 +154,13 @@ int ssc_destroy(ssc_handle* h);
  * ground-truth kernel instead of the integer-threshold kernel), "force_generic" (0/1), "gzip" (0/1: the slabs
  * handed to the sink hold concatenated gzip members -- a valid .gz stream of the same FASTQ bytes -- compressed on
  * the GPU, one member per 32 pairs, Huffman-coded with a table fitted to the first batch, or stored where that code would
- * expand the member past its bytes + 23, so gzip mode fails only where plain output does; the plain bytes of
+ * expand the member past its bytes + 23, so gzip mode fails only where plain output does, with every kernel and profile; the plain bytes of
  * SeqWriter::write are the default), "bgzf" (0/1, default 0; no effect without gzip: every gzip member is written as a BGZF
  * block -- FLG = FEXTRA and the 8 bytes 06 00 'B' 'C' 02 00 BSIZE(2, = block length - 1) after the 10-byte header, the
  * DEFLATE data unchanged, a stored block raw + 31 bytes -- so bgzip, samtools and other htslib readers can decompress in
- * parallel and seek.  A block holds the records of 32 pairs (interleaved: of both mates), at most 39 199 bytes; in PE output
+ * parallel and seek.  A block holds the records of 32 pairs (interleaved: of both mates), at most 32 x the plan's worst-case
+ * record (header + 2 x (read length + 96) + 4 bytes; both mates interleaved) + 31 bytes: 39 199 up to read length 160, 59 167
+ * at read length 320 with 64-byte names, interleaved; in PE output
  * block k of file 1 and block k of file 2 hold the same pairs.  The slabs and ssc_generate_device hold whole blocks, gz_bytes
  * counts them.  The library does not write the 28-byte BGZF end-of-file block, since it cannot know which call is the last:
  * the writer appends 1f 8b 08 04 00 00 00 00 00 ff 06 00 42 43 02 00 1b 00 03 00 00 00 00 00 00 00 00 00 (ssh_writer_bgzf

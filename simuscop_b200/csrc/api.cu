@@ -90,7 +90,7 @@ cudaError_t create(Event& e, unsigned flags = cudaEventDisableTiming) { return c
 struct BufferSet {
 	DevBuf<uint8_t> d_out[2];                   // [file] dense slabs
 	HostBuf<uint8_t> h_out[2];                  // their host copies (ssc_generate)
-	DevBuf<uint8_t> d_slots;                    // pass-1 blob scratch of the fast kernel, FG_SLOT bytes per record
+	DevBuf<uint8_t> d_slots;                    // ticket blob scratch: the fast kernel's pass 1, the generic kernel's gzip mode
 	size_t file2Off = 0;                        // file 2's blobs start this many bytes into d_slots (0: one file)
 	DevBuf<unsigned long long> d_blobPrefix;
 	DevBuf<int32_t> d_tileStart;
@@ -196,6 +196,7 @@ struct ssc_handle {
 	int64_t slabPairs = 0;
 	uint64_t slabCap = 0;
 	int slabFiles = 0;                             // output streams the slabs were allocated for (out_files)
+	uint32_t blobBytes = 0;                        // blob scratch per ticket and file the sets were allocated for (ticket_bytes)
 	BufferSet set[2];
 	struct { bool valid = false; int buf = 0; ssc::GenParams P; } pending;   // generated (scan queued), blobs not yet moved
 	DevBuf<int64_t> d_cenStarts;                  // ssc_gc_census scratch (grow-only)
@@ -230,6 +231,15 @@ bool interleaved(const ssc_handle* h) { return h->interleave && h->dt.paired; }
 // output streams of ssc_generate / ssc_generate_device: 2 for two-file PE, 1 for SE and interleaved PE
 int out_files(const ssc_handle* h) { return h->dt.paired && !h->interleave ? 2 : 1; }
 
+// Bytes of blob scratch per ticket and file: the pitch of one file's ticket blobs and of their gzip members (interleaved: one
+// blob of both mates at twice this).  The fast kernel's tickets take FG_SLOT bytes per record.  The generic kernel writes
+// ticket blobs only in gzip mode; its records are longer (up to 924 bytes at RL 320 with 64-byte names), so the pitch is its
+// tile of the plan's worst-case records plus a stored BGZF block, rounded to 16 bytes.
+uint32_t ticket_bytes(const ssc_handle* h) {
+	int qm = 0; size_t sb = 0;
+	if (!h->gzip || use_fast(h, &qm, &sb)) return FG_CHUNK * FG_SLOT;
+	return (uint32_t)(((uint64_t)GEN_TILE_PAIRS * (uint64_t)h->maxRecBytes + ssc::GZ_BGZF_STORED_EXTRA + 15) / 16 * 16);
+}
 
 int ensure_batch_resources(ssc_handle* h, bool needHost) {
 	int64_t pairs = std::min<int64_t>(h->batchPairs, std::max<int64_t>(h->emittedPairs, 1));
@@ -250,6 +260,18 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 	}
 	int nFiles = h->dt.paired ? 2 : 1;             // halves of the blob scratch (interleaved: one blob of both mates across both)
 	const int slabFiles = out_files(h);
+	// where tickets go through blobs (the fast kernel, gzip mode), a ticket's blob of worst-case records (interleaved: both mates),
+	// and in gzip mode its stored member, fit the blob pitch, which is a multiple of 16; a stored member fits one BGZF block.  The
+	// fast kernel's fixed slots hold any plan it takes (RL <= 160).
+	const uint32_t blobBytes = ticket_bytes(h);
+	int qm = 0; size_t sb = 0;
+	if (h->gzip || use_fast(h, &qm, &sb)) {
+		const uint64_t mates = interleaved(h) ? 2 : 1, pitch = blobBytes * mates;
+		const uint64_t maxBlob = (uint64_t)GEN_TILE_PAIRS * (uint64_t)h->maxRecBytes * mates;
+		if (pitch % 16 || maxBlob + gzExtra > pitch || (h->gzip && maxBlob + gzExtra > (uint64_t)ssc::GZ_BGZF_MAX_BLOCK))
+			return fail(SSC_ERR_INVALID, "a ticket of %d records of up to %d bytes does not fit its blob pitch of %llu bytes", GEN_TILE_PAIRS,
+			            h->maxRecBytes * (int)mates, (unsigned long long)pitch);
+	}
 	{
 		// the fast kernel addresses its blob scratch (FG_SLOT bytes per record, both mates) with 32-bit offsets
 		const int64_t maxFast = (int64_t)(((1ull << 32) - (1ull << 20)) / ((uint64_t)FG_SLOT * (uint64_t)nFiles));
@@ -258,15 +280,15 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 			cap = slab_cap(pairs);
 		}
 	}
-	if (pairs != h->slabPairs || cap != h->slabCap || slabFiles != h->slabFiles) {
-		h->slabPairs = 0; h->slabCap = 0; h->slabFiles = 0;   // committed below, once every allocation has succeeded
+	if (pairs != h->slabPairs || cap != h->slabCap || slabFiles != h->slabFiles || blobBytes != h->blobBytes) {
+		h->slabPairs = 0; h->slabCap = 0; h->slabFiles = 0; h->blobBytes = 0;   // committed below, once every allocation has succeeded
 		h->pending.valid = false;
 		h->d_gzBlobs[0].release(); h->d_gzBlobs[1].release();   // sized by the slabs: allocated below when gzip is on
 		h->gzBlobBytes = 0;
 		int nTiles = (int)(pairs / 16) + 2;   // enough for every kernel's tile size
 		for (BufferSet& S : h->set) {
 			// file 2's blobs behind file 1's: the kernel addresses both from one base pointer with 32-bit cursors
-			const size_t fileBytes = (size_t)pairs * FG_SLOT + 256;
+			const size_t fileBytes = (size_t)(pairs / GEN_TILE_PAIRS) * blobBytes + 256;
 			CK(S.d_slots.alloc(fileBytes * nFiles));
 			S.file2Off = nFiles == 2 ? fileBytes : 0;
 			CK(S.d_blobPrefix.alloc(nTiles));
@@ -278,12 +300,10 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 			CK(S.d_tileState.alloc(nTiles));
 			CK(S.d_ticket.alloc(1));
 		}
-		h->slabPairs = pairs; h->slabCap = cap; h->slabFiles = slabFiles;
+		h->slabPairs = pairs; h->slabCap = cap; h->slabFiles = slabFiles; h->blobBytes = blobBytes;
 	}
-	// gzip members: one per ticket blob, at the blob's pitch (interleaved: twice the per-file pitch, one file).  A BGZF block is
-	// at most 19 584 + 31 bytes (interleaved 39 168 + 31) in a pitch of 20 480 (40 960)
-	static_assert(FG_SLOT * FG_CHUNK >= 19584 + ssc::GZ_BGZF_STORED_EXTRA, "a BGZF block fits its ticket's member pitch");
-	const size_t gzBytes = (size_t)h->slabPairs * FG_SLOT * (interleaved(h) ? 2 : 1) + 64;
+	// gzip members: one per ticket blob, at the blob's pitch (interleaved: twice the per-file pitch, one file)
+	const size_t gzBytes = (size_t)(h->slabPairs / GEN_TILE_PAIRS) * h->blobBytes * (interleaved(h) ? 2 : 1) + 64;
 	if (h->gzip && h->gzBlobBytes != gzBytes) {
 		h->gzBlobBytes = 0;
 		for (int f = 0; f < 2; f++) CK(h->d_gzBlobs[f].alloc(f < (interleaved(h) ? 1 : 2) ? gzBytes : 0));
@@ -434,17 +454,20 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 	P.cap1 = h->slabCap; P.cap2 = h->slabCap;
 	P.result = S.d_result.p;
 	int grid = std::min(nTiles, h->smCount);
+	const bool ilv = interleaved(h);
+	cudaEvent_t te;
+	if (fast || h->gzip) {
+		// the generation kernel writes one blob per ticket and file into the scratch, pass 2 (scan of the blob lengths + one move per
+		// blob, in gzip mode per member) the dense slab.  Interleaved: one blob per ticket over both halves of the scratch, so twice
+		// the per-file pitch
+		P.dense1 = P.out1; P.dense2 = P.out2;
+		P.out1 = S.d_slots.p; P.out2 = S.file2Off ? S.d_slots.p + S.file2Off : nullptr;
+		P.blobPitch = h->blobBytes * (ilv ? 2u : 1u);
+		P.file2Off = (uint32_t)S.file2Off;
+	}
 	if (fast) {
 		h->stats.gen_kernel = 1; h->stats.gen_nch = ssc::fast_nch(h->dt.RL); h->stats.gen_qmode = qsmem;
 		h->stats.gen_smem_bytes = (int32_t)fastSmem;
-		// pass 1 writes one blob per ticket and file into the scratch, pass 2 (scan of the blob lengths + one move per blob) the dense slab
-		P.dense1 = P.out1; P.dense2 = P.out2;
-		P.out1 = S.d_slots.p; P.out2 = S.file2Off ? S.d_slots.p + S.file2Off : nullptr;
-		// interleaved: one blob per ticket over both halves of the scratch, so twice the per-file pitch
-		const bool ilv = interleaved(h);
-		P.blobPitch = (uint32_t)(FG_CHUNK * FG_SLOT * (ilv ? 2 : 1));
-		P.file2Off = (uint32_t)S.file2Off;
-		cudaEvent_t te;
 		if (!h->gzip) {
 			int movedBuf = -1;
 			if (h->pending.valid) {
@@ -481,36 +504,37 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 			// later work on this stream (the next launch reuses the blob scratch, copies read the dense slab) comes after the mover
 			if (movedBuf >= 0) CK(cudaStreamWaitEvent(s, h->set[movedBuf].evMoved, 0));
 			return SSC_OK;
-		} else {
-			// gzip mode: blobs -> (first batch of a plan: fit the Huffman table to a sample) -> one gzip member per blob -> pass 2 on the members
-			int rc = flush_pending(h);
-			if (rc) return rc;
-			grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount);
-			if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
-			CK(time_begin(h, s, &h->stats.gen_kernel_ms, &te));
-			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, ilv));
-			if (te) CK(cudaEventRecord(te, s));
-			CK(time_begin(h, s, &h->stats.compact_kernel_ms, &te));
-			if (!h->haveGz) { rc = build_gz_tables(h, P, nTiles); if (rc) return rc; }
-			CK(cudaMemsetAsync(h->d_gzLens.p, 0, sizeof(unsigned long long) * nTiles, s));
-			CK(ssc::launch_deflate_blobs(P.out1, P.out2, P.tileState, nTiles, P.blobPitch, h->d_gzBlobs[0].p, h->d_gzBlobs[1].p, h->d_gzLens.p,
-			                             P.blobPitch, h->d_gzTab.p + (h->bgzf ? 1 : 0), h->smCount, s));
-			ssc::GenParams P2 = P;
-			P2.out1 = h->d_gzBlobs[0].p; P2.out2 = h->d_gzBlobs[1].p; P2.tileState = h->d_gzLens.p;
-			CK(ssc::launch_pass2(P2, h->smCount, s));
-			if (te) CK(cudaEventRecord(te, s));
-			h->stats.launches += 4;
 		}
+		int rc = flush_pending(h);
+		if (rc) return rc;
+		grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount);
+		if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
+		CK(time_begin(h, s, &h->stats.gen_kernel_ms, &te));
+		CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, ilv));
+		if (te) CK(cudaEventRecord(te, s));
+		h->stats.launches += 1;
 	} else {
-		if (h->gzip) return fail(SSC_ERR_INVALID, "gzip output needs the fast kernel (kmer 3, read length 33..160)");
 		int rc = flush_pending(h);
 		if (rc) return rc;
 		ssc::GenVariant v = ssc::choose_variant(h->dt, h->fp64, h->smemLimit);
 		if (!v.ok) return fail(SSC_ERR_INVALID, "no kernel variant for read length %d / kmer %d", h->dt.RL, h->dt.K);
 		h->stats.gen_kernel = v.fp64 ? 4 : v.k3 ? 2 : 3; h->stats.gen_nch = GEN_NCH; h->stats.gen_qmode = -1;
 		h->stats.gen_smem_bytes = (int32_t)v.smemBytes;
-		CK(ssc::launch_generate(P, v, grid, s, interleaved(h)));
+		CK(ssc::launch_generate(P, v, grid, s, ilv, h->gzip));
 		h->stats.launches += 1;
+	}
+	if (h->gzip) {
+		// blobs -> (first batch of a plan: fit the Huffman table to a sample) -> one gzip member per blob -> pass 2 on the members
+		CK(time_begin(h, s, &h->stats.compact_kernel_ms, &te));
+		if (!h->haveGz) { const int rc = build_gz_tables(h, P, nTiles); if (rc) return rc; }
+		CK(cudaMemsetAsync(h->d_gzLens.p, 0, sizeof(unsigned long long) * nTiles, s));
+		CK(ssc::launch_deflate_blobs(P.out1, P.out2, P.tileState, nTiles, P.blobPitch, h->d_gzBlobs[0].p, h->d_gzBlobs[1].p, h->d_gzLens.p,
+		                             P.blobPitch, h->d_gzTab.p + (h->bgzf ? 1 : 0), h->smCount, s));
+		ssc::GenParams P2 = P;
+		P2.out1 = h->d_gzBlobs[0].p; P2.out2 = h->d_gzBlobs[1].p; P2.tileState = h->d_gzLens.p;
+		CK(ssc::launch_pass2(P2, h->smCount, s));
+		if (te) CK(cudaEventRecord(te, s));
+		h->stats.launches += 3;
 	}
 	return result_to_host(h, buf, s);
 }

@@ -55,7 +55,7 @@ struct BatchResult {
 	unsigned long long bases, reads, pairs, hapBytes;
 	unsigned int errorFlags;   // bit0: slab overflow, bit1: read outgrew scratch, bit2: too many indel events
 	unsigned int pad;
-	unsigned long long rawBytes;   // fast kernel: FASTQ bytes generated (bytes1/bytes2 are compressed sizes in gzip mode)
+	unsigned long long rawBytes;   // FASTQ bytes generated: fast kernel, generic kernel in gzip mode (bytes1/bytes2 are compressed sizes in gzip mode)
 };
 
 struct GenParams {
@@ -80,10 +80,10 @@ struct GenParams {
 	unsigned long long* tileState;
 	unsigned long long* blobPrefix;   // fast kernel: exclusive prefix of the blob lengths (pass 2)
 	unsigned int* ticket;       // work counter of the generation kernel (tiles / tickets of FG_CHUNK pairs), zeroed per launch
-	uint8_t* out1; uint8_t* out2;       // generic kernel: final slabs; fast kernel: blob scratch (pass 1: out2 == out1 + file2Off)
-	uint32_t blobPitch;                 // fast kernel: bytes from the blob of ticket j to the blob of ticket j + 1 (pass 1 output, pass 2 / deflate input)
+	uint8_t* out1; uint8_t* out2;       // generic kernel: final slabs (gzip mode: blob scratch); fast kernel: blob scratch (pass 1: out2 == out1 + file2Off)
+	uint32_t blobPitch;                 // ticket blobs: bytes from the blob of ticket j to the blob of ticket j + 1 (pass 1 output, pass 2 / deflate input)
 	uint32_t file2Off;                  // fast kernel, pass 1: file 2's blobs start this many bytes behind file 1's (one allocation, 32-bit cursors)
-	uint8_t* dense1; uint8_t* dense2;   // fast kernel: final slabs (pass 2)
+	uint8_t* dense1; uint8_t* dense2;   // ticket blobs: final slabs (pass 2)
 	unsigned long long cap1, cap2;
 	BatchResult* result;
 	// array output (generate_slots_kernel<NCH, QP, true>): out1 = reads of the batch's first pair, [pair][mate][2][pitch];

@@ -8,11 +8,15 @@
 // Bytes absent from the sample still get codes, of 14-15 bits: a later blob full of them (a 64-byte name that is not in
 // the sample, N-run qualities) can code to nearly twice its size.  So, as zlib does, a member whose coded form would be
 // longer than its raw bytes + 23 is written as one stored block instead (gzip header, 0x01, LEN, NLEN, the raw bytes,
-// CRC-32, ISIZE): no member exceeds its blob + 23 bytes (a blob is at most 32 x 612 = 19 584 bytes, its scratch 20 480; an
-// interleaved blob of both mates at most 39 168, its scratch 40 960: still within the 16-bit LEN of one stored block).
+// CRC-32, ISIZE): no member exceeds its blob + 23 bytes.  The blobs come from either generation kernel, one per ticket of 32
+// pairs: the fast kernel's are at most 32 x 612 = 19 584 bytes in a scratch pitch of 20 480 (interleaved, both mates: 39 168 in
+// 40 960); the generic kernel's (gzip mode, RL up to 320) at most 32 worst-case records of the plan, 29 568 bytes at RL 320 with
+// 64-byte names (interleaved 59 136), in a pitch of that + 31 rounded to 16 (api.cu, ticket_bytes): still within the 16-bit LEN
+// of one stored block.  The member pitch is the blob pitch.
 // BGZF (the "bgzf" option, DESIGN 13): the same member with FLG = FEXTRA and the 8-byte BC field after the 10-byte header, so
 // the tables carry an 18-byte header in the prefix and the DEFLATE bits follow 64 bits later; the warp writes BSIZE (member
-// length - 1) once the length is known.  A stored member is then raw + 31 bytes, and no block exceeds 39 199 bytes (< 65 536).
+// length - 1) once the length is known.  A stored member is then raw + 31 bytes, and no block exceeds the 65 536 bytes BGZF
+// allows (39 199 from the fast kernel, 59 167 from the generic kernel).
 //
 // Kernel: one warp per (ticket, file); interleaved output is one file (the second file's jobs have length 0).  A round takes 256 bytes (two 32-bit words per lane): LUT -> up to 2 x 60 bits
 // per lane, warp scan of the bit counts, OR into a shared-memory round buffer (two buffers in turn: the one just

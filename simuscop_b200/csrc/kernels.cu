@@ -16,6 +16,7 @@
 #include <cstdint>
 
 #include "device_types.h"
+#include "gz.h"
 #include "kernels.h"
 #include "philox.cuh"
 
@@ -342,7 +343,10 @@ __device__ __forceinline__ void copy_out(const uint8_t* sm, int len, uint8_t* g,
 // ILV (interleaved output, PE): mate 2's record goes right behind mate 1's in the warp's first stage buffer, whose neighbour is
 // its second one (2 x STAGE_CAP hold both mates of GEN_PPW pairs), and the one slab P.out1 receives mate 1, mate 2 of every
 // pair in turn; off2, the second length of the look-back and P.out2 stay unused.
-template <bool K3, bool FP64, bool ILV>
+// BLOB (gzip output): a tile is one ticket of GEN_TILE_PAIRS = FG_CHUNK pairs, written as the fast kernel writes its tickets:
+// file f's records to out_f + tile * P.blobPitch, the packed lengths len1 << 31 | len2 to P.tileState[tile] (no flags, no
+// look-back), for the deflate kernel and pass 2, which writes result->bytes1/2.  The FASTQ bytes go to result->rawBytes.
+template <bool K3, bool FP64, bool ILV, bool BLOB>
 __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParams P) {
 	extern __shared__ __align__(16) uint8_t smem[];
 	const DevTables& t = P.t;
@@ -386,6 +390,7 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 	const int nMates = t.paired ? 2 : 1;
 	const int chunksRL = (RL + 31) >> 5;
 	unsigned long long accBases = 0, accReads = 0, accPairs = 0, accHap = 0;
+	unsigned long long accRaw = 0;   // BLOB: FASTQ bytes of the CTA's tiles (thread 0)
 
 	while (true) {
 		__syncthreads();   // staging of the previous tile fully copied out; tables visible
@@ -635,7 +640,9 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 			const unsigned long long packed = ((tot >> 32) << 31) | (tot & 0x7fffffffull);
 			volatile unsigned long long* st = P.tileState;
 			unsigned long long excl = 0;
-			if (tile == 0) {
+			if (BLOB) {
+				if (lane == 0) { st[tile] = packed; accRaw += (tot >> 32) + (tot & 0xffffffffull); }
+			} else if (tile == 0) {
 				if (lane == 0) st[0] = ST_P | packed;
 			} else {
 				if (lane == 0) st[tile] = ST_A | packed;
@@ -657,7 +664,7 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 				}
 				if (lane == 0) st[tile] = ST_P | (excl + packed);
 			}
-			if (lane == 0) {
+			if (!BLOB && lane == 0) {
 				s_tileBase = excl;
 				if (tile == P.nTiles - 1) {
 					const unsigned long long fin = excl + packed;
@@ -667,7 +674,20 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 			}
 		}
 		__syncthreads();
-		{
+		if (BLOB) {
+			// the blob and the bytes of a stored block must fit the pitch: the deflate kernel writes a member that coding would
+			// expand as one stored block, at the same pitch
+			const unsigned long long wo = s_warpOff[warp];
+			const unsigned long long o1 = wo >> 32, o2 = wo & 0xffffffffull;
+			const unsigned long long lim = P.blobPitch - (uint32_t)GZ_BGZF_STORED_EXTRA;
+			if (o1 + (unsigned)off1 > lim || o2 + (unsigned)off2 > lim) {
+				if (lane == 0) atomicOr(&P.result->errorFlags, 1u);
+			} else {
+				const size_t blob = (size_t)tile * P.blobPitch;
+				copy_out(s_stage1, off1, P.out1 + blob + o1, lane);
+				if (t.paired && !ILV) copy_out(s_stage2, off2, P.out2 + blob + o2, lane);
+			}
+		} else {
 			const unsigned long long tb = s_tileBase;
 			const unsigned long long wo = s_warpOff[warp];
 			const unsigned long long g1 = (tb >> 31) + (wo >> 32);
@@ -690,15 +710,16 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 	if (threadIdx.x == 0) {
 		atomicAdd(&P.result->bases, s_stats[0]); atomicAdd(&P.result->reads, s_stats[1]);
 		atomicAdd(&P.result->pairs, s_stats[2]); atomicAdd(&P.result->hapBytes, s_stats[3]);
+		if (BLOB) atomicAdd(&P.result->rawBytes, accRaw);
 	}
 }
 
 // ----------------------------------------------------------------------------------------
 // host-side launchers
 // ----------------------------------------------------------------------------------------
-template <bool K3, bool FP64, bool ILV>
+template <bool K3, bool FP64, bool ILV, bool BLOB>
 static cudaError_t launch_variant(const GenParams& P, int grid, size_t smemBytes, cudaStream_t stream) {
-	auto kern = generate_kernel<K3, FP64, ILV>;
+	auto kern = generate_kernel<K3, FP64, ILV, BLOB>;
 	cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemBytes);
 	if (e != cudaSuccess) return e;
 	kern<<<grid, GEN_THREADS, smemBytes, stream>>>(P);
@@ -724,15 +745,16 @@ GenVariant choose_variant(const DevTables& t, bool fp64, int smemLimit) {
 	return v;
 }
 
-cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream, bool interleaved) {
-	if (interleaved) {
-		if (v.fp64) return launch_variant<false, true, true>(P, grid, v.smemBytes, stream);
-		if (v.k3) return launch_variant<true, false, true>(P, grid, v.smemBytes, stream);
-		return launch_variant<false, false, true>(P, grid, v.smemBytes, stream);
-	}
-	if (v.fp64) return launch_variant<false, true, false>(P, grid, v.smemBytes, stream);
-	if (v.k3) return launch_variant<true, false, false>(P, grid, v.smemBytes, stream);
-	return launch_variant<false, false, false>(P, grid, v.smemBytes, stream);
+template <bool ILV, bool BLOB>
+static cudaError_t launch_tables(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream) {
+	if (v.fp64) return launch_variant<false, true, ILV, BLOB>(P, grid, v.smemBytes, stream);
+	if (v.k3) return launch_variant<true, false, ILV, BLOB>(P, grid, v.smemBytes, stream);
+	return launch_variant<false, false, ILV, BLOB>(P, grid, v.smemBytes, stream);
+}
+
+cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream, bool interleaved, bool blobs) {
+	if (blobs) return interleaved ? launch_tables<true, true>(P, v, grid, stream) : launch_tables<false, true>(P, v, grid, stream);
+	return interleaved ? launch_tables<true, false>(P, v, grid, stream) : launch_tables<false, false>(P, v, grid, stream);
 }
 
 // ----------------------------------------------------------------------------------------

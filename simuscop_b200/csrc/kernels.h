@@ -35,7 +35,8 @@ struct GenVariant {
 };
 
 GenVariant choose_variant(const DevTables& t, bool fp64, int smemLimit);
-cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream, bool interleaved);   // interleaved: PE, one slab
+// interleaved: PE, one slab; blobs: gzip output, one ticket blob per tile and file (P.out1/out2 blob scratch, P.blobPitch, P.tileState)
+cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream, bool interleaved, bool blobs);
 bool fast_supported(const DevTables& t, int smemLimit, int* qmode, size_t* smemBytes);   // qmode: 8 / 16 / 2 / 0, see gen_fast.cu
 int fast_choose_qbins(int B, int RL);
 int fast_nch(int RL);
