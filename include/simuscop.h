@@ -114,14 +114,14 @@ typedef struct ssc_stats {
 	uint64_t pairs_emitted;
 	uint64_t reads_emitted;
 	uint64_t bases_emitted;    /* sum of emitted read lengths */
-	uint64_t fastq_bytes;      /* bytes of FASTQ written to HBM */
+	uint64_t fastq_bytes;      /* bytes of FASTQ written to HBM ("bam": bytes of the BAM records before compression) */
 	uint64_t hap_bytes;        /* algorithmic haplotype bytes read: ceil(len/4)+ceil(len/8) per fragment */
 	uint64_t d2h_bytes;
 	uint64_t h2d_bytes;
 	double   gen_kernel_ms;    /* CUDA-event time of the generation kernel alone (ssc_generate_device) */
 	double   compact_kernel_ms;/* CUDA-event time of the compaction kernel alone (ssc_generate_device) */
 	uint64_t timed_batches;    /* launches covered by gen_kernel_ms */
-	uint64_t gz_bytes;         /* gzip mode: compressed bytes written to the slabs, BGZF blocks with "bgzf" (fastq_bytes stays the plain size) */
+	uint64_t gz_bytes;         /* gzip mode: compressed bytes written to the slabs, BGZF blocks with "bgzf" or "bam" (fastq_bytes stays the plain size) */
 	uint64_t bin_bytes;        /* algorithmic bin-record bytes read: 64 bytes per distinct bin of every generated batch */
 	double   mover_kernel_ms;  /* CUDA-event time of the concurrent blob mover (concurrent_move > 0) on its own stream, under the
 	                              generation kernel of the next batch (ssc_generate_device) */
@@ -169,7 +169,22 @@ int ssc_destroy(ssc_handle* h);
  * `bwa mem -p` and `bowtie2 --interleaved` read; the sink gets it as buf1/len1 with buf2 == NULL, len2 == 0,
  * ssc_generate_device returns it in *bytes1 with *bytes2 = 0, ssc_stats counts the same fastq_bytes / gz_bytes totals; with
  * gzip, one member per 32 pairs of both mates; no effect on SE plans and on ssc_generate_reads; like gzip it may be set
- * between calls and takes effect at the next one), "concurrent_move" (n > 0: the blobs of batch k are moved by a
+ * between calls and takes effect at the next one), "bam" (0/1, default 0: the slabs hold BGZF blocks of unaligned BAM records
+ * (SAM specification v1, section 4.2) instead of FASTQ, whatever "gzip", "bgzf" and "interleave" say.  Each read is one record:
+ * refID, pos, next_refID, next_pos -1, mapq 0, bin 4680, no CIGAR, tlen 0, flag 77 / 141 for PE mate 1 / 2 and 4 for SE (0x10 is
+ * never set: a read is stored as its FASTQ record has it), read_name = the FASTQ name without '@' and without "/1" or "/2"
+ * (both mates of a pair have the same name), l_seq = the read's length, the FASTQ bases as 4-bit codes (first base in the
+ * high nibble, a zero pad nibble behind an odd-length read), the FASTQ qualities - 33, and RG:Z:<id> when
+ * ssc_set_read_group has set an id.  The records are those of the interleaved FASTQ of the same range, in the same order; a
+ * PE plan writes ONE stream (buf1/len1 of the sink, *bytes1 of ssc_generate_device), mate 1 and mate 2 of each pair in turn.
+ * A block holds the records of 32 pairs (both mates), at most 32 x 2 x (36 + name + 21 + (RL + 97) / 2 + RL + 96 + 68) + 31
+ * bytes.  The Huffman table is fitted to the first batch of BAM records, and fitted anew at the next call whenever the option
+ * changes.  gz_bytes counts the BGZF bytes, fastq_bytes the BAM record bytes.  A plan whose segment names hold, after the
+ * '@', a byte outside the SAM QNAME characters [!-?A-~] is refused with SSC_ERR_INVALID before anything is generated (the
+ * message names the segment and the byte), also for an empty pair range, so that a caller can check a plan that way before
+ * it opens its output; the handle stays usable.  The library writes neither the BAM header
+ * (ssc_bam_header) nor the BGZF end-of-file block: the caller's writer does (ssh_writer_bgzf appends the EOF block).  No
+ * effect on ssc_generate_reads; may be set between calls and takes effect at the next one), "concurrent_move" (n > 0: the blobs of batch k are moved by a
  * bulk-copy kernel on n SMs, on a second stream, while the generation kernel of batch k+1 runs on the others; default 9 of
  * 148 SMs, 0 below 64 SMs; 0, or n at least the GPU's SM count: a stand-alone kernel after every batch), "max_ctas" (> 0 caps the grid of the generation
  * kernel; 0 = one CTA per SM), "no_splice" (0/1, tests: reads with indel events take the position-by-position path
@@ -179,6 +194,16 @@ int ssc_destroy(ssc_handle* h);
  * symbols), 2 = only the ref == call rows in shared memory, 0 = all in global memory.  A mode that does not apply or does
  * not fit the shared memory leaves the profile to the generic kernel; ssc_stats shows what ran). */
 int ssc_set_option(ssc_handle* h, const char* key, int64_t value);
+
+/* Read group of the "bam" output: every record then ends in the tag RG:Z:<id>.  id: 1..64 bytes of [!-~]; NULL or "" removes
+ * the tag (the default).  Anything else is refused with SSC_ERR_INVALID.  May be set between calls. */
+int ssc_set_read_group(ssc_handle* h, const char* id);
+
+/* Host-only (no GPU, no handle): the header of a BAM stream as one stored BGZF block -- "BAM\1", l_text and the text
+ * "@HD\tVN:1.6\tSO:unsorted\tGO:query\n", plus "@RG\tID:<id>\tSM:<id>\n" when read_group is neither NULL nor "", and
+ * n_ref = 0 -- written to out.  A BAM file of the "bam" option is this block, the handles' blocks, then the BGZF EOF block.
+ * Returns the block size, 0 when it does not fit `cap`, or -1 on a bad read group (see ssc_set_read_group). */
+int64_t ssc_bam_header(const char* read_group, uint8_t* out, size_t cap);
 
 int ssc_set_profile(ssc_handle* h, const ssc_profile_tables* t);
 

@@ -76,7 +76,12 @@ int ssh_writer_close(ssh_writer* w, uint64_t* bytes1, uint64_t* bytes2);
  * SIMUSCOP_INTERLEAVE=1 writes a PE sample to <output>/<stem>.fq (.fq.gz with SIMUSCOP_GZIP=1), mate 1 and mate 2 of each pair
  * in turn, instead of <stem>_1 / <stem>_2; SIMUSCOP_STDOUT=1 writes the reads (PE interleaved) to standard output and no
  * FASTQ file, and refuses a configuration with more than one sample; SIMUSCOP_BGZF=1 (implies SIMUSCOP_GZIP=1) writes every
- * .fq.gz as BGZF, ended by the EOF block, with its block index <name>.fq.gz.gzi beside it (standard output: no index). */
+ * .fq.gz as BGZF, ended by the EOF block, with its block index <name>.fq.gz.gzi beside it (standard output: no index);
+ * SIMUSCOP_BAM=1 writes every sample, PE or SE, as unaligned BAM to <output>/<stem>.bam (standard output with SIMUSCOP_STDOUT=1):
+ * the header block of ssc_bam_header with read group <stem>, the records of the handles' "bam" option (RG:Z:<stem>), the BGZF
+ * EOF block, and no index; it takes precedence over SIMUSCOP_GZIP, SIMUSCOP_BGZF and SIMUSCOP_INTERLEAVE.  A stem longer than
+ * the 64 bytes of a read group id gives its first bytes and "~<sample index>"; bytes outside [!-~] become '_'.  A sample whose
+ * read names are not valid BAM names is refused before its file is opened. */
 int ssh_run(ssh_job* job, int device);
 
 #ifdef __cplusplus

@@ -16,6 +16,7 @@
 #include <vector>
 
 #include "../../include/simuscop.h"
+#include "bam.cuh"
 #include "device_types.h"
 #include "kernels.h"
 #include "tables.h"
@@ -132,8 +133,12 @@ struct ssc_handle {
 	bool gzip = false;            // slabs hold gzip members (one per ticket blob) instead of plain FASTQ
 	bool bgzf = false;            // "bgzf": with gzip, every member is a BGZF block (no effect without gzip)
 	bool interleave = false;      // "interleave": a PE plan's mates go to one stream, mate 1 and mate 2 of each pair in turn
+	bool bam = false;             // "bam": BGZF blocks of unaligned BAM records (PE: both mates in one stream), whatever gzip / bgzf / interleave say
+	int rgLen = 0;                // ssc_set_read_group: bytes of the id in d_rg (0: no RG tag)
+	DevBuf<char> d_rg;
 	size_t gzBlobBytes = 0;       // allocation of d_gzBlobs[0] (interleaved: both mates per ticket)
 	bool haveGz = false;          // Huffman / CRC tables of the current plan are on the device
+	bool gzBam = false;           // ... fitted to BAM records (refitted when the output format changes)
 	DevBuf<ssc::GzTables> d_gzTab;      // [0] gzip members, [1] BGZF blocks: one Huffman table, two member headers
 	DevBuf<uint8_t> d_gzBlobs[2];
 	DevBuf<unsigned long long> d_gzLens;
@@ -190,7 +195,10 @@ struct ssc_handle {
 	std::vector<char> names;                         // host copy of the name blob and of the segments' name ranges (ssc_segment_name)
 	std::vector<int32_t> segNameOff, segNameLen;
 	int64_t nDevBins = 0, plannedPairs = 0, emittedPairs = 0;
-	int maxRecBytes = 0;
+	int maxRecBytes = 0;                             // worst-case FASTQ record of the plan
+	int maxName = 0;                                 // longest segment name of the plan, '@' included
+	int64_t badQnameSeg = -1;                        // first segment whose name is not a valid BAM read name (-1: none)
+	int badQnameByte = 0;
 
 	// batch resources
 	int64_t slabPairs = 0;
@@ -225,11 +233,23 @@ bool use_fast(const ssc_handle* h, int* qmode, size_t* smemBytes) {
 	return ssc::fast_supported(h->dt, h->smemLimit, qmode, smemBytes);
 }
 
-// PE plan with the "interleave" option: one output stream holding both mates (the option has no effect on SE plans)
-bool interleaved(const ssc_handle* h) { return h->interleave && h->dt.paired; }
+// PE plan with the "interleave" or the "bam" option: one output stream holding both mates (no effect on SE plans)
+bool interleaved(const ssc_handle* h) { return (h->interleave || h->bam) && h->dt.paired; }
 
 // output streams of ssc_generate / ssc_generate_device: 2 for two-file PE, 1 for SE and interleaved PE
-int out_files(const ssc_handle* h) { return h->dt.paired && !h->interleave ? 2 : 1; }
+int out_files(const ssc_handle* h) { return h->dt.paired && !interleaved(h) ? 2 : 1; }
+
+// the slabs hold compressed members (gzip, or BAM, which always goes through the gzip arm) / BGZF blocks
+bool gz_mode(const ssc_handle* h) { return h->gzip || h->bam; }
+bool bgzf_mode(const ssc_handle* h) { return h->bam || (h->gzip && h->bgzf); }
+
+// Worst-case record bytes of the plan in the running format.  FASTQ: header + 2 x (RL + 96) + 4.  BAM: 36 fixed bytes, the name
+// without '@' and its two fields and NUL (name + 21), the 4-bit codes and qualities of RL + 96 bases, RG:Z:<id> NUL.
+int rec_bytes(const ssc_handle* h) {
+	if (!h->bam) return h->maxRecBytes;
+	const uint32_t m = (uint32_t)h->dt.RL + 96u;
+	return ssc::BAM_FIXED + (int)ssc::bam_tail_bytes((uint32_t)h->maxName + 21u, m, (uint32_t)h->rgLen);
+}
 
 // Bytes of blob scratch per ticket and file: the pitch of one file's ticket blobs and of their gzip members (interleaved: one
 // blob of both mates at twice this).  The fast kernel's tickets take FG_SLOT bytes per record.  The generic kernel writes
@@ -237,8 +257,8 @@ int out_files(const ssc_handle* h) { return h->dt.paired && !h->interleave ? 2 :
 // tile of the plan's worst-case records plus a stored BGZF block, rounded to 16 bytes.
 uint32_t ticket_bytes(const ssc_handle* h) {
 	int qm = 0; size_t sb = 0;
-	if (!h->gzip || use_fast(h, &qm, &sb)) return FG_CHUNK * FG_SLOT;
-	return (uint32_t)(((uint64_t)GEN_TILE_PAIRS * (uint64_t)h->maxRecBytes + ssc::GZ_BGZF_STORED_EXTRA + 15) / 16 * 16);
+	if (!gz_mode(h) || use_fast(h, &qm, &sb)) return FG_CHUNK * FG_SLOT;
+	return (uint32_t)(((uint64_t)GEN_TILE_PAIRS * (uint64_t)rec_bytes(h) + ssc::GZ_BGZF_STORED_EXTRA + 15) / 16 * 16);
 }
 
 int ensure_batch_resources(ssc_handle* h, bool needHost) {
@@ -247,8 +267,8 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 	// gzip mode: a member is at most its blob plus the bytes of a stored block (gz.cu: 23, a BGZF block 31), and there is one
 	// member per ticket.  Interleaved output: a slab holds both mates of a pair.  The scan packs a slab length into 31 bits, so
 	// the slab bound stays below 2^31 in every mode: the clamp budgets the stored-block bytes as ceil(extra / 32) = 1 per pair.
-	const uint64_t recBytes = (uint64_t)h->maxRecBytes * (interleaved(h) ? 2u : 1u);
-	const uint64_t gzExtra = h->gzip ? (uint64_t)(h->bgzf ? ssc::GZ_BGZF_STORED_EXTRA : ssc::GZ_STORED_EXTRA) : 0;
+	const uint64_t recBytes = (uint64_t)rec_bytes(h) * (interleaved(h) ? 2u : 1u);
+	const uint64_t gzExtra = gz_mode(h) ? (uint64_t)(bgzf_mode(h) ? ssc::GZ_BGZF_STORED_EXTRA : ssc::GZ_STORED_EXTRA) : 0;
 	const uint64_t perPair = recBytes + (gzExtra + FG_CHUNK - 1) / FG_CHUNK;
 	auto slab_cap = [&](int64_t n) { return (uint64_t)n * recBytes + 4096 + (uint64_t)(n / FG_CHUNK) * gzExtra; };
 	uint64_t cap = slab_cap(pairs);
@@ -265,12 +285,12 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 	// fast kernel's fixed slots hold any plan it takes (RL <= 160).
 	const uint32_t blobBytes = ticket_bytes(h);
 	int qm = 0; size_t sb = 0;
-	if (h->gzip || use_fast(h, &qm, &sb)) {
+	if (gz_mode(h) || use_fast(h, &qm, &sb)) {
 		const uint64_t mates = interleaved(h) ? 2 : 1, pitch = blobBytes * mates;
-		const uint64_t maxBlob = (uint64_t)GEN_TILE_PAIRS * (uint64_t)h->maxRecBytes * mates;
-		if (pitch % 16 || maxBlob + gzExtra > pitch || (h->gzip && maxBlob + gzExtra > (uint64_t)ssc::GZ_BGZF_MAX_BLOCK))
+		const uint64_t maxBlob = (uint64_t)GEN_TILE_PAIRS * (uint64_t)rec_bytes(h) * mates;
+		if (pitch % 16 || maxBlob + gzExtra > pitch || (gz_mode(h) && maxBlob + gzExtra > (uint64_t)ssc::GZ_BGZF_MAX_BLOCK))
 			return fail(SSC_ERR_INVALID, "a ticket of %d records of up to %d bytes does not fit its blob pitch of %llu bytes", GEN_TILE_PAIRS,
-			            h->maxRecBytes * (int)mates, (unsigned long long)pitch);
+			            rec_bytes(h) * (int)mates, (unsigned long long)pitch);
 	}
 	{
 		// the fast kernel addresses its blob scratch (FG_SLOT bytes per record, both mates) with 32-bit offsets
@@ -304,7 +324,7 @@ int ensure_batch_resources(ssc_handle* h, bool needHost) {
 	}
 	// gzip members: one per ticket blob, at the blob's pitch (interleaved: twice the per-file pitch, one file)
 	const size_t gzBytes = (size_t)(h->slabPairs / GEN_TILE_PAIRS) * h->blobBytes * (interleaved(h) ? 2 : 1) + 64;
-	if (h->gzip && h->gzBlobBytes != gzBytes) {
+	if (gz_mode(h) && h->gzBlobBytes != gzBytes) {
 		h->gzBlobBytes = 0;
 		for (int f = 0; f < 2; f++) CK(h->d_gzBlobs[f].alloc(f < (interleaved(h) ? 1 : 2) ? gzBytes : 0));
 		h->gzBlobBytes = gzBytes;
@@ -356,6 +376,7 @@ int build_gz_tables(ssc_handle* h, const ssc::GenParams& P, int nTiles) {
 	CK(cudaMemcpyAsync(h->d_gzTab.p, tab.data(), 2 * sizeof(ssc::GzTables), cudaMemcpyHostToDevice, h->compute));   // stream order with the deflate kernel
 	CK(cudaStreamSynchronize(h->compute));          // tab is freed on return
 	h->haveGz = true;
+	h->gzBam = h->bam;
 	return SSC_OK;
 }
 
@@ -423,6 +444,7 @@ ssc::GenParams batch_params(ssc_handle* h, int64_t emitLo, int64_t emitHi, bool 
 	P.insLim = h->dt.insEnable ? h->dt.insT + 1u : 0u;
 	P.delLim = h->dt.delEnable ? h->dt.delT + 1u : 0u;
 	P.alwaysSlow = (h->dt.insEnable && h->dt.insT == 0xFFFFFFFFu) || (h->dt.delEnable && h->dt.delT == 0xFFFFFFFFu);
+	P.rg = h->d_rg.p; P.rgLen = h->rgLen;
 	for (int r = 0; r < 10; r++) {
 		P.rk[2 * r] = (uint32_t)h->seed + (uint32_t)r * 0x9E3779B9u;
 		P.rk[2 * r + 1] = (uint32_t)(h->seed >> 32) + (uint32_t)r * 0xBB67AE85u;
@@ -456,7 +478,8 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 	int grid = std::min(nTiles, h->smCount);
 	const bool ilv = interleaved(h);
 	cudaEvent_t te;
-	if (fast || h->gzip) {
+	const bool gz = gz_mode(h);
+	if (fast || gz) {
 		// the generation kernel writes one blob per ticket and file into the scratch, pass 2 (scan of the blob lengths + one move per
 		// blob, in gzip mode per member) the dense slab.  Interleaved: one blob per ticket over both halves of the scratch, so twice
 		// the per-file pitch
@@ -468,7 +491,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 	if (fast) {
 		h->stats.gen_kernel = 1; h->stats.gen_nch = ssc::fast_nch(h->dt.RL); h->stats.gen_qmode = qsmem;
 		h->stats.gen_smem_bytes = (int32_t)fastSmem;
-		if (!h->gzip) {
+		if (!gz) {
 			int movedBuf = -1;
 			if (h->pending.valid) {
 				// pass 2b of the previous batch on the mover stream, under this batch's generation kernel (which leaves it the SMs);
@@ -487,7 +510,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 			grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount - (movedBuf >= 0 ? h->moverCtas : 0));
 			if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
 			CK(time_begin(h, s, &h->stats.gen_kernel_ms, &te));
-			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, ilv));
+			CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, ilv, false));
 			if (te) CK(cudaEventRecord(te, s));
 			// pass 2a on the mover stream, behind the previous batch's move: only the moves and the host need its offsets and
 			// totals, so the compute stream goes straight on to the next batch
@@ -510,7 +533,7 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 		grid = std::min((nTiles + FG_GEN - 1) / FG_GEN, h->smCount);
 		if (h->maxCtas > 0) grid = std::min(grid, h->maxCtas);
 		CK(time_begin(h, s, &h->stats.gen_kernel_ms, &te));
-		CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, ilv));
+		CK(ssc::launch_generate_fast(P, qsmem, fastSmem, grid, s, ilv, h->bam));
 		if (te) CK(cudaEventRecord(te, s));
 		h->stats.launches += 1;
 	} else {
@@ -520,16 +543,17 @@ int launch_batch(ssc_handle* h, int buf, int64_t emitLo, int64_t emitHi) {
 		if (!v.ok) return fail(SSC_ERR_INVALID, "no kernel variant for read length %d / kmer %d", h->dt.RL, h->dt.K);
 		h->stats.gen_kernel = v.fp64 ? 4 : v.k3 ? 2 : 3; h->stats.gen_nch = GEN_NCH; h->stats.gen_qmode = -1;
 		h->stats.gen_smem_bytes = (int32_t)v.smemBytes;
-		CK(ssc::launch_generate(P, v, grid, s, ilv, h->gzip));
+		CK(ssc::launch_generate(P, v, grid, s, ilv, gz, h->bam));
 		h->stats.launches += 1;
 	}
-	if (h->gzip) {
-		// blobs -> (first batch of a plan: fit the Huffman table to a sample) -> one gzip member per blob -> pass 2 on the members
+	if (gz) {
+		// blobs -> (first batch of a plan or of a changed format, FASTQ or BAM: fit the Huffman table to a sample) -> one gzip member
+		// per blob -> pass 2 on the members
 		CK(time_begin(h, s, &h->stats.compact_kernel_ms, &te));
-		if (!h->haveGz) { const int rc = build_gz_tables(h, P, nTiles); if (rc) return rc; }
+		if (!h->haveGz || h->gzBam != h->bam) { const int rc = build_gz_tables(h, P, nTiles); if (rc) return rc; }
 		CK(cudaMemsetAsync(h->d_gzLens.p, 0, sizeof(unsigned long long) * nTiles, s));
 		CK(ssc::launch_deflate_blobs(P.out1, P.out2, P.tileState, nTiles, P.blobPitch, h->d_gzBlobs[0].p, h->d_gzBlobs[1].p, h->d_gzLens.p,
-		                             P.blobPitch, h->d_gzTab.p + (h->bgzf ? 1 : 0), h->smCount, s));
+		                             P.blobPitch, h->d_gzTab.p + (bgzf_mode(h) ? 1 : 0), h->smCount, s));
 		ssc::GenParams P2 = P;
 		P2.out1 = h->d_gzBlobs[0].p; P2.out2 = h->d_gzBlobs[1].p; P2.tileState = h->d_gzLens.p;
 		CK(ssc::launch_pass2(P2, h->smCount, s));
@@ -558,8 +582,8 @@ int check_result(ssc_handle* h, const ssc::BatchResult& r) {
 	h->stats.pairs_emitted += r.pairs;
 	h->stats.reads_emitted += r.reads;
 	h->stats.bases_emitted += r.bases;
-	h->stats.fastq_bytes += h->gzip ? r.rawBytes : r.bytes1 + r.bytes2;
-	if (h->gzip) h->stats.gz_bytes += r.bytes1 + r.bytes2;
+	h->stats.fastq_bytes += gz_mode(h) ? r.rawBytes : r.bytes1 + r.bytes2;
+	if (gz_mode(h)) h->stats.gz_bytes += r.bytes1 + r.bytes2;
 	h->stats.hap_bytes += r.hapBytes;
 	return SSC_OK;
 }
@@ -634,6 +658,7 @@ int ssc_set_option(ssc_handle* h, const char* key, int64_t value) {
 	if (!strcmp(key, "gzip")) { h->gzip = value != 0; return SSC_OK; }
 	if (!strcmp(key, "bgzf")) { h->bgzf = value != 0; return SSC_OK; }        // takes effect with gzip, at the next call
 	if (!strcmp(key, "interleave")) { h->interleave = value != 0; return SSC_OK; }   // slabs re-sized at the next call if they must
+	if (!strcmp(key, "bam")) { h->bam = value != 0; return SSC_OK; }                 // likewise; the Huffman table is refitted
 	if (!strcmp(key, "concurrent_move")) {
 		if (value < 0 || value > 64) return fail(SSC_ERR_INVALID, "concurrent_move: 0 (off) .. 64 SMs");
 		h->moverCtas = value < h->smCount ? (int)value : 0;     // the generation kernel needs SMs beside the mover
@@ -1176,6 +1201,14 @@ int ssc_set_plan(ssc_handle* h, uint64_t seed, const ssc_bin* bins, int64_t n_bi
 	h->names.swap(nm);
 	h->segNameOff.resize((size_t)n_segs); h->segNameLen.resize((size_t)n_segs);
 	for (int64_t k = 0; k < n_segs; k++) { h->segNameOff[(size_t)k] = segs[k].name_offset; h->segNameLen[(size_t)k] = segs[k].name_len; }
+	// BAM output takes names made of the SAM QNAME characters [!-?A-~] only: the first segment with another byte after its '@'
+	h->badQnameSeg = -1;
+	for (int64_t k = 0; k < n_segs && h->badQnameSeg < 0; k++)
+		for (int32_t i = 1; i < segs[k].name_len; i++) {
+			const uint8_t c = (uint8_t)h->names[(size_t)(segs[k].name_offset + i)];
+			if (c < '!' || c > '~' || c == '@') { h->badQnameSeg = k; h->badQnameByte = c; break; }
+		}
+	h->maxName = maxName;
 	h->stats.h2d_bytes += nDev * sizeof(ssc::DevBin) + devEmitBase.size() * 8;
 	// worst-case record bytes per pair per file: header + 2*(RL + 96) + 4
 	h->maxRecBytes = maxName + 10 + 1 + 10 + 3 + 2 * (RL + 96) + 4;
@@ -1183,6 +1216,13 @@ int ssc_set_plan(ssc_handle* h, uint64_t seed, const ssc_bin* bins, int64_t n_bi
 	if (planned_pairs) *planned_pairs = h->plannedPairs;
 	if (emitted_pairs) *emitted_pairs = h->emittedPairs;
 	return SSC_OK;
+}
+
+// BAM output of a plan whose read names are not all valid QNAMEs is refused before anything is generated
+static int check_bam_names(const ssc_handle* h) {
+	if (!h->bam || h->badQnameSeg < 0) return SSC_OK;
+	return fail(SSC_ERR_INVALID, "bam: segment %lld: its name holds byte 0x%02x, which a BAM read name may not hold (SAM QNAME [!-?A-~])",
+	            (long long)h->badQnameSeg, h->badQnameByte);
 }
 
 // The pipeline of ssc_generate.  Every error return goes through bail() in ssc_generate.
@@ -1200,7 +1240,7 @@ static int generate_batches(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc
 	// copies of batch k-1 (file 1 / file 2 on two streams), which run under the sink of batch k-2.  h_out[k & 1] was consumed by
 	// the sink of batch k-2 an iteration before the copy of batch k is issued.
 	int qm = 0; size_t sb = 0;
-	const bool moverCompletes = use_fast(h, &qm, &sb) && !h->gzip && h->moverCtas > 0;   // batch k's dense slab under launch k+1
+	const bool moverCompletes = use_fast(h, &qm, &sb) && !gz_mode(h) && h->moverCtas > 0;   // batch k's dense slab under launch k+1
 	auto launch = [&](int k) -> int {
 		// the dense slab this launch writes: d_out[(k-1) & 1] when the mover completes the previous batch under it, else
 		// d_out[k & 1]; its last reader is the copy of the batch two before the one that now lands there
@@ -1257,6 +1297,7 @@ int ssc_generate(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, ssc_sink_fn si
 	if (!h || !sink) return fail(SSC_ERR_INVALID, "null argument");
 	if (!h->havePlan) return fail(SSC_ERR_STATE, "ssc_set_plan must precede ssc_generate");
 	if (pair_lo < 0 || pair_hi < pair_lo) return fail(SSC_ERR_INVALID, "bad pair range");
+	if (check_bam_names(h)) return SSC_ERR_INVALID;
 	CK(cudaSetDevice(h->device));
 	const int rc = generate_batches(h, pair_lo, pair_hi, sink, user);
 	return rc ? bail(h, rc) : SSC_OK;
@@ -1313,6 +1354,7 @@ int ssc_generate_device(ssc_handle* h, int64_t pair_lo, int64_t pair_hi, uint64_
 	if (!h) return fail(SSC_ERR_INVALID, "null handle");
 	if (!h->havePlan) return fail(SSC_ERR_STATE, "ssc_set_plan must precede ssc_generate_device");
 	if (pair_lo < 0 || pair_hi < pair_lo) return fail(SSC_ERR_INVALID, "bad pair range");
+	if (check_bam_names(h)) return SSC_ERR_INVALID;
 	CK(cudaSetDevice(h->device));
 	uint64_t b1 = 0, b2 = 0, nb = 0;
 	float ms = 0;
@@ -1445,6 +1487,49 @@ int64_t ssc_gzip_member_host(const uint8_t* in, uint32_t n, const uint8_t* sampl
 	const char* err = ssc::gz_build_tables(hist, &tab);
 	if (err[0]) { fail(SSC_ERR_INVALID, "gzip tables: %s", err); return -1; }
 	return (int64_t)ssc::gz_member_host(&tab, in, n, out, cap);
+}
+
+// a read group id: 1..64 bytes of [!-~]
+static bool valid_read_group(const char* id, size_t n) {
+	if (n < 1 || n > 64) return false;
+	for (size_t i = 0; i < n; i++) if ((uint8_t)id[i] < '!' || (uint8_t)id[i] > '~') return false;
+	return true;
+}
+
+int ssc_set_read_group(ssc_handle* h, const char* id) {
+	if (!h) return fail(SSC_ERR_INVALID, "null handle");
+	const size_t n = id ? strlen(id) : 0;
+	if (n == 0) { h->rgLen = 0; return SSC_OK; }
+	if (!valid_read_group(id, n)) return fail(SSC_ERR_INVALID, "read group id must be 1..64 printable characters without spaces ([!-~])");
+	CK(cudaSetDevice(h->device));
+	if (!h->d_rg.p) CK(h->d_rg.alloc(64));
+	// in stream order behind the kernels of earlier calls, which read the old id
+	CK(cudaMemcpyAsync(h->d_rg.p, id, n, cudaMemcpyHostToDevice, h->compute));
+	CK(cudaStreamSynchronize(h->compute));
+	h->rgLen = (int)n;
+	return SSC_OK;
+}
+
+int64_t ssc_bam_header(const char* read_group, uint8_t* out, size_t cap) {
+	const size_t n = read_group ? strlen(read_group) : 0;
+	if ((n && !valid_read_group(read_group, n)) || (!out && cap)) { fail(SSC_ERR_INVALID, "ssc_bam_header: bad argument"); return -1; }
+	std::string text = "@HD\tVN:1.6\tSO:unsorted\tGO:query\n";
+	if (n) text += "@RG\tID:" + std::string(read_group, n) + "\tSM:" + std::string(read_group, n) + "\n";
+	std::vector<uint8_t> raw = {'B', 'A', 'M', 1};
+	auto le32 = [](std::vector<uint8_t>& v, uint32_t x) { for (int k = 0; k < 4; k++) v.push_back((uint8_t)(x >> (8 * k))); };
+	le32(raw, (uint32_t)text.size());
+	raw.insert(raw.end(), text.begin(), text.end());
+	le32(raw, 0);                                   // n_ref
+	// one stored BGZF block: header with the BC field, a final stored DEFLATE block, CRC-32, ISIZE
+	const size_t total = raw.size() + ssc::GZ_BGZF_STORED_EXTRA;
+	if (cap < total) return 0;
+	std::vector<uint8_t> b = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, (uint8_t)((total - 1) & 0xff), (uint8_t)((total - 1) >> 8),
+	                          1, (uint8_t)(raw.size() & 0xff), (uint8_t)(raw.size() >> 8), (uint8_t)(~raw.size() & 0xff), (uint8_t)((~raw.size() >> 8) & 0xff)};
+	b.insert(b.end(), raw.begin(), raw.end());
+	le32(b, ssc::gz_crc32_host(raw.data(), raw.size()));
+	le32(b, (uint32_t)raw.size());
+	memcpy(out, b.data(), b.size());
+	return (int64_t)b.size();
 }
 
 int ssc_issue_floor(ssc_handle* h, int mode, int read_length, int64_t n_pairs, int reps, double* ms_per_launch) {

@@ -92,6 +92,9 @@ struct GenParams {
 	int64_t* rdPairId;
 	int32_t* rdSegment; int32_t* rdPos; int32_t* rdFrag;
 	uint32_t pitch;
+	// BAM output: the read group id every record carries as RG:Z (device memory, rgLen bytes, 0 = no tag)
+	const char* rg;
+	int rgLen;
 };
 
 }  // namespace ssc

@@ -33,6 +33,7 @@
 #include <cuda_runtime.h>
 #include <cstdint>
 
+#include "bam.cuh"
 #include "device_types.h"
 #include "kernels.h"
 #include "philox.cuh"
@@ -405,17 +406,30 @@ __device__ __forceinline__ void splice_read(const WarpCtx& w, const IndelPlan& p
 	__syncwarp();
 }
 
+// Output modes of generate_slots_kernel (see there)
+enum { OUT_FASTQ = 0, OUT_ARRAYS = 1, OUT_INTERLEAVED = 2, OUT_BAM = 3 };
+
+// One base of a chunk: the character to pB, the quality to pQ (lanes inside the read); BAM: see bam_put_base, pB is the
+// chunk's byte of 4-bit codes for this lane pair, and every lane of the warp must call it.
+template <int OUT>
+__device__ __forceinline__ void put_base(uint8_t* pB, uint8_t* pQ, bool in, uint32_t ch, uint32_t q, int lane) {
+	if (OUT == OUT_BAM) bam_put_base(pB, pQ, in, ch, q, lane);
+	else if (in) { *pB = (uint8_t)ch; *pQ = (uint8_t)q; }
+}
+
 // Per-base work of a read of m <= 32 * NCH bases whose source sequence is packed at index dOff (store orientation) of
 // win: the fast path's phase C with the position bins of the post-indel length (Profile.cpp:1671), rolled.
-// ARRAYS: the qualities lie `pitch` bytes behind the bases (array output) instead of m + 3 (FASTQ record).
-template <int NCH, int QP, bool ARRAYS>
+// OUT_ARRAYS: the qualities lie `pitch` bytes behind the bases (array output) instead of m + 3 (FASTQ record); OUT_BAM: the
+// bases are 4-bit codes, (m + 1) / 2 bytes, the qualities behind them.
+template <int NCH, int QP, int OUT>
 __device__ __forceinline__ void emit_packed(const WarpCtx& w, const uint32_t* win, int dOff, bool rev, int m, uint32_t lut0, uint32_t lutN,
                                             uint8_t* stage, int H, uint32_t pitch, const uint32_t (&x2)[NCH], const uint32_t (&x3)[NCH]) {
+	constexpr bool ARRAYS = OUT == OUT_ARRAYS, BAM = OUT == OUT_BAM;
 	const int lane = w.lane;
 	const uint32_t inv = (m > 1) ? (0xffffffffu / (uint32_t)m + 1u) : 0xffffffffu;
 	const int chunksM = (m + 31) >> 5;
-	uint8_t* pB = stage + H + lane;                 // this lane's base of the current chunk; its quality follows m + 3 bytes later
-	uint8_t* pQ = ARRAYS ? pB + pitch : pB + m + 3;
+	uint8_t* pB = stage + H + (BAM ? lane >> 1 : lane);   // this lane's base of the current chunk; its quality follows m + 3 bytes later
+	uint8_t* pQ = ARRAYS ? pB + pitch : BAM ? stage + H + ((m + 1) >> 1) + lane : pB + m + 3;
 	uint32_t a2[NCH], a3[NCH];
 #pragma unroll
 	for (int k = 0; k < NCH; k++) { a2[k] = x2[k]; a3[k] = x3[k]; }
@@ -434,8 +448,8 @@ __device__ __forceinline__ void emit_packed(const WarpCtx& w, const uint32_t* wi
 		uint32_t ch, q;
 		if (QP == 16) {
 			lookup16(w, rowIdx, binIdx, u2, u3, false, 0u, ch, q);
-			if (j < m) { *pB = (uint8_t)ch; *pQ = (uint8_t)q; }
-			pB += 32; pQ += 32;
+			put_base<OUT>(pB, pQ, j < m, ch, q, lane);
+			pB += BAM ? 16 : 32; pQ += 32;
 			continue;
 		}
 		const uint4 sr = w.sub[rowIdx + binIdx];
@@ -453,19 +467,18 @@ __device__ __forceinline__ void emit_packed(const WarpCtx& w, const uint32_t* wi
 			q = qual_lookup<QP>(w.q, r16 >> 2, r16 & 3u, binIdx, w.B, u3);
 			ch = __byte_perm(w.baseChars, 0, 0x4440u | (r16 & 3u));
 		}
-		if (j < m) {
-			*pB = (uint8_t)ch;
-			*pQ = (uint8_t)q;
-		}
-		pB += 32; pQ += 32;
+		put_base<OUT>(pB, pQ, j < m, ch, q, lane);
+		pB += BAM ? 16 : 32; pQ += 32;
 	}
 }
 
 // Step 2b.  x2/x3: the substitution / quality draws of output positions 32c+lane, c < NCH (registers of the caller).
-// Writes bases/quals into stage[H ..] (qualities as in emit_packed).
-template <int NCH, int QP, bool ARRAYS>
+// Writes bases/quals into stage[H ..] (qualities as in emit_packed).  OUT_BAM: every lane runs the per-base work, lanes past
+// the read end on the position bin of base m - 1, so that the warp packs the 4-bit codes together.
+template <int NCH, int QP, int OUT>
 __device__ __forceinline__ void emit_mapped(const WarpCtx& w, const IndelPlan& pl, int mate, bool rev, int relFirst,
                                             uint8_t* stage, int H, uint32_t pitch, const uint32_t (&x2)[NCH], const uint32_t (&x3)[NCH]) {
+	constexpr bool ARRAYS = OUT == OUT_ARRAYS, BAM = OUT == OUT_BAM;
 	const int RL = w.RL, lane = w.lane, m = pl.m, nEv = pl.nEv;
 	const uint2 e0 = pl.e0;
 	const uint2* evs = (const uint2*)w.ev;
@@ -516,20 +529,23 @@ __device__ __forceinline__ void emit_mapped(const WarpCtx& w, const IndelPlan& p
 		const uint32_t r1 = __shfl_sync(0xffffffffu, both, (lane + 31) & 31), r2 = __shfl_sync(0xffffffffu, both, (lane + 30) & 31);
 		const uint32_t p1 = lane >= 1 ? (r1 & 7u) : (r1 >> 4), p2 = lane >= 2 ? (r2 & 7u) : (r2 >> 4);
 		prev = code;
-		if (j < m) {
+		if (BAM || j < m) {
 			const uint32_t cur = code & 3u;
 			const uint32_t v6 = (p2 & 3u) | ((p1 & 3u) << 2) | (cur << 4);
 			const uint32_t n3 = (p2 >> 2) | ((p1 >> 2) << 1) | ((code >> 2) << 2);          // bit 2 = the base itself
 			const uint32_t var = j >= 2 ? 0u : (j == 0 ? 2u : 3u);                          // 'X' padded contexts
 			const uint32_t rowIdx = *(const uint16_t*)(w.lutB + var * 128u + v6 * 2u);
-			const uint32_t binIdx = __umulhi((uint32_t)(j * w.B), inv);
+			const uint32_t binIdx = __umulhi((uint32_t)((BAM && j >= m ? m - 1 : j) * w.B), inv);
 			uint32_t ch, q;
 			if (QP == 16) {
 				if (n3 & 4u) { ch = 'N'; q = (uint32_t)w.minQ + __umulhi(20u, u3); }   // randomInteger(33, 53), Profile.cpp:1583
 				else lookup16(w, rowIdx, binIdx, u2, u3, n3 != 0u, cur, ch, q);
-				stB[c * 32] = (uint8_t)ch;
-				if (ARRAYS) stB[pitch + c * 32] = (uint8_t)q;
-				else stB[m + 3 + c * 32] = (uint8_t)q;
+				if (BAM) bam_put_base(stage + H + 16 * c + (lane >> 1), stage + H + ((m + 1) >> 1) + j, j < m, ch, q, lane);
+				else {
+					stB[c * 32] = (uint8_t)ch;
+					if (ARRAYS) stB[pitch + c * 32] = (uint8_t)q;
+					else stB[m + 3 + c * 32] = (uint8_t)q;
+				}
 				continue;
 			}
 			const uint4 sr = w.sub[rowIdx + binIdx];
@@ -549,9 +565,12 @@ __device__ __forceinline__ void emit_mapped(const WarpCtx& w, const IndelPlan& p
 				q = qual_lookup<QP>(w.q, r16 >> 2, r16 & 3u, binIdx, w.B, u3);
 				ch = __byte_perm(w.baseChars, 0, 0x4440u | (r16 & 3u));
 			}
-			stB[c * 32] = (uint8_t)ch;
-			if (ARRAYS) stB[pitch + c * 32] = (uint8_t)q;
-			else stB[m + 3 + c * 32] = (uint8_t)q;
+			if (BAM) bam_put_base(stage + H + 16 * c + (lane >> 1), stage + H + ((m + 1) >> 1) + j, j < m, ch, q, lane);
+			else {
+				stB[c * 32] = (uint8_t)ch;
+				if (ARRAYS) stB[pitch + c * 32] = (uint8_t)q;
+				else stB[m + 3 + c * 32] = (uint8_t)q;
+			}
 		}
 	}
 }
@@ -792,14 +811,15 @@ __device__ __forceinline__ void clear_rows(uint8_t* row0, int m, uint32_t pitch,
 // their own.  OUT_FASTQ: one blob per ticket and file (PE: file 2's blob P.file2Off bytes behind file 1's); OUT_INTERLEAVED
 // (PE only): one blob per ticket holding mate 1, mate 2 of every pair in turn, at pitch 2 x FG_CHUNK x FG_SLOT over both halves
 // of the scratch.  Mate 2's header is written at the cursor behind mate 1's record, which is known once mate 1's indel scan
-// has fixed its length.
+// has fixed its length.  OUT_BAM: the same blobs (PE: the interleaved layout) hold unaligned BAM records (bam.cuh): the name
+// comes from the header code without '@', mate suffix and line feed, and the 36 fixed bytes and the read group tag are
+// written once the read's length is known.
 // ---------------------------------------------------------------------------------------------
-enum { OUT_FASTQ = 0, OUT_ARRAYS = 1, OUT_INTERLEAVED = 2 };
-
 template <int NCH, int QP, int OUT>
 __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __grid_constant__ GenParams P) {
 	constexpr bool ARRAYS = OUT == OUT_ARRAYS;
 	constexpr bool ILV = OUT == OUT_INTERLEAVED;
+	constexpr bool BAM = OUT == OUT_BAM;
 	extern __shared__ __align__(16) uint8_t smem[];
 	const DevTables& t = P.t;
 	const int lane = threadIdx.x & 31;
@@ -1047,9 +1067,11 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 			if (dc.w) qd = dsrc;
 			const uint32_t dg = qd - 10u * (__umulhi(qd, 0xCCCCCCCDu) >> 3) + '0';
 			const int nameLen = (int)((nameNd >> 17) & 127u), nameOff = (int)(nameNd & 0x1ffffu);
-			const int H = ARRAYS ? 0 : nameLen + nd1 + 1 + nd2 + (t.paired ? 2 : 0) + 1;   // array output: no header
-			const int hWords = (H + 31) >> 5;
-			const uint32_t slash = t.paired ? (uint32_t)'/' : (uint32_t)'\n';
+			// BAM: the name (header characters 1 .. nameEnd, the last one a NUL) starts at byte 36 of the record
+			const int nameEnd = nameLen + nd1 + 1 + nd2;
+			const int H = ARRAYS ? 0 : BAM ? BAM_FIXED + nameEnd : nameLen + nd1 + 1 + nd2 + (t.paired ? 2 : 0) + 1;   // array output: no header
+			const int hWords = ((BAM ? nameEnd + 1 : H) + 31) >> 5;
+			const uint32_t slash = BAM ? 0u : t.paired ? (uint32_t)'/' : (uint32_t)'\n';
 			const int mateAt = t.paired ? H - 2 : -1;
 			uint32_t hdr = 0;                                                        // interleaved: this lane's header characters, byte r
 #pragma unroll
@@ -1067,12 +1089,14 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 				if (r < 2 && k < 0) ch = (uint8_t)P.names[nameOff + i];          // names are at most 64 bytes
 				// straight into both records of the pair (the cursors of file 1 / file 2 are posA / posB here); only the mate
 				// digit in front of the final '\n' differs
-				if (i < H) {
+				if (BAM) {
+					if (i >= 1 && i <= nameEnd) P.out1[posA + (BAM_FIXED - 1) + i] = (uint8_t)ch;
+				} else if (i < H) {
 					const bool mateDigit = i == mateAt;
 					P.out1[posA + i] = (uint8_t)(mateDigit ? (uint32_t)'1' : ch);
 					if (t.paired && !ILV) P.out1[posB + i] = (uint8_t)(mateDigit ? (uint32_t)'2' : ch);
 				}
-				if (ILV) hdr |= (ch & 0xffu) << (8 * r);                               // mate 2's header, written behind mate 1's record
+				if (ILV || BAM) hdr |= (ch & 0xffu) << (8 * r);                        // mate 2's header (name), written behind mate 1's record
 			}
 
 #pragma unroll 1
@@ -1121,6 +1145,8 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 					const uint8_t* subMB = (const uint8_t*)subM;
 					uint8_t* st1 = stage + H + lane;
 					uint8_t* st2 = ARRAYS ? st1 + P.pitch : st1 + RL + 3;
+					uint8_t* sq1 = stage + H + (lane >> 1);                               // BAM: bases, 16 bytes per chunk
+					uint8_t* sq2 = stage + H + ((RL + 1) >> 1) + lane;                     // BAM: qualities
 #pragma unroll
 					for (int c = 0; c < NCH; c++) {
 						const uint32_t v6 = __funnelshift_r(dptr[c * dstep], dptr[c * dstep + 1], dsh) & 63u;
@@ -1150,7 +1176,9 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 							q = qual_lookup<QP>(w.q, r16 >> 2, call, binOf[c], B, x3[c]);
 							ch = __byte_perm(baseChars, 0, 0x4440u | call);
 						}
-						if (c < NCH - 1) {
+						if (BAM) {
+							put_base<OUT>(sq1 + c * 16, sq2 + c * 32, c < NCH - 1 || jLast < RL, ch, q, lane);
+						} else if (c < NCH - 1) {
 							st1[c * 32] = (uint8_t)ch;
 							st2[c * 32] = (uint8_t)q;
 						} else if (ARRAYS) {
@@ -1168,7 +1196,7 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 						}
 					}
 					if (ARRAYS) clear_rows(stage, 32 * NCH, P.pitch, lane);
-					else if (!foldTail && lane == 0) { stage[H + m] = '\n'; stage[H + m + 1] = '+'; stage[H + m + 2] = '\n'; stage[H + 2 * m + 3] = '\n'; }
+					else if (!BAM && !foldTail && lane == 0) { stage[H + m] = '\n'; stage[H + m + 1] = '+'; stage[H + m + 2] = '\n'; stage[H + 2 * m + 3] = '\n'; }
 				} else {
 					uint32_t evbits = 0;
 #pragma unroll
@@ -1190,33 +1218,48 @@ __global__ void __launch_bounds__(FG_THREADS, 1) generate_slots_kernel(const __g
 					const bool hasN = __any_sync(0xffffffffu, lane >= 16 && lane < 25 && s_win[lane] != 0u);
 					if (hasN || m > 32 * NCH || P.noSplice) {
 						const int relFirst = rev ? (dOff + RL - 1) : dOff;
-						emit_mapped<NCH, QP, ARRAYS>(w, pl, mate, rev, relFirst, stage, H, P.pitch, x2, x3);
+						emit_mapped<NCH, QP, OUT>(w, pl, mate, rev, relFirst, stage, H, P.pitch, x2, x3);
 					} else {
 						if (pl.nEv) splice_read(w, pl, rev, dOff);
-						emit_packed<NCH, QP, ARRAYS>(w, pl.nEv ? w.outw : s_win, dOff, rev, m, rev ? lutRev0 : lutFwd0, rev ? 128u : 0u, stage, H,
+						emit_packed<NCH, QP, OUT>(w, pl.nEv ? w.outw : s_win, dOff, rev, m, rev ? lutRev0 : lutFwd0, rev ? 128u : 0u, stage, H,
 						                             P.pitch, x2, x3);
 					}
 					if (ARRAYS) clear_rows(stage, m, P.pitch, lane);
-					else if (lane == 0) { stage[H + m] = '\n'; stage[H + m + 1] = '+'; stage[H + m + 2] = '\n'; stage[H + 2 * m + 3] = '\n'; }
+					else if (!BAM && lane == 0) { stage[H + m] = '\n'; stage[H + m + 1] = '+'; stage[H + m + 2] = '\n'; stage[H + 2 * m + 3] = '\n'; }
 				}
 				if (ARRAYS && lane == 0) P.rdLength[readIdx] = (int16_t)m;
-				posA += (uint32_t)(H + 2 * m + 4);
-				if (ILV) {
-					if (mate == 0) {
+				if (BAM) {
+					const uint32_t tail = bam_tail_bytes((uint32_t)nameEnd, (uint32_t)m, (uint32_t)P.rgLen);
+					bam_fixed(stage, (uint32_t)nameEnd, t.paired ? (mate == 0 ? BAM_FLAG_PE1 : BAM_FLAG_PE2) : BAM_FLAG_SE, (uint32_t)m,
+					          (uint32_t)P.rgLen, lane);
+					bam_read_group(stage + BAM_FIXED + tail - P.rgLen - 4, P.rg, P.rgLen, lane);
+					posA += (uint32_t)BAM_FIXED + tail;
+					if (mate == 0 && nMates == 2) {
 #pragma unroll
-						for (int r = 0; r < 3; r++) {
+						for (int r = 0; r < 3; r++) {                                        // mate 2's name is mate 1's
 							const int i = lane + 32 * r;
-							if (i < H) P.out1[posA + i] = (uint8_t)(i == mateAt ? (uint32_t)'2' : (hdr >> (8 * r)) & 0xffu);
+							if (i >= 1 && i <= nameEnd) P.out1[posA + (BAM_FIXED - 1) + i] = (uint8_t)((hdr >> (8 * r)) & 0xffu);
 						}
 					}
-				} else if (nMates == 2) { const uint32_t tswap = posA; posA = posB; posB = tswap; }
+				} else {
+					posA += (uint32_t)(H + 2 * m + 4);
+					if (ILV) {
+						if (mate == 0) {
+#pragma unroll
+							for (int r = 0; r < 3; r++) {
+								const int i = lane + 32 * r;
+								if (i < H) P.out1[posA + i] = (uint8_t)(i == mateAt ? (uint32_t)'2' : (hdr >> (8 * r)) & 0xffu);
+							}
+						}
+					} else if (nMates == 2) { const uint32_t tswap = posA; posA = posB; posB = tswap; }
+				}
 				acc += (uint32_t)m;                                                    // bases of the ticket (<= 2^14)
 				__syncwarp();
 			}
 		}
 		{
 			const uint32_t ticket = (uint32_t)chunk;
-			const uint32_t len1 = posA - blobBase, len2 = (nMates == 2 && !ILV) ? posB - blobBase - P.file2Off : 0u;
+			const uint32_t len1 = posA - blobBase, len2 = (nMates == 2 && !ILV && !BAM) ? posB - blobBase - P.file2Off : 0u;
 			if (lane == 0) {
 				if (!ARRAYS) P.tileState[ticket] = ((unsigned long long)len1 << 31) | len2;   // blob lengths, scanned by pass 2
 				const uint32_t nPairs = (uint32_t)count;
@@ -1317,8 +1360,9 @@ static cudaError_t launch_fast_instance(const GenParams& P, int qmode, size_t sm
 }
 
 // P.out1/out2 = blob scratch, P.dense1/dense2 = final slabs, P.nTiles = tickets of FG_CHUNK pairs.  Launches pass 1.
-// interleaved (PE): one blob per ticket, P.blobPitch = 2 x FG_CHUNK x FG_SLOT.
-cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream, bool interleaved) {
+// interleaved (PE): one blob per ticket, P.blobPitch = 2 x FG_CHUNK x FG_SLOT.  bam: BAM records, PE in the interleaved layout.
+cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream, bool interleaved, bool bam) {
+	if (bam) return launch_fast_instance<OUT_BAM>(P, qmode, smemBytes, grid, stream);
 	return interleaved ? launch_fast_instance<OUT_INTERLEAVED>(P, qmode, smemBytes, grid, stream)
 	                   : launch_fast_instance<OUT_FASTQ>(P, qmode, smemBytes, grid, stream);
 }

@@ -15,6 +15,7 @@
 #include <cuda_runtime.h>
 #include <cstdint>
 
+#include "bam.cuh"
 #include "device_types.h"
 #include "gz.h"
 #include "kernels.h"
@@ -346,7 +347,8 @@ __device__ __forceinline__ void copy_out(const uint8_t* sm, int len, uint8_t* g,
 // BLOB (gzip output): a tile is one ticket of GEN_TILE_PAIRS = FG_CHUNK pairs, written as the fast kernel writes its tickets:
 // file f's records to out_f + tile * P.blobPitch, the packed lengths len1 << 31 | len2 to P.tileState[tile] (no flags, no
 // look-back), for the deflate kernel and pass 2, which writes result->bytes1/2.  The FASTQ bytes go to result->rawBytes.
-template <bool K3, bool FP64, bool ILV, bool BLOB>
+// BAM (with BLOB; PE with ILV): unaligned BAM records (bam.cuh) instead of FASTQ; rawBytes counts their bytes.
+template <bool K3, bool FP64, bool ILV, bool BLOB, bool BAM>
 __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParams P) {
 	extern __shared__ __align__(16) uint8_t smem[];
 	const DevTables& t = P.t;
@@ -556,15 +558,19 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 
 				// ---- record header
 				uint8_t* stage = (mate == 0 || ILV) ? s_stage1 + off1 : s_stage2 + off2;
-				const int H = write_header(stage, P.names + bin.name_off, bin.name_len, posmod, fragCount,
+				// BAM: the header without a mate suffix, one byte in front of the name's place, so that its '@' lands in the fixed
+				// fields and its line feed on the name's NUL (both overwritten below)
+				const int H = BAM ? BAM_FIXED - 1 + write_header(stage + (BAM_FIXED - 1), P.names + bin.name_off, bin.name_len, posmod, fragCount, 0, lane)
+				                  : write_header(stage, P.names + bin.name_off, bin.name_len, posmod, fragCount,
 				                           t.paired ? (mate + 1) : 0, lane);
-				if (lane == 0) { stage[H + m] = '\n'; stage[H + m + 1] = '+'; stage[H + m + 2] = '\n'; stage[H + 2 * m + 3] = '\n'; }
+				if (!BAM && lane == 0) { stage[H + m] = '\n'; stage[H + m + 1] = '+'; stage[H + m + 2] = '\n'; stage[H + 2 * m + 3] = '\n'; }
 
 				// ---- phase C: substitution + quality at output position j
 				const uint32_t inv = (m > 1) ? (0xffffffffu / (uint32_t)m + 1u) : 0xffffffffu;
 				const int chunksM = (m + 31) >> 5;
 				const uint4* subM = subTab + ((mate == 1 && t.useCdf2) ? t.nSub : 0);
 				const double* fsub = (mate == 1 && t.useCdf2) ? t.f_sub2 : t.f_sub1;
+				uint32_t bch = 0, bq = 0;   // BAM: the base and quality characters of emit, stored by the whole warp
 				auto emit = [&](int j, uint32_t u2, uint32_t u3) {
 					const uint32_t cur = s_src[j];
 					int row = 0; uint32_t bad = cur & 4u;
@@ -601,22 +607,52 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 							q = qualSym[qrow * t.qualPitch + k];
 						}
 					}
-					stage[H + j] = ch;
-					stage[H + m + 3 + j] = q;
-				};
-#pragma unroll
-				for (int c = 0; c < GEN_NCH; c++) {
-					const int j = c * 32 + lane;
-					if (c < chunksM && j < m) {
-						if (c < chunksRL) emit(j, x2[c], x3[c]);
-						else { u32x4 blk = draw_block(P.seed, pair, mate, STREAM_CYCLE, 0, (uint32_t)j); emit(j, blk.z, blk.w); }
+					if (BAM) { bch = ch; bq = q; }
+					else {
+						stage[H + j] = ch;
+						stage[H + m + 3 + j] = q;
 					}
+				};
+				if (BAM) {
+					// the 4-bit codes of a chunk are packed by the whole warp, every lane inside the read or not
+#pragma unroll
+					for (int c = 0; c < GEN_NCH; c++) {
+						const int j = c * 32 + lane;
+						if (c < chunksM) {
+							if (j < m) {
+								if (c < chunksRL) emit(j, x2[c], x3[c]);
+								else { u32x4 blk = draw_block(P.seed, pair, mate, STREAM_CYCLE, 0, (uint32_t)j); emit(j, blk.z, blk.w); }
+							}
+							bam_put_base(stage + H + (j >> 1), stage + H + ((m + 1) >> 1) + j, j < m, bch, bq, lane);
+						}
+					}
+					for (int c = GEN_NCH; c < chunksM; c++) {
+						const int j = c * 32 + lane;
+						if (j < m) { u32x4 blk = draw_block(P.seed, pair, mate, STREAM_CYCLE, 0, (uint32_t)j); emit(j, blk.z, blk.w); }
+						bam_put_base(stage + H + (j >> 1), stage + H + ((m + 1) >> 1) + j, j < m, bch, bq, lane);
+					}
+					__syncwarp();                                   // the header's '@' and line feed are in place
+					const uint32_t lReadName = (uint32_t)(H - BAM_FIXED), tail = bam_tail_bytes(lReadName, (uint32_t)m, (uint32_t)P.rgLen);
+					if (lane == 0) stage[H - 1] = 0;
+					bam_fixed(stage, lReadName, t.paired ? (mate == 0 ? BAM_FLAG_PE1 : BAM_FLAG_PE2) : BAM_FLAG_SE, (uint32_t)m,
+					          (uint32_t)P.rgLen, lane);
+					bam_read_group(stage + BAM_FIXED + tail - P.rgLen - 4, P.rg, P.rgLen, lane);
+					off1 += BAM_FIXED + (int)tail;
+				} else {
+#pragma unroll
+					for (int c = 0; c < GEN_NCH; c++) {
+						const int j = c * 32 + lane;
+						if (c < chunksM && j < m) {
+							if (c < chunksRL) emit(j, x2[c], x3[c]);
+							else { u32x4 blk = draw_block(P.seed, pair, mate, STREAM_CYCLE, 0, (uint32_t)j); emit(j, blk.z, blk.w); }
+						}
+					}
+					for (int c = GEN_NCH; c < chunksM; c++) {
+						const int j = c * 32 + lane;
+						if (j < m) { u32x4 blk = draw_block(P.seed, pair, mate, STREAM_CYCLE, 0, (uint32_t)j); emit(j, blk.z, blk.w); }
+					}
+					if (mate == 0 || ILV) off1 += H + 2 * m + 4; else off2 += H + 2 * m + 4;
 				}
-				for (int c = GEN_NCH; c < chunksM; c++) {
-					const int j = c * 32 + lane;
-					if (j < m) { u32x4 blk = draw_block(P.seed, pair, mate, STREAM_CYCLE, 0, (uint32_t)j); emit(j, blk.z, blk.w); }
-				}
-				if (mate == 0 || ILV) off1 += H + 2 * m + 4; else off2 += H + 2 * m + 4;
 				accBases += (unsigned long long)m;
 				accReads += 1;
 				__syncwarp();
@@ -717,9 +753,9 @@ __global__ void __launch_bounds__(GEN_THREADS, 1) generate_kernel(const GenParam
 // ----------------------------------------------------------------------------------------
 // host-side launchers
 // ----------------------------------------------------------------------------------------
-template <bool K3, bool FP64, bool ILV, bool BLOB>
+template <bool K3, bool FP64, bool ILV, bool BLOB, bool BAM>
 static cudaError_t launch_variant(const GenParams& P, int grid, size_t smemBytes, cudaStream_t stream) {
-	auto kern = generate_kernel<K3, FP64, ILV, BLOB>;
+	auto kern = generate_kernel<K3, FP64, ILV, BLOB, BAM>;
 	cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemBytes);
 	if (e != cudaSuccess) return e;
 	kern<<<grid, GEN_THREADS, smemBytes, stream>>>(P);
@@ -745,14 +781,15 @@ GenVariant choose_variant(const DevTables& t, bool fp64, int smemLimit) {
 	return v;
 }
 
-template <bool ILV, bool BLOB>
+template <bool ILV, bool BLOB, bool BAM = false>
 static cudaError_t launch_tables(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream) {
-	if (v.fp64) return launch_variant<false, true, ILV, BLOB>(P, grid, v.smemBytes, stream);
-	if (v.k3) return launch_variant<true, false, ILV, BLOB>(P, grid, v.smemBytes, stream);
-	return launch_variant<false, false, ILV, BLOB>(P, grid, v.smemBytes, stream);
+	if (v.fp64) return launch_variant<false, true, ILV, BLOB, BAM>(P, grid, v.smemBytes, stream);
+	if (v.k3) return launch_variant<true, false, ILV, BLOB, BAM>(P, grid, v.smemBytes, stream);
+	return launch_variant<false, false, ILV, BLOB, BAM>(P, grid, v.smemBytes, stream);
 }
 
-cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream, bool interleaved, bool blobs) {
+cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream, bool interleaved, bool blobs, bool bam) {
+	if (bam) return interleaved ? launch_tables<true, true, true>(P, v, grid, stream) : launch_tables<false, true, true>(P, v, grid, stream);
 	if (blobs) return interleaved ? launch_tables<true, true>(P, v, grid, stream) : launch_tables<false, true>(P, v, grid, stream);
 	return interleaved ? launch_tables<true, false>(P, v, grid, stream) : launch_tables<false, false>(P, v, grid, stream);
 }

@@ -35,12 +35,13 @@ struct GenVariant {
 };
 
 GenVariant choose_variant(const DevTables& t, bool fp64, int smemLimit);
-// interleaved: PE, one slab; blobs: gzip output, one ticket blob per tile and file (P.out1/out2 blob scratch, P.blobPitch, P.tileState)
-cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream, bool interleaved, bool blobs);
+// interleaved: PE, one slab; blobs: gzip output, one ticket blob per tile and file (P.out1/out2 blob scratch, P.blobPitch, P.tileState);
+// bam: BAM records in such blobs (blobs must be set; PE: interleaved)
+cudaError_t launch_generate(const GenParams& P, const GenVariant& v, int grid, cudaStream_t stream, bool interleaved, bool blobs, bool bam);
 bool fast_supported(const DevTables& t, int smemLimit, int* qmode, size_t* smemBytes);   // qmode: 8 / 16 / 2 / 0, see gen_fast.cu
 int fast_choose_qbins(int B, int RL);
 int fast_nch(int RL);
-cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream, bool interleaved);
+cudaError_t launch_generate_fast(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream, bool interleaved, bool bam);
 cudaError_t launch_generate_reads(const GenParams& P, int qmode, size_t smemBytes, int grid, cudaStream_t stream);
 cudaError_t launch_scan_blobs(const GenParams& P, cudaStream_t stream);
 cudaError_t launch_move_blobs(const GenParams& P, int smCount, cudaStream_t stream);

@@ -13,7 +13,8 @@ from .paths import LIB_CUDA
 SYMBOLS = ["ssc_last_error", "ssc_version", "ssc_create", "ssc_destroy", "ssc_set_option", "ssc_set_profile",
            "ssc_genome_reserve", "ssc_genome_append", "ssc_genome_size", "ssc_reference_upload", "ssc_reference_upload_fasta", "ssc_reference_prefetch_fasta", "ssc_reference_adopt_prefetched", "ssc_genome_append_ref", "ssc_genome_poke", "ssc_genome_read", "ssc_gc_census", "ssc_set_plan", "ssc_generate",
            "ssc_generate_device", "ssc_read_shape", "ssc_generate_reads", "ssc_segment_name", "ssc_get_stats", "ssc_reset_stats",
-           "ssc_table_lookup_host", "ssc_sub_lookup_host", "ssc_gzip_member_host", "ssc_issue_floor"]
+           "ssc_table_lookup_host", "ssc_sub_lookup_host", "ssc_gzip_member_host", "ssc_issue_floor", "ssc_set_read_group",
+           "ssc_bam_header"]
 
 _lib = None
 
@@ -60,6 +61,9 @@ def lib():
         L.ssc_gzip_member_host.argtypes = [C.c_char_p, C.c_uint32, C.c_char_p, C.c_size_t, C.c_void_p, C.c_size_t]
         L.ssc_gzip_member_host.restype = C.c_int64
         L.ssc_issue_floor.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int, C.POINTER(C.c_double)]
+        L.ssc_set_read_group.argtypes = [C.c_void_p, C.c_char_p]
+        L.ssc_bam_header.argtypes = [C.c_char_p, C.c_void_p, C.c_size_t]
+        L.ssc_bam_header.restype = C.c_int64
         _lib = L
     return _lib
 
@@ -67,6 +71,17 @@ def lib():
 def _ck(rc):
     if rc != 0:
         raise SscError("ssc error %d: %s" % (rc, lib().ssc_last_error().decode(errors="replace")))
+
+
+def bam_header(read_group=None):
+    """The header of a BAM stream of the "bam" option as one BGZF block (ssc_bam_header; needs no GPU): @HD, an @RG line
+    with ID and SM = read_group when it is given, no references."""
+    rg = read_group.encode() if isinstance(read_group, str) else read_group
+    buf = C.create_string_buffer(1024)
+    n = lib().ssc_bam_header(rg, buf, len(buf))
+    if n <= 0:
+        raise SscError("ssc_bam_header: %s" % lib().ssc_last_error().decode(errors="replace"))
+    return buf.raw[:n]
 
 
 def _read_views(reads, length, pair_id, segment, pos, frag):
@@ -98,6 +113,11 @@ class Generator:
 
     def set_option(self, key, value):
         _ck(lib().ssc_set_option(self.h, key.encode(), int(value)))
+
+    def set_read_group(self, read_group):
+        """RG:Z:<read_group> on every record of the "bam" output; None or "" removes the tag (ssc_set_read_group)."""
+        rg = read_group.encode() if isinstance(read_group, str) else read_group
+        _ck(lib().ssc_set_read_group(self.h, rg))
 
     def load_plan(self, plan, seed):
         """Upload profile tables, haplotype store and bins of a planfile.Plan."""

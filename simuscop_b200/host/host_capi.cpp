@@ -256,6 +256,19 @@ int turn_sink(void* user, const char* b1, size_t l1, const char* b2, size_t l2, 
 	return e ? 1 : 0;
 }
 
+// Read group of sample s in BAM output: its stem, which a BAM read group id takes when it is 1..64 bytes of [!-~].  A longer
+// stem (an abundance file with several or long population names) keeps its first bytes and ends in "~<s>", which keeps the ids
+// of one run distinct; other bytes become '_'.
+std::string bam_read_group(const std::string& stem, int s) {
+	std::string id = stem;
+	for (char& c : id) if ((unsigned char)c < '!' || (unsigned char)c > '~') c = '_';
+	if (id.size() > 64) {
+		const std::string tail = "~" + std::to_string(s);
+		id = id.substr(0, 64 - tail.size()) + tail;
+	}
+	return id.empty() ? "sample~" + std::to_string(s) : id;
+}
+
 // SIMUSCOP_TRUTH_VCF=1: <output>/<stem>.truth.vcf of sample s, written once the sample is prepared
 int write_truth(sschost::Job& J, int s) {
 	const char* t = getenv("SIMUSCOP_TRUTH_VCF");
@@ -431,11 +444,16 @@ int ssh_run(ssh_job* job, int device) {
 	if (devIds.empty()) devIds.push_back(device);
 	sschost::Job& J = job->job;
 	// SIMUSCOP_STDOUT=1: the reads of the one sample go to standard output (PE interleaved) and no FASTQ file is written;
-	// SIMUSCOP_INTERLEAVE=1: a PE sample is written to <output>/<stem>.fq[.gz], mate 1 and mate 2 of each pair in turn
+	// SIMUSCOP_INTERLEAVE=1: a PE sample is written to <output>/<stem>.fq[.gz], mate 1 and mate 2 of each pair in turn;
+	// SIMUSCOP_BAM=1: every sample, PE or SE, is written as unaligned BAM to <output>/<stem>.bam, read group = the stem (see
+	// bam_read_group; takes
+	// precedence over SIMUSCOP_GZIP, SIMUSCOP_BGZF and SIMUSCOP_INTERLEAVE)
 	const char* soEnv = getenv("SIMUSCOP_STDOUT");
 	const bool toStdout = soEnv && atoi(soEnv) != 0;
+	const char* bamEnv = getenv("SIMUSCOP_BAM");
+	const bool bam = bamEnv && atoi(bamEnv) != 0;
 	const char* ilEnv = getenv("SIMUSCOP_INTERLEAVE");
-	const bool interleave = J.cfg.paired() && (toStdout || (ilEnv && atoi(ilEnv) != 0));
+	const bool interleave = !bam && J.cfg.paired() && (toStdout || (ilEnv && atoi(ilEnv) != 0));
 	if (toStdout && J.samples.size() > 1) {
 		std::cerr << "Error: SIMUSCOP_STDOUT=1 writes one sample, this configuration yields " << J.samples.size()
 		          << " (one per row of the abundance file); write them to files instead" << std::endl;
@@ -456,8 +474,9 @@ int ssh_run(ssh_job* job, int device) {
 	// (the block index `bgzip -i` writes; none on standard output); implies SIMUSCOP_GZIP=1
 	const char* gzEnv = getenv("SIMUSCOP_GZIP");
 	const char* bgzfEnv = getenv("SIMUSCOP_BGZF");
-	const bool bgzf = bgzfEnv && atoi(bgzfEnv) != 0;
-	const bool gz = bgzf || (gzEnv && atoi(gzEnv) != 0);
+	const bool bgzf = !bam && bgzfEnv && atoi(bgzfEnv) != 0;
+	const bool gz = !bam && (bgzf || (gzEnv && atoi(gzEnv) != 0));
+	if (bam) for (auto* d : devs) ssc_set_option(d, "bam", 1);
 	if (gz) for (auto* d : devs) ssc_set_option(d, "gzip", 1);
 	if (bgzf) for (auto* d : devs) ssc_set_option(d, "bgzf", 1);
 	if (interleave) for (auto* d : devs) ssc_set_option(d, "interleave", 1);
@@ -465,8 +484,8 @@ int ssh_run(ssh_job* job, int device) {
 	for (int s = 0; s < (int)J.samples.size() && !rc; s++) {
 		const std::string prefix = J.cfg.str["output"] + "/" + J.samples[s].stem;
 		const bool paired = J.cfg.paired();
-		const std::string ext = gz ? ".fq.gz" : ".fq";
-		const bool twoFiles = paired && !interleave;
+		const std::string ext = bam ? ".bam" : gz ? ".fq.gz" : ".fq";
+		const bool twoFiles = paired && !interleave && !bam;
 		const std::string f1 = toStdout ? "<standard output>" : (twoFiles ? prefix + "_1" + ext : prefix + ext);
 		const std::string f2 = twoFiles ? prefix + "_2" + ext : "";
 		std::string dump;
@@ -476,6 +495,14 @@ int ssh_run(ssh_job* job, int device) {
 		if (rc) { std::cerr << "Error: " << ssc_last_error() << std::endl; break; }
 		rc = write_truth(J, s);
 		if (rc) break;
+		const std::string rg = bam_read_group(J.samples[s].stem, s);
+		if (bam) {
+			for (auto* d : devs)
+				if ((rc = ssc_set_read_group(d, rg.c_str()))) break;
+			// the read names are checked before the output is opened: an empty range runs the check and generates nothing
+			if (!rc) rc = ssc_generate(devs[0], 0, 0, [](void*, const char*, size_t, const char*, size_t, int64_t, int64_t) { return 0; }, nullptr);
+		}
+		if (rc) { std::cerr << "Error: " << ssc_last_error() << std::endl; break; }
 		// one ordered writer per sample.  One GPU: a single ssc_generate call over the whole job (the library pipelines kernel,
 		// device->host copy and sink).  Several GPUs: the job is cut into batches, batch k goes to GPU k mod G, and every
 		// finished slab waits at the writer's turnstile until all earlier batches are in the file -- one pass of I/O, no part
@@ -489,6 +516,17 @@ int ssh_run(ssh_job* job, int device) {
 			const std::string i1 = f1 + ".gzi", i2 = f2 + ".gzi";
 			if (ssh_writer_bgzf(w, toStdout ? nullptr : i1.c_str(), twoFiles ? i2.c_str() : nullptr))
 				sschost::die(-1, "Error: can not open the BGZF index file of:\n" + f1);
+		}
+		if (bam) {
+			// BGZF blocks without an index (unaligned records have no coordinates), the header block in front of turn 0
+			uint8_t hdr[512];
+			const int64_t n = ssc_bam_header(rg.c_str(), hdr, sizeof(hdr));
+			if (n <= 0 || ssh_writer_bgzf(w, nullptr, nullptr) || w->write_slabs((const char*)hdr, (size_t)n, nullptr, 0)) {
+				std::cerr << "Error: writing the BAM header of " << f1 << " failed" << std::endl;
+				ssh_writer_close(w, nullptr, nullptr);
+				rc = SSC_ERR_SINK;
+				break;
+			}
 		}
 		if (G == 1) {
 			rc = ssc_generate(devs[0], 0, planned, writer_sink, w);

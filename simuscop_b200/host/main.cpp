@@ -3,8 +3,9 @@
 //   SIMUSCOP_SEED (default: wall clock, like the reference), SIMUSCOP_DEVICE (default 0),
 //   SIMUSCOP_DUMP_PLAN=<prefix>, SIMUSCOP_BATCH_PAIRS, SIMUSCOP_GZIP=1 (<name>.fq.gz, compressed on the GPU),
 //   SIMUSCOP_BGZF=1 (<name>.fq.gz as BGZF blocks + its <name>.fq.gz.gzi index: parallel decompression, random access),
-//   SIMUSCOP_INTERLEAVE=1 (PE: one <name>.fq, mates in turn), SIMUSCOP_STDOUT=1 (the reads to standard output, e.g.
-//   `simuReads config | bwa mem -p ref.fa -`).  Every message goes to stderr, so stdout carries FASTQ bytes only.
+//   SIMUSCOP_INTERLEAVE=1 (PE: one <name>.fq, mates in turn), SIMUSCOP_BAM=1 (<name>.bam: unaligned BAM, read group
+//   <name>, PE and SE; before SIMUSCOP_GZIP / BGZF / INTERLEAVE), SIMUSCOP_STDOUT=1 (the reads to standard output, e.g.
+//   `simuReads config | bwa mem -p ref.fa -`).  Every message goes to stderr, so stdout carries FASTQ or BAM bytes only.
 #include <signal.h>
 
 #include <chrono>
